@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (this repo's CUDA path)
     python bench.py --impl reference --gpus N --steps K ...  (the reference's CPU algorithm, oracle port)
+    python bench.py ... --dump-outputs DIR                   (also write W, H and the losses of the timed steps as .npy)
 
 One "step" = one full MU iteration (update_motifs! + update_feature_maps! incl. the loss,
 src/algs/alternating.jl:51-54) over the whole synthetic data set.  N > 1 shards the time axis
@@ -31,6 +32,9 @@ CONFIGS = {
     "c5": dict(N=512, T=1 << 24, K=128, L=32),     # spectrogram-shaped, HALS (--alg hals)
 }
 SEED_DATA, SEED_INIT, P_H, NOISE = 1234, 0, 0.05, 0.1
+# --dump-outputs: each factor is written whole up to DUMP_ELEMS values (24 MiB in fp32), else as a fixed, seeded sample of
+# units (W) or columns (H), so that two builds run with the same arguments can be compared entry for entry
+DUMP_ELEMS, DUMP_SEED = 6 << 20, 2024
 
 
 def peaks():
@@ -314,6 +318,8 @@ def run_ours(args, cfg, name):
         lt = torch.tensor([launches], dtype=torch.float64, device=f"cuda:{local_rank}")
         dist.all_reduce(lt)
         launches = int(lt.item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, shard, losses, rank, world, dist)
     ms_per_step = ms / args.steps
     value = 1e3 / ms_per_step
     engine = shard.get_engine()
@@ -533,6 +539,38 @@ def run_ours(args, cfg, name):
         dist.destroy_process_group()
 
 
+def dump_sample(n, keep, seed):
+    """Sorted indices of a fixed, seeded sample of `keep` out of range(n); all of range(n) when keep >= n."""
+    import numpy as np
+
+    if keep >= n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=keep, replace=False))
+
+
+def dump_outputs(outdir, shard, losses, rank, world, dist):
+    """Writes what the timed loop leaves its caller as OUTDIR/W.npy (K x N x L), H.npy (K x T) in the fit's float32 and
+    loss.npy (the loss of every timed step, float64).  A factor larger than DUMP_ELEMS keeps a seeded sample of its units
+    (W) or columns (H); the columns of H are gathered over the ranks, so the files do not depend on the GPU count."""
+    import numpy as np
+
+    K, N, L = shard.K, shard.N, shard.L
+    W, H_own = shard.get_factors()
+    cols = dump_sample(shard.T, DUMP_ELEMS // K, DUMP_SEED)
+    mine = np.ascontiguousarray(H_own[:, cols[(cols >= shard.t0) & (cols < shard.t1)] - shard.t0])
+    parts = [mine]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, mine)
+    if rank != 0:
+        return
+    units = dump_sample(N, DUMP_ELEMS // (K * L), DUMP_SEED + 1)
+    os.makedirs(outdir, exist_ok=True)
+    np.save(os.path.join(outdir, "W.npy"), np.ascontiguousarray(W[:, units, :]))
+    np.save(os.path.join(outdir, "H.npy"), np.concatenate(parts, axis=1))      # ranks own ascending column ranges
+    np.save(os.path.join(outdir, "loss.npy"), np.asarray(losses, dtype=np.float64))
+
+
 def _tensor_roofline(name, world, dom, engine, achieved_tf, pk, Fc_rank, per_launch_ms, K, L, prof, contr_share):
     # dram__bytes_read.sum + dram__bytes_write.sum of the dominant kernel from one `ncu --set full` capture of this very
     # workload (profiles/r1_ncu_full_corr_c4_lockstep.md); only known for the 1-GPU c4 correlation launch
@@ -588,7 +626,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-direct", action="store_true", help="skip the direct-loss figure")
     ap.add_argument("--no-calibrated", action="store_true", help="skip the calibrated-expansion figure (63 more iterations)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write W.npy, H.npy (float32; a seeded sample of units / columns where a "
+                         "factor exceeds 24 MiB) and loss.npy (every timed step, float64) to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     cfg = dict(CONFIGS[args.config])
     name = args.config
     if args.T:
