@@ -7,14 +7,14 @@ whose kernels are hand-written CUDA for sm_100a (csrc/).  Import as ``cmf_jl_b20
 from ._lib import CMFError, F32, F64, HALS, MULT, SO_PATH  # noqa: F401
 from .model import (  # noqa: F401
     AbstractCFUpdate, AlternatingOptimizer, CNMF_results, HALSUpdate, MultUpdate, PGDUpdate, compute_loss,
-    converged, corr_w, fit, fit_cnmf, init_rand, num_components, num_iter, num_lags, num_units,
+    converged, corr_w, fit, fit_cnmf, fit_cnmf_batch, init_rand, num_components, num_iter, num_lags, num_units,
     tensor_conv, tensor_transconv, compute_resids, shift_and_stack,
 )
 from .io import gen_synthetic, load_model, parameter_sweep, save_model  # noqa: F401
 from .sharded import DeviceShard, LibraryFit, ShardedMultFit, ShardPlan  # noqa: F401
 
 __all__ = [
-    "fit_cnmf", "init_rand", "MultUpdate", "HALSUpdate", "PGDUpdate", "AbstractCFUpdate", "AlternatingOptimizer",
+    "fit_cnmf", "fit_cnmf_batch", "init_rand", "MultUpdate", "HALSUpdate", "PGDUpdate", "AbstractCFUpdate", "AlternatingOptimizer",
     "fit", "CNMF_results", "converged", "compute_loss", "tensor_conv", "tensor_transconv", "corr_w",
     "num_lags", "num_units", "num_components", "num_iter", "ShardPlan", "DeviceShard",
     "ShardedMultFit", "LibraryFit", "compute_resids", "shift_and_stack", "CMFError", "gen_synthetic", "save_model", "load_model", "parameter_sweep",

@@ -109,6 +109,7 @@ struct cmf_ctx {
     bool numH_dot_valid = false;     // scal[4] == <numH, H> of the current numH and H (left there by the MU update of H)
     bool gram_valid = false;         // exchange buffer 1 holds the local Gram/tail partial of the current H
     bool have_data = false, have_factors = false;
+    int64_t R = 0;                   // restarts of a batch handle (cmf_create_batch); 0 = a handle of one factor set
     // optional per-kernel-class event timing (bench.py's roofline): class -> list of event pairs
     bool profiling = false;
     struct ProfEv { int which; cudaEvent_t a, b; };
@@ -186,6 +187,15 @@ struct cmf_ctx {
     virtual void prim_corr(const void *, void *) { no_multi(); }
     virtual void prim_resids(void *) { no_multi(); }
     virtual void prim_shift_and_stack(void *) { no_multi(); }
+    // batch handles (R > 0): R restarts of MultUpdate on one data set
+    virtual void batch_set_factors(const void *, const void *) { no_multi(); }
+    virtual void batch_get_factors(void *, void *) { no_multi(); }
+    virtual void batch_scale_partials(double *) { no_multi(); }
+    virtual void batch_scale(const double *) { no_multi(); }
+    virtual void batch_loss(double *) { no_multi(); }
+    virtual void batch_set_state(const double *, const int *) { no_multi(); }
+    virtual void batch_update_motifs() { no_multi(); }
+    virtual void batch_update_feature_maps() { no_multi(); }
 };
 
 enum { PROF_CONV = 0, PROF_TRANSCONV = 1, PROF_CORR = 2, PROF_SWEEP = 3, PROF_NCLASS = 4 };
@@ -325,6 +335,7 @@ struct Ctx : cmf_ctx {
     }
 
     void init() {
+        if (R > 0) { init_batch(); return; }
         CK(cudaSetDevice(device));
         CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         own_stream = true;
@@ -1000,9 +1011,10 @@ struct Ctx : cmf_ctx {
         if (own_stream && stream) cudaStreamDestroy(stream);
     }
 
-    void plan_split(int64_t Nin, int64_t tau_hi, int &nsplit, int64_t &split_len) {
+    // splits of the tau sum of corr_kernel so that the grid has ~592 CTAs; Kc components (default K), nrest restarts
+    void plan_split(int64_t Nin, int64_t tau_hi, int &nsplit, int64_t &split_len, int64_t Kc = 0, int64_t nrest = 1) {
         const int64_t ngrp = cdiv(L, 8);
-        const int64_t bxy = cdiv(Nin, 128) * cdiv(K * ngrp, CORR_PB);
+        const int64_t bxy = cdiv(Nin, 128) * cdiv((Kc ? Kc : K) * ngrp, CORR_PB) * nrest;
         int64_t ns = std::min<int64_t>(std::max<int64_t>(cdiv(592, bxy), 1), 64);
         split_len = cdiv(cdiv(tau_hi, ns), CORR_BTAU) * CORR_BTAU;
         if (split_len < CORR_BTAU) split_len = CORR_BTAU;
@@ -1047,15 +1059,18 @@ struct Ctx : cmf_ctx {
 
     // ---------------------------------------------------------------- kernel launch helpers
     // est over local columns [t_lo, t_hi) from (Wsrc, Hsrc) with dims (Kc, Lc).
+    // nrest > 1: restart z of a batch handle (W rows l*ld + z*Kc + k, H columns t*ld + z*Kc + k with ld = nrest*Kc) writes
+    // its partials at partial + z*part_rs
     void launch_conv(const S *Wsrc, const S *Hsrc, int64_t Kc, int64_t Lc, int64_t h_lo, int64_t h_hi,
                      int64_t t_lo, int64_t t_hi, int flags, S *out, double *partial, uint64_t seed = 0,
-                     double noise = 0.0) {
+                     double noise = 0.0, int nrest = 1, int64_t part_rs = 0) {
         if (t_hi <= t_lo) return;
         ConvArgs<S> a;
         a.Wi = Wsrc; a.H = Hsrc; a.X = X.p; a.out = out; a.partial = partial;
         a.N = N; a.K = Kc; a.L = Lc; a.t_lo = t_lo; a.t_hi = t_hi; a.h_lo = h_lo; a.h_hi = h_hi;
         a.flags = flags; a.seed = seed; a.t_global0 = t0; a.noise = noise;
         a.mask = pgd_mask.n ? pgd_mask.p : nullptr; a.lossf = pgd_loss;
+        a.ldw = a.ldh = nrest * Kc; a.w_rs = Kc * N; a.h_rs = Kc; a.part_rs = part_rs;
         const int Lpad = (int)(cdiv(Lc, 8) * 8);
         const int HW = BT + Lpad - 1;
         const size_t ws_bytes = (size_t)CONV_LC * BN * sizeof(S);
@@ -1066,7 +1081,7 @@ struct Ctx : cmf_ctx {
         const size_t smem = (size_t)KC * HW * sizeof(S) + ws_bytes;
         auto kern = conv_kernel<S, TN, TT, TY>;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        dim3 grid((unsigned)cdiv(t_hi - t_lo, BT), (unsigned)cdiv(N, BN));
+        dim3 grid((unsigned)cdiv(t_hi - t_lo, BT), (unsigned)cdiv(N, BN), (unsigned)nrest);
         prof_begin(PROF_CONV);
         kern<<<grid, dim3(16, TY), smem, stream>>>(a);
         prof_end();
@@ -1074,8 +1089,9 @@ struct Ctx : cmf_ctx {
     }
     int conv_nblocks(int64_t t_lo, int64_t t_hi) const { return (int)(cdiv(N, BN) * cdiv(t_hi - t_lo, BT)); }
 
-    void reduce_scalar(const double *part, int64_t n, double *dst) {
-        reduce_sum_kernel<<<1, 1024, 0, stream>>>(part, n, dst);
+    // nrest > 1: dst[r] = sum of part[r*n .. r*n+n)
+    void reduce_scalar(const double *part, int64_t n, double *dst, int nrest = 1) {
+        reduce_sum_kernel<<<(unsigned)nrest, 1024, 0, stream>>>(part, n, dst);
         post_launch();
     }
     double fetch_scalar(const double *dst) {
@@ -1085,9 +1101,11 @@ struct Ctx : cmf_ctx {
         return v;
     }
 
-    // out[t][k] for t in [0, t_out)
+    // out[t][k] for t in [0, t_out).  nrest > 1: restart z uses Wg + z*wg_rs, Xin + z*x_rs and writes out + z*out_rs with
+    // row stride ldo (no split over units).  split_need != nullptr: launch nothing, return the elements of tr_part the call needs.
     void launch_transconv(const S *Wg, const S *Xin, S *out, int64_t Nin, int64_t Kout, int64_t Lin,
-                          int64_t ldx, int64_t t_out, int64_t x_cols) {
+                          int64_t ldx, int64_t t_out, int64_t x_cols, int nrest = 1, int64_t wg_rs = 0, int64_t x_rs = 0,
+                          int64_t out_rs = 0, int64_t ldo = 0, size_t *split_need = nullptr) {
         if (t_out <= 0) return;
         // choose TK / kgroups minimising padding
         int best_tk = 8, best_kg = 1;
@@ -1105,29 +1123,34 @@ struct Ctx : cmf_ctx {
         TransArgs<S> a;
         a.Wg = Wg; a.Xin = Xin; a.out = out; a.Nin = Nin; a.Kout = Kout; a.Lin = Lin; a.ldx = ldx;
         a.t_out = t_out; a.x_cols = x_cols; a.kgroups = best_kg; a.tgroups = tg;
+        a.wg_rs = wg_rs; a.x_rs = x_rs; a.out_rs = out_rs; a.ldo = ldo ? ldo : Kout;
         const int BTt = tg * 8, Lpad = (int)(cdiv(Lin, 8) * 8);
         const int XW = BTt + Lpad, XWP = XW + XW / 8 + 1, KP = best_kg * best_tk;
         const size_t smem = ((size_t)TR_NC * XWP + (size_t)8 * TR_NC * KP) * sizeof(S);
         REQUIRE(smem <= 200 * 1024, "transconv: L too large for the shared-memory window");
-        dim3 grid((unsigned)cdiv(t_out, BTt), (unsigned)cdiv(Kout, KP));
+        dim3 grid((unsigned)cdiv(t_out, BTt), (unsigned)cdiv(Kout, KP), (unsigned)nrest);
         const int nthr = best_kg * tg;
         // small problems (configs 1-2: T = 2000 gives 8 CTAs) do not fill the device over (t, k) tiles alone: split the sum over
         // units across blockIdx.z into partial outputs and add them in a fixed order (deterministic)
         int nsplit = 1;
         a.n_chunk = cdiv(Nin, TR_NC) * TR_NC; a.part_stride = 0;
         const int64_t ctas = (int64_t)grid.x * grid.y;
-        if (ctas < 296 && Nin >= 64) {
+        if (nrest == 1 && ctas < 296 && Nin >= 64) {
             const int64_t want = std::min<int64_t>(std::min<int64_t>(cdiv(Nin, 32), cdiv(296, ctas)), 32);
             a.n_chunk = cdiv(cdiv(Nin, want), TR_NC) * TR_NC;
             nsplit = (int)cdiv(Nin, a.n_chunk);
             if (nsplit > 1) {
                 a.part_stride = t_out * Kout;
                 const size_t need = (size_t)nsplit * (size_t)a.part_stride;
+                if (split_need) { *split_need = need; return; }
                 if (tr_part.n < need) tr_part.alloc(need);
                 a.out = tr_part.p;
+                a.ldo = Kout;
                 grid.z = (unsigned)nsplit;
             }
         }
+        if (split_need) { *split_need = 0; return; }
+        a.nsplit = nsplit;
 #define LAUNCH_TR(TKV)                                                                             \
     {                                                                                              \
         auto kern = transconv_kernel<S, TKV, 8>;                                                   \
@@ -1146,28 +1169,41 @@ struct Ctx : cmf_ctx {
     }
     DevBuf<S> tr_part;     // partial outputs of the N-split transposed convolution
 
-    // out_S / out_D [(l*K+k)*Nin + n] = sum_tau hm(tau-l)[k] Xin[tau][n]
+    // out_S / out_D [(l*K+k)*Nin + n] = sum_tau hm(tau-l)[k] Xin[tau][n].  hm = Hs (default: this handle's H) with Kc
+    // components (default K) and row stride ldh (default Kc).  nrest > 1 is the per-restart Gram of a batch handle: Xin and
+    // Hs are both the stacked H, restart z reads its Kc columns at offset z*Kc and writes out + z*out_rs.
     void launch_corr(const S *Xin, int64_t Nin, int64_t ldx, int64_t tau_hi, int nsplit, int64_t split_len,
-                     S *out_s, double *out_d) {
+                     S *out_s, double *out_d, const S *Hs = nullptr, int64_t Kc = 0, int64_t ldh = 0, int nrest = 1,
+                     int64_t out_rs = 0) {
+        if (!Hs) Hs = H;
+        if (!Kc) Kc = K;
         CorrArgs<S> a;
-        a.H = H; a.Xin = Xin; a.part = corr_part.p; a.Nin = Nin; a.K = K; a.L = L; a.ldx = ldx;
+        a.H = Hs; a.Xin = Xin; a.part = corr_part.p; a.Nin = Nin; a.K = Kc; a.L = L; a.ldx = ldx;
         a.u_hi = Tl; a.tau_hi = tau_hi; a.split_len = split_len;
+        a.ldh = ldh ? ldh : Kc; a.nsplit = nsplit;
+        const int64_t n = L * Kc * Nin;
+        a.h_rs = a.x_rs = nrest > 1 ? Kc : 0; a.part_rs = (int64_t)nsplit * n;
         const int64_t ngrp = cdiv(L, 8);
-        dim3 grid((unsigned)cdiv(Nin, 128), (unsigned)cdiv(K * ngrp, CORR_PB), (unsigned)nsplit);
+        dim3 grid((unsigned)cdiv(Nin, 128), (unsigned)cdiv(Kc * ngrp, CORR_PB), (unsigned)(nsplit * nrest));
         if (Nin == N) prof_begin(PROF_CORR);
         corr_kernel<S><<<grid, dim3(16, 16), 0, stream>>>(a);
         prof_end();
         post_launch();
-        const int64_t n = KL() * Nin;
-        reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, nsplit, n, out_s, out_d);
+        reduce_partials_kernel<S><<<dim3((unsigned)cdiv(n, 256), (unsigned)nrest), 256, 0, stream>>>(corr_part.p, nsplit, n, out_s, out_d, out_rs);
         post_launch();
     }
 
+    static GemmRows rows(int64_t ld) { return GemmRows{ld, INT64_MAX, 0, 0}; }
     template <bool TB>
     void launch_gemm(const S *A, const S *B, S *C, int64_t M, int64_t Nn, int64_t Kg, int64_t lda, int64_t ldb,
                      int64_t ldc) {
-        dim3 grid((unsigned)cdiv(Nn, 64), (unsigned)cdiv(M, 64));
-        gemm_kernel<S, TB><<<grid, 256, 0, stream>>>(A, B, C, M, Nn, Kg, lda, ldb, ldc);
+        launch_gemm_rows<TB>(A, B, C, M, Nn, Kg, rows(lda), rows(ldb), rows(ldc), 1);
+    }
+    template <bool TB>
+    void launch_gemm_rows(const S *A, const S *B, S *C, int64_t M, int64_t Nn, int64_t Kg, GemmRows ra, GemmRows rb, GemmRows rc,
+                          int nrest) {
+        dim3 grid((unsigned)cdiv(Nn, 64), (unsigned)cdiv(M, 64), (unsigned)nrest);
+        gemm_kernel<S, TB><<<grid, 256, 0, stream>>>(A, B, C, M, Nn, Kg, ra, rb, rc);
         post_launch();
     }
 
@@ -1248,7 +1284,7 @@ struct Ctx : cmf_ctx {
         const int64_t lo = std::max<int64_t>(t0 - (L - 1), 0), hi = std::min(t1 + (L - 1), T);
         REQUIRE(first_col <= lo, "set_factors: host H starts after the shard's left halo");
         CK(cudaMemcpyAsync(Wtmp.p, Wh, Wi.n * sizeof(S), cudaMemcpyHostToDevice, stream));
-        w_julia_to_internal<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L);
+        w_julia_to_internal<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, K);
         post_launch();
         CK(cudaMemsetAsync(Hbuf.p, 0, Hbuf.n * sizeof(S), stream));
         const S *src = static_cast<const S *>(Hh) + (lo - first_col) * K;
@@ -1267,7 +1303,7 @@ struct Ctx : cmf_ctx {
         // W in Julia order (k + K*(n + N*l)) so the draw for element (k,n,l) does not depend on layout
         uniform_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, KL() * N, seed, 100, 0);
         post_launch();
-        w_julia_to_internal<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L);
+        w_julia_to_internal<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, K);
         post_launch();
         const int64_t lo = std::max<int64_t>(t0 - (L - 1), 0), hi = std::min(t1 + (L - 1), T);
         CK(cudaMemsetAsync(Hbuf.p, 0, Hbuf.n * sizeof(S), stream));
@@ -1307,12 +1343,187 @@ struct Ctx : cmf_ctx {
 
     void get_factors(void *Wo, void *Ho) override {
         if (Wo) {
-            w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L);
+            w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, K);
             post_launch();
             CK(cudaMemcpyAsync(Wo, Wtmp.p, Wi.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         }
         if (Ho) CK(cudaMemcpyAsync(Ho, H, (size_t)(Tl * K) * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
+    }
+
+    // ---------------------------------------------------------------- batch of R MultUpdate restarts (cmf_create_batch)
+    // Restart-stacked layout: H is [t][R*K] with column r*K + k, Wi has rows j' = l*R*K + r*K + k.  numW (mult.jl:32) and numH
+    // (mult.jl:47) are linear in the factor they contract with X, so ONE correlation and ONE transposed convolution with R*K
+    // components serve every restart and X is read once per step.  Everything else is block-diagonal per restart and runs as
+    // one launch with a restart grid index, so the launches of an iteration do not depend on R.
+    int64_t RK() const { return R * K; }
+    int64_t b_exch() const { return L * K * K + (L - 1) * K + 1; }   // doubles of one restart's Gram + H tail block in exch1
+    int64_t b_tail_blocks() const { return cdiv((2 * L - 1) * K, 256); }
+    DevBuf<double> b_reg, b_vals;    // [R][4] = (l1W, l2W, l1H, l2H) per restart; R per-restart scalars
+    DevBuf<int> b_active;            // 0 = the restart has converged: the updates leave its factors alone
+    GemmRows b_wrows() const { return GemmRows{N, K, RK() * N, K * N}; }   // W_r: rows l*K + k of restart r
+    GemmRows b_grows() const { return GemmRows{KL(), INT64_MAX, 0, KL() * KL()}; }   // G_r / S2_r: K L x K L blocks
+
+    // Walks every device buffer of a batch handle: returns the bytes, and allocates them when `alloc` is set (so the footprint
+    // checked before allocating is what is allocated).
+    size_t batch_buffers(bool alloc) {
+        size_t bytes = 0;
+        auto take = [&](auto &buf, int64_t count) {
+            bytes += (size_t)count * sizeof(*buf.p);
+            if (alloc) buf.alloc((size_t)count);
+        };
+        const int64_t hal = L - 1, KLR = L * RK();
+        plan_split(N, Tl + hal, nsplit_w, split_w, RK(), 1);
+        plan_split(K, Tl + hal, nsplit_g, split_g, K, R);
+        size_t tr_need = 0;
+        launch_transconv(nullptr, nullptr, nullptr, N, RK(), L, N, Tl, Tl + hal, 1, 0, 0, 0, 0, &tr_need);
+        const int nb = conv_nblocks(0, Tl);
+        take(X, (Tl + hal) * N);
+        take(Hbuf, (Tl + 2 * hal) * RK());
+        take(Wi, KLR * N); take(Wtmp, KLR * N); take(numW, KLR * N); take(denW, KLR * N);
+        take(GS, R * KL() * KL());
+        take(Cf, R * (2 * L - 1) * K * K);
+        take(numH, Tl * RK()); take(denH, Tl * RK());
+        take(exch1, R * b_exch());
+        take(corr_part, std::max<int64_t>((int64_t)nsplit_w * KLR * N, R * nsplit_g * KL() * K));
+        take(loss_part, std::max<int64_t>(2 * nb * R, 4096));
+        take(tail_part, R * b_tail_blocks() * hal * K);
+        take(tr_part, (int64_t)tr_need);
+        take(scal, 8);
+        take(b_reg, 4 * R); take(b_vals, R); take(b_active, R);
+        return bytes;
+    }
+
+    void init_batch() {
+        CK(cudaSetDevice(device));
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const size_t need = batch_buffers(false);
+        if (need > free_b)
+            throw CmfError(CMF_ERR_ARG, "cmf_create_batch: " + std::to_string(R) + " restarts need " + std::to_string(need) +
+                                            " bytes of device memory; " + std::to_string(free_b) + " bytes are free");
+        CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        own_stream = true;
+        H = nullptr;
+        batch_buffers(true);
+        H = Hbuf.p + (L - 1) * RK();
+        conv_blocks_max = conv_nblocks(0, Tl);
+        CK(cudaStreamSynchronize(stream));
+    }
+
+    // host: R Julia blocks W (K x N x L) and H (K x T); numH stages H (it is recomputed before every use)
+    void batch_set_factors(const void *Wh, const void *Hh) override {
+        REQUIRE(Wh && Hh, "cmf_set_factors_batch: null pointer");
+        CK(cudaMemcpyAsync(Wtmp.p, Wh, Wtmp.n * sizeof(S), cudaMemcpyHostToDevice, stream));
+        w_julia_to_internal<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, RK());
+        post_launch();
+        CK(cudaMemsetAsync(Hbuf.p, 0, Hbuf.n * sizeof(S), stream));
+        CK(cudaMemcpyAsync(numH.p, Hh, numH.n * sizeof(S), cudaMemcpyHostToDevice, stream));
+        h_stack_kernel<S><<<(unsigned)cdiv(RK() * Tl, 256), 256, 0, stream>>>(numH.p, H, K, Tl, R, 1);
+        post_launch();
+        CK(cudaStreamSynchronize(stream));
+        have_factors = true;
+    }
+    void batch_get_factors(void *Wo, void *Ho) override {
+        REQUIRE(have_factors, "no factors");
+        if (Wo) {
+            w_internal_to_julia<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, RK());
+            post_launch();
+            CK(cudaMemcpyAsync(Wo, Wtmp.p, Wtmp.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
+        }
+        if (Ho) {
+            h_stack_kernel<S><<<(unsigned)cdiv(RK() * Tl, 256), 256, 0, stream>>>(H, numH.p, K, Tl, R, 0);
+            post_launch();
+            CK(cudaMemcpyAsync(Ho, numH.p, numH.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
+        }
+        CK(cudaStreamSynchronize(stream));
+    }
+
+    // out[2r] = <X, est_r>, out[2r+1] = ||est_r||^2 (model.jl:119-120), each summed over the conv blocks in the order of
+    // init_scale_partials
+    void batch_scale_partials(double *out) override {
+        REQUIRE(have_data && have_factors, "cmf_init_scale_partials_batch: data and factors must be set");
+        const int nb = conv_nblocks(0, Tl);
+        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p, 0, 0.0, (int)R, 2 * nb);
+        std::vector<double> hp((size_t)(2 * nb * R));
+        CK(cudaMemcpyAsync(hp.data(), loss_part.p, hp.size() * sizeof(double), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (int64_t r = 0; r < R; ++r) {
+            const double *p = hp.data() + 2 * nb * r;
+            double a = 0.0, b = 0.0;
+            for (int i = 0; i < nb; ++i) { a += p[2 * i]; b += p[2 * i + 1]; }
+            out[2 * r] = a; out[2 * r + 1] = b;
+        }
+    }
+    void batch_scale(const double *s) override {
+        CK(cudaMemcpyAsync(b_vals.p, s, (size_t)R * sizeof(double), cudaMemcpyHostToDevice, stream));
+        scale_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, S(1), (int64_t)Wi.n, b_vals.p, N, K, RK());
+        post_launch();
+        scale_kernel<S><<<(unsigned)cdiv((int64_t)Hbuf.n, 256), 256, 0, stream>>>(Hbuf.p, S(1), (int64_t)Hbuf.n, b_vals.p, 1, K, RK());
+        post_launch();
+        CK(cudaStreamSynchronize(stream));
+    }
+
+    // relative loss of every restart (mult.jl:55-57): one direct conv + residual pass with a restart index, one deterministic
+    // reduction per restart, one copy of R doubles
+    void batch_loss(double *out) override {
+        REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
+        const int nb = conv_nblocks(0, Tl);
+        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p, 0, 0.0, (int)R, nb);
+        reduce_scalar(loss_part.p, nb, b_vals.p, (int)R);
+        CK(cudaMemcpyAsync(out, b_vals.p, (size_t)R * sizeof(double), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (int64_t r = 0; r < R; ++r) out[r] = std::sqrt(std::max(out[r], 0.0)) / data_norm;
+    }
+
+    // reg = R x (l1W, l2W, l1H, l2H) and / or the R active flags (either may be NULL)
+    void batch_set_state(const double *reg, const int *active) override {
+        if (reg) CK(cudaMemcpyAsync(b_reg.p, reg, (size_t)(4 * R) * sizeof(double), cudaMemcpyHostToDevice, stream));
+        if (active) CK(cudaMemcpyAsync(b_active.p, active, (size_t)R * sizeof(int), cudaMemcpyHostToDevice, stream));
+        CK(cudaStreamSynchronize(stream));
+    }
+
+    // update_motifs! (mult.jl:23-39) of every active restart
+    void batch_update_motifs() override {
+        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
+        launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, RK(), RK());          // numW, all restarts
+        launch_corr(H, K, RK(), Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p, H, K, RK(), (int)R, b_exch());   // Gram_r
+        if (L > 1) {
+            h_tail_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl,
+                                                                                                   1, RK(), b_exch());
+            post_launch();
+        }
+        build_G_kernel<S><<<dim3((unsigned)cdiv(KL() * KL(), 256), (unsigned)R), 256, 0, stream>>>(exch1.p, exch1.p + L * K * K, GS.p,
+                                                                                                    K, L, b_exch());
+        post_launch();
+        launch_gemm_rows<false>(GS.p, Wi.p, denW.p, KL(), N, KL(), b_grows(), b_wrows(), b_wrows(), (int)R);   // denomW_r = G_r W_r
+        mu_update_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, numW.p, denW.p, S(0), S(0), (int64_t)Wi.n,
+                                                                                     b_reg.p, b_active.p, N, K, RK());
+        post_launch();
+    }
+
+    // update_feature_maps! (mult.jl:42-58, without the loss) of every active restart
+    void batch_update_feature_maps() override {
+        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
+        launch_transconv(Wi.p, X.p, numH.p, N, RK(), L, N, Tl, Tl + (L - 1));                                // numH, all restarts
+        launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), (int)R);     // S2_r = W_r W_r'
+        lag_table_kernel<S><<<dim3((unsigned)cdiv((2 * L - 1) * K * K, 256), (unsigned)R), 256, 0, stream>>>(GS.p, Cf.p, K, L, K, KL(),
+                                                                                                          KL() * KL());
+        post_launch();
+        launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, RK(), Tl, Tl + 2 * (L - 1), (int)R, (2 * L - 1) * K * K, K, K, RK());
+        if (L > 1) {                                                                                          // truncated tail
+            const int nb = (int)b_tail_blocks();
+            const int64_t prs = (int64_t)nb * (L - 1) * K;
+            denomH_tail_prefix_kernel<S><<<dim3((unsigned)nb, (unsigned)K, (unsigned)R), 256, (size_t)8 * (size_t)(L - 1) * sizeof(double),
+                                           stream>>>(GS.p, H, tail_part.p, K, L, Tl, -(L - 1), K, KL(), RK(), KL() * KL(), prs);
+            post_launch();
+            denomH_tail_reduce_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(tail_part.p, denH.p, K, L,
+                                                                                                                Tl, nb, RK(), prs);
+            post_launch();
+        }
+        mu_update_kernel<S><<<(unsigned)cdiv(Tl * RK(), 256), 256, 0, stream>>>(H, numH.p, denH.p, S(0), S(0), Tl * RK(), b_reg.p + 2,
+                                                                                 b_active.p, 1, K, RK());
+        post_launch();
     }
 
     // ---------------------------------------------------------------- MU (src/algs/mult.jl)
@@ -1332,7 +1543,7 @@ struct Ctx : cmf_ctx {
         else if (tc_active()) { tc_split_H(true); tc_split_H(false); tc_gram(); }
         else launch_corr(H, K, K, Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p);
         if (L > 1) {
-            h_tail_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl, is_last ? 1 : 0);
+            h_tail_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl, is_last ? 1 : 0, K, 0);
             post_launch();
         }
     }
@@ -1394,9 +1605,10 @@ struct Ctx : cmf_ctx {
         }
         const size_t need = (size_t)nb * (size_t)(L - 1) * (size_t)K;
         if (tail_part.n < need) tail_part.alloc(need);
-        denomH_tail_prefix_kernel<S><<<dim3((unsigned)nb, (unsigned)K), 256, smem, stream>>>(GS.p, H, tail_part.p, K, L, Tl, -(L - 1), s2_ks, s2_ld);
+        denomH_tail_prefix_kernel<S><<<dim3((unsigned)nb, (unsigned)K), 256, smem, stream>>>(GS.p, H, tail_part.p, K, L, Tl, -(L - 1), s2_ks, s2_ld,
+                                                                                            K, 0, 0);
         post_launch();
-        denomH_tail_reduce_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(tail_part.p, denH.p, K, L, Tl, nb);
+        denomH_tail_reduce_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(tail_part.p, denH.p, K, L, Tl, nb, K, 0);
         post_launch();
     }
 
@@ -1791,7 +2003,7 @@ struct Ctx : cmf_ctx {
     void prim_corr(const void *X_host, void *out_host) override {
         set_data(X_host, 0);
         launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
-        w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(numW.p, Wtmp.p, K, N, L);
+        w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(numW.p, Wtmp.p, K, N, L, K);
         post_launch();
         CK(cudaMemcpyAsync(out_host, Wtmp.p, Wtmp.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
@@ -1818,7 +2030,8 @@ struct Ctx : cmf_ctx {
     }
 };
 
-cmf_ctx *make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device) {
+cmf_ctx *make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device,
+                  int64_t R = 0) {
     REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
     REQUIRE(L <= T, "need L <= T (src/common.jl:28-31)");
     REQUIRE(0 <= t0 && t0 < t1 && t1 <= T, "bad shard range");
@@ -1838,6 +2051,7 @@ cmf_ctx *make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64
     c->N = N; c->T = T; c->t0 = t0; c->t1 = t1; c->Tl = t1 - t0; c->K = K; c->L = L;
     c->dtype = dtype; c->alg = alg; c->device = device;
     c->is_first = (t0 == 0); c->is_last = (t1 == T);
+    c->R = R;
     try {
         if (dtype == CMF_F64) static_cast<Ctx<double> *>(c)->init();
         else static_cast<Ctx<float> *>(c)->init();
@@ -2161,6 +2375,7 @@ void r_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int chec
 
 void r_set_engine(cmf_ctx *h, int engine) {
     REQUIRE(engine >= 0 && engine <= 2, "engine must be 0 (SIMT), 1 (tcgen05, time domain) or 2 (tcgen05, frequency domain)");
+    if (h->R > 0 && engine != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles run the SIMT engine (0) only");
     if (engine == 2 && !h->fd_available())
         throw CmfError(CMF_ERR_UNSUPPORTED, "the frequency-domain engine needs an fp32 handle with K <= 128, L <= 256, N % 8 == 0 on sm_100 and room for the spectrum of X");
     if (engine < 2) h->fd_release();               // the spectrum of X and the time-domain planes never coexist
@@ -2190,6 +2405,58 @@ void attach_comm(cmf_ctx *h, ncclComm_t comm, int rank, int world, bool owned) {
         CK(cudaEventCreateWithFlags(&h->ev_b, cudaEventDisableTiming));
     }
     r_agree_engine(h);
+}
+
+// Every call that takes or returns ONE factor set refuses a batch handle and names the call to use instead.
+void single_set(cmf_handle h, const char *use) {
+    if (h && h->R > 0) throw CmfError(CMF_ERR_ARG, std::string("this is a batch handle (cmf_create_batch): use ") + use);
+}
+void no_batch_split(cmf_handle h) {
+    if (h && h->R > 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles have no split-phase calls: use cmf_fit_batch");
+}
+cmf_ctx *batch_handle(cmf_handle h) {
+    REQUIRE(h && h->R > 0, "not a batch handle (cmf_create_batch)");
+    return h;
+}
+
+// src/algs/alternating.jl:16-71 for R restarts at once.  Restart r keeps its own history and early stop; once it has
+// converged its factors are frozen (active flag 0) while the others go on.  The loop ends when every restart has stopped or
+// max_itr / max_time is reached; the elapsed time is the batch's own, shared by all restarts.
+void b_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
+           const double *l1W, const double *l2W, const double *l1H, const double *l2H, double *loss_hist,
+           std::vector<double> &time_hist, int64_t cap, int64_t *n_hist, int *converged_early) {
+    const int64_t R = h->R;
+    std::vector<double> reg((size_t)(4 * R));
+    for (int64_t r = 0; r < R; ++r) { reg[4 * r] = l1W[r]; reg[4 * r + 1] = l2W[r]; reg[4 * r + 2] = l1H[r]; reg[4 * r + 3] = l2H[r]; }
+    std::vector<int> active((size_t)R, 1);
+    h->batch_set_state(reg.data(), active.data());
+    std::vector<double> loss((size_t)R);
+    h->batch_loss(loss.data());                                     // alternating.jl:37
+    for (int64_t r = 0; r < R; ++r) { loss_hist[r * cap] = loss[r]; n_hist[r] = 1; converged_early[r] = 0; }
+    time_hist.assign(1, 0.0);
+    int64_t itr = 1, n_active = R;
+    while (n_active > 0 && (max_itr < 0 || itr <= max_itr) && time_hist.back() <= max_time) {   // alternating.jl:45
+        ++itr;
+        REQUIRE((int64_t)time_hist.size() < cap, "history capacity exhausted");
+        auto t_start = std::chrono::steady_clock::now();
+        if (!eval_mode) h->batch_update_motifs();
+        h->batch_update_feature_maps();
+        h->batch_loss(loss.data());
+        time_hist.push_back(time_hist.back() + std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count());
+        bool stopped = false;
+        for (int64_t r = 0; r < R; ++r) {
+            if (!active[r]) continue;
+            double *lh = loss_hist + r * cap;
+            lh[n_hist[r]++] = loss[r];
+            if (check_convergence && converged(lh, n_hist[r], patience, tol)) {   // alternating.jl:63-66
+                converged_early[r] = 1;
+                active[r] = 0;
+                --n_active;
+                stopped = true;
+            }
+        }
+        if (stopped && n_active > 0) h->batch_set_state(nullptr, active.data());
+    }
 }
 
 }  // namespace
@@ -2409,16 +2676,16 @@ int cmf_set_data_norm(cmf_handle h, double norm) {
     return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->data_norm = norm; r->data_sumsq_global = norm * norm; }); });
 }
 int cmf_set_factors(cmf_handle h, const void *W, const void *H, int64_t first_col) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->set_factors(W, H, first_col); }); });
+    return guarded([&] { single_set(h, "cmf_set_factors_batch"); on_ranks(h, [&](cmf_ctx *r) { r->set_factors(W, H, first_col); }); });
 }
 int cmf_exchange_halos(cmf_handle h) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { c_halo_exchange(r); r->h_changed(); }); });
+    return guarded([&] { no_batch_split(h); on_ranks(h, [&](cmf_ctx *r) { c_halo_exchange(r); r->h_changed(); }); });
 }
 int cmf_init_rand(cmf_handle h, uint64_t seed) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->init_rand(seed); }); });
+    return guarded([&] { single_set(h, "cmf_set_factors_batch with drawn factors"); on_ranks(h, [&](cmf_ctx *r) { r->init_rand(seed); }); });
 }
 int cmf_init_scale_partials(cmf_handle h, double out[2]) {
-    return guarded([&] {
+    return guarded([&] { single_set(h, "cmf_init_scale_partials_batch");
         REQUIRE(out, "null output");
         on_ranks(h, [&](cmf_ctx *r) {
             double v[2];
@@ -2428,10 +2695,10 @@ int cmf_init_scale_partials(cmf_handle h, double out[2]) {
     });
 }
 int cmf_scale_factors(cmf_handle h, double s) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->scale_factors(s); }); });
+    return guarded([&] { single_set(h, "cmf_scale_factors_batch"); on_ranks(h, [&](cmf_ctx *r) { r->scale_factors(s); }); });
 }
 int cmf_get_factors(cmf_handle h, void *W_out, void *H_out) {
-    return guarded([&] {
+    return guarded([&] { single_set(h, "cmf_get_factors_batch");
         const bool grp = h && h->multi;
         on_ranks(h, [&](cmf_ctx *r) {
             REQUIRE(r->have_factors, "no factors");
@@ -2443,11 +2710,11 @@ int cmf_get_factors(cmf_handle h, void *W_out, void *H_out) {
 }
 
 int cmf_update_motifs(cmf_handle h, double l1W, double l2W) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r_update_motifs(r, l1W, l2W); }); });
+    return guarded([&] { single_set(h, "cmf_fit_batch"); on_ranks(h, [&](cmf_ctx *r) { r_update_motifs(r, l1W, l2W); }); });
 }
 
 int cmf_update_feature_maps(cmf_handle h, double l1H, double l2H, double *loss_out) {
-    return guarded([&] {
+    return guarded([&] { single_set(h, "cmf_fit_batch");
         on_ranks(h, [&](cmf_ctx *r) {
             const double loss = r_update_feature_maps(r, l1H, l2H);
             if (loss_out && (r->rank() == 0 || !h->multi)) *loss_out = loss;
@@ -2456,7 +2723,7 @@ int cmf_update_feature_maps(cmf_handle h, double l1H, double l2H, double *loss_o
 }
 
 int cmf_loss(cmf_handle h, double *loss_out) {
-    return guarded([&] {
+    return guarded([&] { single_set(h, "cmf_loss_batch");
         REQUIRE(loss_out, "null output");
         on_ranks(h, [&](cmf_ctx *r) {
             REQUIRE(r->world() > 1 || (r->is_first && r->is_last), "shards without a communicator use cmf_loss_partial");
@@ -2469,7 +2736,7 @@ int cmf_loss(cmf_handle h, double *loss_out) {
 int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience,
             double tol, double l1W, double l2W, double l1H, double l2H, double *loss_hist, double *time_hist,
             int64_t cap, int64_t *n_hist, int *converged_early) {
-    return guarded([&] {
+    return guarded([&] { single_set(h, "cmf_fit_batch");
         REQUIRE(loss_hist && time_hist && n_hist, "null history pointers");
         REQUIRE(patience >= 1, "patience must be >= 1 (src/algs/alternating.jl:30)");
         REQUIRE(cap >= 1, "history capacity must be >= 1");
@@ -2490,13 +2757,13 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
 }
 
 int cmf_w_partials(cmf_handle h) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_partials(); });
+    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_partials(); });
 }
 int cmf_w_apply(cmf_handle h, double l1W, double l2W) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_apply(l1W, l2W); });
+    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_apply(l1W, l2W); });
 }
 int cmf_h_update(cmf_handle h, double l1H, double l2H) {
-    return guarded([&] {
+    return guarded([&] { no_batch_split(h);
         REQUIRE(h && !h->multi, "single-rank call");
         DevGuard g(h->device);
         REQUIRE(h->alg == CMF_MULT, "the split-phase H update is MultUpdate only");
@@ -2504,13 +2771,13 @@ int cmf_h_update(cmf_handle h, double l1H, double l2H) {
     });
 }
 int cmf_loss_partial(cmf_handle h, double *sumsq_out) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sumsq_out, "null output"); DevGuard g(h->device); *sumsq_out = h->loss_partial(); });
+    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sumsq_out, "null output"); DevGuard g(h->device); *sumsq_out = h->loss_partial(); });
 }
 int cmf_exchange_buffer(cmf_handle h, int which, void **dev_ptr, int64_t *count, int *dtype) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(dev_ptr && count && dtype, "null output"); h->exchange_buffer(which, dev_ptr, count, dtype); });
+    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(dev_ptr && count && dtype, "null output"); h->exchange_buffer(which, dev_ptr, count, dtype); });
 }
 int cmf_halo_buffers(cmf_handle h, void **sl, void **sr, void **rl, void **rr, int64_t *count) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sl && sr && rl && rr && count, "null output"); h->halo_buffers(sl, sr, rl, rr, count); });
+    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sl && sr && rl && rr && count, "null output"); h->halo_buffers(sl, sr, rl, rr, count); });
 }
 int cmf_sync(cmf_handle h) {
     return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { CK(cudaStreamSynchronize(r->stream)); }); });
@@ -2583,6 +2850,7 @@ int cmf_set_engine(cmf_handle h, int engine) {
 int cmf_set_loss_mode(cmf_handle h, int mode) {
     return guarded([&] {
         REQUIRE(mode == 0 || mode == 1, "loss mode must be 0 (direct) or 1 (expansion)");
+        if (h && h->R > 0 && mode != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles evaluate the loss by the direct pass (mode 0) only");
         on_ranks(h, [&](cmf_ctx *r) { r->loss_mode = mode; r->loss_mode_explicit = true; r->calib_reset(); });
     });
 }
@@ -2680,6 +2948,52 @@ int cmf_shift_and_stack(int64_t K, int64_t T, int64_t L, int dtype, const void *
             c->prim_shift_and_stack(out);
         } catch (...) { delete c; throw; }
         delete c;
+    });
+}
+
+int cmf_create_batch(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int dtype, int alg, int64_t R, int device) {
+    return guarded([&] {
+        REQUIRE(out != nullptr, "null output pointer");
+        REQUIRE(R >= 1 && R <= 32768, "R (restarts) must be in 1..32768");
+        REQUIRE(alg == CMF_MULT || alg == CMF_HALS || alg == CMF_PGD, "alg must be 0 (mult), 1 (hals) or 2 (pgd)");
+        if (alg != CMF_MULT)
+            throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts serve MultUpdate only (HALS sweeps run sequentially per restart; PGD is not batched)");
+        REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
+        REQUIRE(R * K * cdiv(L, 8) <= (int64_t)CORR_PB * 65535 && R * K <= 4 * 65535, "R*K too large for one launch grid");
+        if (L > 769) throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts need L <= 769");
+        DevRestore g;
+        *out = make_ctx(N, T, 0, T, K, L, dtype, alg, device, R);
+    });
+}
+int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H) {
+    return guarded([&] { DevGuard g(batch_handle(h)->device); h->batch_set_factors(W, H); });
+}
+int cmf_get_factors_batch(cmf_handle h, void *W_out, void *H_out) {
+    return guarded([&] { DevGuard g(batch_handle(h)->device); h->batch_get_factors(W_out, H_out); });
+}
+int cmf_init_scale_partials_batch(cmf_handle h, double *out) {
+    return guarded([&] { REQUIRE(out, "null output"); DevGuard g(batch_handle(h)->device); h->batch_scale_partials(out); });
+}
+int cmf_scale_factors_batch(cmf_handle h, const double *s) {
+    return guarded([&] { REQUIRE(s, "null scale factors"); DevGuard g(batch_handle(h)->device); h->batch_scale(s); });
+}
+int cmf_loss_batch(cmf_handle h, double *loss_out) {
+    return guarded([&] { REQUIRE(loss_out, "null output"); DevGuard g(batch_handle(h)->device); h->batch_loss(loss_out); });
+}
+int cmf_fit_batch(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
+                  const double *l1W, const double *l2W, const double *l1H, const double *l2H, double *loss_hist, double *time_hist,
+                  int64_t cap, int64_t *n_hist, int *converged_early) {
+    return guarded([&] {
+        batch_handle(h);
+        REQUIRE(l1W && l2W && l1H && l2H, "null regulariser arrays");
+        REQUIRE(loss_hist && time_hist && n_hist && converged_early, "null history pointers");
+        REQUIRE(patience >= 1, "patience must be >= 1 (src/algs/alternating.jl:30)");
+        REQUIRE(cap >= 1, "history capacity must be >= 1");
+        DevGuard g(h->device);
+        std::vector<double> th;
+        b_fit(h, max_itr, max_time, eval_mode, check_convergence, patience, tol, l1W, l2W, l1H, l2H, loss_hist, th, cap, n_hist,
+              converged_early);
+        std::copy(th.begin(), th.end(), time_hist);
     });
 }
 

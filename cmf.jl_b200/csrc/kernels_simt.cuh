@@ -44,14 +44,20 @@ __device__ __forceinline__ double block_sum(double v, double *red) {
     return r;
 }
 
-// Deterministic second stage: one block sums `n` doubles in a fixed order.
+// Deterministic second stage: block b sums the `n` doubles in[b*n .. b*n+n) in a fixed order into out[b]
+// (one block per restart of a batch handle; a single block otherwise).
 __global__ void reduce_sum_kernel(const double *__restrict__ in, int64_t n, double *__restrict__ out) {
     __shared__ double red[32];
+    in += (int64_t)blockIdx.x * n;
     double s = 0.0;
     for (int64_t i = threadIdx.x; i < n; i += blockDim.x) s += in[i];
     s = block_sum(s, red);
-    if (threadIdx.x == 0) out[0] = s;
+    if (threadIdx.x == 0) out[blockIdx.x] = s;
 }
+
+// Restart r of a batch handle owns components [r*K, r*K + K) of the stacked component axis (width RK = R*K).  For an array
+// whose component index is (i / inner) % RK -- W in the internal layout (inner = N), H (inner = 1) -- this is r.
+__device__ __forceinline__ int64_t restart_of(int64_t i, int64_t inner, int64_t K, int64_t RK) { return ((i / inner) % RK) / K; }
 
 // ------------------------------------------------------------------------------------------
 // conv (+ residual, + loss):   est[t][n] = sum_{l<L,k<K} Wi[l*K+k][n] * H[t-l][k]
@@ -81,6 +87,9 @@ struct ConvArgs {
     int KC;               // components staged per H window
     const S *mask;        // flags 32|64: optional mask [t][N] (nullptr = all ones)
     int lossf;            // flags 32|64: 0 SquareLoss, 1 AbsoluteLoss
+    // restart blockIdx.z of a batch handle: W rows (l*ldw + k) and H columns t*ldh + k from Wi + z*w_rs and H + z*h_rs,
+    // partials from partial + z*part_rs (single handles: ldw = ldh = K, one z)
+    int64_t ldw, ldh, w_rs, h_rs, part_rs;
 };
 
 __device__ __forceinline__ uint64_t mix64(uint64_t z) {
@@ -116,6 +125,8 @@ __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
     const int tid = ty * 16 + tx, nthr = 16 * TY;
     const int64_t n0 = (int64_t)blockIdx.y * BN;          // grid.x runs over time tiles (can be > 65535)
     const int64_t t0 = a.t_lo + (int64_t)blockIdx.x * BT;
+    const S *Wr = a.Wi + (int64_t)blockIdx.z * a.w_rs, *Hr = a.H + (int64_t)blockIdx.z * a.h_rs;
+    double *partial = a.partial ? a.partial + (int64_t)blockIdx.z * a.part_rs : nullptr;
 
     S acc[TT][TN];
 #pragma unroll
@@ -131,7 +142,7 @@ __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
             const int k = idx % kc, i = idx / kc;
             const int64_t t = t0 - (Lpad - 1) + i;
             S v = S(0);
-            if (t >= a.h_lo && t < a.h_hi) v = a.H[t * K + kc0 + k];
+            if (t >= a.h_lo && t < a.h_hi) v = Hr[t * a.ldh + kc0 + k];
             Hs[(size_t)k * HW + i] = v;
         }
         for (int k = 0; k < kc; ++k) {
@@ -143,7 +154,7 @@ __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
                     const int n = idx % BN, dl = idx / BN;
                     const int64_t l = lc0 + dl;
                     S v = S(0);
-                    if (l < L && n0 + n < N) v = a.Wi[((l * K) + kc0 + k) * N + n0 + n];
+                    if (l < L && n0 + n < N) v = Wr[((l * a.ldw) + kc0 + k) * N + n0 + n];
                     Ws[dl * BN + n] = v;
                 }
                 __syncthreads();
@@ -208,14 +219,14 @@ __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
     }
     if (a.flags & (4 | 64)) {
         sq = block_sum(sq, red);
-        if (tid == 0) a.partial[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = sq;
+        if (tid == 0) partial[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = sq;
     }
     if (a.flags & 16) {
         const size_t b = (size_t)blockIdx.y * gridDim.x + blockIdx.x;
         dxe = block_sum(dxe, red);
-        if (tid == 0) a.partial[2 * b] = dxe;
+        if (tid == 0) partial[2 * b] = dxe;
         sq = block_sum(sq, red);
-        if (tid == 0) a.partial[2 * b + 1] = sq;
+        if (tid == 0) partial[2 * b + 1] = sq;
     }
 }
 
@@ -233,8 +244,11 @@ struct TransArgs {
     int64_t Nin, Kout, Lin, ldx;
     int64_t t_out, x_cols;
     int kgroups, tgroups;
-    int64_t n_chunk;      // units summed by one CTA (blockIdx.z selects the chunk; a multiple of TR_NC); Nin rounded up = no split
+    int64_t n_chunk;      // units summed by one CTA (blockIdx.z % nsplit selects the chunk; a multiple of TR_NC); Nin rounded up = no split
     int64_t part_stride;  // elements between the partial outputs of consecutive chunks (0 = no split: `out` is the result)
+    int nsplit;           // chunks per restart: blockIdx.z / nsplit is the restart (single handles: one restart)
+    int64_t wg_rs, x_rs, out_rs;   // per-restart offsets of Wg, Xin and out
+    int64_t ldo;          // row stride of out (Kout, or R*K when restarts write their columns of a stacked array)
 };
 
 // out[i] = sum_z part[z * stride + i] in the fixed order z = 0, 1, ... (deterministic; the N-split of transconv_kernel)
@@ -265,6 +279,8 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
     const int kg = tid % kgroups, tg = tid / kgroups;
     const int64_t t0 = (int64_t)blockIdx.x * BT;
     const int64_t kb = (int64_t)blockIdx.y * KP;     // first k of this block
+    const int64_t rs = blockIdx.z / a.nsplit, zs = blockIdx.z % a.nsplit;
+    const S *Wg = a.Wg + rs * a.wg_rs, *Xin = a.Xin + rs * a.x_rs;
 
     S acc[TT][TK];
 #pragma unroll
@@ -272,7 +288,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
 #pragma unroll
         for (int i = 0; i < TK; ++i) acc[j][i] = S(0);
 
-    const int64_t n_lo = (int64_t)blockIdx.z * a.n_chunk, n_hi = min(a.Nin, n_lo + a.n_chunk);
+    const int64_t n_lo = zs * a.n_chunk, n_hi = min(a.Nin, n_lo + a.n_chunk);
     for (int64_t nc0 = n_lo; nc0 < n_hi; nc0 += TR_NC) {
         __syncthreads();
         // stage X window (transposed): Xs[n][phys(i)] = Xin[(t0+i)*ldx + nc0 + n]
@@ -280,7 +296,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
             const int n = idx % TR_NC, i = idx / TR_NC;
             const int64_t t = t0 + i;
             S v = S(0);
-            if (t < a.x_cols && nc0 + n < n_hi) v = a.Xin[t * a.ldx + nc0 + n];
+            if (t < a.x_cols && nc0 + n < n_hi) v = Xin[t * a.ldx + nc0 + n];
             Xs[(size_t)n * XWP + i + i / 8] = v;
         }
         for (int lc0 = 0; lc0 < Lpad; lc0 += 8) {
@@ -291,7 +307,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
                 const int64_t l = lc0 + dl;
                 S v = S(0);
                 if (l < a.Lin && kb + k < a.Kout && nc0 + n < n_hi)
-                    v = a.Wg[((l * a.Kout) + kb + k) * a.Nin + nc0 + n];
+                    v = Wg[((l * a.Kout) + kb + k) * a.Nin + nc0 + n];
                 Ws[((size_t)dl * TR_NC + n) * KP + k] = v;
             }
             __syncthreads();
@@ -329,7 +345,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
 #pragma unroll
         for (int i = 0; i < TK; ++i) {
             const int64_t k = kb + kg * TK + i;
-            if (k < a.Kout) a.out[(int64_t)blockIdx.z * a.part_stride + t * a.Kout + k] = acc[j][i];
+            if (k < a.Kout) a.out[rs * a.out_rs + zs * a.part_stride + t * a.ldo + k] = acc[j][i];
         }
     }
 }
@@ -349,6 +365,9 @@ struct CorrArgs {
     int64_t u_hi;    // owned columns (H valid for u in [0,u_hi))
     int64_t tau_hi;  // Xin valid for tau in [0, tau_hi)
     int64_t split_len;
+    int64_t ldh;     // row stride of H (K, or R*K for the per-restart Gram of a batch handle)
+    int nsplit;      // splits per restart: blockIdx.z / nsplit is the restart (single handles: one restart)
+    int64_t h_rs, x_rs, part_rs;   // per-restart offsets of H, Xin and part
 };
 
 constexpr int CORR_BTAU = 32;
@@ -366,9 +385,11 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
     const int64_t ngrp = (a.L + 7) / 8;
     const bool pvalid = p < a.K * ngrp;
     const int64_t k = pvalid ? p % a.K : 0, l0 = pvalid ? (p / a.K) * 8 : 0;
-    const int64_t tau_a = (int64_t)blockIdx.z * a.split_len;
+    const int64_t rs = blockIdx.z / a.nsplit, zs = blockIdx.z % a.nsplit;
+    const S *Hr = a.H + rs * a.h_rs, *Xr = a.Xin + rs * a.x_rs;
+    const int64_t tau_a = zs * a.split_len;
     const int64_t tau_b = min(a.tau_hi, tau_a + a.split_len);
-    double *part = a.part + (size_t)blockIdx.z * (size_t)(a.L * a.K * a.Nin);
+    double *part = a.part + rs * a.part_rs + (size_t)zs * (size_t)(a.L * a.K * a.Nin);
 
     S acc[8][TN];
 #pragma unroll
@@ -402,7 +423,7 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
             const int n = idx % BN, dt = idx / BN;
             const int64_t tau = tau0 + dt;
             S v = S(0);
-            if (tau < tau_b && n0 + n < a.Nin) v = a.Xin[tau * a.ldx + n0 + n];
+            if (tau < tau_b && n0 + n < a.Nin) v = Xr[tau * a.ldx + n0 + n];
             Xs[dt][n] = v;
         }
         for (int idx = tid; idx < CORR_PB * HWN; idx += 256) {
@@ -412,7 +433,7 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
             if (q < a.K * ngrp) {
                 const int64_t kk = q % a.K, ll0 = (q / a.K) * 8;
                 const int64_t u = tau0 - ll0 - 7 + i;
-                if (u >= 0 && u < a.u_hi) v = a.H[u * a.K + kk];
+                if (u >= 0 && u < a.u_hi) v = Hr[u * a.ldh + kk];
             }
             Hs[pp][i] = v;
         }
@@ -444,12 +465,16 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
     flush();
 }
 
-// out[i] = (S) sum_s part[s][i]   (fixed order -> deterministic)
+// out[i] = (S) sum_s part[s][i]   (fixed order -> deterministic); restart blockIdx.y reads part + y*nsplit*n and writes
+// out + y*out_rs
 template <typename S>
 __global__ void reduce_partials_kernel(const double *__restrict__ part, int nsplit, int64_t n,
-                                       S *__restrict__ out, double *__restrict__ out_d) {
+                                       S *__restrict__ out, double *__restrict__ out_d, int64_t out_rs = 0) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    part += (int64_t)blockIdx.y * nsplit * n;
+    if (out) out += (int64_t)blockIdx.y * out_rs;
+    if (out_d) out_d += (int64_t)blockIdx.y * out_rs;
     double s = 0.0;
     for (int sp = 0; sp < nsplit; ++sp) s += part[(size_t)sp * n + i];
     if (out) out[i] = (S)s;
@@ -459,16 +484,27 @@ __global__ void reduce_partials_kernel(const double *__restrict__ part, int nspl
 // ------------------------------------------------------------------------------------------
 // plain GEMM  C[M][Nn] = A[M][Kg] * B   (row-major; TRANSB: B is [Nn][Kg], else [Kg][Nn])
 //   64x64 tile, BK 16, 256 threads, 4x4 micro-tile.  Used for G*Wi and Wi*Wi' (<1% of the FLOPs).
+//   Each operand's rows are addressed through a GemmRows; blockIdx.z is the restart of a batch handle.
 // ------------------------------------------------------------------------------------------
+// Row j of a GEMM operand starts at (j / grp) * ldg + (j % grp) * ld, restart z at z * rs.  Row-major with leading dimension
+// ld: grp = INT64_MAX.  W_r of a batch handle, rows j = l*K + k at (l*R*K + r*K + k)*N: grp = K, ldg = R*K*N, ld = N, rs = K*N.
+struct GemmRows {
+    int64_t ld, grp, ldg, rs;
+    __device__ __forceinline__ int64_t at(int64_t j) const { return (j / grp) * ldg + (j % grp) * ld; }
+};
+
 template <typename S, bool TRANSB>
 __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, const S *__restrict__ B,
                                                    S *__restrict__ C, int64_t M, int64_t Nn,
-                                                   int64_t Kg, int64_t lda, int64_t ldb, int64_t ldc) {
+                                                   int64_t Kg, GemmRows ra, GemmRows rb, GemmRows rc) {
     constexpr int BM = 64, BNt = 64, BK = 16;
     __shared__ S As[BK][BM + 1];
     __shared__ S Bs[BK][BNt + 1];
     const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
     const int64_t m0 = (int64_t)blockIdx.y * BM, c0 = (int64_t)blockIdx.x * BNt;
+    A += (int64_t)blockIdx.z * ra.rs;
+    B += (int64_t)blockIdx.z * rb.rs;
+    C += (int64_t)blockIdx.z * rc.rs;
     S acc[4][4];
 #pragma unroll
     for (int i = 0; i < 4; ++i)
@@ -479,18 +515,18 @@ __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, cons
         for (int idx = tid; idx < BM * BK; idx += 256) {
             const int kk = idx % BK, mm = idx / BK;
             S v = S(0);
-            if (m0 + mm < M && k0 + kk < Kg) v = A[(m0 + mm) * lda + k0 + kk];
+            if (m0 + mm < M && k0 + kk < Kg) v = A[ra.at(m0 + mm) + k0 + kk];
             As[kk][mm] = v;
         }
         for (int idx = tid; idx < BNt * BK; idx += 256) {
             S v = S(0);
             if (TRANSB) {
                 const int kk = idx % BK, nn = idx / BK;
-                if (c0 + nn < Nn && k0 + kk < Kg) v = B[(c0 + nn) * ldb + k0 + kk];
+                if (c0 + nn < Nn && k0 + kk < Kg) v = B[rb.at(c0 + nn) + k0 + kk];
                 Bs[kk][nn] = v;
             } else {
                 const int nn = idx % BNt, kk = idx / BNt;
-                if (c0 + nn < Nn && k0 + kk < Kg) v = B[(k0 + kk) * ldb + c0 + nn];
+                if (c0 + nn < Nn && k0 + kk < Kg) v = B[rb.at(k0 + kk) + c0 + nn];
                 Bs[kk][nn] = v;
             }
         }
@@ -513,7 +549,7 @@ __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, cons
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int64_t m = m0 + ty * 4 + i, c = c0 + tx * 4 + j;
-            if (m < M && c < Nn) C[m * ldc + c] = acc[i][j];
+            if (m < M && c < Nn) C[rc.at(m) + c] = acc[i][j];
         }
 }
 
@@ -523,10 +559,11 @@ __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, cons
 // ------------------------------------------------------------------------------------------
 template <typename S>
 __global__ void build_G_kernel(const double *__restrict__ Rg, const double *__restrict__ Ht,
-                               S *__restrict__ G, int64_t K, int64_t L) {
+                               S *__restrict__ G, int64_t K, int64_t L, int64_t rg_rs = 0) {
     const int64_t KL = K * L;
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= KL * KL) return;
+    Rg += (int64_t)blockIdx.y * rg_rs; Ht += (int64_t)blockIdx.y * rg_rs; G += (int64_t)blockIdx.y * KL * KL;   // restart y
     const int64_t jp = idx % KL, j = idx / KL;
     const int64_t k = j % K, l = j / K, kp = jp % K, lp = jp / K;
     double g = (l >= lp) ? Rg[((l - lp) * K + k) * K + kp] : Rg[((lp - l) * K + kp) * K + k];
@@ -584,10 +621,13 @@ __global__ void s2_dot_G_diag_kernel(const S *__restrict__ S2, int64_t Ks, int64
 // Cf[(d+L-1)][k][k'] = sum_{l, 0<=l-d<L} S2[(l,k)][(l-d,k')]      (S2 = W W' over the unfolded rows)
 // S2 is addressed as S2[(l*Ks + k) * ld + (l'*Ks + k')]: (Ks, ld) = (K, K*L) for the SIMT product and
 // (Kp, rows_u) for the tensor-core product over the padded rows.
+// Restart blockIdx.y of a batch handle: S2 + y*s2_rs, Cf + y*(2L-1)*K*K.
 template <typename S>
-__global__ void lag_table_kernel(const S *__restrict__ S2, S *__restrict__ Cf, int64_t K, int64_t L, int64_t Ks, int64_t ld) {
+__global__ void lag_table_kernel(const S *__restrict__ S2, S *__restrict__ Cf, int64_t K, int64_t L, int64_t Ks, int64_t ld,
+                                 int64_t s2_rs = 0) {
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (2 * L - 1) * K * K) return;
+    S2 += (int64_t)blockIdx.y * s2_rs; Cf += (int64_t)blockIdx.y * (2 * L - 1) * K * K;
     const int64_t kp = idx % K, k = (idx / K) % K, d = idx / (K * K) - (L - 1);
     double s = 0.0;
     for (int64_t l = (d > 0 ? d : 0); l < L && l - d < L; ++l) s += (double)S2[(l * Ks + k) * ld + (l - d) * Ks + kp];
@@ -630,12 +670,15 @@ __global__ void __launch_bounds__(256) denomH_tail_kernel(const S *__restrict__ 
 //   C_w[d][k][k'] = sum_{l<w, 0<=l-d<L} S2[(l,k)][(l-d,k')]        (w = 1 .. L-1, one more lag l = w-1 per step)
 // in a register while w grows, and den[Tl-w][k] = sum_{d,k'} C_w[d][k][k'] H[Tl-w+d][k'].  Warp sums go to shared
 // memory, block sums to part[block][c][k] (c = L-1-w, the tail column index); denomH_tail_reduce_kernel adds the blocks
-// in order (deterministic).  grid (ceil((2L-1)K / 256), K), dynamic smem 8*(L-1) doubles.
+// in order (deterministic).  grid (ceil((2L-1)K / 256), K, restarts), dynamic smem 8*(L-1) doubles.  Restart z of a batch
+// handle reads S2 + z*s2_rs and H + z*K (row stride ldh) and writes part + z*part_rs.
 template <typename S>
 __global__ void __launch_bounds__(256) denomH_tail_prefix_kernel(const S *__restrict__ S2, const S *__restrict__ H,
                                                                   double *__restrict__ part, int64_t K, int64_t L, int64_t Tl,
-                                                                  int64_t h_lo, int64_t Ks, int64_t ld) {
+                                                                  int64_t h_lo, int64_t Ks, int64_t ld, int64_t ldh,
+                                                                  int64_t s2_rs, int64_t part_rs) {
     extern __shared__ double tail_sm[];                 // [8 warps][L-1]
+    S2 += (int64_t)blockIdx.z * s2_rs; H += (int64_t)blockIdx.z * K; part += (int64_t)blockIdx.z * part_rs;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t k = blockIdx.y;
     const bool live = e < (2 * L - 1) * K;
@@ -668,7 +711,7 @@ __global__ void __launch_bounds__(256) denomH_tail_prefix_kernel(const S *__rest
         pre += cur[q];
         const int64_t u = Tl - w + d;
         double v = 0.0;
-        if (live && pre != S(0) && u >= h_lo) v = (double)(pre * H[u * K + kp]);
+        if (live && pre != S(0) && u >= h_lo) v = (double)(pre * H[u * ldh + kp]);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
         if (lane == 0) tail_sm[warp * Lm + (w - 1)] = v;
@@ -682,27 +725,38 @@ __global__ void __launch_bounds__(256) denomH_tail_prefix_kernel(const S *__rest
     }
 }
 
+// restart blockIdx.y: part + y*part_rs, den + y*K with row stride ldd
 template <typename S>
 __global__ void denomH_tail_reduce_kernel(const double *__restrict__ part, S *__restrict__ den, int64_t K, int64_t L, int64_t Tl,
-                                          int nblocks) {
+                                          int nblocks, int64_t ldd, int64_t part_rs) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;     // c * K + k
     if (i >= (L - 1) * K) return;
+    part += (int64_t)blockIdx.y * part_rs; den += (int64_t)blockIdx.y * K;
     const int64_t c = i / K, k = i - c * K, t = Tl - (L - 1) + c;
     if (t < 0) return;
     double s = 0.0;
     for (int b = 0; b < nblocks; ++b) s += part[(int64_t)b * (L - 1) * K + i];
-    den[t * K + k] = (S)s;
+    den[t * ldd + k] = (S)s;
 }
 
 // ------------------------------------------------------------------------------------------
 // element-wise pieces
 // ------------------------------------------------------------------------------------------
 // src/algs/mult.jl:37-38 / :51-52   x <- max(eps, x * num / (den + l1 + 2*l2*x + eps))
+// Batch handles pass reg != nullptr: restart r = restart_of(i, inner, K, RK) takes l1 = reg[4r], l2 = reg[4r+1] and is
+// left alone while active[r] == 0 (a converged restart is frozen).
 template <typename S>
 __global__ void mu_update_kernel(S *__restrict__ x, const S *__restrict__ num, const S *__restrict__ den,
-                                 S l1, S l2, int64_t n) {
+                                 S l1, S l2, int64_t n, const double *__restrict__ reg = nullptr,
+                                 const int *__restrict__ active = nullptr, int64_t inner = 1, int64_t K = 1, int64_t RK = 1) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if (reg) {
+        const int64_t r = restart_of(i, inner, K, RK);
+        if (!active[r]) return;
+        l1 = (S)reg[4 * r];
+        l2 = (S)reg[4 * r + 1];
+    }
     const S eps = (S)CMF_EPS;
     S v = x[i];
     v = v * (num[i] / (den[i] + l1 + S(2) * l2 * v + eps));
@@ -734,10 +788,14 @@ __global__ void __launch_bounds__(256) mu_update_vec4_kernel(float4 *__restrict_
     }
 }
 
+// s_r != nullptr (batch handles): restart restart_of(i, inner, K, RK) is scaled by s_r[r]
 template <typename S>
-__global__ void scale_kernel(S *__restrict__ x, S s, int64_t n) {
+__global__ void scale_kernel(S *__restrict__ x, S s, int64_t n, const double *__restrict__ s_r = nullptr, int64_t inner = 1,
+                             int64_t K = 1, int64_t RK = 1) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) x[i] *= s;
+    if (i >= n) return;
+    if (s_r) s = (S)s_r[restart_of(i, inner, K, RK)];
+    x[i] *= s;
 }
 
 // partial[block] = sum over a grid-stride slice of a[i]*b[i]  (b may alias a)
@@ -752,20 +810,34 @@ __global__ void dot_partial_kernel(const S *__restrict__ a, const S *__restrict_
     if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
-// Julia W[k + K*(n + N*l)]  <->  Wi[(l*K + k)*N + n]
+// Julia W[k + K*(n + N*l)]  <->  Wi[(l*ldk + k)*N + n]; ldk = K, or R*K for the stacked W of a batch handle, whose restart
+// blockIdx.y has its Julia block at Wj + y*K*N*L and its rows at Wi + y*K*N
 template <typename S>
-__global__ void w_julia_to_internal(const S *__restrict__ Wj, S *__restrict__ Wi, int64_t K, int64_t N, int64_t L) {
+__global__ void w_julia_to_internal(const S *__restrict__ Wj, S *__restrict__ Wi, int64_t K, int64_t N, int64_t L, int64_t ldk) {
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= K * N * L) return;
+    Wj += (int64_t)blockIdx.y * K * N * L; Wi += (int64_t)blockIdx.y * K * N;
     const int64_t n = idx % N, k = (idx / N) % K, l = idx / (N * K);
-    Wi[idx] = Wj[k + K * (n + N * l)];
+    Wi[(l * ldk + k) * N + n] = Wj[k + K * (n + N * l)];
 }
 template <typename S>
-__global__ void w_internal_to_julia(const S *__restrict__ Wi, S *__restrict__ Wj, int64_t K, int64_t N, int64_t L) {
+__global__ void w_internal_to_julia(const S *__restrict__ Wi, S *__restrict__ Wj, int64_t K, int64_t N, int64_t L, int64_t ldk) {
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= K * N * L) return;
+    Wj += (int64_t)blockIdx.y * K * N * L; Wi += (int64_t)blockIdx.y * K * N;
     const int64_t k = idx % K, n = (idx / K) % N, l = idx / (K * N);
-    Wj[idx] = Wi[(l * K + k) * N + n];
+    Wj[idx] = Wi[(l * ldk + k) * N + n];
+}
+
+// H of a batch handle: R host blocks K x T (blk[r][t][k]) <-> the stacked device array st[t][r*K + k]
+template <typename S>
+__global__ void h_stack_kernel(const S *__restrict__ src, S *__restrict__ dst, int64_t K, int64_t T, int64_t R, int to_stacked) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;     // index into the stacked array
+    if (i >= R * K * T) return;
+    const int64_t c = i % (R * K), t = i / (R * K), r = c / K, k = c % K;
+    const int64_t b = (r * T + t) * K + k;
+    if (to_stacked) dst[i] = src[b];
+    else dst[b] = src[i];
 }
 
 // tail[c][k] (double) = H[Tl-(L-1)+c][k]; zeros when this shard is not the last one
@@ -778,13 +850,15 @@ __global__ void shift_stack_kernel(const S *__restrict__ H, S *__restrict__ out,
     out[e] = (t >= l) ? H[(t - l) * K + k] : S(0);
 }
 
+// restart blockIdx.y of a batch handle: H + y*K with row stride ldh, tail + y*tail_rs
 template <typename S>
 __global__ void h_tail_kernel(const S *__restrict__ H, double *__restrict__ tail, int64_t K, int64_t L,
-                              int64_t Tl, int is_last) {
+                              int64_t Tl, int is_last, int64_t ldh, int64_t tail_rs) {
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (L - 1) * K) return;
+    H += (int64_t)blockIdx.y * K; tail += (int64_t)blockIdx.y * tail_rs;
     const int64_t c = idx / K, k = idx % K;
-    tail[idx] = is_last ? (double)H[(Tl - (L - 1) + c) * K + k] : 0.0;
+    tail[idx] = is_last ? (double)H[(Tl - (L - 1) + c) * ldh + k] : 0.0;
 }
 
 // ------------------------------------------------------------------------------------------

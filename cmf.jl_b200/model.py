@@ -417,6 +417,121 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
     return res
 
 
+def _per_restart(name, v, R):
+    a = np.asarray(v, dtype=np.float64)
+    if a.ndim == 0:
+        return np.full(R, float(a))
+    if a.shape != (R,):
+        raise ValueError(f"{name} must be a scalar or have one value per restart ({R}), got shape {a.shape}")
+    return np.ascontiguousarray(a)
+
+
+def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, *, seeds=None, **kwargs):
+    """R MultUpdate fits of the same data in ONE library handle and one device loop (cmf_fit_batch).
+
+    Restart r equals ``fit_cnmf(data, L, K, alg="mult", seed=seeds[r], l1W=l1W[r], ...)`` -- or the fit from
+    ``W_init=W_init[r], H_init=H_init[r]`` -- with every other keyword the same: same initial draws and alpha rescale, same
+    ``loss_hist`` and early stop.  ``seeds`` is a sequence of R seeds; otherwise ``W_init`` (R x K x N x L) and ``H_init``
+    (R x K x T) are both given.  ``l1W``, ``l2W``, ``l1H``, ``l2H`` are scalars or length-R sequences.  A restart that meets
+    the early stop is frozen while the others go on.  The one deliberate difference from R separate fits: ``max_time`` and
+    ``time_hist`` use the batch's wall clock, so every restart has the same ``time_hist`` (cut to its own length).
+    Returns a list of R ``CNMF_results``.  MultUpdate, fp64 / fp32, one GPU, the SIMT engine."""
+    kw = _normalise_kwargs(kwargs)
+    printer = kw.get("printer", print)
+    verbose = kw.get("verbose", False)
+    layout = kw.get("layout", "LNK")
+    if layout not in ("LNK", "KNL"):
+        raise ValueError("layout must be 'LNK' or 'KNL'")
+    dtype = parse_dtype(kw.get("dtype", "f64"))
+    device = kw.get("device", 0)
+    rule_cls = _resolve_alg(alg)
+    data = np.asarray(data)
+    if data.ndim != 2:
+        raise ValueError("data must be an N x T matrix")
+    N, T = data.shape
+    L, K = int(L), int(K)
+    W0, H0 = kw.get("W_init"), kw.get("H_init")
+    if seeds is not None:
+        if W0 is not None or H0 is not None:
+            raise ValueError("give either seeds or the W_init / H_init stacks, not both")
+        seeds = list(seeds)
+        R = len(seeds)
+    elif W0 is not None and H0 is not None:
+        W0, H0 = np.asarray(W0), np.asarray(H0)
+        if W0.ndim != 4 or H0.ndim != 3 or W0.shape[0] != H0.shape[0]:
+            raise ValueError(f"W_init must be R x {(K, N, L)} and H_init R x {(K, T)}; got {W0.shape}, {H0.shape}")
+        R = W0.shape[0]
+        if W0.shape[1:] != (K, N, L) or H0.shape[1:] != (K, T):
+            raise ValueError(f"W_init must be R x {(K, N, L)} and H_init R x {(K, T)}; got {W0.shape}, {H0.shape}")
+    else:
+        raise ValueError("fit_cnmf_batch needs seeds, or both the W_init and H_init stacks")
+    if R < 1:
+        raise ValueError("a batch needs at least one restart")
+    regs = {k: _per_restart(k, kw.get(k, 0.0), R) for k in ("l1W", "l2W", "l1H", "l2H")}
+    if int(kw.get("ngpu", 1) or 1) > 1:
+        raise CMFError(3, "batched restarts run on one GPU")
+
+    if seeds is not None:                                 # model.jl:64-67, 116-117: W drawn first, then H
+        W0, H0 = np.empty((R, K, N, L)), np.empty((R, K, T))
+        for r, seed in enumerate(seeds):
+            rng = np.random.default_rng(seed)
+            W0[r], H0[r] = rng.random((K, N, L)), rng.random((K, T))
+    # restart-major host stacks, each block column-major (include/cmf_sm100.h)
+    Wj = julia_array(np.moveaxis(W0, 0, -1), dtype)
+    Hj = julia_array(np.moveaxis(H0, 0, -1), dtype)
+
+    lib = _lib.load()
+    h = ctypes.c_void_p()
+    check(lib.cmf_create_batch(ctypes.byref(h), N, T, K, L, dtype, rule_cls._ALG, R, device))
+    dptr = lambda a: a.ctypes.data_as(ctypes.POINTER(ctypes.c_double))  # noqa: E731
+    try:
+        if kw.get("engine") is not None:
+            check(lib.cmf_set_engine(h, int(kw["engine"])))
+        if kw.get("loss_mode") is not None:
+            check(lib.cmf_set_loss_mode(h, int(kw["loss_mode"])))
+        check(lib.cmf_set_data(h, fptr(julia_array(data, dtype)), 0))
+        check(lib.cmf_set_factors_batch(h, fptr(Wj), fptr(Hj)))
+        if seeds is not None:                             # model.jl:119-122, per restart
+            part = np.zeros(2 * R)
+            check(lib.cmf_init_scale_partials_batch(h, dptr(part)))
+            s = np.sqrt(np.abs(part[0::2] / part[1::2]))
+            check(lib.cmf_scale_factors_batch(h, dptr(s)))
+        unbounded = not (max_itr < math.inf)
+        cap = 1 + (int(max_itr) if not unbounded else 1_000_000)
+        loss_hist = np.zeros(R * cap)
+        time_hist = np.zeros(cap)
+        n = np.zeros(R, dtype=np.int64)
+        early = np.zeros(R, dtype=np.int32)
+        verbose and _emit(printer, "Starting ", False)
+        check(lib.cmf_fit_batch(
+            h, -1 if unbounded else int(max_itr), float(max_time),
+            int(bool(kw.get("eval_mode", False))), int(bool(kw.get("check_convergence", True))),
+            int(kw.get("patience", 3)), float(kw.get("tol", 1e-4)),
+            dptr(regs["l1W"]), dptr(regs["l2W"]), dptr(regs["l1H"]), dptr(regs["l2H"]),
+            dptr(loss_hist), dptr(time_hist), cap, n.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+            early.ctypes.data_as(ctypes.POINTER(ctypes.c_int))))
+        verbose and _emit(printer, "." * (int(n.max()) - 1), False)
+        for r in range(R):
+            if early[r]:
+                _emit(printer, "Converged early.")        # alternating.jl:64, once per restart that stopped early
+        verbose and _emit(printer, " fit!")
+        dt = np_dtype(dtype)
+        Wo = np.empty((K, N, L, R), dtype=dt, order="F")
+        Ho = np.empty((K, T, R), dtype=dt, order="F")
+        check(lib.cmf_get_factors_batch(h, fptr(Wo), fptr(Ho)))
+    finally:
+        lib.cmf_destroy(h)
+    out = []
+    for r in range(R):
+        W, H = Wo[..., r], np.asfortranarray(Ho[..., r])
+        W = np.ascontiguousarray(W.transpose(2, 1, 0)) if layout == "LNK" else np.asfortranarray(W)
+        nr = int(n[r])
+        res = CNMF_results(data, W, H, list(time_hist[:nr]), list(loss_hist[r * cap: r * cap + nr]), layout)
+        res.engine_info = dict(direct=nr, expansion=0, interval=0, last_err=0.0, engine=0, loss_mode=0, restarts=R)
+        out.append(res)
+    return out
+
+
 def _host_rescaled(data, W, H, dtype, device):
     rule = MultUpdate(data, W, H, dtype=dtype, device=device, sync_host=False)
     try:

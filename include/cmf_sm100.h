@@ -163,6 +163,50 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
             double *loss_hist, double *time_hist, int64_t cap, int64_t *n_hist,
             int *converged_early);
 
+/* ---- batched restarts: R MultUpdate fits of ONE data set in one handle ------------------------
+ *
+ * Random restarts and regulariser sweeps fit the same data many times.  A batch handle holds R factor sets of the same
+ * (K, L) over one copy of X and steps all of them with one launch per kernel: numW (mult.jl:32) and numH (mult.jl:47) of
+ * all restarts are one correlation / one transposed convolution with R*K components (X is read once per step), and the
+ * per-restart pieces (Gram, G*W, W*W', lag tables, denomH, ratio updates, loss) are launches with a restart index.  The
+ * launches of an iteration do not depend on R.  MultUpdate, fp64 and fp32, SIMT engine (0), one GPU, a single shard.
+ *
+ * Host arrays hold the R restarts one after another, each in the layout of the single-set calls: W is R blocks of
+ * K x N x L, H is R blocks of K x T; per-restart vectors have R entries.
+ *
+ * These calls work on a batch handle as on any other: cmf_set_data / cmf_synth_data (X is stored once), cmf_get_data,
+ * cmf_data_sumsq, cmf_destroy, cmf_sync, cmf_launch_count, cmf_stream, cmf_set_stream, cmf_profile, cmf_set_engine(h, 0),
+ * cmf_get_engine, cmf_last_error.  Calls that take or return ONE factor set (cmf_set_factors, cmf_init_rand,
+ * cmf_init_scale_partials, cmf_scale_factors, cmf_get_factors, cmf_update_motifs, cmf_update_feature_maps, cmf_loss,
+ * cmf_fit) return CMF_ERR_ARG with a message naming the batch call to use.  The split-phase calls, engines 1 and 2 and
+ * loss mode 1 return CMF_ERR_UNSUPPORTED. */
+
+/* Like cmf_create with R >= 1 restarts.  alg must be CMF_MULT (HALS / PGD: CMF_ERR_UNSUPPORTED).  The device footprint
+ * (about (4 R K L N + 3 R K T + (T + L) N) elements plus small per-restart tables) is computed before anything is
+ * allocated; when it exceeds the free device memory the call fails with CMF_ERR_ARG and a message stating the bytes needed.
+ * Argument checks come before any device query, as for cmf_create. */
+int cmf_create_batch(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int dtype, int alg, int64_t R,
+                     int device);
+/* W: R blocks of K x N x L, H: R blocks of K x T (restart r at W + r*K*N*L, H + r*K*T). */
+int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H);
+int cmf_get_factors_batch(cmf_handle h, void *W_out, void *H_out);
+/* out[2r] = <X, est_r>, out[2r+1] = ||est_r||^2 (model.jl:119-120); the host applies cmf_scale_factors_batch with
+ * s[r] = sqrt(|out[2r] / out[2r+1]|) (model.jl:121-122).  Each sum runs in the order of cmf_init_scale_partials. */
+int cmf_init_scale_partials_batch(cmf_handle h, double *out /* 2R */);
+int cmf_scale_factors_batch(cmf_handle h, const double *s /* R */);
+/* compute_loss(data, W_r, H_r) of every restart (src/common.jl:54-55). */
+int cmf_loss_batch(cmf_handle h, double *loss_out /* R */);
+/* cmf_fit for every restart, restart r with its own l1W[r], l2W[r], l1H[r], l2H[r] and its own early stop.  Restart r
+ * writes loss_hist[r*cap .. r*cap + n_hist[r]) and converged_early[r].  A restart that meets the early stop of
+ * alternating.jl:63-66 is frozen: nothing updates its factors again while the others go on.  The loop ends when every
+ * restart has stopped or max_itr / max_time is reached.  max_time and time_hist use the batch's own wall clock, so every
+ * restart shares time_hist (its first n_hist[r] entries are restart r's) -- the one difference from R separate cmf_fit
+ * calls, whose clocks would each measure one fit. */
+int cmf_fit_batch(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience,
+                  double tol, const double *l1W, const double *l2W, const double *l1H, const double *l2H,
+                  double *loss_hist /* R x cap, restart-major */, double *time_hist /* cap */, int64_t cap,
+                  int64_t *n_hist /* R */, int *converged_early /* R */);
+
 /* ---- split-phase steps for time-sharded fits (MultUpdate only) -------------------------- */
 
 /* 1. local W-side partials: numW (src/algs/mult.jl:32), the H cross-correlation that yields

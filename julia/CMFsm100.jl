@@ -205,4 +205,68 @@ function fit_cnmf_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, alg=:mult,
     return CNMF_results(data, W, H, time_hist[1:n[]], loss_hist[1:n[]])
 end
 
+per_restart(v, R) = v isa Number ? fill(Cdouble(v), R) : (length(v) == R ? convert(Vector{Cdouble}, v) :
+                                                          throw(ArgumentError("need a scalar or one value per restart ($R)")))
+
+"""
+    fit_cnmf_batch_sm100(data; L=10, K=5, max_itr=100, max_time=Inf, seeds=nothing, W_init=nothing, H_init=nothing, kwargs...)
+
+R MultUpdate fits of the same data in ONE batch handle and ONE `cmf_fit_batch` call (include/cmf_sm100.h).  Restart r
+equals `fit_cnmf_sm100(data; seed=seeds[r], l1W=l1W[r], ...)` -- or the fit from `W_init[:,:,:,r]`, `H_init[:,:,r]`
+(stacks K x N x L x R and K x T x R, restart last, which is the library's restart-major host layout) -- with every other
+keyword the same.  `l1W`, `l2W`, `l1H`, `l2H` are scalars or length-R vectors.  A restart that meets the early stop is
+frozen while the others go on; `max_time` and `time_hist` use the batch's own clock (shared by all restarts).  Returns a
+vector of R `CNMF_results`.  MultUpdate only, one GPU.
+"""
+function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, max_itr=100, max_time=Inf, seeds=nothing,
+                              W_init=nothing, H_init=nothing, layout=:LNK, device::Integer=0, kwargs...) where {T<:Union{Float32,Float64}}
+    kw = Dict{Symbol,Any}(kwargs)
+    for (a, b) in ((:l1_W, :l1W), (:l2_W, :l2W), (:l1_H, :l1H), (:l2_H, :l2H))
+        haskey(kw, a) && (kw[b] = pop!(kw, a))
+    end
+    N, Tt = size(data)
+    if seeds !== nothing
+        (W_init === nothing && H_init === nothing) || throw(ArgumentError("give seeds or the W_init / H_init stacks, not both"))
+        R = length(seeds)
+        W0 = zeros(T, K, N, L, R); H0 = zeros(T, K, Tt, R)
+        for (r, s) in enumerate(seeds)                             # the draws and rescale of fit_cnmf_sm100 (model.jl:64-70)
+            Random.seed!(s)
+            Wr, Hr = init_rand(data, L, K, tensor_conv)
+            W0[:, :, :, r] .= Wr; H0[:, :, r] .= Hr
+        end
+    else
+        (W_init === nothing || H_init === nothing) && throw(ArgumentError("need seeds, or both W_init and H_init"))
+        W0 = convert(Array{T,4}, W_init); H0 = convert(Array{T,3}, H_init)
+        R = size(W0, 4)
+        (size(W0)[1:3] == (K, N, L) && size(H0) == (K, Tt, R)) || throw(ArgumentError("W_init must be K x N x L x R, H_init K x T x R"))
+    end
+    regs = [per_restart(get(kw, k, 0), R) for k in (:l1W, :l2W, :l1H, :l2H)]
+    out = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:cmf_create_batch, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Cint, Cint, Int64, Cint),
+                out, N, Tt, K, L, dtype_code(T), CMF_MULT, R, device))
+    h = out[]
+    try
+        check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h, data, 0))
+        check(ccall((:cmf_set_factors_batch, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}), h, W0, H0))
+        cap = isfinite(max_itr) ? Int(max_itr) + 1 : 1_000_001
+        loss_hist = zeros(Cdouble, cap, R); time_hist = zeros(Cdouble, cap)
+        n = zeros(Int64, R); early = zeros(Cint, R)
+        check(ccall((:cmf_fit_batch, LIB), Cint,
+            (Ptr{Cvoid}, Int64, Cdouble, Cint, Cint, Cint, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Int64, Ptr{Int64}, Ptr{Cint}),
+            h, isfinite(max_itr) ? Int(max_itr) : -1, Float64(max_time),
+            get(kw, :eval_mode, false), get(kw, :check_convergence, true), get(kw, :patience, 3), get(kw, :tol, 1e-4),
+            regs[1], regs[2], regs[3], regs[4], loss_hist, time_hist, cap, n, early))
+        for r in 1:R
+            early[r] != 0 && println("Converged early.")          # alternating.jl:64, once per restart that stopped early
+        end
+        W = similar(W0); H = similar(H0)
+        check(ccall((:cmf_get_factors_batch, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}), h, W, H))
+        return [CNMF_results(data, layout == :LNK ? permutedims(W[:, :, :, r], (3, 2, 1)) : W[:, :, :, r], H[:, :, r],
+                             time_hist[1:n[r]], loss_hist[1:n[r], r]) for r in 1:R]
+    finally
+        ccall((:cmf_destroy, LIB), Cint, (Ptr{Cvoid},), h)
+    end
+end
+
 end # module
