@@ -391,7 +391,7 @@ struct Ctx : cmf_ctx {
     }
     void mark_w_dirty() { tcs.w_dirty = true; fds.w_dirty = true; fds.wx_dirty = true; }
 
-    // ---------------------------------------------------------------- frequency-domain engine (fp32, K <= 64, L <= 256)
+    // ---------------------------------------------------------------- frequency-domain engine (fp32, K <= 128, L <= 256)
     void fd_setup() {
         if constexpr (!std::is_same<S, float>::value) { return; } else {
             FdState &f = fds;

@@ -276,7 +276,9 @@ int cmf_set_loss_guard(cmf_handle h, double guard, int max_interval);
  * calibrated regime) and the relative error of the last checked prediction.  Any output pointer may be NULL. */
 int cmf_get_loss_stats(cmf_handle h, int64_t *n_direct, int64_t *n_expansion, int *interval, double *last_err);
 /* Overlap-save layout of the frequency-domain engine on this handle (first rank of a group): block length B (the smallest
- * power of two >= 8L, at most 1024, the next one when memory is short; CMF_FD_B overrides), hop V = B - L + 1 and the number of
+ * power of two >= 8L, at most 1024; halved when the half is still >= 4L and >= 64 and the shard is so short that the longer
+ * block does not cut the per-frequency product work by at least 3 %; the next power of two when memory is short; CMF_FD_B
+ * overrides with a power of two in [max(4L, 64), 1024], other values are ignored), hop V = B - L + 1 and the number of
  * blocks (padded to a multiple of 16) whose spectrum the two data-sized products stream.  Zeros when engine 2 is not in force. */
 int cmf_get_fd_layout(cmf_handle h, int *block_len, int *hop, int64_t *nblocks);
 /* The engine currently selected (0 / 1 / 2). */
