@@ -281,6 +281,7 @@ struct FdState {
     int64_t nblk2 = 0;
     DevBuf<__nv_bfloat16> Xf_hi, Xf_lo, Ah_hi, Ah_lo, Aw_hi, Aw_lo, Hf_hi, Hf_lo, Ac_hi, Ac_lo;
     DevBuf<float> Of, Df, Gf, Yf;
+    DevBuf<float2> tw;                    // twiddle table of the transforms (fd::twiddle_kernel)
     DevBuf<__nv_bfloat16> Awm_hi, Awm_lo; // direct loss pass: spectrum of W as the A operand of TC_FQX (allocated on first use)
     int64_t nbc = 0;                      // blocks per chunk of the direct loss pass (Yf holds F x nbc x 2 x N floats)
     bool wx_dirty = true;
@@ -290,12 +291,38 @@ struct FdState {
     std::string why;                      // reason the engine is unavailable
     void release() {
         Xf_hi.free(); Xf_lo.free(); Ah_hi.free(); Ah_lo.free(); Aw_hi.free(); Aw_lo.free(); Of.free(); Df.free();
-        Hf_hi.free(); Hf_lo.free(); Gf.free(); Ac_hi.free(); Ac_lo.free();
+        Hf_hi.free(); Hf_lo.free(); Gf.free(); Ac_hi.free(); Ac_lo.free(); tw.free();
         Yf.free(); Awm_hi.free(); Awm_lo.free(); nbc = 0; wx_dirty = true;
         ok = tried = false;
         x_dirty = w_dirty = h_dirty = true; hf2_valid = false;
     }
 };
+
+// The transforms are compiled per block length (log2 B = 6 .. 10) and tile width C: fd_with_b calls fn(LOGB) and fd_with_bc
+// calls fn(LOGB, C) with std::integral_constant arguments for the plan's values.  fd_cols_h never picks C = 32 at B = 1024
+// (the tile would not fit in shared memory).
+template <typename Fn>
+void fd_with_b(int logB, Fn &&fn) {
+    switch (logB) {
+    case 6: fn(std::integral_constant<int, 6>{}); break;
+    case 7: fn(std::integral_constant<int, 7>{}); break;
+    case 8: fn(std::integral_constant<int, 8>{}); break;
+    case 9: fn(std::integral_constant<int, 9>{}); break;
+    case 10: fn(std::integral_constant<int, 10>{}); break;
+    default: REQUIRE(false, "frequency-domain transforms: block length must be a power of two in [64, 1024]");
+    }
+}
+template <typename Fn>
+void fd_with_bc(int logB, int C, Fn &&fn) {
+    fd_with_b(logB, [&](auto lb) {
+        switch (C) {
+        case 8: fn(lb, std::integral_constant<int, 8>{}); break;
+        case 16: fn(lb, std::integral_constant<int, 16>{}); break;
+        case 32: fn(lb, std::integral_constant<int, 32>{}); break;
+        default: REQUIRE(false, "frequency-domain transforms: unsupported tile width");
+        }
+    });
+}
 
 template <typename S>
 struct Ctx : cmf_ctx {
@@ -460,6 +487,9 @@ struct Ctx : cmf_ctx {
             f.Of.alloc(of); f.Df.alloc(df);
             f.Hf_hi.alloc(hf); f.Hf_lo.alloc(hf); f.Gf.alloc(gf);
             f.Ac_hi.alloc(ac); f.Ac_lo.alloc(ac);
+            f.tw.alloc((size_t)f.B);
+            fd::twiddle_kernel<<<(unsigned)cdiv(f.B, 256), 256, 0, stream>>>(f.tw.p, f.B);
+            post_launch();
             __nv_bfloat16 *xs[2] = {f.Xf_hi.p, f.Xf_lo.p}, *as[2] = {f.Ah_hi.p, f.Ah_lo.p}, *ws[2] = {f.Aw_hi.p, f.Aw_lo.p};
             const uint64_t rows = (uint64_t)f.F * (uint64_t)f.nblkp;
             for (int i = 0; i < 2; ++i) {
@@ -475,14 +505,28 @@ struct Ctx : cmf_ctx {
             CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQC>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
             CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQX>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
 
-            const int big = (int)fd_smem(fd_cols_h()), small_ = (int)fd_smem(16);
-            CK(cudaFuncSetAttribute(fd::fft_x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, small_));
-            CK(cudaFuncSetAttribute(fd::ifft_resid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, small_));
-            CK(cudaFuncSetAttribute(fd::fft_w_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, small_));
-            CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, small_));
-            CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, small_));
-            CK(cudaFuncSetAttribute(fd::fft_h_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-            CK(cudaFuncSetAttribute(fd::ifft_numH_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+            // shared memory of every transform instantiation of this block length (each C the H side may pick)
+            fd_with_b(f.logB, [&](auto lb) {
+                constexpr int LB = decltype(lb)::value;
+                const int x16 = (int)fd_smem(16), w = (int)fd_smem(fd_cols_w());
+                CK(cudaFuncSetAttribute(fd::fft_x_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
+                CK(cudaFuncSetAttribute(fd::ifft_resid_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
+                fd_with_bc(f.logB, fd_cols_w(), [&](auto, auto c) {
+                    constexpr int CW = decltype(c)::value;
+                    CK(cudaFuncSetAttribute(fd::fft_w_kernel<LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+                    CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<float, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+                    CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<double, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+                });
+                for (int ch : {8, 16, 32}) {
+                    if (LB == 10 && ch == 32) continue;
+                    const int h = (int)fd_smem(ch);
+                    fd_with_bc(f.logB, ch, [&](auto, auto c) {
+                        constexpr int CH = decltype(c)::value;
+                        CK(cudaFuncSetAttribute(fd::fft_h_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
+                        CK(cudaFuncSetAttribute(fd::ifft_numH_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
+                    });
+                }
+            });
             f.x_dirty = f.w_dirty = f.h_dirty = true;
             f.ok = true;
         }
@@ -500,13 +544,50 @@ struct Ctx : cmf_ctx {
     // complex columns per CTA of the W-side transforms (fft_w / ifft_numW): as for the H side, 8 at B = 1024 keeps three CTAs per SM
     int fd_cols_w() const { return fds.B >= 1024 ? 8 : 16; }
     size_t fd_smem(int C) const { return ((size_t)fds.B * (size_t)C + (size_t)fds.B) * sizeof(float2); }   // tile + full-circle twiddle table
+    // launches of the transforms whose tile width the host picks (fd_cols_h / fd_cols_w)
+    // spectrum of nb blocks of H (hop V, first column t_off) -> hi / lo; full: see fft_h_kernel
+    void fd_fft_h(__nv_bfloat16 *hi, __nv_bfloat16 *lo, int64_t nb, int V, int full, int64_t t_off) {
+        const int C = fd_cols_h();
+        fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
+            fd::fft_h_kernel<decltype(lb)::value, decltype(c)::value><<<(unsigned)(nb * (fds.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
+                H, hi, lo, K, Tl, Tl + (L - 1), V, nb, full, t_off, fds.Kq, fd_order(nb), fds.tw.p);
+        });
+    }
+    // Of (blocks of row stride nblkp_) -> the owned columns of out, nb blocks of hop V
+    void fd_ifft_numH(const float *Of, float *out, int64_t nb, int V, int64_t nblkp_) {
+        const int C = fd_cols_h();
+        fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
+            fd::ifft_numH_kernel<decltype(lb)::value, decltype(c)::value><<<(unsigned)(nb * (fds.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
+                Of, out, K, Tl, V, nblkp_, fds.Kq, fd_order(nb), fds.tw.p);
+        });
+    }
+    // spectrum of the Lw lags of src[(l*K+k)][Nw] -> hi / lo (see fft_w_kernel)
+    void fd_fft_w(const float *src, __nv_bfloat16 *hi, __nv_bfloat16 *lo, int64_t Nw, int64_t Lw, int64_t ldw, int64_t coff, int xmode) {
+        const int C = fd_cols_w();
+        fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
+            fd::fft_w_kernel<decltype(lb)::value, decltype(c)::value><<<dim3((unsigned)cdiv(Nw, 2 * C), (unsigned)K), fd::NT, fd_smem(C), stream>>>(
+                src, hi, lo, Nw, K, Lw, ldw, coff, xmode, fds.Kq, fds.tw.p);
+        });
+    }
+    // Df (rows of ldi) -> the first L lags of out[(l*K+k)][Nw]
+    template <typename OutT>
+    void fd_ifft_numW(const float *Df, OutT *out, int64_t Nw, int64_t ldi) {
+        const int C = fd_cols_w();
+        fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
+            fd::ifft_numW_kernel<OutT, decltype(lb)::value, decltype(c)::value><<<dim3((unsigned)cdiv(Nw, 2 * C), (unsigned)K), fd::NT, fd_smem(C), stream>>>(
+                Df, out, Nw, ldi, K, L, fds.Kq, fds.tw.p);
+        });
+    }
 
     void fd_build_X() {
         if constexpr (std::is_same<S, float>::value) {
             FdState &f = fds;
             if (!f.x_dirty) return;
             dim3 grid((unsigned)(f.nblkp * cdiv(N, 32)));
-            fd::fft_x_kernel<<<grid, fd::NT, fd_smem(16), stream>>>(X.p, f.Xf_hi.p, f.Xf_lo.p, N, Tl + (L - 1), f.B, f.logB, f.V, f.nblkp, fd_order(f.nblkp));
+            fd_with_b(f.logB, [&](auto lb) {
+                fd::fft_x_kernel<decltype(lb)::value><<<grid, fd::NT, fd_smem(16), stream>>>(X.p, f.Xf_hi.p, f.Xf_lo.p, N, Tl + (L - 1), f.V, f.nblkp,
+                                                                                            fd_order(f.nblkp), f.tw.p);
+            });
             post_launch();
             f.x_dirty = false;
         }
@@ -529,7 +610,7 @@ struct Ctx : cmf_ctx {
             tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mXfMN[0], f.mXfMN[1], q);
             prof_end();
             post_launch();
-            fd::ifft_numW_kernel<float><<<dim3((unsigned)cdiv(N, 2 * fd_cols_w()), (unsigned)K), fd::NT, fd_smem(fd_cols_w()), stream>>>(f.Df.p, numW.p, N, N, K, L, f.B, f.logB, f.Kq, fd_cols_w());
+            fd_ifft_numW(f.Df.p, numW.p, N, N);
             post_launch();
         }
     }
@@ -538,10 +619,8 @@ struct Ctx : cmf_ctx {
     void fd_denomH() {
         if constexpr (std::is_same<S, float>::value) {
             FdState &f = fds;
-            fd::fft_w_kernel<<<dim3((unsigned)cdiv(K, 2 * fd_cols_w()), (unsigned)K), fd::NT, fd_smem(fd_cols_w()), stream>>>(
-                Cf.p, f.Ac_hi.p, f.Ac_lo.p, K, K, 2 * L - 1, f.B, f.logB, f.MR, f.Kq, 0, f.Kq, fd_cols_w());
+            fd_fft_w(Cf.p, f.Ac_hi.p, f.Ac_lo.p, K, 2 * L - 1, f.MR, f.Kq, 0);
             post_launch();
-            const int C = fd_cols_h();
             fd_denomH_prefetch();
             f.hf2_valid = false;                                   // consumed below; Hf is shared with the Gram / loss passes
             tc::Params q = tc_base_params();
@@ -554,8 +633,7 @@ struct Ctx : cmf_ctx {
             const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
             tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAc[0], f.mAc[1], f.mHf2K[0], f.mHf2K[1], q);
             post_launch();
-            fd::ifft_numH_kernel<<<(unsigned)(f.nblk2 * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                f.Of.p, denH.p, K, Tl, f.B, f.logB, f.V2, f.nblk2, C, f.Kq, fd_order(f.nblk2));
+            fd_ifft_numH(f.Of.p, denH.p, f.nblk2, f.V2, f.nblk2);
             post_launch();
         }
     }
@@ -565,9 +643,7 @@ struct Ctx : cmf_ctx {
         if constexpr (std::is_same<S, float>::value) {
             FdState &f = fds;
             if (!fd_active() || f.hf2_valid) return;
-            const int C = fd_cols_h();
-            fd::fft_h_kernel<<<(unsigned)(f.nblk2 * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                H, f.Hf_hi.p, f.Hf_lo.p, K, Tl, Tl + (L - 1), f.B, f.logB, f.V2, f.nblk2, C, 1, -(L - 1), f.Kq, fd_order(f.nblk2));
+            fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblk2, f.V2, 1, -(L - 1));
             post_launch();
             f.hf2_valid = true;
         }
@@ -602,13 +678,11 @@ struct Ctx : cmf_ctx {
             const size_t need_lp = (size_t)(f.nblk * ntile32);
             if (loss_part.n < need_lp) loss_part.alloc(std::max<size_t>(need_lp, 4096));
             if (f.wx_dirty) {
-                fd::fft_w_kernel<<<dim3((unsigned)cdiv(N, 2 * fd_cols_w()), (unsigned)K), fd::NT, fd_smem(fd_cols_w()), stream>>>(Wi.p, f.Awm_hi.p, f.Awm_lo.p, N, K, L, f.B, f.logB, 2 * N, N, 1, f.Kq, fd_cols_w());
+                fd_fft_w(Wi.p, f.Awm_hi.p, f.Awm_lo.p, N, L, 2 * N, N, 1);
                 post_launch();
                 f.wx_dirty = false;
             }
-            const int C = fd_cols_h();
-            fd::fft_h_kernel<<<(unsigned)(f.nblk * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                H, f.Hf_hi.p, f.Hf_lo.p, K, Tl, Tl + (L - 1), f.B, f.logB, f.V, f.nblk, C, 1, -(L - 1), f.Kq, fd_order(f.nblk));
+            fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblk, f.V, 1, -(L - 1));
             post_launch();
             prof_begin(PROF_CONV);
             for (int64_t b0 = 0; b0 < f.nblk; b0 += f.nbc) {
@@ -624,8 +698,10 @@ struct Ctx : cmf_ctx {
                 const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
                 tc::tc_kernel<tc::TC_FQX><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAwm[0], f.mAwm[1], f.mHcK[0], f.mHcK[1], q);
                 post_launch();
-                fd::ifft_resid_kernel<<<(unsigned)(cur * ntile32), fd::NT, fd_smem(16), stream>>>(
-                    f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.B, f.logB, f.V, cur, b0, fd_order(cur));
+                fd_with_b(f.logB, [&](auto lb) {
+                    fd::ifft_resid_kernel<decltype(lb)::value><<<(unsigned)(cur * ntile32), fd::NT, fd_smem(16), stream>>>(
+                        f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.V, cur, b0, fd_order(cur), f.tw.p);
+                });
                 post_launch();
             }
             prof_end();
@@ -638,9 +714,7 @@ struct Ctx : cmf_ctx {
         if constexpr (std::is_same<S, float>::value) {
             FdState &f = fds;
             if (!f.h_dirty) return;
-            const int C = fd_cols_h();
-            fd::fft_h_kernel<<<(unsigned)(f.nblkp * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                H, f.Ah_hi.p, f.Ah_lo.p, K, Tl, Tl + (L - 1), f.B, f.logB, f.V, f.nblkp, C, 0, 0, f.Kq, fd_order(f.nblkp));
+            fd_fft_h(f.Ah_hi.p, f.Ah_lo.p, f.nblkp, f.V, 0, 0);
             post_launch();
             f.h_dirty = false;
         }
@@ -651,9 +725,7 @@ struct Ctx : cmf_ctx {
             FdState &f = fds;
             f.hf2_valid = false;
             fd_spectrum_H();
-            const int C = fd_cols_h();
-            fd::fft_h_kernel<<<(unsigned)(f.nblkp * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                H, f.Hf_hi.p, f.Hf_lo.p, K, Tl, Tl + (L - 1), f.B, f.logB, f.V, f.nblkp, C, 1, 0, f.Kq, fd_order(f.nblkp));
+            fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblkp, f.V, 1, 0);
             post_launch();
             tc::Params q = tc_base_params();
             q.nprod = 3;
@@ -665,7 +737,7 @@ struct Ctx : cmf_ctx {
             const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
             tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mHfMN[0], f.mHfMN[1], q);
             post_launch();
-            fd::ifft_numW_kernel<double><<<dim3((unsigned)cdiv(K, 2 * fd_cols_w()), (unsigned)K), fd::NT, fd_smem(fd_cols_w()), stream>>>(f.Gf.p, exch1.p, K, f.Kq, K, L, f.B, f.logB, f.Kq, fd_cols_w());
+            fd_ifft_numW(f.Gf.p, exch1.p, K, f.Kq);
             post_launch();
         }
     }
@@ -675,7 +747,7 @@ struct Ctx : cmf_ctx {
             FdState &f = fds;
             fd_build_X();
             if (f.w_dirty) {
-                fd::fft_w_kernel<<<dim3((unsigned)cdiv(N, 2 * fd_cols_w()), (unsigned)K), fd::NT, fd_smem(fd_cols_w()), stream>>>(Wi.p, f.Aw_hi.p, f.Aw_lo.p, N, K, L, f.B, f.logB, 2 * N, N, 0, f.Kq, fd_cols_w());
+                fd_fft_w(Wi.p, f.Aw_hi.p, f.Aw_lo.p, N, L, 2 * N, N, 0);
                 post_launch();
                 f.w_dirty = false;
             }
@@ -691,9 +763,7 @@ struct Ctx : cmf_ctx {
             tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAw[0], f.mAw[1], f.mXfK[0], f.mXfK[1], q);
             prof_end();
             post_launch();
-            const int C = fd_cols_h();
-            fd::ifft_numH_kernel<<<(unsigned)(f.nblk * (f.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                f.Of.p, numH.p, K, Tl, f.B, f.logB, f.V, f.nblkp, C, f.Kq, fd_order(f.nblk));
+            fd_ifft_numH(f.Of.p, numH.p, f.nblk, f.V, f.nblkp);
             post_launch();
         }
     }
