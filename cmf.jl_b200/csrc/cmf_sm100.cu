@@ -168,8 +168,6 @@ struct cmf_ctx {
     virtual double loss_partial() { no_multi(); }
     virtual int loss_partial_dev() { no_multi(); }                 // leaves 1 (direct) or 2 (expansion) doubles in scalars()
     virtual double *scalars() { no_multi(); }                      // device buffer of 8 doubles
-    virtual void hals_update_motifs(double, double) { no_multi(); }
-    virtual double hals_update_feature_maps(double, double) { no_multi(); }
     virtual void hals_h_prepare() { no_multi(); }                  // Q = denomH - numH on the owned columns
     virtual void hals_h_local(void **, void **, int64_t *) { no_multi(); }     // device pointers of the local Q and H (owned columns), element count
     virtual void hals_h_full(void **, void **) { no_multi(); }     // rank 0 of a sharded fit: full-T Q and H buffers (allocated on first use)
@@ -389,147 +387,152 @@ struct Ctx : cmf_ctx {
         loss_part.alloc((size_t)std::max(2 * conv_blocks_max, 4096));
         // the tensor-core engine is set up right away only where it is the default (big contractions); small problems
         // build it lazily on cmf_set_engine(h, 1)
-        if (sizeof(S) == 4 && N >= 256 && Tl >= 4096 && K * L >= 256) {
-            tc_setup();
-            // frequency-domain engine by default where it wins: enough lags that 2*L direct flops per element exceed the
-            // ~8.5 of the per-frequency products, and room for the spectrum of X (CMF_ENGINE_DEFAULT=1 keeps engine 1)
-            const char *e = getenv("CMF_ENGINE_DEFAULT");
-            if (tcs.ok && engine == 1 && L >= 8 && K <= fd::KQ_MAX && !(e && atoi(e) == 1)) {
-                fd_setup();
-                // with this engine the expansion loss is the default too: the direct pass would cost 10x the iteration
-                if (fds.ok) { engine = 2; loss_mode = 1; }
+        if constexpr (is_f32) {
+            if (N >= 256 && Tl >= 4096 && K * L >= 256) {
+                tc_setup();
+                // frequency-domain engine by default where it wins: enough lags that 2*L direct flops per element exceed the
+                // ~8.5 of the per-frequency products, and room for the spectrum of X (CMF_ENGINE_DEFAULT=1 keeps engine 1)
+                const char *e = getenv("CMF_ENGINE_DEFAULT");
+                if (tcs.ok && engine == 1 && L >= 8 && K <= fd::KQ_MAX && !(e && atoi(e) == 1)) {
+                    fd_setup();
+                    // with this engine the expansion loss is the default too: the direct pass would cost 10x the iteration
+                    if (fds.ok) { engine = 2; loss_mode = 1; }
+                }
             }
         }
         CK(cudaStreamSynchronize(stream));
     }
 
     // ---------------------------------------------------------------- tcgen05 engine (fp32 only)
+    // Engines 1 and 2 exist for fp32 handles only.  The contraction dispatchers (section "contractions"), the direct loss
+    // pass and the runtime entries (init, tc_available, fd_available, fd_denomH_prefetch) test this; the tc_* / fd_* methods
+    // are reached only through them.  fd_active() implies tc_active().
+    static constexpr bool is_f32 = std::is_same<S, float>::value;
     bool tc_active() const { return engine >= 1 && tcs.ok; }
     bool fd_active() const { return engine == 2 && tcs.ok && fds.ok; }
     bool fd_available() override {
-        if (!tc_available()) return false;
-        if (!fds.ok && !fds.tried) fd_setup();
-        if (fds.ok) { tcs.X_hi.free(); tcs.X_lo.free(); tcs.x_dirty = true; }   // the two engines never hold both copies of X
+        if constexpr (is_f32) {
+            if (!tc_available()) return false;
+            if (!fds.ok && !fds.tried) fd_setup();
+            if (fds.ok) { tcs.X_hi.free(); tcs.X_lo.free(); tcs.x_dirty = true; }   // the two engines never hold both copies of X
+        }
         return fds.ok;
     }
     void fd_release() override { fds.release(); }
     void fd_layout(int *B, int *V, int64_t *nblk) override {
         *B = fd_active() ? fds.B : 0; *V = fd_active() ? fds.V : 0; *nblk = fd_active() ? fds.nblkp : 0;
     }
-    void mark_w_dirty() { tcs.w_dirty = true; fds.w_dirty = true; fds.wx_dirty = true; }
 
     // ---------------------------------------------------------------- frequency-domain engine (fp32, K <= 128, L <= 256)
     void fd_setup() {
-        if constexpr (!std::is_same<S, float>::value) { return; } else {
-            FdState &f = fds;
-            f.tried = true;
-            if (!tcs.ok) { f.why = "needs the tcgen05 engine"; return; }
-            if (K > fd::KQ_MAX || L > 256 || N < 16) { f.why = "needs K <= 128, L <= 256, N >= 16"; return; }
-            f.Kq = (K <= 64) ? 64 : 128;
-            f.MR = 2 * f.Kq;
-            // block length: the smallest power of two >= 8L, at most 1024 (>= 4L always: L <= 256).  A/B on B200 with the round-2
-            // transforms, same box: c4 (L = 100) 512 -> 45.9 ms, 1024 -> 43.2 ms per iteration; c3 (L = 50) 256 -> 3.86, 512 -> 3.48,
-            // 1024 -> 3.92 ms: the products move and multiply (B / V)(F / (B/2)) ~ 1.24 / 1.11 / 1.05 times the size of X at
-            // B = 4L.. / 8L.. / 16L.., the transforms get longer
-            int B0 = 64;
-            while (B0 < 8 * L && B0 < 1024) B0 *= 2;
-            while (B0 < 4 * L) B0 *= 2;
-            // ... unless this shard is so short that the longer block only adds padding: the numH product works on tiles of 256
-            // blocks, so its work goes like F * 256 * ceil(blocks / 256), the numW product's like F * blocks.  A rank of an
-            // 8-GPU c4 fit (524288 columns) has 1270 blocks of 512 (5 tiles, 1 % padding) or 567 blocks of 1024 (3 tiles, 26 %
-            // padding): the shorter block is kept when the longer one does not win at least 3 % on that count.
-            if (B0 / 2 >= 4 * L && B0 / 2 >= 64) {
-                auto work = [&](int B) {
-                    const int64_t nb = cdiv(Tl, (int64_t)(B - (int)L + 1));
-                    return (double)(B / 2 + 1) * (double)(cdiv(nb, tc::BN) * tc::BN + cdiv(nb, 16) * 16);
-                };
-                if (work(B0) > 0.97 * work(B0 / 2)) B0 /= 2;
-            }
-            int forced = 0;
-            if (const char *e = getenv("CMF_FD_B")) {
-                const int want = atoi(e);
-                if (want >= 4 * L && want >= 64 && want <= 1024 && (want & (want - 1)) == 0) forced = want;
-            }
-            tcs.X_hi.free(); tcs.X_lo.free(); tcs.x_dirty = true;
-            size_t free_b = 0, total_b = 0;
-            CK(cudaMemGetInfo(&free_b, &total_b));
-            // what this handle allocates later, beside the spectra: the HALS round kernel's component-major copies of H and
-            // Delta H and its ring of block partials; the direct loss pass's spectrum of W and a minimal chunk buffer
-            size_t later = (size_t)1 << 30;
-            if (alg == CMF_HALS) later += (size_t)2 * (size_t)(Tl + 2048) * (size_t)K * 4 + (size_t)hals2::RING * (size_t)cdiv(K, hals2::GS) * (size_t)K * hals2::CW * 4;
-            size_t xf = 0, ah = 0, aw = 0, of = 0, df = 0, hf = 0, gf = 0, ac = 0;
-            bool fits = false;
-            // the next power of two moves fewer bytes still (hop / length grows), so it is the fallback when the first choice does
-            // not fit beside the data
-            for (int B = forced ? forced : B0; B <= (forced ? forced : std::min(2 * B0, 1024)); B *= 2) {
-                int logB = 0;
-                while ((1 << logB) < B) ++logB;
-                f.B = B; f.logB = logB; f.V = B - (int)L + 1; f.F = B / 2 + 1;
-                f.nblk = cdiv(Tl, f.V);
-                f.nblkp = cdiv(f.nblk, 16) * 16;
-                xf = (size_t)f.F * (size_t)f.nblkp * 2 * (size_t)N + 64;
-                ah = (size_t)f.F * (size_t)f.nblkp * 2 * f.MR + 64;
-                aw = (size_t)f.F * f.MR * 2 * (size_t)N + 64;
-                f.V2 = B - 2 * (int)L + 2;
-                f.nblk2 = cdiv(Tl, f.V2);
-                of = (size_t)f.F * (size_t)std::max(f.nblkp, f.nblk2) * f.MR; df = (size_t)f.F * f.MR * (size_t)N;
-                // Hf serves the Gram partial (nblkp blocks) and, later on the same stream, denomH (nblk2 blocks)
-                hf = (size_t)f.F * (size_t)std::max(f.nblkp, f.nblk2) * 2 * f.Kq + 256; gf = (size_t)f.F * f.MR * f.Kq;
-                ac = (size_t)f.F * f.MR * f.MR;
-                const size_t need = 4 * (xf + ah + aw + hf + ac) + 4 * (of + df + gf);
-                const size_t loss_pass = 4 * aw + (size_t)256 * (size_t)f.F * 2 * (size_t)N * sizeof(float);
-                if (need + later + loss_pass <= free_b) { fits = true; break; }
-            }
-            if (!fits) { f.why = "not enough device memory for the spectrum of X"; return; }
-            f.Xf_hi.alloc(xf); f.Xf_lo.alloc(xf);
-            f.Ah_hi.alloc(ah); f.Ah_lo.alloc(ah);
-            f.Aw_hi.alloc(aw); f.Aw_lo.alloc(aw);
-            f.Of.alloc(of); f.Df.alloc(df);
-            f.Hf_hi.alloc(hf); f.Hf_lo.alloc(hf); f.Gf.alloc(gf);
-            f.Ac_hi.alloc(ac); f.Ac_lo.alloc(ac);
-            f.tw.alloc((size_t)f.B);
-            fd::twiddle_kernel<<<(unsigned)cdiv(f.B, 256), 256, 0, stream>>>(f.tw.p, f.B);
-            post_launch();
-            __nv_bfloat16 *xs[2] = {f.Xf_hi.p, f.Xf_lo.p}, *as[2] = {f.Ah_hi.p, f.Ah_lo.p}, *ws[2] = {f.Aw_hi.p, f.Aw_lo.p};
-            const uint64_t rows = (uint64_t)f.F * (uint64_t)f.nblkp;
-            for (int i = 0; i < 2; ++i) {
-                f.mXfK[i] = make_map_2d(xs[i], (uint64_t)(2 * N), rows, (uint64_t)N * 4, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                f.mXfMN[i] = make_map_mn(xs[i], rows * 2, (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 4);
-                f.mAw[i] = make_map_2d(ws[i], (uint64_t)(2 * N), (uint64_t)f.F * f.MR, (uint64_t)N * 4, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                f.mAh[i] = make_map_mn(as[i], rows * 2, (uint64_t)f.MR * 2, (uint64_t)(f.MR / 64), tc::BK, 2);
-                f.mHfMN[i] = make_map_mn(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, rows * 2, (uint64_t)f.Kq * 2, (uint64_t)(f.Kq / 64), tc::BK, 4);
-                f.mAc[i] = make_map_2d(i == 0 ? f.Ac_hi.p : f.Ac_lo.p, f.MR, (uint64_t)f.F * f.MR, (uint64_t)f.MR * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                f.mHf2K[i] = make_map_2d(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, f.MR, (uint64_t)f.F * (uint64_t)f.nblk2, (uint64_t)f.MR * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-            }
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQC>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQX>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-
-            // shared memory of every transform instantiation of this block length (each C the H side may pick)
-            fd_with_b(f.logB, [&](auto lb) {
-                constexpr int LB = decltype(lb)::value;
-                const int x16 = (int)fd_smem(16), w = (int)fd_smem(fd_cols_w());
-                CK(cudaFuncSetAttribute(fd::fft_x_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
-                CK(cudaFuncSetAttribute(fd::ifft_resid_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
-                fd_with_bc(f.logB, fd_cols_w(), [&](auto, auto c) {
-                    constexpr int CW = decltype(c)::value;
-                    CK(cudaFuncSetAttribute(fd::fft_w_kernel<LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
-                    CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<float, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
-                    CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<double, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
-                });
-                for (int ch : {8, 16, 32}) {
-                    if (LB == 10 && ch == 32) continue;
-                    const int h = (int)fd_smem(ch);
-                    fd_with_bc(f.logB, ch, [&](auto, auto c) {
-                        constexpr int CH = decltype(c)::value;
-                        CK(cudaFuncSetAttribute(fd::fft_h_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
-                        CK(cudaFuncSetAttribute(fd::ifft_numH_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
-                    });
-                }
-            });
-            f.x_dirty = f.w_dirty = f.h_dirty = true;
-            f.ok = true;
+        FdState &f = fds;
+        f.tried = true;
+        if (!tcs.ok) { f.why = "needs the tcgen05 engine"; return; }
+        if (K > fd::KQ_MAX || L > 256 || N < 16) { f.why = "needs K <= 128, L <= 256, N >= 16"; return; }
+        f.Kq = (K <= 64) ? 64 : 128;
+        f.MR = 2 * f.Kq;
+        // block length: the smallest power of two >= 8L, at most 1024 (>= 4L always: L <= 256).  A/B on B200 with the round-2
+        // transforms, same box: c4 (L = 100) 512 -> 45.9 ms, 1024 -> 43.2 ms per iteration; c3 (L = 50) 256 -> 3.86, 512 -> 3.48,
+        // 1024 -> 3.92 ms: the products move and multiply (B / V)(F / (B/2)) ~ 1.24 / 1.11 / 1.05 times the size of X at
+        // B = 4L.. / 8L.. / 16L.., the transforms get longer
+        int B0 = 64;
+        while (B0 < 8 * L && B0 < 1024) B0 *= 2;
+        while (B0 < 4 * L) B0 *= 2;
+        // ... unless this shard is so short that the longer block only adds padding: the numH product works on tiles of 256
+        // blocks, so its work goes like F * 256 * ceil(blocks / 256), the numW product's like F * blocks.  A rank of an
+        // 8-GPU c4 fit (524288 columns) has 1270 blocks of 512 (5 tiles, 1 % padding) or 567 blocks of 1024 (3 tiles, 26 %
+        // padding): the shorter block is kept when the longer one does not win at least 3 % on that count.
+        if (B0 / 2 >= 4 * L && B0 / 2 >= 64) {
+            auto work = [&](int B) {
+                const int64_t nb = cdiv(Tl, (int64_t)(B - (int)L + 1));
+                return (double)(B / 2 + 1) * (double)(cdiv(nb, tc::BN) * tc::BN + cdiv(nb, 16) * 16);
+            };
+            if (work(B0) > 0.97 * work(B0 / 2)) B0 /= 2;
         }
+        int forced = 0;
+        if (const char *e = getenv("CMF_FD_B")) {
+            const int want = atoi(e);
+            if (want >= 4 * L && want >= 64 && want <= 1024 && (want & (want - 1)) == 0) forced = want;
+        }
+        tcs.X_hi.free(); tcs.X_lo.free(); tcs.x_dirty = true;
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        // what this handle allocates later, beside the spectra: the HALS round kernel's component-major copies of H and
+        // Delta H and its ring of block partials; the direct loss pass's spectrum of W and a minimal chunk buffer
+        size_t later = (size_t)1 << 30;
+        if (alg == CMF_HALS) later += (size_t)2 * (size_t)(Tl + 2048) * (size_t)K * 4 + (size_t)hals2::RING * (size_t)cdiv(K, hals2::GS) * (size_t)K * hals2::CW * 4;
+        size_t xf = 0, ah = 0, aw = 0, of = 0, df = 0, hf = 0, gf = 0, ac = 0;
+        bool fits = false;
+        // the next power of two moves fewer bytes still (hop / length grows), so it is the fallback when the first choice does
+        // not fit beside the data
+        for (int B = forced ? forced : B0; B <= (forced ? forced : std::min(2 * B0, 1024)); B *= 2) {
+            int logB = 0;
+            while ((1 << logB) < B) ++logB;
+            f.B = B; f.logB = logB; f.V = B - (int)L + 1; f.F = B / 2 + 1;
+            f.nblk = cdiv(Tl, f.V);
+            f.nblkp = cdiv(f.nblk, 16) * 16;
+            xf = (size_t)f.F * (size_t)f.nblkp * 2 * (size_t)N + 64;
+            ah = (size_t)f.F * (size_t)f.nblkp * 2 * f.MR + 64;
+            aw = (size_t)f.F * f.MR * 2 * (size_t)N + 64;
+            f.V2 = B - 2 * (int)L + 2;
+            f.nblk2 = cdiv(Tl, f.V2);
+            of = (size_t)f.F * (size_t)std::max(f.nblkp, f.nblk2) * f.MR; df = (size_t)f.F * f.MR * (size_t)N;
+            // Hf serves the Gram partial (nblkp blocks) and, later on the same stream, denomH (nblk2 blocks)
+            hf = (size_t)f.F * (size_t)std::max(f.nblkp, f.nblk2) * 2 * f.Kq + 256; gf = (size_t)f.F * f.MR * f.Kq;
+            ac = (size_t)f.F * f.MR * f.MR;
+            const size_t need = 4 * (xf + ah + aw + hf + ac) + 4 * (of + df + gf);
+            const size_t loss_pass = 4 * aw + (size_t)256 * (size_t)f.F * 2 * (size_t)N * sizeof(float);
+            if (need + later + loss_pass <= free_b) { fits = true; break; }
+        }
+        if (!fits) { f.why = "not enough device memory for the spectrum of X"; return; }
+        f.Xf_hi.alloc(xf); f.Xf_lo.alloc(xf);
+        f.Ah_hi.alloc(ah); f.Ah_lo.alloc(ah);
+        f.Aw_hi.alloc(aw); f.Aw_lo.alloc(aw);
+        f.Of.alloc(of); f.Df.alloc(df);
+        f.Hf_hi.alloc(hf); f.Hf_lo.alloc(hf); f.Gf.alloc(gf);
+        f.Ac_hi.alloc(ac); f.Ac_lo.alloc(ac);
+        f.tw.alloc((size_t)f.B);
+        fd::twiddle_kernel<<<(unsigned)cdiv(f.B, 256), 256, 0, stream>>>(f.tw.p, f.B);
+        post_launch();
+        __nv_bfloat16 *xs[2] = {f.Xf_hi.p, f.Xf_lo.p}, *as[2] = {f.Ah_hi.p, f.Ah_lo.p}, *ws[2] = {f.Aw_hi.p, f.Aw_lo.p};
+        const uint64_t rows = (uint64_t)f.F * (uint64_t)f.nblkp;
+        for (int i = 0; i < 2; ++i) {
+            f.mXfK[i] = make_map_2d(xs[i], (uint64_t)(2 * N), rows, (uint64_t)N * 4, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+            f.mXfMN[i] = make_map_mn(xs[i], rows * 2, (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 4);
+            f.mAw[i] = make_map_2d(ws[i], (uint64_t)(2 * N), (uint64_t)f.F * f.MR, (uint64_t)N * 4, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            f.mAh[i] = make_map_mn(as[i], rows * 2, (uint64_t)f.MR * 2, (uint64_t)(f.MR / 64), tc::BK, 2);
+            f.mHfMN[i] = make_map_mn(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, rows * 2, (uint64_t)f.Kq * 2, (uint64_t)(f.Kq / 64), tc::BK, 4);
+            f.mAc[i] = make_map_2d(i == 0 ? f.Ac_hi.p : f.Ac_lo.p, f.MR, (uint64_t)f.F * f.MR, (uint64_t)f.MR * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            f.mHf2K[i] = make_map_2d(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, f.MR, (uint64_t)f.F * (uint64_t)f.nblk2, (uint64_t)f.MR * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+        }
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQC>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_FQX>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+
+        // shared memory of every transform instantiation of this block length (each C the H side may pick)
+        fd_with_b(f.logB, [&](auto lb) {
+            constexpr int LB = decltype(lb)::value;
+            const int x16 = (int)fd_smem(16), w = (int)fd_smem(fd_cols_w());
+            CK(cudaFuncSetAttribute(fd::fft_x_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
+            CK(cudaFuncSetAttribute(fd::ifft_resid_kernel<LB>, cudaFuncAttributeMaxDynamicSharedMemorySize, x16));
+            fd_with_bc(f.logB, fd_cols_w(), [&](auto, auto c) {
+                constexpr int CW = decltype(c)::value;
+                CK(cudaFuncSetAttribute(fd::fft_w_kernel<LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+                CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<float, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+                CK(cudaFuncSetAttribute(fd::ifft_numW_kernel<double, LB, CW>, cudaFuncAttributeMaxDynamicSharedMemorySize, w));
+            });
+            for (int ch : {8, 16, 32}) {
+                if (LB == 10 && ch == 32) continue;
+                const int h = (int)fd_smem(ch);
+                fd_with_bc(f.logB, ch, [&](auto, auto c) {
+                    constexpr int CH = decltype(c)::value;
+                    CK(cudaFuncSetAttribute(fd::fft_h_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
+                    CK(cudaFuncSetAttribute(fd::ifft_numH_kernel<LB, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, h));
+                });
+            }
+        });
+        f.x_dirty = f.w_dirty = f.h_dirty = true;
+        f.ok = true;
     }
     // component pairs per CTA of the H-side transforms: 32 (all 64 rows) while the tile fits in shared memory
     int fd_cols_h() const {
@@ -580,67 +583,61 @@ struct Ctx : cmf_ctx {
     }
 
     void fd_build_X() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            if (!f.x_dirty) return;
-            dim3 grid((unsigned)(f.nblkp * cdiv(N, 32)));
-            fd_with_b(f.logB, [&](auto lb) {
-                fd::fft_x_kernel<decltype(lb)::value><<<grid, fd::NT, fd_smem(16), stream>>>(X.p, f.Xf_hi.p, f.Xf_lo.p, N, Tl + (L - 1), f.V, f.nblkp,
-                                                                                            fd_order(f.nblkp), f.tw.p);
-            });
-            post_launch();
-            f.x_dirty = false;
-        }
+        FdState &f = fds;
+        if (!f.x_dirty) return;
+        dim3 grid((unsigned)(f.nblkp * cdiv(N, 32)));
+        fd_with_b(f.logB, [&](auto lb) {
+            fd::fft_x_kernel<decltype(lb)::value><<<grid, fd::NT, fd_smem(16), stream>>>(X.p, f.Xf_hi.p, f.Xf_lo.p, N, Tl + (L - 1), f.V, f.nblkp,
+                                                                                        fd_order(f.nblkp), f.tw.p);
+        });
+        post_launch();
+        f.x_dirty = false;
     }
     // numW through the spectrum of X (mult.jl:32)
     void fd_corr() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            fd_build_X();
-            fd_spectrum_H();
-            tc::Params q = tc_base_params();
-            q.nprod = 3;
-            q.tiles_n = cdiv(N, tc::BN);
-            q.nkb = f.nblkp * 2 / tc::BK;
-            q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
-            q.fq_rows = f.nblkp * 2;
-            q.out = f.Df.p; q.Mrows = f.MR; q.Ncols = N; q.ldo = N;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            prof_begin(PROF_CORR);
-            tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mXfMN[0], f.mXfMN[1], q);
-            prof_end();
-            post_launch();
-            fd_ifft_numW(f.Df.p, numW.p, N, N);
-            post_launch();
-        }
+        FdState &f = fds;
+        fd_build_X();
+        fd_spectrum_H();
+        tc::Params q = tc_base_params();
+        q.nprod = 3;
+        q.tiles_n = cdiv(N, tc::BN);
+        q.nkb = f.nblkp * 2 / tc::BK;
+        q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
+        q.fq_rows = f.nblkp * 2;
+        q.out = f.Df.p; q.Mrows = f.MR; q.Ncols = N; q.ldo = N;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        prof_begin(PROF_CORR);
+        tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mXfMN[0], f.mXfMN[1], q);
+        prof_end();
+        post_launch();
+        fd_ifft_numW(f.Df.p, numW.p, N, N);
+        post_launch();
     }
     // denomH = C (*) H through the spectrum of H (mult.jl:44,48): the numH product with the lag table in place of W and
     // H (both halos) in place of X; needs lag_tables() done.  The last L-1 columns are overwritten by the truncated tail.
     void fd_denomH() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            fd_fft_w(Cf.p, f.Ac_hi.p, f.Ac_lo.p, K, 2 * L - 1, f.MR, f.Kq, 0);
-            post_launch();
-            fd_denomH_prefetch();
-            f.hf2_valid = false;                                   // consumed below; Hf is shared with the Gram / loss passes
-            tc::Params q = tc_base_params();
-            q.nprod = 3;
-            q.tiles_n = cdiv(f.nblk2, tc::BN);
-            q.nkb = f.MR / tc::BK;
-            q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
-            q.fq_rows = f.nblk2;
-            q.out = f.Of.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAc[0], f.mAc[1], f.mHf2K[0], f.mHf2K[1], q);
-            post_launch();
-            fd_ifft_numH(f.Of.p, denH.p, f.nblk2, f.V2, f.nblk2);
-            post_launch();
-        }
+        FdState &f = fds;
+        fd_fft_w(Cf.p, f.Ac_hi.p, f.Ac_lo.p, K, 2 * L - 1, f.MR, f.Kq, 0);
+        post_launch();
+        fd_denomH_prefetch();
+        f.hf2_valid = false;                                   // consumed below; Hf is shared with the Gram / loss passes
+        tc::Params q = tc_base_params();
+        q.nprod = 3;
+        q.tiles_n = cdiv(f.nblk2, tc::BN);
+        q.nkb = f.MR / tc::BK;
+        q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
+        q.fq_rows = f.nblk2;
+        q.out = f.Of.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAc[0], f.mAc[1], f.mHf2K[0], f.mHf2K[1], q);
+        post_launch();
+        fd_ifft_numH(f.Of.p, denH.p, f.nblk2, f.V2, f.nblk2);
+        post_launch();
     }
     // the H-only part of fd_denomH: spectrum of the blocks of H (hop V2, both halos).  Depends on H alone, so a sharded fit runs it
     // while the all-gather of the new W is in flight (r_update_motifs).
     void fd_denomH_prefetch() override {
-        if constexpr (std::is_same<S, float>::value) {
+        if constexpr (is_f32) {
             FdState &f = fds;
             if (!fd_active() || f.hf2_valid) return;
             fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblk2, f.V2, 1, -(L - 1));
@@ -652,198 +649,189 @@ struct Ctx : cmf_ctx {
     // blocks (TC_FQX), inverse transform, subtract X, sum of squares (ifft_resid_kernel); returns the number of partials.
     // ~5x cheaper than the time-domain TC_CONV pass at c4, and free of the cancellation of the expansion.
     int64_t fd_conv_loss() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            f.hf2_valid = false;
-            const int64_t ntile32 = cdiv(N, 32);
-            if (f.Awm_hi.n == 0) {
-                const size_t aw = (size_t)f.F * 2 * f.MR * (size_t)N + 64;
-                size_t free_b = 0, total_b = 0;
-                CK(cudaMemGetInfo(&free_b, &total_b));
-                const size_t per_block = (size_t)f.F * 2 * (size_t)N * sizeof(float);          // Yf bytes per block
-                REQUIRE(free_b > 4 * aw + 256 * per_block + ((size_t)1 << 29), "not enough device memory for the frequency-domain loss pass");
-                size_t budget = std::min<size_t>((free_b - 4 * aw - ((size_t)1 << 29)) / 2, (size_t)12 << 30);
-                int64_t nbc = (int64_t)(budget / per_block) / tc::BN * tc::BN;
-                nbc = std::max<int64_t>(tc::BN, std::min<int64_t>(nbc, cdiv(f.nblk, tc::BN) * tc::BN));
-                if (const char *e = getenv("CMF_FD_NBC")) { const int64_t v = atoll(e); if (v >= tc::BN && v % tc::BN == 0 && v < nbc) nbc = v; }   // tests: force several chunks
-                f.nbc = nbc;
-                f.Awm_hi.alloc(aw); f.Awm_lo.alloc(aw);
-                f.Yf.alloc((size_t)f.F * (size_t)nbc * 2 * (size_t)N);
-                for (int i = 0; i < 2; ++i) {
-                    f.mAwm[i] = make_map_mn(i == 0 ? f.Awm_hi.p : f.Awm_lo.p, (uint64_t)f.F * 2 * f.MR, (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 2);
-                    f.mHcK[i] = make_map_2d(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, f.MR, (uint64_t)f.F * (uint64_t)f.nblk, (uint64_t)f.MR * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                }
-                f.wx_dirty = true;
+        FdState &f = fds;
+        f.hf2_valid = false;
+        const int64_t ntile32 = cdiv(N, 32);
+        if (f.Awm_hi.n == 0) {
+            const size_t aw = (size_t)f.F * 2 * f.MR * (size_t)N + 64;
+            size_t free_b = 0, total_b = 0;
+            CK(cudaMemGetInfo(&free_b, &total_b));
+            const size_t per_block = (size_t)f.F * 2 * (size_t)N * sizeof(float);          // Yf bytes per block
+            REQUIRE(free_b > 4 * aw + 256 * per_block + ((size_t)1 << 29), "not enough device memory for the frequency-domain loss pass");
+            size_t budget = std::min<size_t>((free_b - 4 * aw - ((size_t)1 << 29)) / 2, (size_t)12 << 30);
+            int64_t nbc = (int64_t)(budget / per_block) / tc::BN * tc::BN;
+            nbc = std::max<int64_t>(tc::BN, std::min<int64_t>(nbc, cdiv(f.nblk, tc::BN) * tc::BN));
+            if (const char *e = getenv("CMF_FD_NBC")) { const int64_t v = atoll(e); if (v >= tc::BN && v % tc::BN == 0 && v < nbc) nbc = v; }   // tests: force several chunks
+            f.nbc = nbc;
+            f.Awm_hi.alloc(aw); f.Awm_lo.alloc(aw);
+            f.Yf.alloc((size_t)f.F * (size_t)nbc * 2 * (size_t)N);
+            for (int i = 0; i < 2; ++i) {
+                f.mAwm[i] = make_map_mn(i == 0 ? f.Awm_hi.p : f.Awm_lo.p, (uint64_t)f.F * 2 * f.MR, (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 2);
+                f.mHcK[i] = make_map_2d(i == 0 ? f.Hf_hi.p : f.Hf_lo.p, f.MR, (uint64_t)f.F * (uint64_t)f.nblk, (uint64_t)f.MR * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
             }
-            const size_t need_lp = (size_t)(f.nblk * ntile32);
-            if (loss_part.n < need_lp) loss_part.alloc(std::max<size_t>(need_lp, 4096));
-            if (f.wx_dirty) {
-                fd_fft_w(Wi.p, f.Awm_hi.p, f.Awm_lo.p, N, L, 2 * N, N, 1);
-                post_launch();
-                f.wx_dirty = false;
-            }
-            fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblk, f.V, 1, -(L - 1));
-            post_launch();
-            prof_begin(PROF_CONV);
-            for (int64_t b0 = 0; b0 < f.nblk; b0 += f.nbc) {
-                const int64_t cur = std::min(f.nbc, f.nblk - b0);
-                tc::Params q = tc_base_params();
-                q.nprod = 3;
-                q.tiles_n = cdiv(cur, tc::BN);
-                q.tiles_m = cdiv(N, tc::BM);
-                q.nkb = f.MR / tc::BK;
-                q.MR = f.MR; q.mtiles = 1; q.units = (int64_t)f.F * 2 * q.tiles_m * q.tiles_n;
-                q.fq_rows = f.nblk; q.b_off = b0; q.nbc = cur;
-                q.out = f.Yf.p;
-                const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-                tc::tc_kernel<tc::TC_FQX><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAwm[0], f.mAwm[1], f.mHcK[0], f.mHcK[1], q);
-                post_launch();
-                fd_with_b(f.logB, [&](auto lb) {
-                    fd::ifft_resid_kernel<decltype(lb)::value><<<(unsigned)(cur * ntile32), fd::NT, fd_smem(16), stream>>>(
-                        f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.V, cur, b0, fd_order(cur), f.tw.p);
-                });
-                post_launch();
-            }
-            prof_end();
-            return f.nblk * ntile32;
+            f.wx_dirty = true;
         }
-        return 0;
+        const size_t need_lp = (size_t)(f.nblk * ntile32);
+        if (loss_part.n < need_lp) loss_part.alloc(std::max<size_t>(need_lp, 4096));
+        if (f.wx_dirty) {
+            fd_fft_w(Wi.p, f.Awm_hi.p, f.Awm_lo.p, N, L, 2 * N, N, 1);
+            post_launch();
+            f.wx_dirty = false;
+        }
+        fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblk, f.V, 1, -(L - 1));
+        post_launch();
+        prof_begin(PROF_CONV);
+        for (int64_t b0 = 0; b0 < f.nblk; b0 += f.nbc) {
+            const int64_t cur = std::min(f.nbc, f.nblk - b0);
+            tc::Params q = tc_base_params();
+            q.nprod = 3;
+            q.tiles_n = cdiv(cur, tc::BN);
+            q.tiles_m = cdiv(N, tc::BM);
+            q.nkb = f.MR / tc::BK;
+            q.MR = f.MR; q.mtiles = 1; q.units = (int64_t)f.F * 2 * q.tiles_m * q.tiles_n;
+            q.fq_rows = f.nblk; q.b_off = b0; q.nbc = cur;
+            q.out = f.Yf.p;
+            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+            tc::tc_kernel<tc::TC_FQX><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAwm[0], f.mAwm[1], f.mHcK[0], f.mHcK[1], q);
+            post_launch();
+            fd_with_b(f.logB, [&](auto lb) {
+                fd::ifft_resid_kernel<decltype(lb)::value><<<(unsigned)(cur * ntile32), fd::NT, fd_smem(16), stream>>>(
+                    f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.V, cur, b0, fd_order(cur), f.tw.p);
+            });
+            post_launch();
+        }
+        prof_end();
+        return f.nblk * ntile32;
     }
     // Ah = spectrum of the owned columns of the current H, block by block (shared by numW and the Gram partial)
     void fd_spectrum_H() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            if (!f.h_dirty) return;
-            fd_fft_h(f.Ah_hi.p, f.Ah_lo.p, f.nblkp, f.V, 0, 0);
-            post_launch();
-            f.h_dirty = false;
-        }
+        FdState &f = fds;
+        if (!f.h_dirty) return;
+        fd_fft_h(f.Ah_hi.p, f.Ah_lo.p, f.nblkp, f.V, 0, 0);
+        post_launch();
+        f.h_dirty = false;
     }
     // Gram partial Rg[d][k][k'] = sum_u H[u][k] H[u+d][k'] through the spectrum of H (u owned, u+d into the right halo)
     void fd_gram() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            f.hf2_valid = false;
-            fd_spectrum_H();
-            fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblkp, f.V, 1, 0);
-            post_launch();
-            tc::Params q = tc_base_params();
-            q.nprod = 3;
-            q.tiles_n = 1;
-            q.nkb = f.nblkp * 2 / tc::BK;
-            q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.mtiles;
-            q.fq_rows = f.nblkp * 2;
-            q.out = f.Gf.p; q.Mrows = f.MR; q.Ncols = K; q.ldo = f.Kq;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mHfMN[0], f.mHfMN[1], q);
-            post_launch();
-            fd_ifft_numW(f.Gf.p, exch1.p, K, f.Kq);
-            post_launch();
-        }
+        FdState &f = fds;
+        f.hf2_valid = false;
+        fd_spectrum_H();
+        fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblkp, f.V, 1, 0);
+        post_launch();
+        tc::Params q = tc_base_params();
+        q.nprod = 3;
+        q.tiles_n = 1;
+        q.nkb = f.nblkp * 2 / tc::BK;
+        q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.mtiles;
+        q.fq_rows = f.nblkp * 2;
+        q.out = f.Gf.p; q.Mrows = f.MR; q.Ncols = K; q.ldo = f.Kq;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        tc::tc_kernel<tc::TC_FQC><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAh[0], f.mAh[1], f.mHfMN[0], f.mHfMN[1], q);
+        post_launch();
+        fd_ifft_numW(f.Gf.p, exch1.p, K, f.Kq);
+        post_launch();
     }
     // numH through the spectrum of X (mult.jl:47)
     void fd_transconv() {
-        if constexpr (std::is_same<S, float>::value) {
-            FdState &f = fds;
-            fd_build_X();
-            if (f.w_dirty) {
-                fd_fft_w(Wi.p, f.Aw_hi.p, f.Aw_lo.p, N, L, 2 * N, N, 0);
-                post_launch();
-                f.w_dirty = false;
-            }
-            tc::Params q = tc_base_params();
-            q.nprod = 3;
-            q.tiles_n = cdiv(f.nblkp, tc::BN);
-            q.nkb = cdiv(2 * N, tc::BK);
-            q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
-            q.fq_rows = f.nblkp;
-            q.out = f.Of.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            prof_begin(PROF_TRANSCONV);
-            tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAw[0], f.mAw[1], f.mXfK[0], f.mXfK[1], q);
-            prof_end();
+        FdState &f = fds;
+        fd_build_X();
+        if (f.w_dirty) {
+            fd_fft_w(Wi.p, f.Aw_hi.p, f.Aw_lo.p, N, L, 2 * N, N, 0);
             post_launch();
-            fd_ifft_numH(f.Of.p, numH.p, f.nblk, f.V, f.nblkp);
-            post_launch();
+            f.w_dirty = false;
         }
+        tc::Params q = tc_base_params();
+        q.nprod = 3;
+        q.tiles_n = cdiv(f.nblkp, tc::BN);
+        q.nkb = cdiv(2 * N, tc::BK);
+        q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
+        q.fq_rows = f.nblkp;
+        q.out = f.Of.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        prof_begin(PROF_TRANSCONV);
+        tc::tc_kernel<tc::TC_FQT><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(f.mAw[0], f.mAw[1], f.mXfK[0], f.mXfK[1], q);
+        prof_end();
+        post_launch();
+        fd_ifft_numH(f.Of.p, numH.p, f.nblk, f.V, f.nblkp);
+        post_launch();
     }
     bool tc_available() override {
-        if (!tcs.ok && !tcs.tried) tc_setup();
+        if constexpr (is_f32) {
+            if (!tcs.ok && !tcs.tried) tc_setup();
+        }
         return tcs.ok;
     }
 
     void tc_setup() {
-        if constexpr (!std::is_same<S, float>::value) { return; } else {
-            TcState &t = tcs;
-            t.tried = true;
-            if (K > 128 || N % 8 != 0) return;
-            t.Kp = (int)(cdiv(K, 8) * 8);                          // TMA row strides must be multiples of 16 bytes
-            t.G = 128 / t.Kp;                                      // lags per 128-row tile of the transposed conv
-            t.KLp = cdiv(L * t.Kp, 64) * 64;
-            t.groups = cdiv(L, t.G);
-            t.rows_u = cdiv(L * t.Kp + 128, 128) * 128;             // dense rows l*Kp + k, padded so every 128-row box is in bounds
-            const int64_t hal = L - 1;
-            t.hrows = Tl + hal;                                   // window rows addressed (X columns incl. right halo)
-            cudaDeviceProp prop;
-            CK(cudaGetDeviceProperties(&prop, device));
-            if (prop.major != 10) return;                         // tcgen05 needs sm_100
-            t.num_sms = prop.multiProcessorCount;
-            // the bf16 planes of H (4 x the size of H in bf16) are allocated on first use (tc_h_planes): a handle that runs on
-            // the frequency-domain engine never touches them
-            t.Wc_hi.alloc((size_t)(N * t.KLp)); t.Wc_lo.alloc((size_t)(N * t.KLp));
-            t.Wu_hi.alloc((size_t)(t.rows_u * N)); t.Wu_lo.alloc((size_t)(t.rows_u * N));
-            t.groups_c = cdiv(2 * L - 1, t.G);
-            t.rows_c = cdiv((2 * L - 1) * t.Kp + 128, 128) * 128;
-            t.Cc_hi.alloc((size_t)(t.rows_c * t.Kp)); t.Cc_lo.alloc((size_t)(t.rows_c * t.Kp));
-            t.Gc_hi.alloc((size_t)(KL() * t.KLp)); t.Gc_lo.alloc((size_t)(KL() * t.KLp));
-            if (GS.n < (size_t)(t.rows_u * t.rows_u)) GS.alloc((size_t)(t.rows_u * t.rows_u));
-            // tensor maps (index 0 = hi plane, 1 = lo plane)
-            __nv_bfloat16 *wc[2] = {t.Wc_hi.p, t.Wc_lo.p};
-            __nv_bfloat16 *wu[2] = {t.Wu_hi.p, t.Wu_lo.p};
-            for (int i = 0; i < 2; ++i) {
-                t.mWc[i] = make_map_2d(wc[i], (uint64_t)t.KLp, (uint64_t)N, (uint64_t)t.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                t.mWu[i] = make_map_2d(wu[i], (uint64_t)N, (uint64_t)t.rows_u, (uint64_t)N * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                // denomH: A = C table rows (d'*Kp + k) x Kp
-                __nv_bfloat16 *cc[2] = {t.Cc_hi.p, t.Cc_lo.p};
-                t.mCu[i] = make_map_2d(cc[i], (uint64_t)t.Kp, (uint64_t)t.rows_c, (uint64_t)t.Kp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                __nv_bfloat16 *gc[2] = {t.Gc_hi.p, t.Gc_lo.p};
-                t.mWuB[i] = make_map_2d(wu[i], (uint64_t)N, (uint64_t)t.rows_u, (uint64_t)N * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                t.mWcB[i] = make_map_2d(wc[i], (uint64_t)t.KLp, (uint64_t)N, (uint64_t)t.KLp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                t.mGc[i] = make_map_2d(gc[i], (uint64_t)t.KLp, (uint64_t)KL(), (uint64_t)t.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-            }
-            // correlation work split: balance persistent CTAs, keep splits >= FLUSH_T columns
-            t.tiles_m = cdiv(t.KLp, tc::BM);
-            t.tiles_n = cdiv(N, tc::BN);
-            const int64_t tau = Tl + hal, base = t.tiles_m * t.tiles_n;
-            double best = -1.0;
-            for (int ns = 1; ns <= 16; ++ns) {
-                const int64_t sl = cdiv(cdiv(tau, ns), tc::BK) * tc::BK;
-                if (ns > 1 && sl < tc::FLUSH_T) break;
-                const int64_t units = base * cdiv(tau, sl);
-                const double eff = (double)units / (double)(cdiv(units, t.num_sms) * t.num_sms);
-                if (eff > best + 1e-9) { best = eff; t.nsplit = (int)cdiv(tau, sl); t.split_len = sl; }
-            }
-            // Gram correlation (one n tile): enough splits to fill the machine
-            {
-                const int64_t want = std::max<int64_t>(1, cdiv(2 * t.num_sms, t.tiles_m));
-                const int64_t maxs = std::max<int64_t>(1, tau / tc::FLUSH_T);
-                const int64_t ns = std::min(want, maxs);
-                t.split_len_g = cdiv(cdiv(tau, ns), tc::BK) * tc::BK;
-                t.nsplit_g = (int)cdiv(tau, t.split_len_g);
-            }
-            const size_t need = std::max((size_t)t.nsplit * (size_t)(KL() * N), (size_t)t.nsplit_g * (size_t)(KL() * K));
-            if (corr_part.n < need) corr_part.alloc(need);
-            const size_t need_lp = (size_t)(tc::EPI_WARPS * cdiv(Tl, tc::BN) * cdiv(N, tc::BM));
-            if (loss_part.n < need_lp) loss_part.alloc(std::max<size_t>(need_lp, 4096));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_CONV>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_TRANS>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_CORR>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            t.ok = true;
-            t.x_dirty = t.w_dirty = true;
-            // default engine: tensor cores when the contraction is big enough to fill 128x256 tiles
-            if (N >= 256 && Tl >= 4096 && K * L >= 256) engine = 1;
+        TcState &t = tcs;
+        t.tried = true;
+        if (K > 128 || N % 8 != 0) return;
+        t.Kp = (int)(cdiv(K, 8) * 8);                          // TMA row strides must be multiples of 16 bytes
+        t.G = 128 / t.Kp;                                      // lags per 128-row tile of the transposed conv
+        t.KLp = cdiv(L * t.Kp, 64) * 64;
+        t.groups = cdiv(L, t.G);
+        t.rows_u = cdiv(L * t.Kp + 128, 128) * 128;             // dense rows l*Kp + k, padded so every 128-row box is in bounds
+        const int64_t hal = L - 1;
+        t.hrows = Tl + hal;                                   // window rows addressed (X columns incl. right halo)
+        cudaDeviceProp prop;
+        CK(cudaGetDeviceProperties(&prop, device));
+        if (prop.major != 10) return;                         // tcgen05 needs sm_100
+        t.num_sms = prop.multiProcessorCount;
+        // the bf16 planes of H (4 x the size of H in bf16) are allocated on first use (tc_h_planes): a handle that runs on
+        // the frequency-domain engine never touches them
+        t.Wc_hi.alloc((size_t)(N * t.KLp)); t.Wc_lo.alloc((size_t)(N * t.KLp));
+        t.Wu_hi.alloc((size_t)(t.rows_u * N)); t.Wu_lo.alloc((size_t)(t.rows_u * N));
+        t.groups_c = cdiv(2 * L - 1, t.G);
+        t.rows_c = cdiv((2 * L - 1) * t.Kp + 128, 128) * 128;
+        t.Cc_hi.alloc((size_t)(t.rows_c * t.Kp)); t.Cc_lo.alloc((size_t)(t.rows_c * t.Kp));
+        t.Gc_hi.alloc((size_t)(KL() * t.KLp)); t.Gc_lo.alloc((size_t)(KL() * t.KLp));
+        if (GS.n < (size_t)(t.rows_u * t.rows_u)) GS.alloc((size_t)(t.rows_u * t.rows_u));
+        // tensor maps (index 0 = hi plane, 1 = lo plane)
+        __nv_bfloat16 *wc[2] = {t.Wc_hi.p, t.Wc_lo.p};
+        __nv_bfloat16 *wu[2] = {t.Wu_hi.p, t.Wu_lo.p};
+        for (int i = 0; i < 2; ++i) {
+            t.mWc[i] = make_map_2d(wc[i], (uint64_t)t.KLp, (uint64_t)N, (uint64_t)t.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            t.mWu[i] = make_map_2d(wu[i], (uint64_t)N, (uint64_t)t.rows_u, (uint64_t)N * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            // denomH: A = C table rows (d'*Kp + k) x Kp
+            __nv_bfloat16 *cc[2] = {t.Cc_hi.p, t.Cc_lo.p};
+            t.mCu[i] = make_map_2d(cc[i], (uint64_t)t.Kp, (uint64_t)t.rows_c, (uint64_t)t.Kp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            __nv_bfloat16 *gc[2] = {t.Gc_hi.p, t.Gc_lo.p};
+            t.mWuB[i] = make_map_2d(wu[i], (uint64_t)N, (uint64_t)t.rows_u, (uint64_t)N * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+            t.mWcB[i] = make_map_2d(wc[i], (uint64_t)t.KLp, (uint64_t)N, (uint64_t)t.KLp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+            t.mGc[i] = make_map_2d(gc[i], (uint64_t)t.KLp, (uint64_t)KL(), (uint64_t)t.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
         }
+        // correlation work split: balance persistent CTAs, keep splits >= FLUSH_T columns
+        t.tiles_m = cdiv(t.KLp, tc::BM);
+        t.tiles_n = cdiv(N, tc::BN);
+        const int64_t tau = Tl + hal, base = t.tiles_m * t.tiles_n;
+        double best = -1.0;
+        for (int ns = 1; ns <= 16; ++ns) {
+            const int64_t sl = cdiv(cdiv(tau, ns), tc::BK) * tc::BK;
+            if (ns > 1 && sl < tc::FLUSH_T) break;
+            const int64_t units = base * cdiv(tau, sl);
+            const double eff = (double)units / (double)(cdiv(units, t.num_sms) * t.num_sms);
+            if (eff > best + 1e-9) { best = eff; t.nsplit = (int)cdiv(tau, sl); t.split_len = sl; }
+        }
+        // Gram correlation (one n tile): enough splits to fill the machine
+        {
+            const int64_t want = std::max<int64_t>(1, cdiv(2 * t.num_sms, t.tiles_m));
+            const int64_t maxs = std::max<int64_t>(1, tau / tc::FLUSH_T);
+            const int64_t ns = std::min(want, maxs);
+            t.split_len_g = cdiv(cdiv(tau, ns), tc::BK) * tc::BK;
+            t.nsplit_g = (int)cdiv(tau, t.split_len_g);
+        }
+        const size_t need = std::max((size_t)t.nsplit * (size_t)(KL() * N), (size_t)t.nsplit_g * (size_t)(KL() * K));
+        if (corr_part.n < need) corr_part.alloc(need);
+        const size_t need_lp = (size_t)(tc::EPI_WARPS * cdiv(Tl, tc::BN) * cdiv(N, tc::BM));
+        if (loss_part.n < need_lp) loss_part.alloc(std::max<size_t>(need_lp, 4096));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_CONV>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_TRANS>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_CORR>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        CK(cudaFuncSetAttribute(tc::tc_kernel<tc::TC_PLAIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
+        t.ok = true;
+        t.x_dirty = t.w_dirty = true;
+        // default engine: tensor cores when the contraction is big enough to fill 128x256 tiles
+        if (N >= 256 && Tl >= 4096 && K * L >= 256) engine = 1;
     }
 
     tc::Params tc_base_params() {
@@ -857,223 +845,197 @@ struct Ctx : cmf_ctx {
 
     // the time-domain bf16 planes of X are allocated on first use: the frequency-domain engine never needs them
     void tc_split_X() {
-        if constexpr (std::is_same<S, float>::value) {
-            if (!tcs.ok || !tcs.x_dirty) return;
-            TcState &t = tcs;
-            if (t.X_hi.n == 0) {
-                const int64_t hal = L - 1;
-                t.X_hi.alloc(X.n + 64); t.X_lo.alloc(X.n + 64);      // +64: the 3-D maps may touch one atom past the last row
-                __nv_bfloat16 *xs[2] = {t.X_hi.p, t.X_lo.p};
-                for (int i = 0; i < 2; ++i) {
-                    t.mXk[i] = make_map_2d(xs[i], (uint64_t)N, (uint64_t)(Tl + hal), (uint64_t)N * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                    t.mXmn[i] = make_map_mn(xs[i], (uint64_t)(Tl + hal), (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 4);
-                }
+        if (!tcs.ok || !tcs.x_dirty) return;
+        TcState &t = tcs;
+        if (t.X_hi.n == 0) {
+            const int64_t hal = L - 1;
+            t.X_hi.alloc(X.n + 64); t.X_lo.alloc(X.n + 64);      // +64: the 3-D maps may touch one atom past the last row
+            __nv_bfloat16 *xs[2] = {t.X_hi.p, t.X_lo.p};
+            for (int i = 0; i < 2; ++i) {
+                t.mXk[i] = make_map_2d(xs[i], (uint64_t)N, (uint64_t)(Tl + hal), (uint64_t)N * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+                t.mXmn[i] = make_map_mn(xs[i], (uint64_t)(Tl + hal), (uint64_t)N * 2, (uint64_t)cdiv(N, 64), tc::BK, 4);
             }
-            tc::split_plain_kernel<<<(unsigned)cdiv((int64_t)X.n, 256), 256, 0, stream>>>(X.p, tcs.X_hi.p, tcs.X_lo.p, (int64_t)X.n);
-            post_launch();
-            tcs.x_dirty = false;
         }
+        tc::split_plain_kernel<<<(unsigned)cdiv((int64_t)X.n, 256), 256, 0, stream>>>(X.p, tcs.X_hi.p, tcs.X_lo.p, (int64_t)X.n);
+        post_launch();
+        tcs.x_dirty = false;
     }
     void tc_split_W() {
-        if constexpr (std::is_same<S, float>::value) {
-            if (!tcs.w_dirty) return;
-            tc::split_W_kernel<<<dim3((unsigned)cdiv(N, 32), (unsigned)cdiv(tcs.Kp, 32), (unsigned)L), dim3(32, 8), 0, stream>>>(
-                Wi.p, tcs.Wc_hi.p, tcs.Wc_lo.p, tcs.Wu_hi.p, tcs.Wu_lo.p, N, K, L, tcs.Kp, tcs.KLp);
-            post_launch();
-            tcs.w_dirty = false;
-        }
+        if (!tcs.w_dirty) return;
+        tc::split_W_kernel<<<dim3((unsigned)cdiv(N, 32), (unsigned)cdiv(tcs.Kp, 32), (unsigned)L), dim3(32, 8), 0, stream>>>(
+            Wi.p, tcs.Wc_hi.p, tcs.Wc_lo.p, tcs.Wu_hi.p, tcs.Wu_lo.p, N, K, L, tcs.Kp, tcs.KLp);
+        post_launch();
+        tcs.w_dirty = false;
     }
     // bf16 hi/lo planes of H for the time-domain tensor-core kernels and the maps over them, on first use
     void tc_h_planes() {
-        if constexpr (std::is_same<S, float>::value) {
-            TcState &t = tcs;
-            if (t.Hw_hi.n != 0) return;
-            const int64_t hal = L - 1;
-            const size_t hw_elems = (size_t)((Tl + 2 * hal) * t.Kp + t.KLp + 64);
-            t.Hw_hi.alloc(hw_elems); t.Hw_lo.alloc(hw_elems);
-            t.Hm_hi.alloc(hw_elems); t.Hm_lo.alloc(hw_elems);
-            __nv_bfloat16 *hw[2] = {t.Hw_hi.p, t.Hw_lo.p}, *hm[2] = {t.Hm_hi.p, t.Hm_lo.p};
-            for (int i = 0; i < 2; ++i) {
-                // overlapping-row "window" map: row t starts at element t*Kp and is KLp long
-                t.mHw[i] = make_map_2d(hw[i], (uint64_t)t.KLp, (uint64_t)t.hrows, (uint64_t)t.Kp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-                t.mHm[i] = make_map_mn(hm[i], (uint64_t)t.hrows, (uint64_t)t.Kp * 2, (uint64_t)(t.KLp / 64), tc::BK, 2);
-                // Gram: "X" = H rows from owned column 0 (owned + right halo), [t][Kp] MN-major
-                t.mHmn[i] = make_map_mn(hw[i] + hal * t.Kp, (uint64_t)(Tl + hal), (uint64_t)t.Kp * 2, (uint64_t)cdiv(t.Kp, 64), tc::BK, 4);
-                // denomH: "X" = H rows from the left halo on, K-major
-                t.mHk[i] = make_map_2d(hw[i], (uint64_t)t.Kp, (uint64_t)(Tl + 2 * hal), (uint64_t)t.Kp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
-            }
+        TcState &t = tcs;
+        if (t.Hw_hi.n != 0) return;
+        const int64_t hal = L - 1;
+        const size_t hw_elems = (size_t)((Tl + 2 * hal) * t.Kp + t.KLp + 64);
+        t.Hw_hi.alloc(hw_elems); t.Hw_lo.alloc(hw_elems);
+        t.Hm_hi.alloc(hw_elems); t.Hm_lo.alloc(hw_elems);
+        __nv_bfloat16 *hw[2] = {t.Hw_hi.p, t.Hw_lo.p}, *hm[2] = {t.Hm_hi.p, t.Hm_lo.p};
+        for (int i = 0; i < 2; ++i) {
+            // overlapping-row "window" map: row t starts at element t*Kp and is KLp long
+            t.mHw[i] = make_map_2d(hw[i], (uint64_t)t.KLp, (uint64_t)t.hrows, (uint64_t)t.Kp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
+            t.mHm[i] = make_map_mn(hm[i], (uint64_t)t.hrows, (uint64_t)t.Kp * 2, (uint64_t)(t.KLp / 64), tc::BK, 2);
+            // Gram: "X" = H rows from owned column 0 (owned + right halo), [t][Kp] MN-major
+            t.mHmn[i] = make_map_mn(hw[i] + hal * t.Kp, (uint64_t)(Tl + hal), (uint64_t)t.Kp * 2, (uint64_t)cdiv(t.Kp, 64), tc::BK, 4);
+            // denomH: "X" = H rows from the left halo on, K-major
+            t.mHk[i] = make_map_2d(hw[i], (uint64_t)t.Kp, (uint64_t)(Tl + 2 * hal), (uint64_t)t.Kp * 2, tc::BK, tc::BN, CU_TENSOR_MAP_SWIZZLE_64B);
         }
     }
     void tc_split_H(bool masked) {
-        if constexpr (std::is_same<S, float>::value) {
-            tc_h_planes();
-            const int64_t rows = Tl + 2 * (L - 1);
-            tc::split_H_kernel<<<(unsigned)cdiv(rows * tcs.Kp, 256), 256, 0, stream>>>(
-                Hbuf.p, masked ? tcs.Hm_hi.p : tcs.Hw_hi.p, masked ? tcs.Hm_lo.p : tcs.Hw_lo.p, rows, K, tcs.Kp,
-                L - 1, L - 1 + Tl, masked ? 1 : 0);
-            post_launch();
-        }
+        tc_h_planes();
+        const int64_t rows = Tl + 2 * (L - 1);
+        tc::split_H_kernel<<<(unsigned)cdiv(rows * tcs.Kp, 256), 256, 0, stream>>>(
+            Hbuf.p, masked ? tcs.Hm_hi.p : tcs.Hw_hi.p, masked ? tcs.Hm_lo.p : tcs.Hw_lo.p, rows, K, tcs.Kp,
+            L - 1, L - 1 + Tl, masked ? 1 : 0);
+        post_launch();
     }
 
     // numW via tensor cores (mult.jl:32)
     void tc_corr() {
-        if constexpr (std::is_same<S, float>::value) {
-            if (fd_active()) { fd_corr(); return; }
-            tc_split_X();
-            tc_split_H(true);
-            tc::Params q = tc_base_params();
-            q.tiles_m = tcs.tiles_m; q.tiles_n = tcs.tiles_n; q.split_len = tcs.split_len; q.tau_hi = Tl + (L - 1);
-            q.units = tcs.tiles_m * tcs.tiles_n * tcs.nsplit;
-            q.part = corr_part.p;
-            q.corr_order = 0;   // j tiles fastest: the CTAs that run together share the X tile (A/B: 124 vs 148 ms at T=1M)
-            {
-                const char *e = getenv("CMF_LOCKSTEP");            // k-block window; 0 disables (diagnostics)
-                const int w = e ? atoi(e) : 256;
-                if (w > 0) {
-                    if (lockstep.n == 0) lockstep.alloc(1024);
-                    CK(cudaMemsetAsync(lockstep.p, 0, lockstep.n * sizeof(int), stream));
-                    q.lockstep = lockstep.p; q.lockstep_window = w;
-                }
+        tc_split_X();
+        tc_split_H(true);
+        tc::Params q = tc_base_params();
+        q.tiles_m = tcs.tiles_m; q.tiles_n = tcs.tiles_n; q.split_len = tcs.split_len; q.tau_hi = Tl + (L - 1);
+        q.units = tcs.tiles_m * tcs.tiles_n * tcs.nsplit;
+        q.part = corr_part.p;
+        q.corr_order = 0;   // j tiles fastest: the CTAs that run together share the X tile (A/B: 124 vs 148 ms at T=1M)
+        {
+            const char *e = getenv("CMF_LOCKSTEP");            // k-block window; 0 disables (diagnostics)
+            const int w = e ? atoi(e) : 256;
+            if (w > 0) {
+                if (lockstep.n == 0) lockstep.alloc(1024);
+                CK(cudaMemsetAsync(lockstep.p, 0, lockstep.n * sizeof(int), stream));
+                q.lockstep = lockstep.p; q.lockstep_window = w;
             }
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            prof_begin(PROF_CORR);
-            if (q.lockstep != nullptr) {
-                // CTAs wait on one another inside this launch: co-residency must be guaranteed
-                void *args[] = {&tcs.mHm[0], &tcs.mHm[1], &tcs.mXmn[0], &tcs.mXmn[1], &q};
-                CK(cudaLaunchCooperativeKernel((void *)tc::tc_kernel<tc::TC_CORR>, dim3(grid), dim3(tc::THREADS), args, tc::SMEM_BYTES, stream));
-            } else {
-                tc::tc_kernel<tc::TC_CORR><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mHm[0], tcs.mHm[1], tcs.mXmn[0], tcs.mXmn[1], q);
-            }
-            prof_end();
-            post_launch();
-            const int64_t n = KL() * N;
-            reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, tcs.nsplit, n, numW.p, nullptr);
-            post_launch();
         }
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        prof_begin(PROF_CORR);
+        if (q.lockstep != nullptr) {
+            // CTAs wait on one another inside this launch: co-residency must be guaranteed
+            void *args[] = {&tcs.mHm[0], &tcs.mHm[1], &tcs.mXmn[0], &tcs.mXmn[1], &q};
+            CK(cudaLaunchCooperativeKernel((void *)tc::tc_kernel<tc::TC_CORR>, dim3(grid), dim3(tc::THREADS), args, tc::SMEM_BYTES, stream));
+        } else {
+            tc::tc_kernel<tc::TC_CORR><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mHm[0], tcs.mHm[1], tcs.mXmn[0], tcs.mXmn[1], q);
+        }
+        prof_end();
+        post_launch();
+        const int64_t n = KL() * N;
+        reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, tcs.nsplit, n, numW.p, nullptr);
+        post_launch();
     }
     // plain GEMM out[m*ldo + n] = sum_k A[m][k] B[n][k] on tensor cores (operands given as hi/lo tensor maps)
     void tc_plain(const CUtensorMap *mA, const CUtensorMap *mB, S *out, int64_t Mrows, int64_t Ncols, int64_t Kdim, int64_t ldo, bool sym = false) {
-        if constexpr (std::is_same<S, float>::value) {
-            tc::Params q = tc_base_params();
-            q.sym = (sym && !getenv("CMF_S2_FULL")) ? 1 : 0;
-            q.tiles_n = cdiv(Ncols, tc::BN);
-            q.nkb = cdiv(Kdim, tc::BK);
-            q.units = q.tiles_n * cdiv(Mrows, tc::BM);
-            q.out = out; q.Mrows = Mrows; q.Ncols = Ncols; q.ldo = ldo;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            tc::tc_kernel<tc::TC_PLAIN><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(mA[0], mA[1], mB[0], mB[1], q);
+        tc::Params q = tc_base_params();
+        q.sym = (sym && !getenv("CMF_S2_FULL")) ? 1 : 0;
+        q.tiles_n = cdiv(Ncols, tc::BN);
+        q.nkb = cdiv(Kdim, tc::BK);
+        q.units = q.tiles_n * cdiv(Mrows, tc::BM);
+        q.out = out; q.Mrows = Mrows; q.Ncols = Ncols; q.ldo = ldo;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        tc::tc_kernel<tc::TC_PLAIN><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(mA[0], mA[1], mB[0], mB[1], q);
+        post_launch();
+        if (q.sym) {
+            tc::mirror_upper_kernel<<<dim3((unsigned)cdiv(Mrows, 256), (unsigned)Mrows), 256, 0, stream>>>(out, Mrows, ldo);
             post_launch();
-            if (q.sym) {
-                tc::mirror_upper_kernel<<<dim3((unsigned)cdiv(Mrows, 256), (unsigned)Mrows), 256, 0, stream>>>(out, Mrows, ldo);
-                post_launch();
-            }
         }
     }
     // denomW = G * Wi (mult.jl:28,33): G is built straight into bf16 planes in the K-dim order of Wc
-    void tc_denomW(int64_t j0 = 0, int64_t j1 = -1) {
-        if (j1 < 0) j1 = KL();
-        if constexpr (std::is_same<S, float>::value) {
-            if (getenv("CMF_G_DIRECT"))          // element-wise form (kept for A/B)
-                tc::build_G_split_kernel<<<(unsigned)cdiv(KL() * tcs.KLp, 256), 256, 0, stream>>>(
-                    exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
-            else
-                tc::build_G_split_diag_kernel<<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(
-                    exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
-            post_launch();
-            tc_split_W();
-            if (j0 == 0 && j1 == KL()) {
-                tc_plain(tcs.mGc, tcs.mWcB, denW.p, KL(), N, tcs.KLp, N);
-            } else {
-                // rows [j0, j1) of G only (the W update is sharded by rows over the ranks): A maps over that row block
-                CUtensorMap mg[2];
-                __nv_bfloat16 *gc[2] = {tcs.Gc_hi.p, tcs.Gc_lo.p};
-                for (int i = 0; i < 2; ++i)
-                    mg[i] = make_map_2d(gc[i] + j0 * tcs.KLp, (uint64_t)tcs.KLp, (uint64_t)(j1 - j0), (uint64_t)tcs.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
-                tc_plain(mg, tcs.mWcB, denW.p + j0 * N, j1 - j0, N, tcs.KLp, N);
-            }
+    void tc_denomW(int64_t j0, int64_t j1) {
+        if (getenv("CMF_G_DIRECT"))          // element-wise form (kept for A/B)
+            tc::build_G_split_kernel<<<(unsigned)cdiv(KL() * tcs.KLp, 256), 256, 0, stream>>>(
+                exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
+        else
+            tc::build_G_split_diag_kernel<<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(
+                exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
+        post_launch();
+        tc_split_W();
+        if (j0 == 0 && j1 == KL()) {
+            tc_plain(tcs.mGc, tcs.mWcB, denW.p, KL(), N, tcs.KLp, N);
+        } else {
+            // rows [j0, j1) of G only (the W update is sharded by rows over the ranks): A maps over that row block
+            CUtensorMap mg[2];
+            __nv_bfloat16 *gc[2] = {tcs.Gc_hi.p, tcs.Gc_lo.p};
+            for (int i = 0; i < 2; ++i)
+                mg[i] = make_map_2d(gc[i] + j0 * tcs.KLp, (uint64_t)tcs.KLp, (uint64_t)(j1 - j0), (uint64_t)tcs.KLp * 2, tc::BK, tc::BM, CU_TENSOR_MAP_SWIZZLE_64B);
+            tc_plain(mg, tcs.mWcB, denW.p + j0 * N, j1 - j0, N, tcs.KLp, N);
         }
     }
     // Gram partial Rg[d][k][k'] = sum_u H[u][k] H[u+d][k'] via tensor cores (needs tc_split_H(true) and (false) done)
     void tc_gram() {
-        if constexpr (std::is_same<S, float>::value) {
-            tc::Params q = tc_base_params();
-            q.N = K;                                   // output row stride / column bound: Rg is [L][K][K]
-            q.tiles_m = tcs.tiles_m; q.tiles_n = 1; q.split_len = tcs.split_len_g; q.tau_hi = Tl + (L - 1);
-            q.units = tcs.tiles_m * tcs.nsplit_g;
-            q.part = corr_part.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            tc::tc_kernel<tc::TC_CORR><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mHm[0], tcs.mHm[1], tcs.mHmn[0], tcs.mHmn[1], q);
-            post_launch();
-            const int64_t n = L * K * K;
-            reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, tcs.nsplit_g, n, nullptr, exch1.p);
-            post_launch();
-        }
+        tc::Params q = tc_base_params();
+        q.N = K;                                   // output row stride / column bound: Rg is [L][K][K]
+        q.tiles_m = tcs.tiles_m; q.tiles_n = 1; q.split_len = tcs.split_len_g; q.tau_hi = Tl + (L - 1);
+        q.units = tcs.tiles_m * tcs.nsplit_g;
+        q.part = corr_part.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        tc::tc_kernel<tc::TC_CORR><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mHm[0], tcs.mHm[1], tcs.mHmn[0], tcs.mHmn[1], q);
+        post_launch();
+        const int64_t n = L * K * K;
+        reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, tcs.nsplit_g, n, nullptr, exch1.p);
+        post_launch();
     }
     // denomH = C (*) H via tensor cores (mult.jl:44,48); needs lag_tables() and tc_split_H(false) done
     void tc_denomH(bool resplit_C = true) {
-        if constexpr (std::is_same<S, float>::value) {
-            if (resplit_C) {
-                tc::split_C_kernel<<<(unsigned)cdiv(tcs.rows_c * tcs.Kp, 256), 256, 0, stream>>>(Cf.p, tcs.Cc_hi.p, tcs.Cc_lo.p, K, 2 * L - 1, tcs.Kp, tcs.rows_c);
-                post_launch();
-            }
-            tc::Params q = tc_base_params();
-            q.groups = tcs.groups_c; q.nblocks = cdiv(tcs.Kp, tc::BK); q.own = tc::BN - (tcs.G - 1);
-            q.units = cdiv(Tl, q.own);
-            q.out = denH.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mCu[0], tcs.mCu[1], tcs.mHk[0], tcs.mHk[1], q);
+        if (resplit_C) {
+            tc::split_C_kernel<<<(unsigned)cdiv(tcs.rows_c * tcs.Kp, 256), 256, 0, stream>>>(Cf.p, tcs.Cc_hi.p, tcs.Cc_lo.p, K, 2 * L - 1, tcs.Kp, tcs.rows_c);
             post_launch();
         }
+        tc::Params q = tc_base_params();
+        q.groups = tcs.groups_c; q.nblocks = cdiv(tcs.Kp, tc::BK); q.own = tc::BN - (tcs.G - 1);
+        q.units = cdiv(Tl, q.own);
+        q.out = denH.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mCu[0], tcs.mCu[1], tcs.mHk[0], tcs.mHk[1], q);
+        post_launch();
     }
     // numH via tensor cores (mult.jl:47)
     void tc_transconv() {
-        if constexpr (std::is_same<S, float>::value) {
-            if (fd_active()) { fd_transconv(); return; }
-            tc_split_X();
-            tc_split_W();
-            tc::Params q = tc_base_params();
-            q.groups = tcs.groups; q.nblocks = cdiv(N, tc::BK); q.own = tc::BN - (tcs.G - 1);
-            q.units = cdiv(Tl, q.own);
-            q.out = numH.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            {
-                const char *e = getenv("CMF_LOCKSTEP_TRANS");      // k-block window; 0 (default) disables
-                const int w = e ? atoi(e) : 0;
-                if (w > 0 && q.units >= (int64_t)grid) {
-                    if (lockstep.n == 0) lockstep.alloc(1024);
-                    CK(cudaMemsetAsync(lockstep.p, 0, lockstep.n * sizeof(int), stream));
-                    q.lockstep = lockstep.p; q.lockstep_window = w;
-                }
+        tc_split_X();
+        tc_split_W();
+        tc::Params q = tc_base_params();
+        q.groups = tcs.groups; q.nblocks = cdiv(N, tc::BK); q.own = tc::BN - (tcs.G - 1);
+        q.units = cdiv(Tl, q.own);
+        q.out = numH.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        {
+            const char *e = getenv("CMF_LOCKSTEP_TRANS");      // k-block window; 0 (default) disables
+            const int w = e ? atoi(e) : 0;
+            if (w > 0 && q.units >= (int64_t)grid) {
+                if (lockstep.n == 0) lockstep.alloc(1024);
+                CK(cudaMemsetAsync(lockstep.p, 0, lockstep.n * sizeof(int), stream));
+                q.lockstep = lockstep.p; q.lockstep_window = w;
             }
-            prof_begin(PROF_TRANSCONV);
-            if (q.lockstep != nullptr) {
-                void *args[] = {&tcs.mWu[0], &tcs.mWu[1], &tcs.mXk[0], &tcs.mXk[1], &q};
-                CK(cudaLaunchCooperativeKernel((void *)tc::tc_kernel<tc::TC_TRANS>, dim3(grid), dim3(tc::THREADS), args, tc::SMEM_BYTES, stream));
-            } else {
-                tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWu[0], tcs.mWu[1], tcs.mXk[0], tcs.mXk[1], q);
-            }
-            prof_end();
-            post_launch();
         }
+        prof_begin(PROF_TRANSCONV);
+        if (q.lockstep != nullptr) {
+            void *args[] = {&tcs.mWu[0], &tcs.mWu[1], &tcs.mXk[0], &tcs.mXk[1], &q};
+            CK(cudaLaunchCooperativeKernel((void *)tc::tc_kernel<tc::TC_TRANS>, dim3(grid), dim3(tc::THREADS), args, tc::SMEM_BYTES, stream));
+        } else {
+            tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWu[0], tcs.mWu[1], tcs.mXk[0], tcs.mXk[1], q);
+        }
+        prof_end();
+        post_launch();
     }
     // sum of squared residuals via tensor cores (mult.jl:55-57); returns the number of partials written
     int64_t tc_conv_loss() {
-        if constexpr (std::is_same<S, float>::value) {
-            tc_split_W();
-            tc_split_H(false);
-            tc::Params q = tc_base_params();
-            q.tiles_n = cdiv(N, tc::BM);
-            q.nkb = tcs.KLp / tc::BK;
-            q.units = q.tiles_n * cdiv(Tl, tc::BN);
-            q.X = X.p; q.partial = loss_part.p;
-            const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-            prof_begin(PROF_CONV);
-            tc::tc_kernel<tc::TC_CONV><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWc[0], tcs.mWc[1], tcs.mHw[0], tcs.mHw[1], q);
-            prof_end();
-            post_launch();
-            return tc::EPI_WARPS * q.units;
-        }
-        return 0;
+        tc_split_W();
+        tc_split_H(false);
+        tc::Params q = tc_base_params();
+        q.tiles_n = cdiv(N, tc::BM);
+        q.nkb = tcs.KLp / tc::BK;
+        q.units = q.tiles_n * cdiv(Tl, tc::BN);
+        q.X = X.p; q.partial = loss_part.p;
+        const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
+        prof_begin(PROF_CONV);
+        tc::tc_kernel<tc::TC_CONV><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWc[0], tcs.mWc[1], tcs.mHw[0], tcs.mHw[1], q);
+        prof_end();
+        post_launch();
+        return tc::EPI_WARPS * q.units;
     }
 
     ~Ctx() override {
@@ -1281,7 +1243,7 @@ struct Ctx : cmf_ctx {
     // comes out of the H update for free.  Returns whether the inner product was produced.
     DevBuf<double> mu_part;
     bool launch_mu(S *x, const S *num, const S *den, double l1, double l2, int64_t n, double *dot_dst = nullptr) {
-        if constexpr (std::is_same<S, float>::value) {
+        if constexpr (is_f32) {
             const bool aligned = (((uintptr_t)x | (uintptr_t)num | (uintptr_t)den) & 15) == 0;
             if (aligned && n % 4 == 0 && n >= 4096) {
                 const unsigned grid = (unsigned)std::min<int64_t>(cdiv(n / 4, 256), 148 * 8);
@@ -1299,6 +1261,24 @@ struct Ctx : cmf_ctx {
         return false;
     }
 
+    // ---------------------------------------------------------------- what a change of X, W or H makes stale
+    // Every change of X, W or H goes through these.  Elsewhere a cache flag is written only by engine setup and by the code
+    // that recomputes or consumes the cached operand.
+    void x_changed() {                    // planes / spectrum of X, numH
+        tcs.x_dirty = fds.x_dirty = true;
+        numH_valid = numH_dot_valid = false;
+        calib_reset();
+    }
+    void w_changed() {                    // planes / spectra of W, numH and W W'
+        tcs.w_dirty = fds.w_dirty = fds.wx_dirty = true;
+        numH_valid = numH_dot_valid = false;
+    }
+    void h_changed() override {           // Gram partial, spectra of H; numH too (the HALS sweep leaves Q there)
+        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
+        numH_valid = numH_dot_valid = false;
+    }
+    void factors_replaced() { w_changed(); h_changed(); calib_reset(); }
+
     // ---------------------------------------------------------------- data
     void set_data(const void *Xh, int64_t first_col) override {
         REQUIRE(Xh != nullptr, "set_data: null pointer");
@@ -1315,10 +1295,7 @@ struct Ctx : cmf_ctx {
         CK(cudaStreamSynchronize(stream));
     }
     void finish_data() {
-        tcs.x_dirty = true;
-        fds.x_dirty = true;
-        numH_valid = false; numH_dot_valid = false;
-        calib_reset();
+        x_changed();
         data_sumsq_local = data_sumsq();
         data_norm = std::sqrt(data_sumsq_local);
         pgd_cur_loss = data_norm;
@@ -1361,12 +1338,9 @@ struct Ctx : cmf_ctx {
         CK(cudaMemcpyAsync(H + (lo - t0) * K, src, (size_t)((hi - lo) * K) * sizeof(S), cudaMemcpyHostToDevice, stream));
         CK(cudaStreamSynchronize(stream));
         have_factors = true;
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
+        factors_replaced();
         pgd_stepW = pgd_stepH = 5.0;            // a new rule instance (pgd.jl:147-149)
         pgd_cur_loss = data_norm;
-        calib_reset();
     }
 
     void init_rand(uint64_t seed) override {
@@ -1381,10 +1355,7 @@ struct Ctx : cmf_ctx {
         post_launch();
         CK(cudaStreamSynchronize(stream));
         have_factors = true;
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
-        calib_reset();
+        factors_replaced();
     }
 
     void init_scale_partials(double out[2]) override {
@@ -1405,10 +1376,7 @@ struct Ctx : cmf_ctx {
         post_launch();
         scale_kernel<S><<<(unsigned)cdiv((int64_t)Hbuf.n, 256), 256, 0, stream>>>(Hbuf.p, (S)s, (int64_t)Hbuf.n);
         post_launch();
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
-        calib_reset();
+        factors_replaced();
     }
 
     void get_factors(void *Wo, void *Ho) override {
@@ -1596,22 +1564,46 @@ struct Ctx : cmf_ctx {
         post_launch();
     }
 
-    // ---------------------------------------------------------------- MU (src/algs/mult.jl)
-    void w_partials() override {
-        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        // numW partial over the owned u (mult.jl:32): Xin = X incl. right halo
-        if (tc_active()) tc_corr();
-        else launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
-        // Gram partial Rg[d][k][k'] = sum_u H[u][k] H[u+d][k'] (owned u, right halo for u+d); already resident
-        // when the expansion loss of the previous iteration computed it for the same H
-        if (!gram_valid) gram_partial();
-        gram_valid = false;     // the host all-reduces the buffer in place: it is consumed by this step
-    }
+    // ---------------------------------------------------------------- contractions
+    // Each contraction picks its engine here and nowhere else: SIMT unless the tensor cores are on (never on fp64 handles),
+    // then the frequency-domain engine where it is active, the time-domain one otherwise.
 
+    // numW partial over the owned u (mult.jl:32): Xin = X incl. right halo
+    void compute_numW() {
+        if (!tc_active()) launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
+        else if constexpr (is_f32) { if (fd_active()) fd_corr(); else tc_corr(); }
+    }
+    // numH (mult.jl:47)
+    void compute_numH() {
+        if (!tc_active()) launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
+        else if constexpr (is_f32) { if (fd_active()) fd_transconv(); else tc_transconv(); }
+    }
+    // denomW = G * Wi (mult.jl:28,33) for the unfolded rows [j0, j1); the frequency-domain engine runs it in the time domain
+    void compute_denomW(int64_t j0, int64_t j1) {
+        if (!tc_active()) {
+            build_G();
+            launch_gemm<false>(GS.p + j0 * KL(), Wi.p, denW.p + j0 * N, j1 - j0, N, KL(), KL(), N, N);
+        } else if constexpr (is_f32) {
+            tc_denomW(j0, j1);
+        }
+    }
+    // W W' and its lag tables, then denomH = C (*) H on all owned columns (mult.jl:44,48), then the truncated tail
+    void compute_denomH() {
+        lag_tables();
+        if (!tc_active()) launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, K, Tl, Tl + 2 * (L - 1));
+        else if constexpr (is_f32) {
+            if (fd_active()) fd_denomH();
+            else { tc_split_H(false); tc_denomH(); }
+        }
+        if (is_last && L > 1) launch_denomH_tail();
+    }
+    // Gram partial Rg[d][k][k'] = sum_u H[u][k] H[u+d][k'] (owned u, right halo for u+d) and the H tail block
     void gram_partial() {
-        if (fd_active()) fd_gram();
-        else if (tc_active()) { tc_split_H(true); tc_split_H(false); tc_gram(); }
-        else launch_corr(H, K, K, Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p);
+        if (!tc_active()) launch_corr(H, K, K, Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p);
+        else if constexpr (is_f32) {
+            if (fd_active()) fd_gram();
+            else { tc_split_H(true); tc_split_H(false); tc_gram(); }
+        }
         if (L > 1) {
             h_tail_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl, is_last ? 1 : 0, K, 0);
             post_launch();
@@ -1623,26 +1615,26 @@ struct Ctx : cmf_ctx {
         post_launch();
     }
 
+    // ---------------------------------------------------------------- MU (src/algs/mult.jl)
+    void w_partials() override {
+        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
+        compute_numW();
+        // the Gram partial is already resident when the expansion loss of the previous iteration computed it for the same H
+        if (!gram_valid) gram_partial();
+        gram_valid = false;     // the host all-reduces the buffer in place: it is consumed by this step
+    }
+
     void w_apply(double l1W, double l2W) override {
         if (alg == CMF_HALS) { hals_w_apply(l1W, l2W); return; }
         REQUIRE(alg == CMF_MULT, "the split-phase W update serves MultUpdate and HALSUpdate");
         w_denom_rows(0, KL());
         w_update_rows(l1W, l2W, 0, KL());
     }
-    // denomW = G * Wi (mult.jl:28,33) for the unfolded rows [j0, j1)
-    void w_denom_rows(int64_t j0, int64_t j1) override {
-        if (tc_active()) {
-            tc_denomW(j0, j1);                                                    // on tensor cores
-        } else {
-            build_G();
-            launch_gemm<false>(GS.p + j0 * KL(), Wi.p, denW.p + j0 * N, j1 - j0, N, KL(), KL(), N, N);
-        }
-    }
+    void w_denom_rows(int64_t j0, int64_t j1) override { compute_denomW(j0, j1); }
     // mult.jl:37-38 on the rows [j0, j1) (the whole update when the range is everything)
     void w_update_rows(double l1W, double l2W, int64_t j0, int64_t j1) override {
         launch_mu(Wi.p + j0 * N, numW.p + j0 * N, denW.p + j0 * N, l1W, l2W, (j1 - j0) * N);
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
+        w_changed();
     }
     void w_rows_buffers(void **numw, void **w, int64_t *row_elems) override { *numw = numW.p; *w = Wi.p; *row_elems = N; }
 
@@ -1650,13 +1642,13 @@ struct Ctx : cmf_ctx {
     int64_t s2_ks = 0, s2_ld = 0;
 
     void lag_tables() {
-        if (tc_active()) {
+        if (!tc_active()) {
+            launch_gemm<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, N, N, KL());              // S2 = Wi Wi'
+            s2_ks = K; s2_ld = KL();
+        } else if constexpr (is_f32) {
             tc_split_W();
             tc_plain(tcs.mWu, tcs.mWuB, GS.p, tcs.rows_u, tcs.rows_u, N, tcs.rows_u, true);   // S2 = Wu Wu' on tensor cores (lower tiles + mirror)
             s2_ks = tcs.Kp; s2_ld = tcs.rows_u;
-        } else {
-            launch_gemm<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, N, N, KL());              // S2 = Wi Wi'
-            s2_ks = K; s2_ld = KL();
         }
         lag_table_kernel<S><<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(GS.p, Cf.p, K, L, s2_ks, s2_ld);
         post_launch();
@@ -1684,20 +1676,13 @@ struct Ctx : cmf_ctx {
 
     void h_update(double l1H, double l2H) override {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        if (tc_active()) tc_transconv();
-        else launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));    // numH (mult.jl:47)
-        lag_tables();
-        // denomH = C (*) H on all owned columns (mult.jl:44,48), then the truncated tail
-        if (fd_active()) fd_denomH();
-        else if (tc_active()) { tc_split_H(false); tc_denomH(); }
-        else launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, K, Tl, Tl + 2 * (L - 1));
-        if (is_last && L > 1) {
-            launch_denomH_tail();
-        }
+        compute_numH();
+        compute_denomH();
         // mult.jl:51-52; with the expansion loss in force the update also leaves <numH, H'> in scal[4]
-        numH_dot_valid = launch_mu(H, numH.p, denH.p, l1H, l2H, Tl * K, (loss_mode == 1 && alg == CMF_MULT) ? scal.p + 4 : nullptr);
-        numH_valid = (alg == CMF_MULT);
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
+        const bool dot = launch_mu(H, numH.p, denH.p, l1H, l2H, Tl * K, (loss_mode == 1 && alg == CMF_MULT) ? scal.p + 4 : nullptr);
+        h_changed();
+        numH_valid = (alg == CMF_MULT);     // numH and W W' are still those of the current W
+        numH_dot_valid = dot;
     }
 
     double *scalars() override { return scal.p; }
@@ -1711,13 +1696,12 @@ struct Ctx : cmf_ctx {
         if (loss_mode == 1 && tc_active()) {
             // frequency-domain engine: numH and W W' are cheap, so the expansion also serves calls that find them stale
             // (the loss at the initial factors, after a W-only step, after the HALS sweep overwrote numH)
-            if (!numH_valid && fd_active()) { tc_transconv(); lag_tables(); numH_valid = true; numH_dot_valid = false; }
+            if (!numH_valid && fd_active()) { compute_numH(); lag_tables(); numH_valid = true; numH_dot_valid = false; }
             if (numH_valid) { loss_partial_expansion_dev(); return 2; }
         }
         int64_t nb = conv_nblocks(0, Tl);
-        if (fd_active() && !getenv("CMF_FD_LOSS_TC")) nb = fd_conv_loss();
-        else if (tc_active()) nb = tc_conv_loss();
-        else launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p);  // mult.jl:55-57
+        if (!tc_active()) launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p);  // mult.jl:55-57
+        else if constexpr (is_f32) nb = (fd_active() && !getenv("CMF_FD_LOSS_TC")) ? fd_conv_loss() : tc_conv_loss();
         reduce_scalar(loss_part.p, nb, scal.p);
         CK(cudaMemsetAsync(scal.p + 1, 0, sizeof(double), stream));
         return 1;
@@ -1761,9 +1745,8 @@ struct Ctx : cmf_ctx {
     //   Q = transconv(W, R) = denomH - numH
     // with R = conv(W,H) - X (hals.jl:22).  w_partials() / the Gram all-reduce are shared with MU.
     void hals_w_apply(double l1W, double l2W) {
-        if (tc_active()) tc_denomW();
-        build_G();                                                            // G as a matrix for the sweep (GS)
-        if (!tc_active()) launch_gemm<false>(GS.p, Wi.p, denW.p, KL(), N, KL(), KL(), N, N);
+        compute_denomW(0, KL());
+        if (tc_active()) build_G();                                           // G as a matrix for the sweep (GS; SIMT built it above)
         sub_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(numW.p, denW.p, numW.p, KL() * N);   // P
         post_launch();
         const size_t smem = (size_t)KL() * sizeof(S);
@@ -1772,27 +1755,14 @@ struct Ctx : cmf_ctx {
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kern<<<(unsigned)N, 256, smem, stream>>>(GS.p, numW.p, Wi.p, K, L, N, (S)l1W, (S)l2W);   // hals.jl:90-112
         post_launch();
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
-    }
-
-    void hals_update_motifs(double l1W, double l2W) override {
-        w_partials();
-        hals_w_apply(l1W, l2W);
+        w_changed();
     }
 
     // Q = transconv(W, R) = denomH - numH on the owned columns (left in numH)
     void hals_h_prepare() override {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        if (tc_active()) tc_transconv();
-        else launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
-        lag_tables();
-        if (fd_active()) fd_denomH();
-        else if (tc_active()) { tc_split_H(false); tc_denomH(); }
-        else launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, K, Tl, Tl + 2 * (L - 1));
-        if (is_last && L > 1) {
-            launch_denomH_tail();
-        }
+        compute_numH();
+        compute_denomH();
         sub_kernel<S><<<(unsigned)cdiv(Tl * K, 256), 256, 0, stream>>>(numH.p, denH.p, numH.p, Tl * K);        // Q
         post_launch();
     }
@@ -1813,7 +1783,7 @@ struct Ctx : cmf_ctx {
     DevBuf<unsigned> h2_bar;
     int h2_max_ctas = -1;
     bool hals2_sweep(const S *Qp, S *Hp, int64_t Tt, const S *ct, double l1H, double l2H) {
-        if constexpr (!std::is_same<S, float>::value) { return false; } else {
+        if constexpr (!is_f32) { return false; } else {
             if (L > hals2::LMAX || K > 128 || (L > 1 && ct == nullptr)) return false;
             if (const char *e = getenv("CMF_HALS_SWEEP")) { if (atoi(e) == 1) return false; }      // 1: first-generation wavefront kernel
             const int G = (int)cdiv(K, hals2::GS);
@@ -1919,18 +1889,6 @@ struct Ctx : cmf_ctx {
         prof_end();
         post_launch();
     }
-    void h_changed() override {
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
-        numH_valid = false; numH_dot_valid = false;
-    }
-
-    double hals_update_feature_maps(double l1H, double l2H) override {
-        REQUIRE(is_first && is_last, "single-shard entry; sharded fits go through the communicator path");
-        hals_h_prepare();
-        hals_h_sweep(0, l1H, l2H);
-        h_changed();
-        return loss_partial();                                                // hals.jl:41
-    }
 
     // ---------------------------------------------------------------- PGD (src/algs/pgd.jl, SquareLoss)
     // The gradients are the MU quantities again: dW = 2 (denomW - numW), dH = 2 (denomH - numH) (pgd.jl:206-221).
@@ -1997,19 +1955,16 @@ struct Ctx : cmf_ctx {
             pgd_penalty_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(denW.p, Wi.p, (S)l1W, (S)l2W, KL() * N);
             post_launch();
             pgd_step(Wi.p, denW.p, KL() * N, pgd_stepW, pgd_constrW, N);
-            mark_w_dirty();
-            numH_valid = false; numH_dot_valid = false;
+            w_changed();
             pgd_adapt(pgd_loss_eval(), pgd_stepW);
             return;
         }
         w_partials();
-        if (tc_active()) tc_denomW();
-        else { build_G(); launch_gemm<false>(GS.p, Wi.p, denW.p, KL(), N, KL(), KL(), N, N); }
+        compute_denomW(0, KL());
         pgd_grad_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(denW.p, denW.p, numW.p, Wi.p, (S)l1W, (S)l2W, KL() * N);
         post_launch();
         pgd_step(Wi.p, denW.p, KL() * N, pgd_stepW, pgd_constrW, N);
-        mark_w_dirty();
-        numH_valid = false; numH_dot_valid = false;
+        w_changed();
         pgd_adapt(loss_partial(), pgd_stepW);                                           // pgd.jl:244-252
     }
 
@@ -2021,24 +1976,16 @@ struct Ctx : cmf_ctx {
             pgd_penalty_kernel<S><<<(unsigned)cdiv(Tl * K, 256), 256, 0, stream>>>(denH.p, H, (S)l1H, (S)l2H, Tl * K);
             post_launch();
             pgd_step(H, denH.p, Tl * K, pgd_stepH, pgd_constrH, 1);
-            gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
-            numH_valid = false; numH_dot_valid = false;
+            h_changed();
             pgd_adapt(pgd_loss_eval(), pgd_stepH);
             return pgd_cur_loss;
         }
-        if (tc_active()) tc_transconv();
-        else launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
-        lag_tables();
-        if (fd_active()) fd_denomH();
-        else if (tc_active()) { tc_split_H(false); tc_denomH(); }
-        else launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, K, Tl, Tl + 2 * (L - 1));
-        if (L > 1) {
-            launch_denomH_tail();
-        }
+        compute_numH();
+        compute_denomH();                                                               // is_last: PGD is single-shard
         pgd_grad_kernel<S><<<(unsigned)cdiv(Tl * K, 256), 256, 0, stream>>>(denH.p, denH.p, numH.p, H, (S)l1H, (S)l2H, Tl * K);
         post_launch();
         pgd_step(H, denH.p, Tl * K, pgd_stepH, pgd_constrH, 1);
-        gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
+        h_changed();
         numH_valid = true;                                                              // W unchanged: the expansion loss may reuse numH / W W'
         pgd_adapt(loss_partial(), pgd_stepH);
         return pgd_cur_loss;                                                            // caller: sqrt(cur_loss / datanorm^2), pgd.jl:202
