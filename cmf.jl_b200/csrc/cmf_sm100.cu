@@ -1,7 +1,7 @@
 // libcmf_sm100: C ABI + host orchestration of the B200 CNMF fit path (see include/cmf_sm100.h).
 //
-// One handle = one time-shard on one GPU.  All device memory is owned here; host arrays are
-// copied during the call.  Errors never escape as C++ exceptions.
+// One rank context (Ctx<S>) = one time-shard on one GPU; a handle holds one rank context, or one per device of a
+// multi-GPU group.  All device memory is owned here; host arrays are copied during the call.  Errors never escape as C++ exceptions.
 #include "../../include/cmf_sm100.h"
 
 #include <cuda_runtime.h>
@@ -20,6 +20,7 @@
 #include <vector>
 
 #include <type_traits>
+#include <variant>
 
 #include "kernels_simt.cuh"
 #include "kernels_tc.cuh"
@@ -76,14 +77,12 @@ struct DevBuf {
     ~DevBuf() { free(); }
 };
 
-}  // namespace
-
 // ------------------------------------------------------------------------------------------
-// handle
+// rank context: the state of one time-shard on one GPU that does not depend on the scalar type (Ctx<S> adds the rest)
 // ------------------------------------------------------------------------------------------
-struct cmf_ctx {
+struct RankState {
     int64_t N = 0, T = 0, t0 = 0, t1 = 0, Tl = 0, K = 0, L = 0;
-    int dtype = 0, alg = 0, device = 0, engine = 0;
+    int alg = 0, device = 0, engine = 0;
     bool is_first = true, is_last = true;
     cudaStream_t stream = nullptr;
     bool own_stream = false;
@@ -132,7 +131,7 @@ struct cmf_ctx {
         for (auto &e : prof_events) { cudaEventDestroy(e.a); cudaEventDestroy(e.b); }
         prof_events.clear();
     }
-    virtual ~cmf_ctx() {
+    ~RankState() {
         prof_clear();
         if (ev_a) cudaEventDestroy(ev_a);
         if (ev_b) cudaEventDestroy(ev_b);
@@ -142,63 +141,11 @@ struct cmf_ctx {
     cmf::Comm comm;                  // NCCL communicator of this rank (world == 1: collectives are no-ops)
     cudaStream_t comm_stream = nullptr;  // side stream for collectives that overlap with kernels of the main stream
     cudaEvent_t ev_a = nullptr, ev_b = nullptr;
-    struct cmf_multi *multi = nullptr;   // set on the single-process multi-GPU handle only (cmf_create_multi)
     int world() const { return comm.world; }
     int rank() const { return comm.rank; }
-    [[noreturn]] static void no_multi() { throw std::runtime_error("this call is not available on a multi-GPU group handle"); }
-    virtual void get_data(void *, int) { no_multi(); }
-    virtual bool tc_available() { no_multi(); }
-    virtual bool fd_available() { no_multi(); }
-    virtual void fd_release() { no_multi(); }
-    virtual void set_data(const void *, int64_t) { no_multi(); }
-    virtual void synth_data(uint64_t, int64_t, int64_t, double, double) { no_multi(); }
-    virtual double data_sumsq() { no_multi(); }
-    virtual void set_factors(const void *, const void *, int64_t) { no_multi(); }
-    virtual void init_rand(uint64_t) { no_multi(); }
-    virtual void init_scale_partials(double *) { no_multi(); }
-    virtual void scale_factors(double) { no_multi(); }
-    virtual void get_factors(void *, void *) { no_multi(); }
-    virtual void w_partials() { no_multi(); }
-    virtual void w_apply(double, double) { no_multi(); }
-    virtual void w_denom_rows(int64_t, int64_t) { no_multi(); }
-    virtual void w_update_rows(double, double, int64_t, int64_t) { no_multi(); }
-    virtual void w_rows_buffers(void **, void **, int64_t *) { no_multi(); }
-    virtual void fd_denomH_prefetch() {}
-    virtual void h_update(double, double) { no_multi(); }
-    virtual double loss_partial() { no_multi(); }
-    virtual int loss_partial_dev() { no_multi(); }                 // leaves 1 (direct) or 2 (expansion) doubles in scalars()
-    virtual double *scalars() { no_multi(); }                      // device buffer of 8 doubles
-    virtual void hals_h_prepare() { no_multi(); }                  // Q = denomH - numH on the owned columns
-    virtual void hals_h_local(void **, void **, int64_t *) { no_multi(); }     // device pointers of the local Q and H (owned columns), element count
-    virtual void hals_h_full(void **, void **) { no_multi(); }     // rank 0 of a sharded fit: full-T Q and H buffers (allocated on first use)
-    virtual void hals_h_sweep(int full, double, double) { no_multi(); }
-    virtual void h_changed() { no_multi(); }                       // invalidates what depends on H (after a halo exchange / scatter)
-    virtual void fd_layout(int *, int *, int64_t *) { no_multi(); }
-    virtual void set_pgd_loss(int, const void *) { no_multi(); }
-    virtual void set_pgd_constraints(int, int) { no_multi(); }
-    virtual void pgd_update_motifs(double, double) { no_multi(); }
-    virtual double pgd_update_feature_maps(double, double) { no_multi(); }
-    virtual void exchange_buffer(int, void **, int64_t *, int *) { no_multi(); }
-    virtual void halo_buffers(void **, void **, void **, void **, int64_t *) { no_multi(); }
-    virtual void prim_conv(void *) { no_multi(); }
-    virtual void prim_transconv(const void *, void *) { no_multi(); }
-    virtual void prim_corr(const void *, void *) { no_multi(); }
-    virtual void prim_resids(void *) { no_multi(); }
-    virtual void prim_shift_and_stack(void *) { no_multi(); }
-    // batch handles (R > 0): R restarts of MultUpdate on one data set
-    virtual void batch_set_factors(const void *, const void *) { no_multi(); }
-    virtual void batch_get_factors(void *, void *) { no_multi(); }
-    virtual void batch_scale_partials(double *) { no_multi(); }
-    virtual void batch_scale(const double *) { no_multi(); }
-    virtual void batch_loss(double *) { no_multi(); }
-    virtual void batch_set_state(const double *, const int *) { no_multi(); }
-    virtual void batch_update_motifs() { no_multi(); }
-    virtual void batch_update_feature_maps() { no_multi(); }
 };
 
 enum { PROF_CONV = 0, PROF_TRANSCONV = 1, PROF_CORR = 2, PROF_SWEEP = 3, PROF_NCLASS = 4 };
-
-namespace {
 
 using namespace cmf;
 
@@ -323,7 +270,8 @@ void fd_with_bc(int logB, int C, Fn &&fn) {
 }
 
 template <typename S>
-struct Ctx : cmf_ctx {
+struct Ctx : RankState {
+    static constexpr int dtype = std::is_same<S, double>::value ? CMF_F64 : CMF_F32;
     TcState tcs;
     FdState fds;
     DevBuf<S> X, Hbuf, Wi, Wtmp, numW, denW, GS, Cf, numH, denH, tailC;
@@ -410,7 +358,7 @@ struct Ctx : cmf_ctx {
     static constexpr bool is_f32 = std::is_same<S, float>::value;
     bool tc_active() const { return engine >= 1 && tcs.ok; }
     bool fd_active() const { return engine == 2 && tcs.ok && fds.ok; }
-    bool fd_available() override {
+    bool fd_available() {
         if constexpr (is_f32) {
             if (!tc_available()) return false;
             if (!fds.ok && !fds.tried) fd_setup();
@@ -418,8 +366,8 @@ struct Ctx : cmf_ctx {
         }
         return fds.ok;
     }
-    void fd_release() override { fds.release(); }
-    void fd_layout(int *B, int *V, int64_t *nblk) override {
+    void fd_release() { fds.release(); }
+    void fd_layout(int *B, int *V, int64_t *nblk) {
         *B = fd_active() ? fds.B : 0; *V = fd_active() ? fds.V : 0; *nblk = fd_active() ? fds.nblkp : 0;
     }
 
@@ -636,7 +584,7 @@ struct Ctx : cmf_ctx {
     }
     // the H-only part of fd_denomH: spectrum of the blocks of H (hop V2, both halos).  Depends on H alone, so a sharded fit runs it
     // while the all-gather of the new W is in flight (r_update_motifs).
-    void fd_denomH_prefetch() override {
+    void fd_denomH_prefetch() {
         if constexpr (is_f32) {
             FdState &f = fds;
             if (!fd_active() || f.hf2_valid) return;
@@ -755,7 +703,7 @@ struct Ctx : cmf_ctx {
         fd_ifft_numH(f.Of.p, numH.p, f.nblk, f.V, f.nblkp);
         post_launch();
     }
-    bool tc_available() override {
+    bool tc_available() {
         if constexpr (is_f32) {
             if (!tcs.ok && !tcs.tried) tc_setup();
         }
@@ -1038,7 +986,7 @@ struct Ctx : cmf_ctx {
         return tc::EPI_WARPS * q.units;
     }
 
-    ~Ctx() override {
+    ~Ctx() {
         if (tracing) trace_dump();
         if (own_stream && stream) cudaStreamDestroy(stream);
     }
@@ -1273,14 +1221,14 @@ struct Ctx : cmf_ctx {
         tcs.w_dirty = fds.w_dirty = fds.wx_dirty = true;
         numH_valid = numH_dot_valid = false;
     }
-    void h_changed() override {           // Gram partial, spectra of H; numH too (the HALS sweep leaves Q there)
+    void h_changed() {           // Gram partial, spectra of H; numH too (the HALS sweep leaves Q there)
         gram_valid = false; fds.h_dirty = true; fds.hf2_valid = false;
         numH_valid = numH_dot_valid = false;
     }
     void factors_replaced() { w_changed(); h_changed(); calib_reset(); }
 
     // ---------------------------------------------------------------- data
-    void set_data(const void *Xh, int64_t first_col) override {
+    void set_data(const void *Xh, int64_t first_col) {
         REQUIRE(Xh != nullptr, "set_data: null pointer");
         REQUIRE(first_col <= t0, "set_data: host array starts after the shard's first column");
         const int64_t hi = std::min(t1 + (L - 1), T);
@@ -1289,7 +1237,7 @@ struct Ctx : cmf_ctx {
         CK(cudaMemcpyAsync(X.p, src, (size_t)((hi - t0) * N) * sizeof(S), cudaMemcpyHostToDevice, stream));
         finish_data();
     }
-    void get_data(void *X_out, int with_halo) override {
+    void get_data(void *X_out, int with_halo) {
         const int64_t cols = with_halo ? std::min(t1 + (L - 1), T) - t0 : Tl;
         CK(cudaMemcpyAsync(X_out, X.p, (size_t)(cols * N) * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
@@ -1301,14 +1249,14 @@ struct Ctx : cmf_ctx {
         pgd_cur_loss = data_norm;
         have_data = true;
     }
-    double data_sumsq() override {
+    double data_sumsq() {
         dot_partial_kernel<S><<<1024, 256, 0, stream>>>(X.p, X.p, Tl * N, loss_part.p);
         post_launch();
         reduce_scalar(loss_part.p, 1024, scal.p);
         return fetch_scalar(scal.p);
     }
 
-    void synth_data(uint64_t seed, int64_t Kt, int64_t Lt, double p_h, double noise) override {
+    void synth_data(uint64_t seed, int64_t Kt, int64_t Lt, double p_h, double noise) {
         REQUIRE(Kt >= 1 && Lt >= 1, "synth_data: bad ground-truth dims");
         DevBuf<S> Wt, Ht;
         Wt.alloc((size_t)(Kt * Lt * N));
@@ -1326,7 +1274,7 @@ struct Ctx : cmf_ctx {
     }
 
     // ---------------------------------------------------------------- factors
-    void set_factors(const void *Wh, const void *Hh, int64_t first_col) override {
+    void set_factors(const void *Wh, const void *Hh, int64_t first_col) {
         REQUIRE(Wh && Hh, "set_factors: null pointer");
         const int64_t lo = std::max<int64_t>(t0 - (L - 1), 0), hi = std::min(t1 + (L - 1), T);
         REQUIRE(first_col <= lo, "set_factors: host H starts after the shard's left halo");
@@ -1343,7 +1291,7 @@ struct Ctx : cmf_ctx {
         pgd_cur_loss = data_norm;
     }
 
-    void init_rand(uint64_t seed) override {
+    void init_rand(uint64_t seed) {
         // W in Julia order (k + K*(n + N*l)) so the draw for element (k,n,l) does not depend on layout
         uniform_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wtmp.p, KL() * N, seed, 100, 0);
         post_launch();
@@ -1358,7 +1306,7 @@ struct Ctx : cmf_ctx {
         factors_replaced();
     }
 
-    void init_scale_partials(double out[2]) override {
+    void init_scale_partials(double out[2]) {
         REQUIRE(have_data && have_factors, "init_scale_partials: data and factors must be set");
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p);
@@ -1371,7 +1319,7 @@ struct Ctx : cmf_ctx {
         out[0] = a; out[1] = b;
     }
 
-    void scale_factors(double s) override {
+    void scale_factors(double s) {
         scale_kernel<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wi.p, (S)s, KL() * N);
         post_launch();
         scale_kernel<S><<<(unsigned)cdiv((int64_t)Hbuf.n, 256), 256, 0, stream>>>(Hbuf.p, (S)s, (int64_t)Hbuf.n);
@@ -1379,7 +1327,7 @@ struct Ctx : cmf_ctx {
         factors_replaced();
     }
 
-    void get_factors(void *Wo, void *Ho) override {
+    void get_factors(void *Wo, void *Ho) {
         if (Wo) {
             w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, K);
             post_launch();
@@ -1450,7 +1398,7 @@ struct Ctx : cmf_ctx {
     }
 
     // host: R Julia blocks W (K x N x L) and H (K x T); numH stages H (it is recomputed before every use)
-    void batch_set_factors(const void *Wh, const void *Hh) override {
+    void batch_set_factors(const void *Wh, const void *Hh) {
         REQUIRE(Wh && Hh, "cmf_set_factors_batch: null pointer");
         CK(cudaMemcpyAsync(Wtmp.p, Wh, Wtmp.n * sizeof(S), cudaMemcpyHostToDevice, stream));
         w_julia_to_internal<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, RK());
@@ -1462,7 +1410,7 @@ struct Ctx : cmf_ctx {
         CK(cudaStreamSynchronize(stream));
         have_factors = true;
     }
-    void batch_get_factors(void *Wo, void *Ho) override {
+    void batch_get_factors(void *Wo, void *Ho) {
         REQUIRE(have_factors, "no factors");
         if (Wo) {
             w_internal_to_julia<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, RK());
@@ -1479,7 +1427,7 @@ struct Ctx : cmf_ctx {
 
     // out[2r] = <X, est_r>, out[2r+1] = ||est_r||^2 (model.jl:119-120), each summed over the conv blocks in the order of
     // init_scale_partials
-    void batch_scale_partials(double *out) override {
+    void batch_scale_partials(double *out) {
         REQUIRE(have_data && have_factors, "cmf_init_scale_partials_batch: data and factors must be set");
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p, 0, 0.0, (int)R, 2 * nb);
@@ -1493,7 +1441,7 @@ struct Ctx : cmf_ctx {
             out[2 * r] = a; out[2 * r + 1] = b;
         }
     }
-    void batch_scale(const double *s) override {
+    void batch_scale(const double *s) {
         CK(cudaMemcpyAsync(b_vals.p, s, (size_t)R * sizeof(double), cudaMemcpyHostToDevice, stream));
         scale_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, S(1), (int64_t)Wi.n, b_vals.p, N, K, RK());
         post_launch();
@@ -1504,7 +1452,7 @@ struct Ctx : cmf_ctx {
 
     // relative loss of every restart (mult.jl:55-57): one direct conv + residual pass with a restart index, one deterministic
     // reduction per restart, one copy of R doubles
-    void batch_loss(double *out) override {
+    void batch_loss(double *out) {
         REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p, 0, 0.0, (int)R, nb);
@@ -1515,14 +1463,14 @@ struct Ctx : cmf_ctx {
     }
 
     // reg = R x (l1W, l2W, l1H, l2H) and / or the R active flags (either may be NULL)
-    void batch_set_state(const double *reg, const int *active) override {
+    void batch_set_state(const double *reg, const int *active) {
         if (reg) CK(cudaMemcpyAsync(b_reg.p, reg, (size_t)(4 * R) * sizeof(double), cudaMemcpyHostToDevice, stream));
         if (active) CK(cudaMemcpyAsync(b_active.p, active, (size_t)R * sizeof(int), cudaMemcpyHostToDevice, stream));
         CK(cudaStreamSynchronize(stream));
     }
 
     // update_motifs! (mult.jl:23-39) of every active restart
-    void batch_update_motifs() override {
+    void batch_update_motifs() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
         launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, RK(), RK());          // numW, all restarts
         launch_corr(H, K, RK(), Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p, H, K, RK(), (int)R, b_exch());   // Gram_r
@@ -1541,7 +1489,7 @@ struct Ctx : cmf_ctx {
     }
 
     // update_feature_maps! (mult.jl:42-58, without the loss) of every active restart
-    void batch_update_feature_maps() override {
+    void batch_update_feature_maps() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
         launch_transconv(Wi.p, X.p, numH.p, N, RK(), L, N, Tl, Tl + (L - 1));                                // numH, all restarts
         launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), (int)R);     // S2_r = W_r W_r'
@@ -1616,7 +1564,7 @@ struct Ctx : cmf_ctx {
     }
 
     // ---------------------------------------------------------------- MU (src/algs/mult.jl)
-    void w_partials() override {
+    void w_partials() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
         compute_numW();
         // the Gram partial is already resident when the expansion loss of the previous iteration computed it for the same H
@@ -1624,19 +1572,19 @@ struct Ctx : cmf_ctx {
         gram_valid = false;     // the host all-reduces the buffer in place: it is consumed by this step
     }
 
-    void w_apply(double l1W, double l2W) override {
+    void w_apply(double l1W, double l2W) {
         if (alg == CMF_HALS) { hals_w_apply(l1W, l2W); return; }
         REQUIRE(alg == CMF_MULT, "the split-phase W update serves MultUpdate and HALSUpdate");
         w_denom_rows(0, KL());
         w_update_rows(l1W, l2W, 0, KL());
     }
-    void w_denom_rows(int64_t j0, int64_t j1) override { compute_denomW(j0, j1); }
+    void w_denom_rows(int64_t j0, int64_t j1) { compute_denomW(j0, j1); }
     // mult.jl:37-38 on the rows [j0, j1) (the whole update when the range is everything)
-    void w_update_rows(double l1W, double l2W, int64_t j0, int64_t j1) override {
+    void w_update_rows(double l1W, double l2W, int64_t j0, int64_t j1) {
         launch_mu(Wi.p + j0 * N, numW.p + j0 * N, denW.p + j0 * N, l1W, l2W, (j1 - j0) * N);
         w_changed();
     }
-    void w_rows_buffers(void **numw, void **w, int64_t *row_elems) override { *numw = numW.p; *w = Wi.p; *row_elems = N; }
+    void w_rows_buffers(void **numw, void **w, int64_t *row_elems) { *numw = numW.p; *w = Wi.p; *row_elems = N; }
 
     // layout of the W W' product held in GS: S2[(l*s2_ks + k)*s2_ld + l'*s2_ks + k']
     int64_t s2_ks = 0, s2_ld = 0;
@@ -1674,7 +1622,7 @@ struct Ctx : cmf_ctx {
         post_launch();
     }
 
-    void h_update(double l1H, double l2H) override {
+    void h_update(double l1H, double l2H) {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
         compute_numH();
         compute_denomH();
@@ -1685,13 +1633,13 @@ struct Ctx : cmf_ctx {
         numH_dot_valid = dot;
     }
 
-    double *scalars() override { return scal.p; }
+    double *scalars() { return scal.p; }   // device buffer of 8 doubles
 
     // Leaves the local loss scalars in scal.p without a host synchronisation and returns how many there are:
     //   1 (direct pass):  scal[0] = sum of squared residuals over the owned columns (mult.jl:55-57)
     //   2 (expansion):    scal[0] = <numH, H>, scal[1] = <W W', Htilde Htilde'> over the owned columns
     // scal[1] is zeroed in the direct case so that a fixed-size all-reduce of two doubles serves both.
-    int loss_partial_dev() override {
+    int loss_partial_dev() {
         REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
         if (loss_mode == 1 && tc_active()) {
             // frequency-domain engine: numH and W W' are cheap, so the expansion also serves calls that find them stale
@@ -1708,7 +1656,7 @@ struct Ctx : cmf_ctx {
     }
 
     // local sum of squared residuals (for the expansion: this shard's share of the global identity)
-    double loss_partial() override {
+    double loss_partial() {
         const int n = loss_partial_dev();
         double bc[2];
         CK(cudaMemcpyAsync(bc, scal.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, stream));
@@ -1759,19 +1707,20 @@ struct Ctx : cmf_ctx {
     }
 
     // Q = transconv(W, R) = denomH - numH on the owned columns (left in numH)
-    void hals_h_prepare() override {
+    void hals_h_prepare() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
         compute_numH();
         compute_denomH();
         sub_kernel<S><<<(unsigned)cdiv(Tl * K, 256), 256, 0, stream>>>(numH.p, denH.p, numH.p, Tl * K);        // Q
         post_launch();
     }
-    void hals_h_local(void **q, void **h, int64_t *count) override { *q = numH.p; *h = H; *count = Tl * K; }
+    // device pointers of the local Q and H (owned columns), element count
+    void hals_h_local(void **q, void **h, int64_t *count) { *q = numH.p; *h = H; *count = Tl * K; }
     // rank 0 of a T-sharded HALS fit holds Q, H and Delta H of ALL columns during the sweep: the sweep is a chain of T
     // dependent steps per component (hals.jl:124-128) that more GPUs cannot shorten, so the shards' Q are gathered here,
     // swept once in the reference's order, and the new H is scattered back (DESIGN.md section 6)
     DevBuf<S> Qfull, Hfull, Dfull;
-    void hals_h_full(void **q, void **h) override {
+    void hals_h_full(void **q, void **h) {
         const size_t n = (size_t)(T * K);
         if (Qfull.n < n) { Qfull.alloc(n); Hfull.alloc(n); Dfull.alloc(n); }
         *q = Qfull.p; *h = Hfull.p;
@@ -1859,7 +1808,7 @@ struct Ctx : cmf_ctx {
     }
 
     // wavefront sweep (hals.jl:121-154) over the local shard (single-shard handles) or over the gathered full-T buffers
-    void hals_h_sweep(int full, double l1H, double l2H) override {
+    void hals_h_sweep(int full, double l1H, double l2H) {
         REQUIRE(full || (is_first && is_last), "the local HALS H sweep needs a single-shard handle");
         if (progress.n == 0) hals_setup();
         CK(cudaMemsetAsync(progress.p, 0, progress.n * sizeof(int), stream));
@@ -1921,12 +1870,12 @@ struct Ctx : cmf_ctx {
     int pgd_loss = 0;                 // 0 SquareLoss, 1 AbsoluteLoss
     DevBuf<S> pgd_mask, pgd_ge;       // mask [t][N] (empty = none), loss-gradient scratch [t][N] incl. a zero right halo
     bool pgd_general() const { return pgd_loss != 0 || pgd_mask.n != 0; }
-    void set_pgd_constraints(int cw, int ch) override {
+    void set_pgd_constraints(int cw, int ch) {
         REQUIRE(alg == CMF_PGD, "cmf_set_pgd_constraints: PGD handles only");
         REQUIRE((cw == 0 || cw == 1) && (ch == 0 || ch == 1), "constraint must be 0 (NonnegConstraint) or 1 (UnitNormConstraint)");
         pgd_constrW = cw; pgd_constrH = ch;
     }
-    void set_pgd_loss(int lossf, const void *mask_host) override {
+    void set_pgd_loss(int lossf, const void *mask_host) {
         REQUIRE(alg == CMF_PGD, "the pluggable loss belongs to PGDUpdate handles");
         REQUIRE(lossf == 0 || lossf == 1, "loss_func must be 0 (SquareLoss) or 1 (AbsoluteLoss)");
         pgd_loss = lossf;
@@ -1947,7 +1896,7 @@ struct Ctx : cmf_ctx {
         return fetch_scalar(scal.p);
     }
 
-    void pgd_update_motifs(double l1W, double l2W) override {
+    void pgd_update_motifs(double l1W, double l2W) {
         REQUIRE(is_first && is_last, "PGD is single-shard");
         if (pgd_general()) {
             pgd_loss_gradient();
@@ -1968,7 +1917,7 @@ struct Ctx : cmf_ctx {
         pgd_adapt(loss_partial(), pgd_stepW);                                           // pgd.jl:244-252
     }
 
-    double pgd_update_feature_maps(double l1H, double l2H) override {
+    double pgd_update_feature_maps(double l1H, double l2H) {
         REQUIRE(is_first && is_last, "PGD is single-shard");
         if (pgd_general()) {
             pgd_loss_gradient();
@@ -1992,32 +1941,32 @@ struct Ctx : cmf_ctx {
     }
 
     // ---------------------------------------------------------------- exchange
-    void exchange_buffer(int which, void **p, int64_t *count, int *dt) override {
+    void exchange_buffer(int which, void **p, int64_t *count, int *dt) {
         if (which == 0) { *p = numW.p; *count = KL() * N; *dt = dtype; }
         else if (which == 1) { *p = exch1.p; *count = L * K * K + (L - 1) * K; *dt = CMF_F64; }
         else if (which == 2) { *p = numH.p; *count = Tl * K; *dt = dtype; }   // diagnostics: numH [t][K]
         else if (which == 3) { *p = denH.p; *count = Tl * K; *dt = dtype; }   // diagnostics: denomH [t][K]
         else throw CmfError(CMF_ERR_ARG, "exchange_buffer: which must be 0..3");
     }
-    void halo_buffers(void **sl, void **sr, void **rl, void **rr, int64_t *count) override {
+    void halo_buffers(void **sl, void **sr, void **rl, void **rr, int64_t *count) {
         *sl = H; *sr = H + (Tl - (L - 1)) * K; *rl = Hbuf.p; *rr = H + Tl * K; *count = (L - 1) * K;
     }
 
     // ---------------------------------------------------------------- primitives
-    void prim_conv(void *out_host) override {
+    void prim_conv(void *out_host) {
         DevBuf<S> out;
         out.alloc((size_t)(N * Tl));
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 1, out.p, nullptr);
         CK(cudaMemcpyAsync(out_host, out.p, out.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
     }
-    void prim_transconv(const void *X_host, void *out_host) override {
+    void prim_transconv(const void *X_host, void *out_host) {
         set_data(X_host, 0);
         launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
         CK(cudaMemcpyAsync(out_host, numH.p, numH.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
     }
-    void prim_corr(const void *X_host, void *out_host) override {
+    void prim_corr(const void *X_host, void *out_host) {
         set_data(X_host, 0);
         launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
         w_internal_to_julia<S><<<(unsigned)cdiv(KL() * N, 256), 256, 0, stream>>>(numW.p, Wtmp.p, K, N, L, K);
@@ -2026,7 +1975,7 @@ struct Ctx : cmf_ctx {
         CK(cudaStreamSynchronize(stream));
     }
     // compute_resids (src/common.jl:58-59): conv(W,H) - X through the conv kernel's residual epilogue
-    void prim_resids(void *out_host) override {
+    void prim_resids(void *out_host) {
         REQUIRE(have_data && have_factors, "compute_resids: data and factors must be set");
         DevBuf<S> out;
         out.alloc((size_t)(N * Tl));
@@ -2036,7 +1985,7 @@ struct Ctx : cmf_ctx {
     }
     // shift_and_stack (src/common.jl:133-142): Htilde[(l*K+k), t] = H[k, t-l], zero for t < l (materialised only here, for tests
     // and small problems: the fit itself addresses the same rows through overlapping windows of H)
-    void prim_shift_and_stack(void *out_host) override {
+    void prim_shift_and_stack(void *out_host) {
         REQUIRE(have_factors, "shift_and_stack: factors must be set");
         DevBuf<S> out;
         out.alloc((size_t)(KL() * Tl));
@@ -2047,8 +1996,11 @@ struct Ctx : cmf_ctx {
     }
 };
 
-cmf_ctx *make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device,
-                  int64_t R = 0) {
+// One rank context, initialised on `device`.  S is chosen by the caller from dtype (with_dtype); the dtype check stays here
+// so that the checks run, and fail, in the same order for every create call.
+template <typename S>
+std::unique_ptr<Ctx<S>> make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg,
+                                 int device, int64_t R = 0) {
     REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
     REQUIRE(L <= T, "need L <= T (src/common.jl:28-31)");
     REQUIRE(0 <= t0 && t0 < t1 && t1 <= T, "bad shard range");
@@ -2064,19 +2016,20 @@ cmf_ctx *make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64
     if (e != cudaSuccess || ndev == 0)
         throw CmfError(CMF_ERR_CUDA, std::string("no CUDA device available (") + cudaGetErrorString(e) + "); libcmf_sm100 has no CPU fallback");
     REQUIRE(device >= 0 && device < ndev, "bad device ordinal");
-    cmf_ctx *c = (dtype == CMF_F64) ? static_cast<cmf_ctx *>(new Ctx<double>()) : static_cast<cmf_ctx *>(new Ctx<float>());
+    std::unique_ptr<Ctx<S>> c(new Ctx<S>());
     c->N = N; c->T = T; c->t0 = t0; c->t1 = t1; c->Tl = t1 - t0; c->K = K; c->L = L;
-    c->dtype = dtype; c->alg = alg; c->device = device;
+    c->alg = alg; c->device = device;
     c->is_first = (t0 == 0); c->is_last = (t1 == T);
     c->R = R;
-    try {
-        if (dtype == CMF_F64) static_cast<Ctx<double> *>(c)->init();
-        else static_cast<Ctx<float> *>(c)->init();
-    } catch (...) {
-        delete c;
-        throw;
-    }
+    c->init();
     return c;
+}
+
+// f(S()) with S = double for CMF_F64 and float otherwise (make_ctx rejects any other dtype)
+template <typename F>
+decltype(auto) with_dtype(int dtype, F &&f) {
+    if (dtype == CMF_F64) return f(double());
+    return f(float());
 }
 
 template <typename F>
@@ -2145,76 +2098,84 @@ void shard_range(int64_t T, int world, int rank, int64_t *t0, int64_t *t1) {
     *t1 = *t0 + base + (rank < rem ? 1 : 0);
 }
 
-ncclDataType_t nccl_dt(const cmf_ctx *h) { return h->dtype == CMF_F64 ? ncclFloat64 : ncclFloat32; }
-size_t elem_size(const cmf_ctx *h) { return h->dtype == CMF_F64 ? 8 : 4; }
+template <typename S>
+ncclDataType_t nccl_dt(const Ctx<S> &) { return std::is_same<S, double>::value ? ncclFloat64 : ncclFloat32; }
+template <typename S>
+constexpr size_t elem_size(const Ctx<S> &) { return sizeof(S); }
 
-void c_allreduce(cmf_ctx *h, void *buf, size_t count, ncclDataType_t dt, ncclRedOp_t op = ncclSum) {
-    if (h->world() == 1) return;
-    NK(nccl().AllReduce(buf, buf, count, dt, op, h->comm.comm, h->stream));
+template <typename S>
+void c_allreduce(Ctx<S> &ctx, void *buf, size_t count, ncclDataType_t dt, ncclRedOp_t op = ncclSum) {
+    if (ctx.world() == 1) return;
+    NK(nccl().AllReduce(buf, buf, count, dt, op, ctx.comm.comm, ctx.stream));
 }
 
 // all-reduce of a few host doubles through the handle's scalar buffer (slots 4..7); synchronises the stream
-void c_allreduce_host(cmf_ctx *h, double *vals, int n, ncclRedOp_t op = ncclSum) {
-    if (h->world() == 1) return;
+template <typename S>
+void c_allreduce_host(Ctx<S> &ctx, double *vals, int n, ncclRedOp_t op = ncclSum) {
+    if (ctx.world() == 1) return;
     REQUIRE(n <= 4, "at most 4 scalars");
-    double *d = h->scalars() + 4;
-    CK(cudaMemcpyAsync(d, vals, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    c_allreduce(h, d, (size_t)n, ncclFloat64, op);
-    CK(cudaMemcpyAsync(vals, d, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    double *d = ctx.scalars() + 4;
+    CK(cudaMemcpyAsync(d, vals, n * sizeof(double), cudaMemcpyHostToDevice, ctx.stream));
+    c_allreduce(ctx, d, (size_t)n, ncclFloat64, op);
+    CK(cudaMemcpyAsync(vals, d, n * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
+    CK(cudaStreamSynchronize(ctx.stream));
 }
 
 // L-1 columns of H each way (left neighbour's right halo <- my first L-1 columns; right neighbour's left halo <- my last)
-void c_halo_exchange(cmf_ctx *h) {
-    if (h->world() == 1 || h->L <= 1) return;
+template <typename S>
+void c_halo_exchange(Ctx<S> &ctx) {
+    if (ctx.world() == 1 || ctx.L <= 1) return;
     void *sl, *sr, *rl, *rr;
     int64_t cnt;
-    h->halo_buffers(&sl, &sr, &rl, &rr, &cnt);
+    ctx.halo_buffers(&sl, &sr, &rl, &rr, &cnt);
     NcclApi &a = nccl();
-    const ncclDataType_t dt = nccl_dt(h);
-    const int r = h->rank(), w = h->world();
+    const ncclDataType_t dt = nccl_dt(ctx);
+    const int r = ctx.rank(), w = ctx.world();
     NK(a.GroupStart());
     if (r + 1 < w) {
-        NK(a.Send(sr, (size_t)cnt, dt, r + 1, h->comm.comm, h->stream));
-        NK(a.Recv(rr, (size_t)cnt, dt, r + 1, h->comm.comm, h->stream));
+        NK(a.Send(sr, (size_t)cnt, dt, r + 1, ctx.comm.comm, ctx.stream));
+        NK(a.Recv(rr, (size_t)cnt, dt, r + 1, ctx.comm.comm, ctx.stream));
     }
     if (r > 0) {
-        NK(a.Send(sl, (size_t)cnt, dt, r - 1, h->comm.comm, h->stream));
-        NK(a.Recv(rl, (size_t)cnt, dt, r - 1, h->comm.comm, h->stream));
+        NK(a.Send(sl, (size_t)cnt, dt, r - 1, ctx.comm.comm, ctx.stream));
+        NK(a.Recv(rl, (size_t)cnt, dt, r - 1, ctx.comm.comm, ctx.stream));
     }
     NK(a.GroupEnd());
 }
 
 // ||X||_F over all shards (mult.jl:13, hals.jl:23)
-void r_data_norm(cmf_ctx *h) {
-    double ss = h->data_sumsq_local;
-    c_allreduce_host(h, &ss, 1);
-    h->data_sumsq_global = ss;
-    h->data_norm = std::sqrt(ss);
-    h->pgd_cur_loss = h->data_norm;
+template <typename S>
+void r_data_norm(Ctx<S> &ctx) {
+    double ss = ctx.data_sumsq_local;
+    c_allreduce_host(ctx, &ss, 1);
+    ctx.data_sumsq_global = ss;
+    ctx.data_norm = std::sqrt(ss);
+    ctx.pgd_cur_loss = ctx.data_norm;
 }
 
 // <X, est> and ||est||^2 of the alpha rescale (src/model.jl:119-120), summed over shards
-void r_init_scale_partials(cmf_ctx *h, double out[2]) {
-    h->init_scale_partials(out);
-    c_allreduce_host(h, out, 2);
+template <typename S>
+void r_init_scale_partials(Ctx<S> &ctx, double out[2]) {
+    ctx.init_scale_partials(out);
+    c_allreduce_host(ctx, out, 2);
 }
 
 // sum of squared residuals over ALL shards: one fixed-size all-reduce of the two loss scalars, one read-back
-double r_loss_sumsq(cmf_ctx *h, bool force_direct = false, bool *expansion_used = nullptr) {
-    const int saved = h->loss_mode;
-    if (force_direct) h->loss_mode = 0;
+template <typename S>
+double r_loss_sumsq(Ctx<S> &ctx, bool force_direct = false, bool *expansion_used = nullptr) {
+    const int saved = ctx.loss_mode;
+    if (force_direct) ctx.loss_mode = 0;
     int n;
-    try { n = h->loss_partial_dev(); } catch (...) { h->loss_mode = saved; throw; }
-    h->loss_mode = saved;
-    double *d = h->scalars();
-    c_allreduce(h, d, 2, ncclFloat64);
+    try { n = ctx.loss_partial_dev(); } catch (...) { ctx.loss_mode = saved; throw; }
+    ctx.loss_mode = saved;
+    double *d = ctx.scalars();
+    c_allreduce(ctx, d, 2, ncclFloat64);
     double v[2];
-    CK(cudaMemcpyAsync(v, d, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpyAsync(v, d, 2 * sizeof(double), cudaMemcpyDeviceToHost, ctx.stream));
+    CK(cudaStreamSynchronize(ctx.stream));
     if (expansion_used) *expansion_used = (n == 2);
-    ++(n == 2 ? h->n_loss_expansion : h->n_loss_direct);
-    return n == 2 ? h->data_sumsq_global - 2.0 * v[0] + v[1] : v[0];
+    ++(n == 2 ? ctx.n_loss_expansion : ctx.n_loss_direct);
+    return n == 2 ? ctx.data_sumsq_global - 2.0 * v[0] + v[1] : v[0];
 }
 
 // Loss of the current factors, mult.jl:55-57.  With loss_mode 1 the algebraic expansion serves while the relative loss is
@@ -2224,149 +2185,154 @@ double r_loss_sumsq(cmf_ctx *h, bool force_direct = false, bool *expansion_used 
 // have predicted is checked against it -- agreement to 5e-6 (relative, on the loss) doubles the interval (up to 16), more
 // than 2e-5 halves it, more than 1e-4 three times in a row returns the handle to the direct pass for good.  Values returned
 // at calibration points are the direct pass itself.  Every rank sees the same all-reduced numbers and takes the same branch.
-double r_guarded_loss(cmf_ctx *h) {
-    if (h->loss_mode != 1) return std::sqrt(std::max(r_loss_sumsq(h), 0.0)) / h->data_norm;
+template <typename S>
+double r_guarded_loss(Ctx<S> &ctx) {
+    if (ctx.loss_mode != 1) return std::sqrt(std::max(r_loss_sumsq(ctx), 0.0)) / ctx.data_norm;
     bool exp_used = false;
-    const double se = r_loss_sumsq(h, false, &exp_used);
-    if (!exp_used) return std::sqrt(std::max(se, 0.0)) / h->data_norm;
-    const double g2 = h->loss_guard * h->loss_guard * h->data_sumsq_global;
-    if (!h->calib_have && se > g2) return std::sqrt(se) / h->data_norm;
-    if (h->calib_have && h->calib_left > 0 && se - h->calib_bias > 0.0) {
-        --h->calib_left;
-        return std::sqrt(se - h->calib_bias) / h->data_norm;
+    const double se = r_loss_sumsq(ctx, false, &exp_used);
+    if (!exp_used) return std::sqrt(std::max(se, 0.0)) / ctx.data_norm;
+    const double g2 = ctx.loss_guard * ctx.loss_guard * ctx.data_sumsq_global;
+    if (!ctx.calib_have && se > g2) return std::sqrt(se) / ctx.data_norm;
+    if (ctx.calib_have && ctx.calib_left > 0 && se - ctx.calib_bias > 0.0) {
+        --ctx.calib_left;
+        return std::sqrt(se - ctx.calib_bias) / ctx.data_norm;
     }
-    const double sd = r_loss_sumsq(h, true);
-    if (h->calib_have && sd > 0.0) {
-        const double err = std::fabs((se - h->calib_bias) - sd) / (2.0 * sd);
-        h->calib_last_err = err;
-        if (err > 1e-4) { h->calib_interval = 1; ++h->calib_fail; }
+    const double sd = r_loss_sumsq(ctx, true);
+    if (ctx.calib_have && sd > 0.0) {
+        const double err = std::fabs((se - ctx.calib_bias) - sd) / (2.0 * sd);
+        ctx.calib_last_err = err;
+        if (err > 1e-4) { ctx.calib_interval = 1; ++ctx.calib_fail; }
         else {
-            h->calib_fail = 0;
-            if (err > 2e-5) h->calib_interval = std::max(1, h->calib_interval / 2);
-            else if (err < 5e-6) h->calib_interval = std::min(h->calib_max_interval, h->calib_interval * 2);
+            ctx.calib_fail = 0;
+            if (err > 2e-5) ctx.calib_interval = std::max(1, ctx.calib_interval / 2);
+            else if (err < 5e-6) ctx.calib_interval = std::min(ctx.calib_max_interval, ctx.calib_interval * 2);
         }
-        if (h->calib_fail >= 3) { h->loss_mode = 0; h->calib_reset(); }      // the expansion is not reliable on this problem
+        if (ctx.calib_fail >= 3) { ctx.loss_mode = 0; ctx.calib_reset(); }      // the expansion is not reliable on this problem
     }
-    h->calib_bias = se - sd;
-    h->calib_have = true;
-    h->calib_left = h->calib_interval - 1;
-    return std::sqrt(std::max(sd, 0.0)) / h->data_norm;
+    ctx.calib_bias = se - sd;
+    ctx.calib_have = true;
+    ctx.calib_left = ctx.calib_interval - 1;
+    return std::sqrt(std::max(sd, 0.0)) / ctx.data_norm;
 }
 
 // update_motifs! (mult.jl:23-39 / hals.jl:31-34 / pgd.jl:158-178) on this rank's shard
-void r_update_motifs(cmf_ctx *h, double l1W, double l2W) {
-    if (h->alg == CMF_PGD) { h->pgd_update_motifs(l1W, l2W); return; }
-    h->w_partials();
-    const int64_t KL = h->K * h->L;
-    if (h->world() > 1 && h->alg == CMF_MULT && KL % h->world() == 0 && !getenv("CMF_W_REPLICATED")) {
+template <typename S>
+void r_update_motifs(Ctx<S> &ctx, double l1W, double l2W) {
+    if (ctx.alg == CMF_PGD) { ctx.pgd_update_motifs(l1W, l2W); return; }
+    ctx.w_partials();
+    const int64_t KL = ctx.K * ctx.L;
+    if (ctx.world() > 1 && ctx.alg == CMF_MULT && KL % ctx.world() == 0 && !getenv("CMF_W_REPLICATED")) {
         // MultUpdate: the W update is sharded by unfolded rows j = l*K + k (contiguous row blocks of numW / W):
         // reduce-scatter of numW on the side stream while this rank forms its rows of denomW = G W, update of those
         // rows, all-gather of W.  Same bytes on the wire as an all-reduce; G W, the ratio update and the eps floor cost 1/world.
         NcclApi &a = nccl();
         void *p; int64_t cnt; int dt;
-        h->exchange_buffer(1, &p, &cnt, &dt);
-        c_allreduce(h, p, (size_t)cnt, ncclFloat64);                                   // Gram + H tail (small, needed by G)
+        ctx.exchange_buffer(1, &p, &cnt, &dt);
+        c_allreduce(ctx, p, (size_t)cnt, ncclFloat64);                                   // Gram + H tail (small, needed by G)
         void *nw, *w; int64_t row;
-        h->w_rows_buffers(&nw, &w, &row);
-        const int64_t rows = KL / h->world(), j0 = rows * h->rank(), chunk = rows * row;
-        const size_t es = elem_size(h);
-        CK(cudaEventRecord(h->ev_a, h->stream));
-        CK(cudaStreamWaitEvent(h->comm_stream, h->ev_a, 0));
-        NK(a.ReduceScatter(nw, (char *)nw + (size_t)(j0 * row) * es, (size_t)chunk, nccl_dt(h), ncclSum, h->comm.comm, h->comm_stream));
-        CK(cudaEventRecord(h->ev_b, h->comm_stream));
-        h->w_denom_rows(j0, j0 + rows);
-        CK(cudaStreamWaitEvent(h->stream, h->ev_b, 0));
-        h->w_update_rows(l1W, l2W, j0, j0 + rows);
+        ctx.w_rows_buffers(&nw, &w, &row);
+        const int64_t rows = KL / ctx.world(), j0 = rows * ctx.rank(), chunk = rows * row;
+        const size_t es = elem_size(ctx);
+        CK(cudaEventRecord(ctx.ev_a, ctx.stream));
+        CK(cudaStreamWaitEvent(ctx.comm_stream, ctx.ev_a, 0));
+        NK(a.ReduceScatter(nw, (char *)nw + (size_t)(j0 * row) * es, (size_t)chunk, nccl_dt(ctx), ncclSum, ctx.comm.comm, ctx.comm_stream));
+        CK(cudaEventRecord(ctx.ev_b, ctx.comm_stream));
+        ctx.w_denom_rows(j0, j0 + rows);
+        CK(cudaStreamWaitEvent(ctx.stream, ctx.ev_b, 0));
+        ctx.w_update_rows(l1W, l2W, j0, j0 + rows);
         // all-gather of W on the side stream; the one piece of the H half-step that does not need W (the spectrum of H for
         // denomH) runs meanwhile
-        CK(cudaEventRecord(h->ev_a, h->stream));
-        CK(cudaStreamWaitEvent(h->comm_stream, h->ev_a, 0));
-        NK(a.AllGather((char *)w + (size_t)(j0 * row) * es, w, (size_t)chunk, nccl_dt(h), h->comm.comm, h->comm_stream));
-        CK(cudaEventRecord(h->ev_b, h->comm_stream));
-        if (h->alg == CMF_MULT) h->fd_denomH_prefetch();
-        CK(cudaStreamWaitEvent(h->stream, h->ev_b, 0));
+        CK(cudaEventRecord(ctx.ev_a, ctx.stream));
+        CK(cudaStreamWaitEvent(ctx.comm_stream, ctx.ev_a, 0));
+        NK(a.AllGather((char *)w + (size_t)(j0 * row) * es, w, (size_t)chunk, nccl_dt(ctx), ctx.comm.comm, ctx.comm_stream));
+        CK(cudaEventRecord(ctx.ev_b, ctx.comm_stream));
+        if (ctx.alg == CMF_MULT) ctx.fd_denomH_prefetch();
+        CK(cudaStreamWaitEvent(ctx.stream, ctx.ev_b, 0));
         return;
     }
-    if (h->world() > 1) {
+    if (ctx.world() > 1) {
         void *p; int64_t cnt; int dt;
-        h->exchange_buffer(0, &p, &cnt, &dt);
-        c_allreduce(h, p, (size_t)cnt, dt == CMF_F64 ? ncclFloat64 : ncclFloat32);     // numW            (K*N*L)
-        h->exchange_buffer(1, &p, &cnt, &dt);
-        c_allreduce(h, p, (size_t)cnt, ncclFloat64);                                   // Gram + H tail   (K*K*L + (L-1)*K doubles)
+        ctx.exchange_buffer(0, &p, &cnt, &dt);
+        c_allreduce(ctx, p, (size_t)cnt, dt == CMF_F64 ? ncclFloat64 : ncclFloat32);     // numW            (K*N*L)
+        ctx.exchange_buffer(1, &p, &cnt, &dt);
+        c_allreduce(ctx, p, (size_t)cnt, ncclFloat64);                                   // Gram + H tail   (K*K*L + (L-1)*K doubles)
     }
-    h->w_apply(l1W, l2W);                                                              // identical update on every rank
+    ctx.w_apply(l1W, l2W);                                                              // identical update on every rank
 }
 
 // HALS H sweep of a T-sharded fit: gather Q and H on rank 0, sweep once in the reference's order, scatter H
-void r_hals_sweep_sharded(cmf_ctx *h, double l1H, double l2H) {
+template <typename S>
+void r_hals_sweep_sharded(Ctx<S> &ctx, double l1H, double l2H) {
     NcclApi &a = nccl();
-    const ncclDataType_t dt = nccl_dt(h);
-    const size_t es = elem_size(h);
-    const int w = h->world(), r = h->rank();
+    const ncclDataType_t dt = nccl_dt(ctx);
+    const size_t es = elem_size(ctx);
+    const int w = ctx.world(), r = ctx.rank();
     void *ql, *hl, *qf = nullptr, *hf = nullptr;
     int64_t cnt;
-    h->hals_h_local(&ql, &hl, &cnt);
-    if (r == 0) h->hals_h_full(&qf, &hf);
+    ctx.hals_h_local(&ql, &hl, &cnt);
+    if (r == 0) ctx.hals_h_full(&qf, &hf);
     for (int pass = 0; pass < 2; ++pass) {          // 0: gather Q and H, 1: scatter H
-        if (pass == 1 && r == 0) h->hals_h_sweep(1, l1H, l2H);
+        if (pass == 1 && r == 0) ctx.hals_h_sweep(1, l1H, l2H);
         NK(a.GroupStart());
         if (r == 0) {
             for (int p = 1; p < w; ++p) {
                 int64_t a0, a1;
-                shard_range(h->T, w, p, &a0, &a1);
-                const size_t off = (size_t)(a0 * h->K) * es, c = (size_t)((a1 - a0) * h->K);
+                shard_range(ctx.T, w, p, &a0, &a1);
+                const size_t off = (size_t)(a0 * ctx.K) * es, c = (size_t)((a1 - a0) * ctx.K);
                 if (pass == 0) {
-                    NK(a.Recv((char *)qf + off, c, dt, p, h->comm.comm, h->stream));
-                    NK(a.Recv((char *)hf + off, c, dt, p, h->comm.comm, h->stream));
+                    NK(a.Recv((char *)qf + off, c, dt, p, ctx.comm.comm, ctx.stream));
+                    NK(a.Recv((char *)hf + off, c, dt, p, ctx.comm.comm, ctx.stream));
                 } else {
-                    NK(a.Send((char *)hf + off, c, dt, p, h->comm.comm, h->stream));
+                    NK(a.Send((char *)hf + off, c, dt, p, ctx.comm.comm, ctx.stream));
                 }
             }
         } else if (pass == 0) {
-            NK(a.Send(ql, (size_t)cnt, dt, 0, h->comm.comm, h->stream));
-            NK(a.Send(hl, (size_t)cnt, dt, 0, h->comm.comm, h->stream));
+            NK(a.Send(ql, (size_t)cnt, dt, 0, ctx.comm.comm, ctx.stream));
+            NK(a.Send(hl, (size_t)cnt, dt, 0, ctx.comm.comm, ctx.stream));
         } else {
-            NK(a.Recv(hl, (size_t)cnt, dt, 0, h->comm.comm, h->stream));
+            NK(a.Recv(hl, (size_t)cnt, dt, 0, ctx.comm.comm, ctx.stream));
         }
         NK(a.GroupEnd());
         if (r == 0) {
             if (pass == 0) {
-                CK(cudaMemcpyAsync(qf, ql, (size_t)cnt * es, cudaMemcpyDeviceToDevice, h->stream));
-                CK(cudaMemcpyAsync(hf, hl, (size_t)cnt * es, cudaMemcpyDeviceToDevice, h->stream));
+                CK(cudaMemcpyAsync(qf, ql, (size_t)cnt * es, cudaMemcpyDeviceToDevice, ctx.stream));
+                CK(cudaMemcpyAsync(hf, hl, (size_t)cnt * es, cudaMemcpyDeviceToDevice, ctx.stream));
             } else {
-                CK(cudaMemcpyAsync(hl, hf, (size_t)cnt * es, cudaMemcpyDeviceToDevice, h->stream));
+                CK(cudaMemcpyAsync(hl, hf, (size_t)cnt * es, cudaMemcpyDeviceToDevice, ctx.stream));
             }
         }
     }
 }
 
 // loss = update_feature_maps! (mult.jl:42-58 / hals.jl:37-42 / pgd.jl:181-203)
-double r_update_feature_maps(cmf_ctx *h, double l1H, double l2H) {
-    if (h->alg == CMF_PGD) {
-        const double loss = std::sqrt(h->pgd_update_feature_maps(l1H, l2H)) / h->data_norm;
-        if (h->loss_mode == 1 && !(loss > 0.25)) h->loss_mode = 0;   // PGD adapts its step on this value: no re-evaluation
+template <typename S>
+double r_update_feature_maps(Ctx<S> &ctx, double l1H, double l2H) {
+    if (ctx.alg == CMF_PGD) {
+        const double loss = std::sqrt(ctx.pgd_update_feature_maps(l1H, l2H)) / ctx.data_norm;
+        if (ctx.loss_mode == 1 && !(loss > 0.25)) ctx.loss_mode = 0;   // PGD adapts its step on this value: no re-evaluation
         return loss;
     }
-    if (h->alg == CMF_HALS) {
-        h->hals_h_prepare();
-        if (h->world() == 1) h->hals_h_sweep(0, l1H, l2H);
-        else r_hals_sweep_sharded(h, l1H, l2H);
-        h->h_changed();
+    if (ctx.alg == CMF_HALS) {
+        ctx.hals_h_prepare();
+        if (ctx.world() == 1) ctx.hals_h_sweep(0, l1H, l2H);
+        else r_hals_sweep_sharded(ctx, l1H, l2H);
+        ctx.h_changed();
     } else {
-        h->h_update(l1H, l2H);
+        ctx.h_update(l1H, l2H);
     }
-    c_halo_exchange(h);
-    return r_guarded_loss(h);
+    c_halo_exchange(ctx);
+    return r_guarded_loss(ctx);
 }
 
 // src/algs/alternating.jl:16-71 on one rank (every rank runs the same loop: the loss is all-reduced, and the elapsed
 // time that decides `max_time` is rank 0's, so all ranks take the same branches)
-void r_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
+template <typename S>
+void r_fit(Ctx<S> &ctx, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
            double l1W, double l2W, double l1H, double l2H, std::vector<double> &loss_hist, std::vector<double> &time_hist,
            int64_t cap, int *converged_early) {
     *converged_early = 0;
     loss_hist.clear(); time_hist.clear();
-    loss_hist.push_back(r_guarded_loss(h));   // alternating.jl:37
+    loss_hist.push_back(r_guarded_loss(ctx));   // alternating.jl:37
     time_hist.push_back(0.0);
     int64_t itr = 1;
     const bool timed = max_time < 1e300;
@@ -2374,12 +2340,12 @@ void r_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int chec
         ++itr;
         REQUIRE((int64_t)loss_hist.size() < cap, "history capacity exhausted");
         auto t_start = std::chrono::steady_clock::now();
-        if (!eval_mode) r_update_motifs(h, l1W, l2W);
-        const double loss = r_update_feature_maps(h, l1H, l2H);
+        if (!eval_mode) r_update_motifs(ctx, l1W, l2W);
+        const double loss = r_update_feature_maps(ctx, l1H, l2H);
         double dur = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
-        if (timed && h->world() > 1) {          // rank 0's clock decides for everyone
-            if (h->rank() != 0) dur = 0.0;
-            c_allreduce_host(h, &dur, 1);
+        if (timed && ctx.world() > 1) {          // rank 0's clock decides for everyone
+            if (ctx.rank() != 0) dur = 0.0;
+            c_allreduce_host(ctx, &dur, 1);
         }
         time_hist.push_back(time_hist.back() + dur);
         loss_hist.push_back(loss);
@@ -2390,65 +2356,57 @@ void r_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int chec
     }
 }
 
-void r_set_engine(cmf_ctx *h, int engine) {
+template <typename S>
+void r_set_engine(Ctx<S> &ctx, int engine) {
     REQUIRE(engine >= 0 && engine <= 2, "engine must be 0 (SIMT), 1 (tcgen05, time domain) or 2 (tcgen05, frequency domain)");
-    if (h->R > 0 && engine != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles run the SIMT engine (0) only");
-    if (engine == 2 && !h->fd_available())
+    if (ctx.R > 0 && engine != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles run the SIMT engine (0) only");
+    if (engine == 2 && !ctx.fd_available())
         throw CmfError(CMF_ERR_UNSUPPORTED, "the frequency-domain engine needs an fp32 handle with K <= 128, L <= 256, N % 8 == 0 on sm_100 and room for the spectrum of X");
-    if (engine < 2) h->fd_release();               // the spectrum of X and the time-domain planes never coexist
-    if (engine >= 1 && !h->tc_available())
+    if (engine < 2) ctx.fd_release();               // the spectrum of X and the time-domain planes never coexist
+    if (engine >= 1 && !ctx.tc_available())
         throw CmfError(CMF_ERR_UNSUPPORTED, "tcgen05 engine needs an fp32 MultUpdate handle with K <= 128 and N % 8 == 0 on sm_100");
-    h->engine = engine;
-    if (!h->loss_mode_explicit) h->loss_mode = (engine == 2) ? 1 : 0;   // the expansion is the default of engine 2 only
+    ctx.engine = engine;
+    if (!ctx.loss_mode_explicit) ctx.loss_mode = (engine == 2) ? 1 : 0;   // the expansion is the default of engine 2 only
 }
 
 // every rank must run the same engine (the collectives are matched by program order): take the minimum of what the
 // ranks selected by themselves (shard lengths and free memory may differ by a little)
-void r_agree_engine(cmf_ctx *h) {
-    if (h->world() == 1) return;
-    double e = (double)h->engine;
-    c_allreduce_host(h, &e, 1, ncclMin);
-    if ((int)e != h->engine) r_set_engine(h, (int)e);
+template <typename S>
+void r_agree_engine(Ctx<S> &ctx) {
+    if (ctx.world() == 1) return;
+    double e = (double)ctx.engine;
+    c_allreduce_host(ctx, &e, 1, ncclMin);
+    if ((int)e != ctx.engine) r_set_engine(ctx, (int)e);
 }
 
-void attach_comm(cmf_ctx *h, ncclComm_t comm, int rank, int world, bool owned) {
+template <typename S>
+void attach_comm(Ctx<S> &ctx, ncclComm_t comm, int rank, int world) {
     int64_t a0, a1;
-    shard_range(h->T, world, rank, &a0, &a1);
-    REQUIRE(a0 == h->t0 && a1 == h->t1, "the handle's column range is not the balanced shard of this rank (use cmf_shard_range)");
-    h->comm.comm = comm; h->comm.rank = rank; h->comm.world = world; h->comm.owned = owned;
-    if (world > 1 && !h->comm_stream) {
-        CK(cudaStreamCreateWithFlags(&h->comm_stream, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&h->ev_a, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&h->ev_b, cudaEventDisableTiming));
+    shard_range(ctx.T, world, rank, &a0, &a1);
+    REQUIRE(a0 == ctx.t0 && a1 == ctx.t1, "the handle's column range is not the balanced shard of this rank (use cmf_shard_range)");
+    ctx.comm.comm = comm; ctx.comm.rank = rank; ctx.comm.world = world;
+    if (world > 1 && !ctx.comm_stream) {
+        CK(cudaStreamCreateWithFlags(&ctx.comm_stream, cudaStreamNonBlocking));
+        CK(cudaEventCreateWithFlags(&ctx.ev_a, cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&ctx.ev_b, cudaEventDisableTiming));
     }
-    r_agree_engine(h);
-}
-
-// Every call that takes or returns ONE factor set refuses a batch handle and names the call to use instead.
-void single_set(cmf_handle h, const char *use) {
-    if (h && h->R > 0) throw CmfError(CMF_ERR_ARG, std::string("this is a batch handle (cmf_create_batch): use ") + use);
-}
-void no_batch_split(cmf_handle h) {
-    if (h && h->R > 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles have no split-phase calls: use cmf_fit_batch");
-}
-cmf_ctx *batch_handle(cmf_handle h) {
-    REQUIRE(h && h->R > 0, "not a batch handle (cmf_create_batch)");
-    return h;
+    r_agree_engine(ctx);
 }
 
 // src/algs/alternating.jl:16-71 for R restarts at once.  Restart r keeps its own history and early stop; once it has
 // converged its factors are frozen (active flag 0) while the others go on.  The loop ends when every restart has stopped or
 // max_itr / max_time is reached; the elapsed time is the batch's own, shared by all restarts.
-void b_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
+template <typename S>
+void b_fit(Ctx<S> &ctx, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
            const double *l1W, const double *l2W, const double *l1H, const double *l2H, double *loss_hist,
            std::vector<double> &time_hist, int64_t cap, int64_t *n_hist, int *converged_early) {
-    const int64_t R = h->R;
+    const int64_t R = ctx.R;
     std::vector<double> reg((size_t)(4 * R));
     for (int64_t r = 0; r < R; ++r) { reg[4 * r] = l1W[r]; reg[4 * r + 1] = l2W[r]; reg[4 * r + 2] = l1H[r]; reg[4 * r + 3] = l2H[r]; }
     std::vector<int> active((size_t)R, 1);
-    h->batch_set_state(reg.data(), active.data());
+    ctx.batch_set_state(reg.data(), active.data());
     std::vector<double> loss((size_t)R);
-    h->batch_loss(loss.data());                                     // alternating.jl:37
+    ctx.batch_loss(loss.data());                                     // alternating.jl:37
     for (int64_t r = 0; r < R; ++r) { loss_hist[r * cap] = loss[r]; n_hist[r] = 1; converged_early[r] = 0; }
     time_hist.assign(1, 0.0);
     int64_t itr = 1, n_active = R;
@@ -2456,9 +2414,9 @@ void b_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int chec
         ++itr;
         REQUIRE((int64_t)time_hist.size() < cap, "history capacity exhausted");
         auto t_start = std::chrono::steady_clock::now();
-        if (!eval_mode) h->batch_update_motifs();
-        h->batch_update_feature_maps();
-        h->batch_loss(loss.data());
+        if (!eval_mode) ctx.batch_update_motifs();
+        ctx.batch_update_feature_maps();
+        ctx.batch_loss(loss.data());
         time_hist.push_back(time_hist.back() + std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count());
         bool stopped = false;
         for (int64_t r = 0; r < R; ++r) {
@@ -2472,55 +2430,95 @@ void b_fit(cmf_ctx *h, int64_t max_itr, double max_time, int eval_mode, int chec
                 stopped = true;
             }
         }
-        if (stopped && n_active > 0) h->batch_set_state(nullptr, active.data());
+        if (stopped && n_active > 0) ctx.batch_set_state(nullptr, active.data());
     }
 }
 
+template <typename S>
+using Ranks = std::vector<std::unique_ptr<Ctx<S>>>;
+
 }  // namespace
 
-// single-process multi-GPU group: one rank context per device, one worker thread per rank
-struct cmf_multi {
-    std::vector<cmf_ctx *> ranks;
-    std::vector<ncclComm_t> comms;
-    std::unique_ptr<cmf::Workers> workers;
+// A handle is the list of its rank contexts, all of one dtype.  cmf_create, cmf_create_shard, cmf_create_rank and
+// cmf_create_batch make one rank context; cmf_create_multi with ngpu > 1 makes one per device, each driven by its own worker
+// thread, over NCCL communicators the handle owns.
+struct cmf_ctx {
+    std::variant<Ranks<float>, Ranks<double>> ranks;
+    std::vector<ncclComm_t> comms;             // several rank contexts: one communicator per rank context
+    std::unique_ptr<cmf::Workers> workers;     // several rank contexts: worker i drives rank context i
+    size_t size() const { return std::visit([](auto &v) { return v.size(); }, ranks); }
+    ~cmf_ctx() {
+        if (!workers) return;   // one rank context: cmf_destroy frees it on its device
+        // every rank context and its communicator are freed by the worker that drives them (a failed create leaves gaps)
+        try {
+            std::visit([&](auto &v) {
+                workers->run_all([&](int i) {
+                    auto &r = v[(size_t)i];
+                    if (!r) return;
+                    cudaSetDevice(r->device);
+                    r.reset();
+                    if (comms[(size_t)i]) NcclApi::get().CommDestroy(comms[(size_t)i]);
+                });
+            }, ranks);
+        } catch (...) {}
+    }
 };
 
 namespace {
 
-struct MultiCtx : cmf_ctx {
-    cmf_multi m;
-    ~MultiCtx() override {
-        if (m.workers) {
-            try {
-                m.workers->run_all([&](int i) {
-                    cmf_ctx *r = m.ranks[(size_t)i];
-                    if (!r) return;
-                    cudaSetDevice(r->device);
-                    delete r;
-                    if ((size_t)i < m.comms.size() && m.comms[(size_t)i]) NcclApi::get().CommDestroy(m.comms[(size_t)i]);
-                });
-            } catch (...) {}
-        }
-    }
-};
+template <typename S>
+cmf_ctx *handle_of(std::unique_ptr<Ctx<S>> r) {
+    Ranks<S> v;
+    v.push_back(std::move(r));
+    return new cmf_ctx{std::move(v)};
+}
 
-// runs f(rank context) on the handle itself or, for a group handle, on every rank concurrently (worker threads)
+// A handle with several rank contexts follows two rules: its first rank context speaks for it (it alone writes the loss,
+// the histories, W, the scale partials and the early-stop flag), and a host H or X array starts at that context's first
+// column, so rank context r reads and writes it at column r.t0 - first(h).t0 (0 on every handle of one rank context).
+RankState &first(cmf_handle h) { return std::visit([](auto &v) -> RankState & { return *v.front(); }, h->ranks); }
+RankState &last(cmf_handle h) { return std::visit([](auto &v) -> RankState & { return *v.back(); }, h->ranks); }
+
+// f(Ctx<S> &) on every rank context of the handle: inline on the calling thread for one, concurrently on the workers for
+// several (the ranks meet in NCCL collectives); each under its device
 template <typename F>
 void on_ranks(cmf_handle h, F &&f) {
     REQUIRE(h != nullptr, "null handle");
-    if (h->multi) {
-        cmf_multi *m = h->multi;
-        m->workers->run_all([&](int i) {
-            cmf_ctx *r = m->ranks[(size_t)i];
-            DevGuard g(r->device);
+    std::visit([&](auto &v) {
+        if (v.size() == 1) {
+            DevGuard g(v[0]->device);
+            f(*v[0]);
+            return;
+        }
+        h->workers->run_all([&](int i) {
+            auto &r = *v[(size_t)i];
+            DevGuard g(r.device);
             f(r);
         });
-    } else {
-        DevGuard g(h->device);
-        f(h);
-    }
+    }, h->ranks);
 }
-cmf_ctx *rank0(cmf_handle h) { return h->multi ? h->multi->ranks[0] : h; }
+// f(Ctx<S> &) on the first rank context, on the calling thread and its current device
+template <typename F>
+void on_first(cmf_handle h, F &&f) {
+    std::visit([&](auto &v) { f(*v.front()); }, h->ranks);
+}
+
+// The split-phase, stream and PGD-setup calls drive one rank context.
+void single_rank(cmf_handle h) { REQUIRE(h && h->size() == 1, "single-rank call"); }
+// Every call that takes or returns ONE factor set refuses a batch handle and names the call to use instead.
+void single_set(cmf_handle h, const char *use) {
+    if (h && first(h).R > 0) throw CmfError(CMF_ERR_ARG, std::string("this is a batch handle (cmf_create_batch): use ") + use);
+}
+void no_batch_split(cmf_handle h) {
+    if (h && first(h).R > 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles have no split-phase calls: use cmf_fit_batch");
+}
+void batch_handle(cmf_handle h) { REQUIRE(h && first(h).R > 0, "not a batch handle (cmf_create_batch)"); }
+
+// a handle of one rank context (make_ctx's checks)
+cmf_ctx *make_handle(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device,
+                     int64_t R = 0) {
+    return with_dtype(dtype, [&](auto s) { return handle_of(make_ctx<decltype(s)>(N, T, t0, t1, K, L, dtype, alg, device, R)); });
+}
 
 }  // namespace
 
@@ -2535,7 +2533,7 @@ int cmf_create(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int 
     return guarded([&] {
         REQUIRE(out != nullptr, "null output pointer");
         DevRestore g;
-        *out = make_ctx(N, T, 0, T, K, L, dtype, alg, device);
+        *out = make_handle(N, T, 0, T, K, L, dtype, alg, device);
     });
 }
 
@@ -2544,7 +2542,7 @@ int cmf_create_shard(cmf_handle *out, int64_t N, int64_t T_global, int64_t t_beg
     return guarded([&] {
         REQUIRE(out != nullptr, "null output pointer");
         DevRestore g;
-        *out = make_ctx(N, T_global, t_begin, t_end, K, L, dtype, alg, device);
+        *out = make_handle(N, T_global, t_begin, t_end, K, L, dtype, alg, device);
     });
 }
 
@@ -2579,8 +2577,8 @@ int cmf_create_rank(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L,
         DevRestore g;
         int64_t a0, a1;
         shard_range(T, world, rank, &a0, &a1);
-        cmf_ctx *c = make_ctx(N, T, a0, a1, K, L, dtype, alg, device);
-        try {
+        *out = with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(N, T, a0, a1, K, L, dtype, alg, device);
             ncclComm_t comm = nullptr;
             if (world > 1) {
                 std::lock_guard<std::mutex> lk(g_comm_mu);
@@ -2597,9 +2595,9 @@ int cmf_create_rank(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L,
                     g_comm_cache[key] = comm;            // replaces (and leaks until exit) an older one: it may still serve a live handle
                 }
             }
-            attach_comm(c, comm, rank, world, false);
-        } catch (...) { delete c; throw; }
-        *out = c;
+            attach_comm(*c, comm, rank, world);
+            return handle_of(std::move(c));
+        });
     });
 }
 
@@ -2619,122 +2617,118 @@ int cmf_create_multi(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L
         }
         if (ngpu == 1) {
             DevRestore g;
-            *out = make_ctx(N, T, 0, T, K, L, dtype, alg, devs[0]);
+            *out = make_handle(N, T, 0, T, K, L, dtype, alg, devs[0]);
             return;
         }
         int prev = 0;
         cudaGetDevice(&prev);
-        auto *mc = new MultiCtx();
-        mc->N = N; mc->T = T; mc->t0 = 0; mc->t1 = T; mc->Tl = T; mc->K = K; mc->L = L;
-        mc->dtype = dtype; mc->alg = alg; mc->device = devs[0];
-        mc->multi = &mc->m;
-        try {
-            mc->m.ranks.assign((size_t)ngpu, nullptr);
-            mc->m.comms.assign((size_t)ngpu, nullptr);
-            mc->m.workers.reset(new Workers(ngpu));
-            NK(nccl().CommInitAll(mc->m.comms.data(), ngpu, devs.data()));
-            cudaSetDevice(prev);
-            mc->m.workers->run_all([&](int i) {
-                DevGuard g(devs[(size_t)i]);
-                int64_t a0, a1;
-                shard_range(T, ngpu, i, &a0, &a1);
-                mc->m.ranks[(size_t)i] = make_ctx(N, T, a0, a1, K, L, dtype, alg, devs[(size_t)i]);
-            });
-            mc->m.workers->run_all([&](int i) {
-                cmf_ctx *r = mc->m.ranks[(size_t)i];
-                DevGuard g(r->device);
-                attach_comm(r, mc->m.comms[(size_t)i], i, ngpu, false);
-            });
-        } catch (...) {
-            cudaSetDevice(prev);
-            delete mc;
-            throw;
-        }
-        *out = mc;
+        with_dtype(dtype, [&](auto s) {
+            using S = decltype(s);
+            auto *mc = new cmf_ctx{Ranks<S>((size_t)ngpu)};
+            Ranks<S> &ranks = std::get<Ranks<S>>(mc->ranks);
+            try {
+                mc->comms.assign((size_t)ngpu, nullptr);
+                mc->workers.reset(new Workers(ngpu));
+                NK(nccl().CommInitAll(mc->comms.data(), ngpu, devs.data()));
+                cudaSetDevice(prev);
+                mc->workers->run_all([&](int i) {
+                    DevGuard g(devs[(size_t)i]);
+                    int64_t a0, a1;
+                    shard_range(T, ngpu, i, &a0, &a1);
+                    ranks[(size_t)i] = make_ctx<S>(N, T, a0, a1, K, L, dtype, alg, devs[(size_t)i]);
+                });
+                mc->workers->run_all([&](int i) {
+                    Ctx<S> &r = *ranks[(size_t)i];
+                    DevGuard g(r.device);
+                    attach_comm(r, mc->comms[(size_t)i], i, ngpu);
+                });
+            } catch (...) {
+                cudaSetDevice(prev);
+                delete mc;
+                throw;
+            }
+            *out = mc;
+        });
     });
 }
 
 int cmf_comm_info(cmf_handle h, int *rank_out, int *world_out, int64_t *t_begin, int64_t *t_end) {
     return guarded([&] {
         REQUIRE(h, "null handle");
-        if (rank_out) *rank_out = h->multi ? 0 : h->rank();
-        if (world_out) *world_out = h->multi ? (int)h->multi->ranks.size() : h->world();
-        if (t_begin) *t_begin = h->t0;
-        if (t_end) *t_end = h->t1;
+        if (rank_out) *rank_out = first(h).rank();
+        if (world_out) *world_out = first(h).world();
+        if (t_begin) *t_begin = first(h).t0;
+        if (t_end) *t_end = last(h).t1;
     });
 }
 
 int cmf_destroy(cmf_handle h) {
     return guarded([&] {
         if (!h) return;
-        if (h->multi) { delete h; return; }
-        DevGuard g(h->device);
-        ncclComm_t comm = (h->comm.owned ? h->comm.comm : nullptr);
+        if (h->workers) { delete h; return; }   // ~cmf_ctx frees every rank context on its worker
+        DevGuard g(first(h).device);
         delete h;
-        if (comm) NcclApi::get().CommDestroy(comm);
     });
 }
 
 int cmf_set_data(cmf_handle h, const void *X, int64_t first_col) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->set_data(X, first_col); r_data_norm(r); }); });
+    return guarded([&] { on_ranks(h, [&](auto &r) { r.set_data(X, first_col); r_data_norm(r); }); });
 }
 int cmf_synth_data(cmf_handle h, uint64_t seed, int64_t K_true, int64_t L_true, double p_h, double noise) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->synth_data(seed, K_true, L_true, p_h, noise); r_data_norm(r); }); });
+    return guarded([&] { on_ranks(h, [&](auto &r) { r.synth_data(seed, K_true, L_true, p_h, noise); r_data_norm(r); }); });
 }
 int cmf_data_sumsq(cmf_handle h, double *out) {
     return guarded([&] {
         REQUIRE(out, "null output");
-        cmf_ctx *r = rank0(h);
-        REQUIRE(r->have_data, "no data");
-        *out = (h->multi || r->world() > 1) ? r->data_sumsq_global : r->data_sumsq_local;
+        const RankState &r = first(h);
+        REQUIRE(r.have_data, "no data");
+        *out = r.world() > 1 ? r.data_sumsq_global : r.data_sumsq_local;
     });
 }
 int cmf_set_data_norm(cmf_handle h, double norm) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r->data_norm = norm; r->data_sumsq_global = norm * norm; }); });
+    return guarded([&] { on_ranks(h, [&](auto &r) { r.data_norm = norm; r.data_sumsq_global = norm * norm; }); });
 }
 int cmf_set_factors(cmf_handle h, const void *W, const void *H, int64_t first_col) {
-    return guarded([&] { single_set(h, "cmf_set_factors_batch"); on_ranks(h, [&](cmf_ctx *r) { r->set_factors(W, H, first_col); }); });
+    return guarded([&] { single_set(h, "cmf_set_factors_batch"); on_ranks(h, [&](auto &r) { r.set_factors(W, H, first_col); }); });
 }
 int cmf_exchange_halos(cmf_handle h) {
-    return guarded([&] { no_batch_split(h); on_ranks(h, [&](cmf_ctx *r) { c_halo_exchange(r); r->h_changed(); }); });
+    return guarded([&] { no_batch_split(h); on_ranks(h, [&](auto &r) { c_halo_exchange(r); r.h_changed(); }); });
 }
 int cmf_init_rand(cmf_handle h, uint64_t seed) {
-    return guarded([&] { single_set(h, "cmf_set_factors_batch with drawn factors"); on_ranks(h, [&](cmf_ctx *r) { r->init_rand(seed); }); });
+    return guarded([&] { single_set(h, "cmf_set_factors_batch with drawn factors"); on_ranks(h, [&](auto &r) { r.init_rand(seed); }); });
 }
 int cmf_init_scale_partials(cmf_handle h, double out[2]) {
     return guarded([&] { single_set(h, "cmf_init_scale_partials_batch");
         REQUIRE(out, "null output");
-        on_ranks(h, [&](cmf_ctx *r) {
+        on_ranks(h, [&](auto &r) {
             double v[2];
             r_init_scale_partials(r, v);
-            if (!h->multi || r->rank() == 0) { out[0] = v[0]; out[1] = v[1]; }
+            if (&r == &first(h)) { out[0] = v[0]; out[1] = v[1]; }
         });
     });
 }
 int cmf_scale_factors(cmf_handle h, double s) {
-    return guarded([&] { single_set(h, "cmf_scale_factors_batch"); on_ranks(h, [&](cmf_ctx *r) { r->scale_factors(s); }); });
+    return guarded([&] { single_set(h, "cmf_scale_factors_batch"); on_ranks(h, [&](auto &r) { r.scale_factors(s); }); });
 }
 int cmf_get_factors(cmf_handle h, void *W_out, void *H_out) {
     return guarded([&] { single_set(h, "cmf_get_factors_batch");
-        const bool grp = h && h->multi;
-        on_ranks(h, [&](cmf_ctx *r) {
-            REQUIRE(r->have_factors, "no factors");
-            void *Hp = H_out;
-            if (grp && H_out) Hp = (char *)H_out + (size_t)(r->t0 * r->K) * elem_size(r);     // group handle: H_out is K x T
-            r->get_factors((!grp || r->rank() == 0) ? W_out : nullptr, Hp);
+        on_ranks(h, [&](auto &r) {
+            REQUIRE(r.have_factors, "no factors");
+            void *Hp = H_out ? (char *)H_out + (size_t)((r.t0 - first(h).t0) * r.K) * elem_size(r) : nullptr;
+            r.get_factors(&r == &first(h) ? W_out : nullptr, Hp);
         });
     });
 }
 
 int cmf_update_motifs(cmf_handle h, double l1W, double l2W) {
-    return guarded([&] { single_set(h, "cmf_fit_batch"); on_ranks(h, [&](cmf_ctx *r) { r_update_motifs(r, l1W, l2W); }); });
+    return guarded([&] { single_set(h, "cmf_fit_batch"); on_ranks(h, [&](auto &r) { r_update_motifs(r, l1W, l2W); }); });
 }
 
 int cmf_update_feature_maps(cmf_handle h, double l1H, double l2H, double *loss_out) {
     return guarded([&] { single_set(h, "cmf_fit_batch");
-        on_ranks(h, [&](cmf_ctx *r) {
+        on_ranks(h, [&](auto &r) {
             const double loss = r_update_feature_maps(r, l1H, l2H);
-            if (loss_out && (r->rank() == 0 || !h->multi)) *loss_out = loss;
+            if (loss_out && &r == &first(h)) *loss_out = loss;
         });
     });
 }
@@ -2742,10 +2736,10 @@ int cmf_update_feature_maps(cmf_handle h, double l1H, double l2H, double *loss_o
 int cmf_loss(cmf_handle h, double *loss_out) {
     return guarded([&] { single_set(h, "cmf_loss_batch");
         REQUIRE(loss_out, "null output");
-        on_ranks(h, [&](cmf_ctx *r) {
-            REQUIRE(r->world() > 1 || (r->is_first && r->is_last), "shards without a communicator use cmf_loss_partial");
+        on_ranks(h, [&](auto &r) {
+            REQUIRE(r.world() > 1 || (r.is_first && r.is_last), "shards without a communicator use cmf_loss_partial");
             const double loss = r_guarded_loss(r);
-            if (r->rank() == 0 || !h->multi) *loss_out = loss;
+            if (&r == &first(h)) *loss_out = loss;
         });
     });
 }
@@ -2758,12 +2752,12 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
         REQUIRE(patience >= 1, "patience must be >= 1 (src/algs/alternating.jl:30)");
         REQUIRE(cap >= 1, "history capacity must be >= 1");
         if (converged_early) *converged_early = 0;
-        on_ranks(h, [&](cmf_ctx *r) {
-            REQUIRE(r->world() > 1 || (r->is_first && r->is_last), "shards without a communicator use the split-phase calls");
+        on_ranks(h, [&](auto &r) {
+            REQUIRE(r.world() > 1 || (r.is_first && r.is_last), "shards without a communicator use the split-phase calls");
             std::vector<double> lh, th;
             int early = 0;
             r_fit(r, max_itr, max_time, eval_mode, check_convergence, patience, tol, l1W, l2W, l1H, l2H, lh, th, cap, &early);
-            if (r->rank() == 0 || !h->multi) {
+            if (&r == &first(h)) {
                 std::copy(lh.begin(), lh.end(), loss_hist);
                 std::copy(th.begin(), th.end(), time_hist);
                 *n_hist = (int64_t)lh.size();
@@ -2774,59 +2768,57 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
 }
 
 int cmf_w_partials(cmf_handle h) {
-    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_partials(); });
+    return guarded([&] { no_batch_split(h); single_rank(h); on_ranks(h, [&](auto &r) { r.w_partials(); }); });
 }
 int cmf_w_apply(cmf_handle h, double l1W, double l2W) {
-    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->w_apply(l1W, l2W); });
+    return guarded([&] { no_batch_split(h); single_rank(h); on_ranks(h, [&](auto &r) { r.w_apply(l1W, l2W); }); });
 }
 int cmf_h_update(cmf_handle h, double l1H, double l2H) {
     return guarded([&] { no_batch_split(h);
-        REQUIRE(h && !h->multi, "single-rank call");
-        DevGuard g(h->device);
-        REQUIRE(h->alg == CMF_MULT, "the split-phase H update is MultUpdate only");
-        h->h_update(l1H, l2H);
+        single_rank(h);
+        on_ranks(h, [&](auto &r) {
+            REQUIRE(r.alg == CMF_MULT, "the split-phase H update is MultUpdate only");
+            r.h_update(l1H, l2H);
+        });
     });
 }
 int cmf_loss_partial(cmf_handle h, double *sumsq_out) {
-    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sumsq_out, "null output"); DevGuard g(h->device); *sumsq_out = h->loss_partial(); });
+    return guarded([&] { no_batch_split(h); single_rank(h); REQUIRE(sumsq_out, "null output"); on_ranks(h, [&](auto &r) { *sumsq_out = r.loss_partial(); }); });
 }
 int cmf_exchange_buffer(cmf_handle h, int which, void **dev_ptr, int64_t *count, int *dtype) {
-    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(dev_ptr && count && dtype, "null output"); h->exchange_buffer(which, dev_ptr, count, dtype); });
+    return guarded([&] { no_batch_split(h); single_rank(h); REQUIRE(dev_ptr && count && dtype, "null output"); on_first(h, [&](auto &r) { r.exchange_buffer(which, dev_ptr, count, dtype); }); });
 }
 int cmf_halo_buffers(cmf_handle h, void **sl, void **sr, void **rl, void **rr, int64_t *count) {
-    return guarded([&] { no_batch_split(h); REQUIRE(h && !h->multi, "single-rank call"); REQUIRE(sl && sr && rl && rr && count, "null output"); h->halo_buffers(sl, sr, rl, rr, count); });
+    return guarded([&] { no_batch_split(h); single_rank(h); REQUIRE(sl && sr && rl && rr && count, "null output"); on_first(h, [&](auto &r) { r.halo_buffers(sl, sr, rl, rr, count); }); });
 }
 int cmf_sync(cmf_handle h) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { CK(cudaStreamSynchronize(r->stream)); }); });
+    return guarded([&] { on_ranks(h, [&](auto &r) { CK(cudaStreamSynchronize(r.stream)); }); });
 }
 int cmf_launch_count(cmf_handle h, int64_t *out) {
     return guarded([&] {
         REQUIRE(h && out, "null argument");
-        if (!h->multi) { *out = h->launches; return; }
-        int64_t n = 0;
-        for (cmf_ctx *r : h->multi->ranks) n += r->launches;
-        *out = n;
+        *out = std::visit([](auto &v) { int64_t n = 0; for (auto &r : v) n += r->launches; return n; }, h->ranks);
     });
 }
 int cmf_stream(cmf_handle h, void **stream_out) {
-    return guarded([&] { REQUIRE(h && stream_out, "null argument"); *stream_out = (void *)rank0(h)->stream; });
+    return guarded([&] { REQUIRE(h && stream_out, "null argument"); *stream_out = (void *)first(h).stream; });
 }
 int cmf_get_data(cmf_handle h, void *X_out, int with_halo) {
     return guarded([&] {
         REQUIRE(X_out, "null output");
-        const bool grp = h && h->multi;
-        on_ranks(h, [&](cmf_ctx *r) {
-            REQUIRE(r->have_data, "no data");
-            r->get_data(grp ? (char *)X_out + (size_t)(r->t0 * r->N) * elem_size(r) : X_out, grp ? 0 : with_halo);
+        on_ranks(h, [&](auto &r) {
+            REQUIRE(r.have_data, "no data");
+            // several rank contexts fill one N x T array: no halos
+            r.get_data((char *)X_out + (size_t)((r.t0 - first(h).t0) * r.N) * elem_size(r), h->size() > 1 ? 0 : with_halo);
         });
     });
 }
 int cmf_profile(cmf_handle h, int enable) {
     return guarded([&] {
-        on_ranks(h, [&](cmf_ctx *r) {
-            CK(cudaStreamSynchronize(r->stream));
-            r->prof_clear();
-            r->profiling = enable != 0;
+        on_ranks(h, [&](auto &r) {
+            CK(cudaStreamSynchronize(r.stream));
+            r.prof_clear();
+            r.profiling = enable != 0;
         });
     });
 }
@@ -2834,12 +2826,12 @@ int cmf_profile_read(cmf_handle h, int which, double *ms_total, int64_t *count) 
     return guarded([&] {
         REQUIRE(h && ms_total && count, "null output");
         REQUIRE(which >= 0 && which < PROF_NCLASS, "which must be 0 (conv), 1 (transconv), 2 (corr) or 3 (HALS H sweep)");
-        cmf_ctx *r = rank0(h);
-        DevGuard g(r->device);
-        CK(cudaStreamSynchronize(r->stream));
+        RankState &r = first(h);
+        DevGuard g(r.device);
+        CK(cudaStreamSynchronize(r.stream));
         double tot = 0.0;
         int64_t n = 0;
-        for (auto &e : r->prof_events) {
+        for (auto &e : r.prof_events) {
             if (e.which != which) continue;
             float ms = 0.f;
             CK(cudaEventElapsedTime(&ms, e.a, e.b));
@@ -2852,54 +2844,54 @@ int cmf_profile_read(cmf_handle h, int which, double *ms_total, int64_t *count) 
 }
 int cmf_set_stream(cmf_handle h, void *stream) {
     return guarded([&] {
-        REQUIRE(h && !h->multi, "single-rank call");
-        DevGuard g(h->device);
-        CK(cudaStreamSynchronize(h->stream));
-        if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
-        h->own_stream = false;
-        h->stream = (cudaStream_t)stream;
+        single_rank(h);
+        RankState &r = first(h);
+        DevGuard g(r.device);
+        CK(cudaStreamSynchronize(r.stream));
+        if (r.own_stream && r.stream) cudaStreamDestroy(r.stream);
+        r.own_stream = false;
+        r.stream = (cudaStream_t)stream;
     });
 }
 int cmf_set_engine(cmf_handle h, int engine) {
-    return guarded([&] { on_ranks(h, [&](cmf_ctx *r) { r_set_engine(r, engine); }); });
+    return guarded([&] { on_ranks(h, [&](auto &r) { r_set_engine(r, engine); }); });
 }
 
 int cmf_set_loss_mode(cmf_handle h, int mode) {
     return guarded([&] {
         REQUIRE(mode == 0 || mode == 1, "loss mode must be 0 (direct) or 1 (expansion)");
-        if (h && h->R > 0 && mode != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles evaluate the loss by the direct pass (mode 0) only");
-        on_ranks(h, [&](cmf_ctx *r) { r->loss_mode = mode; r->loss_mode_explicit = true; r->calib_reset(); });
+        if (h && first(h).R > 0 && mode != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles evaluate the loss by the direct pass (mode 0) only");
+        on_ranks(h, [&](auto &r) { r.loss_mode = mode; r.loss_mode_explicit = true; r.calib_reset(); });
     });
 }
 int cmf_set_loss_guard(cmf_handle h, double guard, int max_interval) {
     return guarded([&] {
         REQUIRE(guard >= 0.0, "loss guard must be >= 0");
         REQUIRE(max_interval >= 1 && max_interval <= 1024, "calibration interval must be in [1, 1024]");
-        on_ranks(h, [&](cmf_ctx *r) { r->loss_guard = guard; r->calib_max_interval = max_interval; r->calib_reset(); });
+        on_ranks(h, [&](auto &r) { r.loss_guard = guard; r.calib_max_interval = max_interval; r.calib_reset(); });
     });
 }
 int cmf_get_loss_stats(cmf_handle h, int64_t *n_direct, int64_t *n_expansion, int *interval, double *last_err) {
     return guarded([&] {
         REQUIRE(h, "null handle");
-        cmf_ctx *r = rank0(h);
-        if (n_direct) *n_direct = r->n_loss_direct;
-        if (n_expansion) *n_expansion = r->n_loss_expansion;
-        if (interval) *interval = r->calib_have ? r->calib_interval : 0;
-        if (last_err) *last_err = r->calib_last_err;
+        const RankState &r = first(h);
+        if (n_direct) *n_direct = r.n_loss_direct;
+        if (n_expansion) *n_expansion = r.n_loss_expansion;
+        if (interval) *interval = r.calib_have ? r.calib_interval : 0;
+        if (last_err) *last_err = r.calib_last_err;
     });
 }
 int cmf_get_loss_mode(cmf_handle h, int *mode_out) {
-    return guarded([&] { REQUIRE(h && mode_out, "null argument"); *mode_out = rank0(h)->loss_mode; });
+    return guarded([&] { REQUIRE(h && mode_out, "null argument"); *mode_out = first(h).loss_mode; });
 }
 int cmf_get_fd_layout(cmf_handle h, int *block_len, int *hop, int64_t *nblocks) {
     return guarded([&] {
         REQUIRE(h && block_len && hop && nblocks, "null argument");
-        cmf_ctx *r = rank0(h);
-        r->fd_layout(block_len, hop, nblocks);
+        on_first(h, [&](auto &r) { r.fd_layout(block_len, hop, nblocks); });
     });
 }
 int cmf_get_engine(cmf_handle h, int *engine_out) {
-    return guarded([&] { REQUIRE(h && engine_out, "null argument"); *engine_out = rank0(h)->engine; });
+    return guarded([&] { REQUIRE(h && engine_out, "null argument"); *engine_out = first(h).engine; });
 }
 
 static int current_device() {
@@ -2909,62 +2901,64 @@ static int current_device() {
 }
 
 int cmf_set_pgd_constraints(cmf_handle h, int constrW, int constrH) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); h->set_pgd_constraints(constrW, constrH); });
+    return guarded([&] { single_rank(h); on_first(h, [&](auto &r) { r.set_pgd_constraints(constrW, constrH); }); });
 }
 int cmf_set_pgd_loss(cmf_handle h, int loss_func, const void *mask) {
-    return guarded([&] { REQUIRE(h && !h->multi, "single-rank call"); DevGuard g(h->device); h->set_pgd_loss(loss_func, mask); });
+    return guarded([&] { single_rank(h); on_ranks(h, [&](auto &r) { r.set_pgd_loss(loss_func, mask); }); });
 }
 
 int cmf_tensor_conv(int64_t N, int64_t T, int64_t K, int64_t L, int dtype, const void *W, const void *H, void *out) {
     return guarded([&] {
         REQUIRE(W && H && out, "null pointer");
-        cmf_ctx *c = make_ctx(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
-        try { c->set_factors(W, H, 0); c->prim_conv(out); } catch (...) { delete c; throw; }
-        delete c;
+        with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
+            c->set_factors(W, H, 0);
+            c->prim_conv(out);
+        });
     });
 }
 int cmf_tensor_transconv(int64_t N, int64_t T, int64_t K, int64_t L, int dtype, const void *W, const void *X, void *out) {
     return guarded([&] {
         REQUIRE(W && X && out, "null pointer");
-        cmf_ctx *c = make_ctx(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
-        try {
-            std::vector<char> Hz((size_t)(K * T) * (dtype == CMF_F64 ? 8 : 4), 0);
+        with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
+            std::vector<decltype(s)> Hz((size_t)(K * T), 0);
             c->set_factors(W, Hz.data(), 0);
             c->prim_transconv(X, out);
-        } catch (...) { delete c; throw; }
-        delete c;
+        });
     });
 }
 int cmf_corr_w(int64_t N, int64_t T, int64_t K, int64_t L, int dtype, const void *H, const void *X, void *out) {
     return guarded([&] {
         REQUIRE(H && X && out, "null pointer");
-        cmf_ctx *c = make_ctx(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
-        try {
-            std::vector<char> Wz((size_t)(K * N * L) * (dtype == CMF_F64 ? 8 : 4), 0);
+        with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
+            std::vector<decltype(s)> Wz((size_t)(K * N * L), 0);
             c->set_factors(Wz.data(), H, 0);
             c->prim_corr(X, out);
-        } catch (...) { delete c; throw; }
-        delete c;
+        });
     });
 }
 int cmf_compute_resids(int64_t N, int64_t T, int64_t K, int64_t L, int dtype, const void *X, const void *W, const void *H, void *out) {
     return guarded([&] {
         REQUIRE(X && W && H && out, "null pointer");
-        cmf_ctx *c = make_ctx(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
-        try { c->set_data(X, 0); c->set_factors(W, H, 0); c->prim_resids(out); } catch (...) { delete c; throw; }
-        delete c;
+        with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(N, T, 0, T, K, L, dtype, CMF_MULT, current_device());
+            c->set_data(X, 0);
+            c->set_factors(W, H, 0);
+            c->prim_resids(out);
+        });
     });
 }
 int cmf_shift_and_stack(int64_t K, int64_t T, int64_t L, int dtype, const void *H, void *out) {
     return guarded([&] {
         REQUIRE(H && out, "null pointer");
-        cmf_ctx *c = make_ctx(8, T, 0, T, K, L, dtype, CMF_MULT, current_device());
-        try {
-            std::vector<char> Wz((size_t)(K * 8 * L) * (dtype == CMF_F64 ? 8 : 4), 0);
+        with_dtype(dtype, [&](auto s) {
+            auto c = make_ctx<decltype(s)>(8, T, 0, T, K, L, dtype, CMF_MULT, current_device());
+            std::vector<decltype(s)> Wz((size_t)(K * 8 * L), 0);
             c->set_factors(Wz.data(), H, 0);
             c->prim_shift_and_stack(out);
-        } catch (...) { delete c; throw; }
-        delete c;
+        });
     });
 }
 
@@ -2979,23 +2973,23 @@ int cmf_create_batch(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L
         REQUIRE(R * K * cdiv(L, 8) <= (int64_t)CORR_PB * 65535 && R * K <= 4 * 65535, "R*K too large for one launch grid");
         if (L > 769) throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts need L <= 769");
         DevRestore g;
-        *out = make_ctx(N, T, 0, T, K, L, dtype, alg, device, R);
+        *out = make_handle(N, T, 0, T, K, L, dtype, alg, device, R);
     });
 }
 int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H) {
-    return guarded([&] { DevGuard g(batch_handle(h)->device); h->batch_set_factors(W, H); });
+    return guarded([&] { batch_handle(h); on_ranks(h, [&](auto &r) { r.batch_set_factors(W, H); }); });
 }
 int cmf_get_factors_batch(cmf_handle h, void *W_out, void *H_out) {
-    return guarded([&] { DevGuard g(batch_handle(h)->device); h->batch_get_factors(W_out, H_out); });
+    return guarded([&] { batch_handle(h); on_ranks(h, [&](auto &r) { r.batch_get_factors(W_out, H_out); }); });
 }
 int cmf_init_scale_partials_batch(cmf_handle h, double *out) {
-    return guarded([&] { REQUIRE(out, "null output"); DevGuard g(batch_handle(h)->device); h->batch_scale_partials(out); });
+    return guarded([&] { REQUIRE(out, "null output"); batch_handle(h); on_ranks(h, [&](auto &r) { r.batch_scale_partials(out); }); });
 }
 int cmf_scale_factors_batch(cmf_handle h, const double *s) {
-    return guarded([&] { REQUIRE(s, "null scale factors"); DevGuard g(batch_handle(h)->device); h->batch_scale(s); });
+    return guarded([&] { REQUIRE(s, "null scale factors"); batch_handle(h); on_ranks(h, [&](auto &r) { r.batch_scale(s); }); });
 }
 int cmf_loss_batch(cmf_handle h, double *loss_out) {
-    return guarded([&] { REQUIRE(loss_out, "null output"); DevGuard g(batch_handle(h)->device); h->batch_loss(loss_out); });
+    return guarded([&] { REQUIRE(loss_out, "null output"); batch_handle(h); on_ranks(h, [&](auto &r) { r.batch_loss(loss_out); }); });
 }
 int cmf_fit_batch(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int check_convergence, int patience, double tol,
                   const double *l1W, const double *l2W, const double *l1H, const double *l2H, double *loss_hist, double *time_hist,
@@ -3006,11 +3000,12 @@ int cmf_fit_batch(cmf_handle h, int64_t max_itr, double max_time, int eval_mode,
         REQUIRE(loss_hist && time_hist && n_hist && converged_early, "null history pointers");
         REQUIRE(patience >= 1, "patience must be >= 1 (src/algs/alternating.jl:30)");
         REQUIRE(cap >= 1, "history capacity must be >= 1");
-        DevGuard g(h->device);
-        std::vector<double> th;
-        b_fit(h, max_itr, max_time, eval_mode, check_convergence, patience, tol, l1W, l2W, l1H, l2H, loss_hist, th, cap, n_hist,
-              converged_early);
-        std::copy(th.begin(), th.end(), time_hist);
+        on_ranks(h, [&](auto &r) {
+            std::vector<double> th;
+            b_fit(r, max_itr, max_time, eval_mode, check_convergence, patience, tol, l1W, l2W, l1H, l2H, loss_hist, th, cap, n_hist,
+                  converged_early);
+            std::copy(th.begin(), th.end(), time_hist);
+        });
     });
 }
 

@@ -72,7 +72,6 @@ struct NcclApi {
 struct Comm {
     ncclComm_t comm = nullptr;
     int rank = 0, world = 1;
-    bool owned = true;
 };
 
 // Persistent worker threads of a single-process multi-GPU handle: run_all(fn) runs fn(rank) on every worker
