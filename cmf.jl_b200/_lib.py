@@ -70,6 +70,7 @@ SIGNATURES = {
     "cmf_compute_resids": [_i64, _i64, _i64, _i64, _int, _vp, _vp, _vp, _vp],
     "cmf_shift_and_stack": [_i64, _i64, _i64, _int, _vp, _vp],
     "cmf_create_batch": [_c.POINTER(_h), _i64, _i64, _i64, _i64, _int, _int, _i64, _int],
+    "cmf_create_batch_ranks": [_c.POINTER(_h), _i64, _i64, _c.POINTER(_i64), _i64, _int, _int, _i64, _int],
     "cmf_set_factors_batch": [_h, _vp, _vp],
     "cmf_get_factors_batch": [_h, _vp, _vp],
     "cmf_init_scale_partials_batch": [_h, _c.POINTER(_dbl)],

@@ -13,6 +13,7 @@
 #include <cstring>
 #include <map>
 #include <memory>
+#include <numeric>
 #include <mutex>
 #include <tuple>
 #include <stdexcept>
@@ -108,7 +109,7 @@ struct RankState {
     bool numH_dot_valid = false;     // scal[4] == <numH, H> of the current numH and H (left there by the MU update of H)
     bool gram_valid = false;         // exchange buffer 1 holds the local Gram/tail partial of the current H
     bool have_data = false, have_factors = false;
-    int64_t R = 0;                   // restarts of a batch handle (cmf_create_batch); 0 = a handle of one factor set
+    int64_t R = 0;                   // restarts of a batch handle (cmf_create_batch[_ranks]); 0 = a handle of one factor set
     // optional per-kernel-class event timing (bench.py's roofline): class -> list of event pairs
     bool profiling = false;
     struct ProfEv { int which; cudaEvent_t a, b; };
@@ -1039,18 +1040,18 @@ struct Ctx : RankState {
 
     // ---------------------------------------------------------------- kernel launch helpers
     // est over local columns [t_lo, t_hi) from (Wsrc, Hsrc) with dims (Kc, Lc).
-    // nrest > 1: restart z of a batch handle (W rows l*ld + z*Kc + k, H columns t*ld + z*Kc + k with ld = nrest*Kc) writes
-    // its partials at partial + z*part_rs
+    // per_restart: one grid slice z per restart of a batch handle (rank K_r, W rows l*C + off_r + k, H columns t*C + off_r + k,
+    // Kc = the largest K_r), writing its partials at partial + z*part_rs
     void launch_conv(const S *Wsrc, const S *Hsrc, int64_t Kc, int64_t Lc, int64_t h_lo, int64_t h_hi,
                      int64_t t_lo, int64_t t_hi, int flags, S *out, double *partial, uint64_t seed = 0,
-                     double noise = 0.0, int nrest = 1, int64_t part_rs = 0) {
+                     double noise = 0.0, bool per_restart = false, int64_t part_rs = 0) {
         if (t_hi <= t_lo) return;
         ConvArgs<S> a;
         a.Wi = Wsrc; a.H = Hsrc; a.X = X.p; a.out = out; a.partial = partial;
         a.N = N; a.K = Kc; a.L = Lc; a.t_lo = t_lo; a.t_hi = t_hi; a.h_lo = h_lo; a.h_hi = h_hi;
         a.flags = flags; a.seed = seed; a.t_global0 = t0; a.noise = noise;
         a.mask = pgd_mask.n ? pgd_mask.p : nullptr; a.lossf = pgd_loss;
-        a.ldw = a.ldh = nrest * Kc; a.w_rs = Kc * N; a.h_rs = Kc; a.part_rs = part_rs;
+        a.ldw = a.ldh = per_restart ? b_C : Kc; a.part_rs = part_rs; a.tab = per_restart ? b_tab.p : nullptr;
         const int Lpad = (int)(cdiv(Lc, 8) * 8);
         const int HW = BT + Lpad - 1;
         const size_t ws_bytes = (size_t)CONV_LC * BN * sizeof(S);
@@ -1061,7 +1062,7 @@ struct Ctx : RankState {
         const size_t smem = (size_t)KC * HW * sizeof(S) + ws_bytes;
         auto kern = conv_kernel<S, TN, TT, TY>;
         CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        dim3 grid((unsigned)cdiv(t_hi - t_lo, BT), (unsigned)cdiv(N, BN), (unsigned)nrest);
+        dim3 grid((unsigned)cdiv(t_hi - t_lo, BT), (unsigned)cdiv(N, BN), (unsigned)(per_restart ? R : 1));
         prof_begin(PROF_CONV);
         kern<<<grid, dim3(16, TY), smem, stream>>>(a);
         prof_end();
@@ -1081,11 +1082,13 @@ struct Ctx : RankState {
         return v;
     }
 
-    // out[t][k] for t in [0, t_out).  nrest > 1: restart z uses Wg + z*wg_rs, Xin + z*x_rs and writes out + z*out_rs with
-    // row stride ldo (no split over units).  split_need != nullptr: launch nothing, return the elements of tr_part the call needs.
+    // out[t][k] for t in [0, t_out).  per_restart: denomH of a batch handle, one grid slice per restart (TransArgs::tab), with
+    // Nin = Kout = the largest K_r and row stride ldo (no split over units unless R = 1).  split_need != nullptr: launch
+    // nothing, return the elements of tr_part the call needs.
     void launch_transconv(const S *Wg, const S *Xin, S *out, int64_t Nin, int64_t Kout, int64_t Lin,
-                          int64_t ldx, int64_t t_out, int64_t x_cols, int nrest = 1, int64_t wg_rs = 0, int64_t x_rs = 0,
-                          int64_t out_rs = 0, int64_t ldo = 0, size_t *split_need = nullptr) {
+                          int64_t ldx, int64_t t_out, int64_t x_cols, bool per_restart = false, int64_t ldo = 0,
+                          size_t *split_need = nullptr) {
+        const int nrest = per_restart ? (int)R : 1;
         if (t_out <= 0) return;
         // choose TK / kgroups minimising padding
         int best_tk = 8, best_kg = 1;
@@ -1103,7 +1106,7 @@ struct Ctx : RankState {
         TransArgs<S> a;
         a.Wg = Wg; a.Xin = Xin; a.out = out; a.Nin = Nin; a.Kout = Kout; a.Lin = Lin; a.ldx = ldx;
         a.t_out = t_out; a.x_cols = x_cols; a.kgroups = best_kg; a.tgroups = tg;
-        a.wg_rs = wg_rs; a.x_rs = x_rs; a.out_rs = out_rs; a.ldo = ldo ? ldo : Kout;
+        a.ldo = ldo ? ldo : Kout; a.tab = per_restart ? b_tab.p : nullptr;
         const int BTt = tg * 8, Lpad = (int)(cdiv(Lin, 8) * 8);
         const int XW = BTt + Lpad, XWP = XW + XW / 8 + 1, KP = best_kg * best_tk;
         const size_t smem = ((size_t)TR_NC * XWP + (size_t)8 * TR_NC * KP) * sizeof(S);
@@ -1150,11 +1153,11 @@ struct Ctx : RankState {
     DevBuf<S> tr_part;     // partial outputs of the N-split transposed convolution
 
     // out_S / out_D [(l*K+k)*Nin + n] = sum_tau hm(tau-l)[k] Xin[tau][n].  hm = Hs (default: this handle's H) with Kc
-    // components (default K) and row stride ldh (default Kc).  nrest > 1 is the per-restart Gram of a batch handle: Xin and
-    // Hs are both the stacked H, restart z reads its Kc columns at offset z*Kc and writes out + z*out_rs.
+    // components (default K) and row stride ldh (default Kc).  per_restart is the per-restart Gram of a batch handle: Xin and
+    // Hs are both the stacked H, Nin = Kc = the largest K_r, and restart z reads its K_r columns at off_r and writes
+    // out_d + ex_r (CorrArgs::tab).
     void launch_corr(const S *Xin, int64_t Nin, int64_t ldx, int64_t tau_hi, int nsplit, int64_t split_len,
-                     S *out_s, double *out_d, const S *Hs = nullptr, int64_t Kc = 0, int64_t ldh = 0, int nrest = 1,
-                     int64_t out_rs = 0) {
+                     S *out_s, double *out_d, const S *Hs = nullptr, int64_t Kc = 0, int64_t ldh = 0, bool per_restart = false) {
         if (!Hs) Hs = H;
         if (!Kc) Kc = K;
         CorrArgs<S> a;
@@ -1162,28 +1165,31 @@ struct Ctx : RankState {
         a.u_hi = Tl; a.tau_hi = tau_hi; a.split_len = split_len;
         a.ldh = ldh ? ldh : Kc; a.nsplit = nsplit;
         const int64_t n = L * Kc * Nin;
-        a.h_rs = a.x_rs = nrest > 1 ? Kc : 0; a.part_rs = (int64_t)nsplit * n;
+        const BatchRest *tab = per_restart ? b_tab.p : nullptr;
+        const int nrest = per_restart ? (int)R : 1;
+        a.tab = tab;
         const int64_t ngrp = cdiv(L, 8);
         dim3 grid((unsigned)cdiv(Nin, 128), (unsigned)cdiv(Kc * ngrp, CORR_PB), (unsigned)(nsplit * nrest));
         if (Nin == N) prof_begin(PROF_CORR);
         corr_kernel<S><<<grid, dim3(16, 16), 0, stream>>>(a);
         prof_end();
         post_launch();
-        reduce_partials_kernel<S><<<dim3((unsigned)cdiv(n, 256), (unsigned)nrest), 256, 0, stream>>>(corr_part.p, nsplit, n, out_s, out_d, out_rs);
+        reduce_partials_kernel<S><<<dim3((unsigned)cdiv(n, 256), (unsigned)nrest), 256, 0, stream>>>(corr_part.p, nsplit, n, out_s, out_d, tab, L);
         post_launch();
     }
 
-    static GemmRows rows(int64_t ld) { return GemmRows{ld, INT64_MAX, 0, 0}; }
+    static GemmRows rows(int64_t ld) { return GemmRows{ld, INT64_MAX, 0, RANK_NONE}; }
     template <bool TB>
     void launch_gemm(const S *A, const S *B, S *C, int64_t M, int64_t Nn, int64_t Kg, int64_t lda, int64_t ldb,
                      int64_t ldc) {
-        launch_gemm_rows<TB>(A, B, C, M, Nn, Kg, rows(lda), rows(ldb), rows(ldc), 1);
+        launch_gemm_rows<TB>(A, B, C, M, Nn, Kg, rows(lda), rows(ldb), rows(ldc), false);
     }
+    // per_restart: one grid slice per restart of a batch handle, extents for the largest K_r (GemmRows::rank)
     template <bool TB>
     void launch_gemm_rows(const S *A, const S *B, S *C, int64_t M, int64_t Nn, int64_t Kg, GemmRows ra, GemmRows rb, GemmRows rc,
-                          int nrest) {
-        dim3 grid((unsigned)cdiv(Nn, 64), (unsigned)cdiv(M, 64), (unsigned)nrest);
-        gemm_kernel<S, TB><<<grid, 256, 0, stream>>>(A, B, C, M, Nn, Kg, ra, rb, rc);
+                          bool per_restart) {
+        dim3 grid((unsigned)cdiv(Nn, 64), (unsigned)cdiv(M, 64), (unsigned)(per_restart ? R : 1));
+        gemm_kernel<S, TB><<<grid, 256, 0, stream>>>(A, B, C, M, Nn, Kg, ra, rb, rc, per_restart ? b_tab.p : nullptr, L);
         post_launch();
     }
 
@@ -1337,46 +1343,63 @@ struct Ctx : RankState {
         CK(cudaStreamSynchronize(stream));
     }
 
-    // ---------------------------------------------------------------- batch of R MultUpdate restarts (cmf_create_batch)
-    // Restart-stacked layout: H is [t][R*K] with column r*K + k, Wi has rows j' = l*R*K + r*K + k.  numW (mult.jl:32) and numH
-    // (mult.jl:47) are linear in the factor they contract with X, so ONE correlation and ONE transposed convolution with R*K
-    // components serve every restart and X is read once per step.  Everything else is block-diagonal per restart and runs as
-    // one launch with a restart grid index, so the launches of an iteration do not depend on R.
-    int64_t RK() const { return R * K; }
-    int64_t b_exch() const { return L * K * K + (L - 1) * K + 1; }   // doubles of one restart's Gram + H tail block in exch1
-    int64_t b_tail_blocks() const { return cdiv((2 * L - 1) * K, 256); }
+    // ---------------------------------------------------------------- batch of R MultUpdate restarts (cmf_create_batch[_ranks])
+    // Restart-stacked layout: restart r has rank K_r and owns components [off_r, off_r + K_r) of a stacked component axis of
+    // width C = sum K_r (off_r = sum_{q<r} K_q): H is [t][C] with column off_r + k, Wi has rows j' = l*C + off_r + k.  numW
+    // (mult.jl:32) and numH (mult.jl:47) are linear in the factor they contract with X, so ONE correlation and ONE transposed
+    // convolution with C components serve every restart and X is read once per step.  Everything else is block-diagonal per
+    // restart and runs as one launch with a restart grid index, sized for K = max K_r: each block reads its restart's rank and
+    // offsets from the table b_tab, so the launches of an iteration depend neither on R nor on the ranks.  Equal ranks give
+    // off_r = r*K and the offsets of the uniform layout.
+    std::vector<int64_t> b_K;        // K_r of every restart
+    std::vector<BatchRest> b_rest;   // host copy of b_tab (filled by batch_buffers)
+    int64_t b_C = 0;                 // C = sum K_r
+    DevBuf<BatchRest> b_tab;
+    DevBuf<int> b_col;               // [C]: the restart that owns each stacked component
     DevBuf<double> b_reg, b_vals;    // [R][4] = (l1W, l2W, l1H, l2H) per restart; R per-restart scalars
     DevBuf<int> b_active;            // 0 = the restart has converged: the updates leave its factors alone
-    GemmRows b_wrows() const { return GemmRows{N, K, RK() * N, K * N}; }   // W_r: rows l*K + k of restart r
-    GemmRows b_grows() const { return GemmRows{KL(), INT64_MAX, 0, KL() * KL()}; }   // G_r / S2_r: K L x K L blocks
+    int64_t b_exch(int64_t Kr) const { return L * Kr * Kr + (L - 1) * Kr + 1; }   // doubles of one restart's Gram + H tail block in exch1
+    int64_t b_tail_blocks(int64_t Kr) const { return cdiv((2 * L - 1) * Kr, 256); }
+    GemmRows b_wrows() const { return GemmRows{N, INT64_MAX, b_C * N, RANK_W}; }   // W_r: rows l*K_r + k of restart r
+    GemmRows b_grows() const { return GemmRows{0, INT64_MAX, 0, RANK_G}; }         // G_r / S2_r: K_r L x K_r L blocks
 
     // Walks every device buffer of a batch handle: returns the bytes, and allocates them when `alloc` is set (so the footprint
-    // checked before allocating is what is allocated).
+    // checked before allocating is what is allocated).  Lays out the per-restart blocks in b_rest.
     size_t batch_buffers(bool alloc) {
         size_t bytes = 0;
         auto take = [&](auto &buf, int64_t count) {
             bytes += (size_t)count * sizeof(*buf.p);
             if (alloc) buf.alloc((size_t)count);
         };
-        const int64_t hal = L - 1, KLR = L * RK();
-        plan_split(N, Tl + hal, nsplit_w, split_w, RK(), 1);
+        const int64_t hal = L - 1, KLR = L * b_C;
+        plan_split(N, Tl + hal, nsplit_w, split_w, b_C, 1);
         plan_split(K, Tl + hal, nsplit_g, split_g, K, R);
+        b_rest.assign((size_t)R, BatchRest{});
+        BatchRest e{};                                    // running offsets; the totals after the last restart
+        for (int64_t r = 0; r < R; ++r) {
+            const int64_t Kr = b_K[(size_t)r];
+            e.K = Kr;
+            b_rest[(size_t)r] = e;
+            e.off += Kr; e.gs += (Kr * L) * (Kr * L); e.cf += (2 * L - 1) * Kr * Kr; e.ex += b_exch(Kr);
+            e.cp += (int64_t)nsplit_g * L * Kr * Kr; e.tp += b_tail_blocks(Kr) * hal * Kr;
+        }
         size_t tr_need = 0;
-        launch_transconv(nullptr, nullptr, nullptr, N, RK(), L, N, Tl, Tl + hal, 1, 0, 0, 0, 0, &tr_need);
+        launch_transconv(nullptr, nullptr, nullptr, N, b_C, L, N, Tl, Tl + hal, false, 0, &tr_need);
         const int nb = conv_nblocks(0, Tl);
         take(X, (Tl + hal) * N);
-        take(Hbuf, (Tl + 2 * hal) * RK());
+        take(Hbuf, (Tl + 2 * hal) * b_C);
         take(Wi, KLR * N); take(Wtmp, KLR * N); take(numW, KLR * N); take(denW, KLR * N);
-        take(GS, R * KL() * KL());
-        take(Cf, R * (2 * L - 1) * K * K);
-        take(numH, Tl * RK()); take(denH, Tl * RK());
-        take(exch1, R * b_exch());
-        take(corr_part, std::max<int64_t>((int64_t)nsplit_w * KLR * N, R * nsplit_g * KL() * K));
+        take(GS, e.gs);
+        take(Cf, e.cf);
+        take(numH, Tl * b_C); take(denH, Tl * b_C);
+        take(exch1, e.ex);
+        take(corr_part, std::max<int64_t>((int64_t)nsplit_w * KLR * N, e.cp));
         take(loss_part, std::max<int64_t>(2 * nb * R, 4096));
-        take(tail_part, R * b_tail_blocks() * hal * K);
+        take(tail_part, e.tp);
         take(tr_part, (int64_t)tr_need);
         take(scal, 8);
         take(b_reg, 4 * R); take(b_vals, R); take(b_active, R);
+        take(b_tab, R); take(b_col, b_C);
         return bytes;
     }
 
@@ -1386,26 +1409,32 @@ struct Ctx : RankState {
         CK(cudaMemGetInfo(&free_b, &total_b));
         const size_t need = batch_buffers(false);
         if (need > free_b)
-            throw CmfError(CMF_ERR_ARG, "cmf_create_batch: " + std::to_string(R) + " restarts need " + std::to_string(need) +
-                                            " bytes of device memory; " + std::to_string(free_b) + " bytes are free");
+            throw CmfError(CMF_ERR_ARG, "batch handle: " + std::to_string(R) + " restarts need " + std::to_string(need) +
+                                            " bytes of device memory (" + std::to_string(b_C) + " stacked components); " +
+                                            std::to_string(free_b) + " bytes are free");
         CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         own_stream = true;
         H = nullptr;
         batch_buffers(true);
-        H = Hbuf.p + (L - 1) * RK();
+        H = Hbuf.p + (L - 1) * b_C;
         conv_blocks_max = conv_nblocks(0, Tl);
+        std::vector<int> col((size_t)b_C);
+        for (int64_t r = 0; r < R; ++r)
+            for (int64_t k = 0; k < b_K[(size_t)r]; ++k) col[(size_t)(b_rest[(size_t)r].off + k)] = (int)r;
+        CK(cudaMemcpyAsync(b_tab.p, b_rest.data(), (size_t)R * sizeof(BatchRest), cudaMemcpyHostToDevice, stream));
+        CK(cudaMemcpyAsync(b_col.p, col.data(), col.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
         CK(cudaStreamSynchronize(stream));
     }
 
-    // host: R Julia blocks W (K x N x L) and H (K x T); numH stages H (it is recomputed before every use)
+    // host: R Julia blocks W (K_r x N x L) and H (K_r x T), one after another; numH stages H (it is recomputed before every use)
     void batch_set_factors(const void *Wh, const void *Hh) {
         REQUIRE(Wh && Hh, "cmf_set_factors_batch: null pointer");
         CK(cudaMemcpyAsync(Wtmp.p, Wh, Wtmp.n * sizeof(S), cudaMemcpyHostToDevice, stream));
-        w_julia_to_internal<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, RK());
+        w_julia_to_internal<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wtmp.p, Wi.p, K, N, L, b_C, b_tab.p);
         post_launch();
         CK(cudaMemsetAsync(Hbuf.p, 0, Hbuf.n * sizeof(S), stream));
         CK(cudaMemcpyAsync(numH.p, Hh, numH.n * sizeof(S), cudaMemcpyHostToDevice, stream));
-        h_stack_kernel<S><<<(unsigned)cdiv(RK() * Tl, 256), 256, 0, stream>>>(numH.p, H, K, Tl, R, 1);
+        h_stack_kernel<S><<<(unsigned)cdiv(b_C * Tl, 256), 256, 0, stream>>>(numH.p, H, b_C, Tl, b_tab.p, b_col.p, 1);
         post_launch();
         CK(cudaStreamSynchronize(stream));
         have_factors = true;
@@ -1413,12 +1442,12 @@ struct Ctx : RankState {
     void batch_get_factors(void *Wo, void *Ho) {
         REQUIRE(have_factors, "no factors");
         if (Wo) {
-            w_internal_to_julia<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, RK());
+            w_internal_to_julia<S><<<dim3((unsigned)cdiv(KL() * N, 256), (unsigned)R), 256, 0, stream>>>(Wi.p, Wtmp.p, K, N, L, b_C, b_tab.p);
             post_launch();
             CK(cudaMemcpyAsync(Wo, Wtmp.p, Wtmp.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         }
         if (Ho) {
-            h_stack_kernel<S><<<(unsigned)cdiv(RK() * Tl, 256), 256, 0, stream>>>(H, numH.p, K, Tl, R, 0);
+            h_stack_kernel<S><<<(unsigned)cdiv(b_C * Tl, 256), 256, 0, stream>>>(H, numH.p, b_C, Tl, b_tab.p, b_col.p, 0);
             post_launch();
             CK(cudaMemcpyAsync(Ho, numH.p, numH.n * sizeof(S), cudaMemcpyDeviceToHost, stream));
         }
@@ -1430,7 +1459,7 @@ struct Ctx : RankState {
     void batch_scale_partials(double *out) {
         REQUIRE(have_data && have_factors, "cmf_init_scale_partials_batch: data and factors must be set");
         const int nb = conv_nblocks(0, Tl);
-        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p, 0, 0.0, (int)R, 2 * nb);
+        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p, 0, 0.0, true, 2 * nb);
         std::vector<double> hp((size_t)(2 * nb * R));
         CK(cudaMemcpyAsync(hp.data(), loss_part.p, hp.size() * sizeof(double), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
@@ -1443,9 +1472,9 @@ struct Ctx : RankState {
     }
     void batch_scale(const double *s) {
         CK(cudaMemcpyAsync(b_vals.p, s, (size_t)R * sizeof(double), cudaMemcpyHostToDevice, stream));
-        scale_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, S(1), (int64_t)Wi.n, b_vals.p, N, K, RK());
+        scale_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, S(1), (int64_t)Wi.n, b_vals.p, N, b_col.p, b_C);
         post_launch();
-        scale_kernel<S><<<(unsigned)cdiv((int64_t)Hbuf.n, 256), 256, 0, stream>>>(Hbuf.p, S(1), (int64_t)Hbuf.n, b_vals.p, 1, K, RK());
+        scale_kernel<S><<<(unsigned)cdiv((int64_t)Hbuf.n, 256), 256, 0, stream>>>(Hbuf.p, S(1), (int64_t)Hbuf.n, b_vals.p, 1, b_col.p, b_C);
         post_launch();
         CK(cudaStreamSynchronize(stream));
     }
@@ -1455,7 +1484,7 @@ struct Ctx : RankState {
     void batch_loss(double *out) {
         REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
         const int nb = conv_nblocks(0, Tl);
-        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p, 0, 0.0, (int)R, nb);
+        launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p, 0, 0.0, true, nb);
         reduce_scalar(loss_part.p, nb, b_vals.p, (int)R);
         CK(cudaMemcpyAsync(out, b_vals.p, (size_t)R * sizeof(double), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
@@ -1472,43 +1501,42 @@ struct Ctx : RankState {
     // update_motifs! (mult.jl:23-39) of every active restart
     void batch_update_motifs() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, RK(), RK());          // numW, all restarts
-        launch_corr(H, K, RK(), Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p, H, K, RK(), (int)R, b_exch());   // Gram_r
+        launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, b_C, b_C);          // numW, all restarts
+        launch_corr(H, K, b_C, Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p, H, K, b_C, true);   // Gram_r
         if (L > 1) {
-            h_tail_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl,
-                                                                                                   1, RK(), b_exch());
+            h_tail_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(H, exch1.p, K, L, Tl, 1, b_C,
+                                                                                                   b_tab.p);
             post_launch();
         }
-        build_G_kernel<S><<<dim3((unsigned)cdiv(KL() * KL(), 256), (unsigned)R), 256, 0, stream>>>(exch1.p, exch1.p + L * K * K, GS.p,
-                                                                                                    K, L, b_exch());
+        build_G_kernel<S><<<dim3((unsigned)cdiv(KL() * KL(), 256), (unsigned)R), 256, 0, stream>>>(exch1.p, nullptr, GS.p, K, L,
+                                                                                                    b_tab.p);
         post_launch();
-        launch_gemm_rows<false>(GS.p, Wi.p, denW.p, KL(), N, KL(), b_grows(), b_wrows(), b_wrows(), (int)R);   // denomW_r = G_r W_r
+        launch_gemm_rows<false>(GS.p, Wi.p, denW.p, KL(), N, KL(), b_grows(), b_wrows(), b_wrows(), true);     // denomW_r = G_r W_r
         mu_update_kernel<S><<<(unsigned)cdiv((int64_t)Wi.n, 256), 256, 0, stream>>>(Wi.p, numW.p, denW.p, S(0), S(0), (int64_t)Wi.n,
-                                                                                     b_reg.p, b_active.p, N, K, RK());
+                                                                                     b_reg.p, b_active.p, N, b_col.p, b_C);
         post_launch();
     }
 
     // update_feature_maps! (mult.jl:42-58, without the loss) of every active restart
     void batch_update_feature_maps() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        launch_transconv(Wi.p, X.p, numH.p, N, RK(), L, N, Tl, Tl + (L - 1));                                // numH, all restarts
-        launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), (int)R);     // S2_r = W_r W_r'
+        launch_transconv(Wi.p, X.p, numH.p, N, b_C, L, N, Tl, Tl + (L - 1));                                // numH, all restarts
+        launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), true);       // S2_r = W_r W_r'
         lag_table_kernel<S><<<dim3((unsigned)cdiv((2 * L - 1) * K * K, 256), (unsigned)R), 256, 0, stream>>>(GS.p, Cf.p, K, L, K, KL(),
-                                                                                                          KL() * KL());
+                                                                                                          b_tab.p);
         post_launch();
-        launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, RK(), Tl, Tl + 2 * (L - 1), (int)R, (2 * L - 1) * K * K, K, K, RK());
+        launch_transconv(Cf.p, Hbuf.p, denH.p, K, K, 2 * L - 1, b_C, Tl, Tl + 2 * (L - 1), true, b_C);
         if (L > 1) {                                                                                          // truncated tail
-            const int nb = (int)b_tail_blocks();
-            const int64_t prs = (int64_t)nb * (L - 1) * K;
-            denomH_tail_prefix_kernel<S><<<dim3((unsigned)nb, (unsigned)K, (unsigned)R), 256, (size_t)8 * (size_t)(L - 1) * sizeof(double),
-                                           stream>>>(GS.p, H, tail_part.p, K, L, Tl, -(L - 1), K, KL(), RK(), KL() * KL(), prs);
+            denomH_tail_prefix_kernel<S><<<dim3((unsigned)b_tail_blocks(K), (unsigned)K, (unsigned)R), 256,
+                                           (size_t)8 * (size_t)(L - 1) * sizeof(double), stream>>>(GS.p, H, tail_part.p, K, L, Tl,
+                                                                                                    -(L - 1), K, KL(), b_C, b_tab.p);
             post_launch();
             denomH_tail_reduce_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(tail_part.p, denH.p, K, L,
-                                                                                                                Tl, nb, RK(), prs);
+                                                                                                                Tl, 0, b_C, b_tab.p);
             post_launch();
         }
-        mu_update_kernel<S><<<(unsigned)cdiv(Tl * RK(), 256), 256, 0, stream>>>(H, numH.p, denH.p, S(0), S(0), Tl * RK(), b_reg.p + 2,
-                                                                                 b_active.p, 1, K, RK());
+        mu_update_kernel<S><<<(unsigned)cdiv(Tl * b_C, 256), 256, 0, stream>>>(H, numH.p, denH.p, S(0), S(0), Tl * b_C, b_reg.p + 2,
+                                                                                 b_active.p, 1, b_col.p, b_C);
         post_launch();
     }
 
@@ -1553,7 +1581,7 @@ struct Ctx : RankState {
             else { tc_split_H(true); tc_split_H(false); tc_gram(); }
         }
         if (L > 1) {
-            h_tail_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl, is_last ? 1 : 0, K, 0);
+            h_tail_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(H, exch1.p + L * K * K, K, L, Tl, is_last ? 1 : 0, K);
             post_launch();
         }
     }
@@ -1616,9 +1644,9 @@ struct Ctx : RankState {
         const size_t need = (size_t)nb * (size_t)(L - 1) * (size_t)K;
         if (tail_part.n < need) tail_part.alloc(need);
         denomH_tail_prefix_kernel<S><<<dim3((unsigned)nb, (unsigned)K), 256, smem, stream>>>(GS.p, H, tail_part.p, K, L, Tl, -(L - 1), s2_ks, s2_ld,
-                                                                                            K, 0, 0);
+                                                                                            K);
         post_launch();
-        denomH_tail_reduce_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(tail_part.p, denH.p, K, L, Tl, nb, K, 0);
+        denomH_tail_reduce_kernel<S><<<(unsigned)cdiv((L - 1) * K, 256), 256, 0, stream>>>(tail_part.p, denH.p, K, L, Tl, nb, K);
         post_launch();
     }
 
@@ -1997,10 +2025,11 @@ struct Ctx : RankState {
 };
 
 // One rank context, initialised on `device`.  S is chosen by the caller from dtype (with_dtype); the dtype check stays here
-// so that the checks run, and fail, in the same order for every create call.
+// so that the checks run, and fail, in the same order for every create call.  A batch handle passes the rank of every restart
+// (`ranks`, non-empty) and K = their maximum.
 template <typename S>
 std::unique_ptr<Ctx<S>> make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg,
-                                 int device, int64_t R = 0) {
+                                 int device, const std::vector<int64_t> &ranks = {}) {
     REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
     REQUIRE(L <= T, "need L <= T (src/common.jl:28-31)");
     REQUIRE(0 <= t0 && t0 < t1 && t1 <= T, "bad shard range");
@@ -2020,7 +2049,9 @@ std::unique_ptr<Ctx<S>> make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, i
     c->N = N; c->T = T; c->t0 = t0; c->t1 = t1; c->Tl = t1 - t0; c->K = K; c->L = L;
     c->alg = alg; c->device = device;
     c->is_first = (t0 == 0); c->is_last = (t1 == T);
-    c->R = R;
+    c->R = (int64_t)ranks.size();
+    c->b_K = ranks;
+    c->b_C = std::accumulate(ranks.begin(), ranks.end(), (int64_t)0);
     c->init();
     return c;
 }
@@ -2516,8 +2547,25 @@ void batch_handle(cmf_handle h) { REQUIRE(h && first(h).R > 0, "not a batch hand
 
 // a handle of one rank context (make_ctx's checks)
 cmf_ctx *make_handle(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device,
-                     int64_t R = 0) {
-    return with_dtype(dtype, [&](auto s) { return handle_of(make_ctx<decltype(s)>(N, T, t0, t1, K, L, dtype, alg, device, R)); });
+                     const std::vector<int64_t> &ranks = {}) {
+    return with_dtype(dtype, [&](auto s) { return handle_of(make_ctx<decltype(s)>(N, T, t0, t1, K, L, dtype, alg, device, ranks)); });
+}
+
+// cmf_create_batch and cmf_create_batch_ranks (after their checks of R): restart r has rank ranks[r].  Every check runs
+// before any device query.
+cmf_ctx *make_batch(int64_t N, int64_t T, const std::vector<int64_t> &ranks, int64_t L, int dtype, int alg, int device) {
+    REQUIRE(alg == CMF_MULT || alg == CMF_HALS || alg == CMF_PGD, "alg must be 0 (mult), 1 (hals) or 2 (pgd)");
+    if (alg != CMF_MULT)
+        throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts serve MultUpdate only (HALS sweeps run sequentially per restart; PGD is not batched)");
+    REQUIRE(N >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
+    for (size_t r = 0; r < ranks.size(); ++r) {
+        REQUIRE(ranks[r] >= 1, "dimensions must be positive: K[" + std::to_string(r) + "] = " + std::to_string(ranks[r]));
+        REQUIRE(ranks[r] <= 4 * 65535, "R*K too large for one launch grid: K[" + std::to_string(r) + "] = " + std::to_string(ranks[r]));
+    }
+    const int64_t C = std::accumulate(ranks.begin(), ranks.end(), (int64_t)0), Kmax = *std::max_element(ranks.begin(), ranks.end());
+    REQUIRE(C * cdiv(L, 8) <= (int64_t)CORR_PB * 65535 && C <= 4 * 65535, "R*K too large for one launch grid (the ranks of all restarts add up to " + std::to_string(C) + ")");
+    if (L > 769) throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts need L <= 769");
+    return make_handle(N, T, 0, T, Kmax, L, dtype, alg, device, ranks);
 }
 
 }  // namespace
@@ -2966,14 +3014,18 @@ int cmf_create_batch(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L
     return guarded([&] {
         REQUIRE(out != nullptr, "null output pointer");
         REQUIRE(R >= 1 && R <= 32768, "R (restarts) must be in 1..32768");
-        REQUIRE(alg == CMF_MULT || alg == CMF_HALS || alg == CMF_PGD, "alg must be 0 (mult), 1 (hals) or 2 (pgd)");
-        if (alg != CMF_MULT)
-            throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts serve MultUpdate only (HALS sweeps run sequentially per restart; PGD is not batched)");
-        REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
-        REQUIRE(R * K * cdiv(L, 8) <= (int64_t)CORR_PB * 65535 && R * K <= 4 * 65535, "R*K too large for one launch grid");
-        if (L > 769) throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts need L <= 769");
         DevRestore g;
-        *out = make_handle(N, T, 0, T, K, L, dtype, alg, device, R);
+        *out = make_batch(N, T, std::vector<int64_t>((size_t)R, K), L, dtype, alg, device);
+    });
+}
+int cmf_create_batch_ranks(cmf_handle *out, int64_t N, int64_t T, const int64_t *K, int64_t L, int dtype, int alg, int64_t R,
+                           int device) {
+    return guarded([&] {
+        REQUIRE(out != nullptr, "null output pointer");
+        REQUIRE(K != nullptr, "null rank array K");
+        REQUIRE(R >= 1 && R <= 32768, "R (restarts) must be in 1..32768");
+        DevRestore g;
+        *out = make_batch(N, T, std::vector<int64_t>(K, K + R), L, dtype, alg, device);
     });
 }
 int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H) {

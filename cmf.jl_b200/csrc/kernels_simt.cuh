@@ -55,9 +55,21 @@ __global__ void reduce_sum_kernel(const double *__restrict__ in, int64_t n, doub
     if (threadIdx.x == 0) out[blockIdx.x] = s;
 }
 
-// Restart r of a batch handle owns components [r*K, r*K + K) of the stacked component axis (width RK = R*K).  For an array
-// whose component index is (i / inner) % RK -- W in the internal layout (inner = N), H (inner = 1) -- this is r.
-__device__ __forceinline__ int64_t restart_of(int64_t i, int64_t inner, int64_t K, int64_t RK) { return ((i / inner) % RK) / K; }
+// Restart r of a batch handle: its rank K_r, the first of its components [off, off + K_r) on the stacked component axis
+// (width C = sum K_r), and where its block starts in each per-restart buffer (elements).  Launches with a restart grid index
+// read entry blockIdx.z (or .y); single handles pass no table and are restart 0 at offset 0.
+struct BatchRest {
+    int64_t K, off;
+    int64_t gs;   // G_r / S2_r (K_r L x K_r L) in GS
+    int64_t cf;   // lag table (2L-1) x K_r x K_r in Cf
+    int64_t ex;   // Gram (L K_r^2) + H tail ((L-1) K_r) + 1 in exch1
+    int64_t cp;   // the Gram's nsplit partials (nsplit L K_r^2) in corr_part
+    int64_t tp;   // denomH tail partials (nb_r (L-1) K_r) in tail_part
+};
+
+// Restart of element i of an array whose component index is (i / inner) % C -- W in the internal layout (inner = N), H
+// (inner = 1): col_rest[c] is the restart that owns stacked component c.
+__device__ __forceinline__ int64_t restart_of(int64_t i, int64_t inner, const int *col_rest, int64_t C) { return col_rest[(i / inner) % C]; }
 
 // ------------------------------------------------------------------------------------------
 // conv (+ residual, + loss):   est[t][n] = sum_{l<L,k<K} Wi[l*K+k][n] * H[t-l][k]
@@ -87,9 +99,10 @@ struct ConvArgs {
     int KC;               // components staged per H window
     const S *mask;        // flags 32|64: optional mask [t][N] (nullptr = all ones)
     int lossf;            // flags 32|64: 0 SquareLoss, 1 AbsoluteLoss
-    // restart blockIdx.z of a batch handle: W rows (l*ldw + k) and H columns t*ldh + k from Wi + z*w_rs and H + z*h_rs,
-    // partials from partial + z*part_rs (single handles: ldw = ldh = K, one z)
-    int64_t ldw, ldh, w_rs, h_rs, part_rs;
+    // restart z = blockIdx.z of a batch handle (tab != nullptr): K = tab[z].K, W rows (l*ldw + k) and H columns t*ldh + k from
+    // Wi + tab[z].off*N and H + tab[z].off, partials from partial + z*part_rs (single handles: ldw = ldh = K, one z)
+    int64_t ldw, ldh, part_rs;
+    const BatchRest *tab;
 };
 
 __device__ __forceinline__ uint64_t mix64(uint64_t z) {
@@ -114,7 +127,8 @@ template <typename S, int TN, int TT, int TY>
 __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
     constexpr int BN = 16 * TN, BT = TY * TT;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int64_t N = a.N, K = a.K, L = a.L;
+    const int64_t N = a.N, K = a.tab ? a.tab[blockIdx.z].K : a.K, L = a.L;
+    const int64_t off = a.tab ? a.tab[blockIdx.z].off : 0;
     const int Lpad = (int)((L + 7) / 8 * 8);
     const int HW = BT + Lpad - 1;
     S *Hs = reinterpret_cast<S *>(smem_raw);            // [KC][HW]
@@ -125,7 +139,7 @@ __global__ void __launch_bounds__(16 * TY) conv_kernel(ConvArgs<S> a) {
     const int tid = ty * 16 + tx, nthr = 16 * TY;
     const int64_t n0 = (int64_t)blockIdx.y * BN;          // grid.x runs over time tiles (can be > 65535)
     const int64_t t0 = a.t_lo + (int64_t)blockIdx.x * BT;
-    const S *Wr = a.Wi + (int64_t)blockIdx.z * a.w_rs, *Hr = a.H + (int64_t)blockIdx.z * a.h_rs;
+    const S *Wr = a.Wi + off * N, *Hr = a.H + off;
     double *partial = a.partial ? a.partial + (int64_t)blockIdx.z * a.part_rs : nullptr;
 
     S acc[TT][TN];
@@ -247,8 +261,10 @@ struct TransArgs {
     int64_t n_chunk;      // units summed by one CTA (blockIdx.z % nsplit selects the chunk; a multiple of TR_NC); Nin rounded up = no split
     int64_t part_stride;  // elements between the partial outputs of consecutive chunks (0 = no split: `out` is the result)
     int nsplit;           // chunks per restart: blockIdx.z / nsplit is the restart (single handles: one restart)
-    int64_t wg_rs, x_rs, out_rs;   // per-restart offsets of Wg, Xin and out
-    int64_t ldo;          // row stride of out (Kout, or R*K when restarts write their columns of a stacked array)
+    int64_t ldo;          // row stride of out (Kout, or C when restarts write their columns of a stacked array)
+    // denomH of a batch handle (tab != nullptr): restart z has Nin = Kout = tab[z].K and reads Wg + tab[z].cf (its lag table)
+    // and Xin + tab[z].off, writes out + tab[z].off; Nin / Kout above are the largest K_r (the grid's extent)
+    const BatchRest *tab;
 };
 
 // out[i] = sum_z part[z * stride + i] in the fixed order z = 0, 1, ... (deterministic; the N-split of transconv_kernel)
@@ -280,7 +296,15 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
     const int64_t t0 = (int64_t)blockIdx.x * BT;
     const int64_t kb = (int64_t)blockIdx.y * KP;     // first k of this block
     const int64_t rs = blockIdx.z / a.nsplit, zs = blockIdx.z % a.nsplit;
-    const S *Wg = a.Wg + rs * a.wg_rs, *Xin = a.Xin + rs * a.x_rs;
+    const S *Wg = a.Wg, *Xin = a.Xin;
+    S *out = a.out;
+    int64_t Nin = a.Nin, Kout = a.Kout;
+    if (a.tab) {
+        const BatchRest r = a.tab[rs];
+        Nin = Kout = r.K;
+        if (kb >= Kout) return;                      // past this restart's components
+        Wg += r.cf; Xin += r.off; out += r.off;
+    }
 
     S acc[TT][TK];
 #pragma unroll
@@ -288,7 +312,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
 #pragma unroll
         for (int i = 0; i < TK; ++i) acc[j][i] = S(0);
 
-    const int64_t n_lo = zs * a.n_chunk, n_hi = min(a.Nin, n_lo + a.n_chunk);
+    const int64_t n_lo = zs * a.n_chunk, n_hi = min(Nin, n_lo + a.n_chunk);
     for (int64_t nc0 = n_lo; nc0 < n_hi; nc0 += TR_NC) {
         __syncthreads();
         // stage X window (transposed): Xs[n][phys(i)] = Xin[(t0+i)*ldx + nc0 + n]
@@ -306,8 +330,8 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
                 const int n = idx % TR_NC, k = (idx / TR_NC) % KP, dl = idx / (TR_NC * KP);
                 const int64_t l = lc0 + dl;
                 S v = S(0);
-                if (l < a.Lin && kb + k < a.Kout && nc0 + n < n_hi)
-                    v = Wg[((l * a.Kout) + kb + k) * a.Nin + nc0 + n];
+                if (l < a.Lin && kb + k < Kout && nc0 + n < n_hi)
+                    v = Wg[((l * Kout) + kb + k) * Nin + nc0 + n];
                 Ws[((size_t)dl * TR_NC + n) * KP + k] = v;
             }
             __syncthreads();
@@ -345,7 +369,7 @@ __global__ void __launch_bounds__(256) transconv_kernel(TransArgs<S> a) {
 #pragma unroll
         for (int i = 0; i < TK; ++i) {
             const int64_t k = kb + kg * TK + i;
-            if (k < a.Kout) a.out[rs * a.out_rs + zs * a.part_stride + t * a.ldo + k] = acc[j][i];
+            if (k < Kout) out[zs * a.part_stride + t * a.ldo + k] = acc[j][i];
         }
     }
 }
@@ -365,9 +389,11 @@ struct CorrArgs {
     int64_t u_hi;    // owned columns (H valid for u in [0,u_hi))
     int64_t tau_hi;  // Xin valid for tau in [0, tau_hi)
     int64_t split_len;
-    int64_t ldh;     // row stride of H (K, or R*K for the per-restart Gram of a batch handle)
+    int64_t ldh;     // row stride of H (K, or C for the per-restart Gram of a batch handle)
     int nsplit;      // splits per restart: blockIdx.z / nsplit is the restart (single handles: one restart)
-    int64_t h_rs, x_rs, part_rs;   // per-restart offsets of H, Xin and part
+    // the per-restart Gram of a batch handle (tab != nullptr): restart z has Nin = K = tab[z].K, reads H + tab[z].off and
+    // Xin + tab[z].off and writes part + tab[z].cp; Nin / K above are the largest K_r (the grid's extent)
+    const BatchRest *tab;
 };
 
 constexpr int CORR_BTAU = 32;
@@ -383,13 +409,21 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
     const int64_t n0 = (int64_t)blockIdx.x * BN;
     const int64_t p = (int64_t)blockIdx.y * CORR_PB + ty;
     const int64_t ngrp = (a.L + 7) / 8;
-    const bool pvalid = p < a.K * ngrp;
-    const int64_t k = pvalid ? p % a.K : 0, l0 = pvalid ? (p / a.K) * 8 : 0;
     const int64_t rs = blockIdx.z / a.nsplit, zs = blockIdx.z % a.nsplit;
-    const S *Hr = a.H + rs * a.h_rs, *Xr = a.Xin + rs * a.x_rs;
+    const S *Hr = a.H, *Xr = a.Xin;
+    double *part = a.part;
+    int64_t K = a.K, Nin = a.Nin;
+    if (a.tab) {
+        const BatchRest r = a.tab[rs];
+        K = Nin = r.K;
+        if (n0 >= Nin || (int64_t)blockIdx.y * CORR_PB >= K * ngrp) return;   // past this restart's components
+        Hr += r.off; Xr += r.off; part += r.cp;
+    }
+    const bool pvalid = p < K * ngrp;
+    const int64_t k = pvalid ? p % K : 0, l0 = pvalid ? (p / K) * 8 : 0;
     const int64_t tau_a = zs * a.split_len;
     const int64_t tau_b = min(a.tau_hi, tau_a + a.split_len);
-    double *part = a.part + rs * a.part_rs + (size_t)zs * (size_t)(a.L * a.K * a.Nin);
+    part += (size_t)zs * (size_t)(a.L * K * Nin);
 
     S acc[8][TN];
 #pragma unroll
@@ -408,8 +442,8 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
 #pragma unroll
             for (int j = 0; j < TN; ++j) {
                 const int64_t n = n0 + tx * TN + j;
-                if (n >= a.Nin) continue;
-                double *d = part + (l * a.K + k) * a.Nin + n;
+                if (n >= Nin) continue;
+                double *d = part + (l * K + k) * Nin + n;
                 *d = flushed_once ? (*d + (double)acc[i][j]) : (double)acc[i][j];
                 acc[i][j] = S(0);
             }
@@ -423,15 +457,15 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
             const int n = idx % BN, dt = idx / BN;
             const int64_t tau = tau0 + dt;
             S v = S(0);
-            if (tau < tau_b && n0 + n < a.Nin) v = Xr[tau * a.ldx + n0 + n];
+            if (tau < tau_b && n0 + n < Nin) v = Xr[tau * a.ldx + n0 + n];
             Xs[dt][n] = v;
         }
         for (int idx = tid; idx < CORR_PB * HWN; idx += 256) {
             const int i = idx % HWN, pp = idx / HWN;
             const int64_t q = (int64_t)blockIdx.y * CORR_PB + pp;
             S v = S(0);
-            if (q < a.K * ngrp) {
-                const int64_t kk = q % a.K, ll0 = (q / a.K) * 8;
+            if (q < K * ngrp) {
+                const int64_t kk = q % K, ll0 = (q / K) * 8;
                 const int64_t u = tau0 - ll0 - 7 + i;
                 if (u >= 0 && u < a.u_hi) v = Hr[u * a.ldh + kk];
             }
@@ -465,16 +499,20 @@ __global__ void __launch_bounds__(256) corr_kernel(CorrArgs<S> a) {
     flush();
 }
 
-// out[i] = (S) sum_s part[s][i]   (fixed order -> deterministic); restart blockIdx.y reads part + y*nsplit*n and writes
-// out + y*out_rs
+// out[i] = (S) sum_s part[s][i]   (fixed order -> deterministic).  The per-restart Gram of a batch handle (tab != nullptr):
+// restart blockIdx.y has n = L K_r^2, reads part + tab[y].cp and writes out_d + tab[y].ex
 template <typename S>
 __global__ void reduce_partials_kernel(const double *__restrict__ part, int nsplit, int64_t n,
-                                       S *__restrict__ out, double *__restrict__ out_d, int64_t out_rs = 0) {
+                                       S *__restrict__ out, double *__restrict__ out_d, const BatchRest *tab = nullptr, int64_t L = 0) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        n = L * r.K * r.K;
+        part += r.cp;
+        if (out) out += r.ex;
+        if (out_d) out_d += r.ex;
+    }
     if (i >= n) return;
-    part += (int64_t)blockIdx.y * nsplit * n;
-    if (out) out += (int64_t)blockIdx.y * out_rs;
-    if (out_d) out_d += (int64_t)blockIdx.y * out_rs;
     double s = 0.0;
     for (int sp = 0; sp < nsplit; ++sp) s += part[(size_t)sp * n + i];
     if (out) out[i] = (S)s;
@@ -486,25 +524,43 @@ __global__ void reduce_partials_kernel(const double *__restrict__ part, int nspl
 //   64x64 tile, BK 16, 256 threads, 4x4 micro-tile.  Used for G*Wi and Wi*Wi' (<1% of the FLOPs).
 //   Each operand's rows are addressed through a GemmRows; blockIdx.z is the restart of a batch handle.
 // ------------------------------------------------------------------------------------------
-// Row j of a GEMM operand starts at (j / grp) * ldg + (j % grp) * ld, restart z at z * rs.  Row-major with leading dimension
-// ld: grp = INT64_MAX.  W_r of a batch handle, rows j = l*K + k at (l*R*K + r*K + k)*N: grp = K, ldg = R*K*N, ld = N, rs = K*N.
+// Row j of a GEMM operand starts at (j / grp) * ldg + (j % grp) * ld.  Row-major with leading dimension ld: grp = INT64_MAX.
+// Operands of a batch handle take restart z = blockIdx.z from the table (rank != RANK_NONE):
+//   RANK_W  W_r, rows j = l*K_r + k at (l*C + off_r + k)*N: ld = N, ldg = C*N, grp = K_r, start off_r*N;
+//   RANK_G  G_r / S2_r, a K_r L x K_r L row-major block at gs_r: ld = K_r L.
+// Every extent an operand spans with K_r L rows or columns is K_r L for restart z; M, Nn, Kg passed in are the largest.
+enum { RANK_NONE = 0, RANK_W = 1, RANK_G = 2 };
 struct GemmRows {
-    int64_t ld, grp, ldg, rs;
+    int64_t ld, grp, ldg;
+    int rank;
     __device__ __forceinline__ int64_t at(int64_t j) const { return (j / grp) * ldg + (j % grp) * ld; }
+    // this operand of restart r: sets its row layout and returns its start
+    __device__ __forceinline__ int64_t of(const BatchRest &r, int64_t L) {
+        if (rank == RANK_W) { grp = r.K; return r.off * ld; }
+        ld = r.K * L;
+        return r.gs;
+    }
 };
 
 template <typename S, bool TRANSB>
 __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, const S *__restrict__ B,
                                                    S *__restrict__ C, int64_t M, int64_t Nn,
-                                                   int64_t Kg, GemmRows ra, GemmRows rb, GemmRows rc) {
+                                                   int64_t Kg, GemmRows ra, GemmRows rb, GemmRows rc,
+                                                   const BatchRest *tab = nullptr, int64_t L = 0) {
     constexpr int BM = 64, BNt = 64, BK = 16;
     __shared__ S As[BK][BM + 1];
     __shared__ S Bs[BK][BNt + 1];
     const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
     const int64_t m0 = (int64_t)blockIdx.y * BM, c0 = (int64_t)blockIdx.x * BNt;
-    A += (int64_t)blockIdx.z * ra.rs;
-    B += (int64_t)blockIdx.z * rb.rs;
-    C += (int64_t)blockIdx.z * rc.rs;
+    if (tab) {
+        const BatchRest r = tab[blockIdx.z];
+        const int64_t kl = r.K * L;
+        int64_t &Brows = TRANSB ? Nn : Kg, &Bcols = TRANSB ? Kg : Nn;
+        if (ra.rank) { A += ra.of(r, L); M = kl; if (ra.rank == RANK_G) Kg = kl; }
+        if (rb.rank) { B += rb.of(r, L); Brows = kl; if (rb.rank == RANK_G) Bcols = kl; }
+        if (rc.rank) { C += rc.of(r, L); M = kl; if (rc.rank == RANK_G) Nn = kl; }
+        if (m0 >= M || c0 >= Nn) return;                 // past this restart's block
+    }
     S acc[4][4];
 #pragma unroll
     for (int i = 0; i < 4; ++i)
@@ -557,13 +613,18 @@ __global__ void __launch_bounds__(256) gemm_kernel(const S *__restrict__ A, cons
 // G = Htilde Htilde'  from the Toeplitz part Rg[d][k][k'] and the tail Ht[c][k] = H[T-(L-1)+c][k]
 //   G[(l,k)][(l',k')] = (l>=l' ? Rg[l-l'][k][k'] : Rg[l'-l][k'][k]) - sum_{i<min(l,l')} Ht[L-1-l+i][k] Ht[L-1-l'+i][k']
 // ------------------------------------------------------------------------------------------
+// Batch handles (tab != nullptr): Rg is the base of exch1; restart y = blockIdx.y has K = K_r, its Gram at Rg + ex_r, its tail
+// right after it, and G_r at G + gs_r (Ht unused).
 template <typename S>
 __global__ void build_G_kernel(const double *__restrict__ Rg, const double *__restrict__ Ht,
-                               S *__restrict__ G, int64_t K, int64_t L, int64_t rg_rs = 0) {
+                               S *__restrict__ G, int64_t K, int64_t L, const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = r.K; Rg += r.ex; Ht = Rg + L * K * K; G += r.gs;
+    }
     const int64_t KL = K * L;
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= KL * KL) return;
-    Rg += (int64_t)blockIdx.y * rg_rs; Ht += (int64_t)blockIdx.y * rg_rs; G += (int64_t)blockIdx.y * KL * KL;   // restart y
     const int64_t jp = idx % KL, j = idx / KL;
     const int64_t k = j % K, l = j / K, kp = jp % K, lp = jp / K;
     double g = (l >= lp) ? Rg[((l - lp) * K + k) * K + kp] : Rg[((lp - l) * K + kp) * K + k];
@@ -621,13 +682,16 @@ __global__ void s2_dot_G_diag_kernel(const S *__restrict__ S2, int64_t Ks, int64
 // Cf[(d+L-1)][k][k'] = sum_{l, 0<=l-d<L} S2[(l,k)][(l-d,k')]      (S2 = W W' over the unfolded rows)
 // S2 is addressed as S2[(l*Ks + k) * ld + (l'*Ks + k')]: (Ks, ld) = (K, K*L) for the SIMT product and
 // (Kp, rows_u) for the tensor-core product over the padded rows.
-// Restart blockIdx.y of a batch handle: S2 + y*s2_rs, Cf + y*(2L-1)*K*K.
+// Restart y = blockIdx.y of a batch handle (tab != nullptr): K = Ks = K_r, ld = K_r L, S2 + gs_r, Cf + cf_r.
 template <typename S>
 __global__ void lag_table_kernel(const S *__restrict__ S2, S *__restrict__ Cf, int64_t K, int64_t L, int64_t Ks, int64_t ld,
-                                 int64_t s2_rs = 0) {
+                                 const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = Ks = r.K; ld = r.K * L; S2 += r.gs; Cf += r.cf;
+    }
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (2 * L - 1) * K * K) return;
-    S2 += (int64_t)blockIdx.y * s2_rs; Cf += (int64_t)blockIdx.y * (2 * L - 1) * K * K;
     const int64_t kp = idx % K, k = (idx / K) % K, d = idx / (K * K) - (L - 1);
     double s = 0.0;
     for (int64_t l = (d > 0 ? d : 0); l < L && l - d < L; ++l) s += (double)S2[(l * Ks + k) * ld + (l - d) * Ks + kp];
@@ -671,16 +735,22 @@ __global__ void __launch_bounds__(256) denomH_tail_kernel(const S *__restrict__ 
 // in a register while w grows, and den[Tl-w][k] = sum_{d,k'} C_w[d][k][k'] H[Tl-w+d][k'].  Warp sums go to shared
 // memory, block sums to part[block][c][k] (c = L-1-w, the tail column index); denomH_tail_reduce_kernel adds the blocks
 // in order (deterministic).  grid (ceil((2L-1)K / 256), K, restarts), dynamic smem 8*(L-1) doubles.  Restart z of a batch
-// handle reads S2 + z*s2_rs and H + z*K (row stride ldh) and writes part + z*part_rs.
+// handle (tab != nullptr) has K = Ks = K_r, ld = K_r L, reads S2 + gs_r and H + off_r (row stride ldh) and writes part + tp_r;
+// the grid is sized for the largest K_r and the blocks past restart z's return at once.
 template <typename S>
 __global__ void __launch_bounds__(256) denomH_tail_prefix_kernel(const S *__restrict__ S2, const S *__restrict__ H,
                                                                   double *__restrict__ part, int64_t K, int64_t L, int64_t Tl,
                                                                   int64_t h_lo, int64_t Ks, int64_t ld, int64_t ldh,
-                                                                  int64_t s2_rs, int64_t part_rs) {
+                                                                  const BatchRest *tab = nullptr) {
     extern __shared__ double tail_sm[];                 // [8 warps][L-1]
-    S2 += (int64_t)blockIdx.z * s2_rs; H += (int64_t)blockIdx.z * K; part += (int64_t)blockIdx.z * part_rs;
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t k = blockIdx.y;
+    if (tab) {
+        const BatchRest r = tab[blockIdx.z];
+        K = Ks = r.K; ld = r.K * L;
+        if (k >= K || (int64_t)blockIdx.x * blockDim.x >= (2 * L - 1) * K) return;
+        S2 += r.gs; H += r.off; part += r.tp;
+    }
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = e < (2 * L - 1) * K;
     const int64_t dq = live ? e / K : 0, kp = live ? e - dq * K : 0;
     const int64_t d = dq - (L - 1);
@@ -725,13 +795,17 @@ __global__ void __launch_bounds__(256) denomH_tail_prefix_kernel(const S *__rest
     }
 }
 
-// restart blockIdx.y: part + y*part_rs, den + y*K with row stride ldd
+// Restart y = blockIdx.y of a batch handle (tab != nullptr): K = K_r, part + tp_r with the ceil((2L-1) K_r / 256) blocks of
+// its prefix launch, den + off_r with row stride ldd.
 template <typename S>
 __global__ void denomH_tail_reduce_kernel(const double *__restrict__ part, S *__restrict__ den, int64_t K, int64_t L, int64_t Tl,
-                                          int nblocks, int64_t ldd, int64_t part_rs) {
+                                          int nblocks, int64_t ldd, const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = r.K; nblocks = (int)(((2 * L - 1) * K + 255) / 256); part += r.tp; den += r.off;
+    }
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;     // c * K + k
     if (i >= (L - 1) * K) return;
-    part += (int64_t)blockIdx.y * part_rs; den += (int64_t)blockIdx.y * K;
     const int64_t c = i / K, k = i - c * K, t = Tl - (L - 1) + c;
     if (t < 0) return;
     double s = 0.0;
@@ -743,16 +817,17 @@ __global__ void denomH_tail_reduce_kernel(const double *__restrict__ part, S *__
 // element-wise pieces
 // ------------------------------------------------------------------------------------------
 // src/algs/mult.jl:37-38 / :51-52   x <- max(eps, x * num / (den + l1 + 2*l2*x + eps))
-// Batch handles pass reg != nullptr: restart r = restart_of(i, inner, K, RK) takes l1 = reg[4r], l2 = reg[4r+1] and is
-// left alone while active[r] == 0 (a converged restart is frozen).
+// Batch handles pass reg != nullptr: restart r = restart_of(i, inner, col_rest, C) takes l1 = reg[4r], l2 = reg[4r+1] and
+// is left alone while active[r] == 0 (a converged restart is frozen).
 template <typename S>
 __global__ void mu_update_kernel(S *__restrict__ x, const S *__restrict__ num, const S *__restrict__ den,
                                  S l1, S l2, int64_t n, const double *__restrict__ reg = nullptr,
-                                 const int *__restrict__ active = nullptr, int64_t inner = 1, int64_t K = 1, int64_t RK = 1) {
+                                 const int *__restrict__ active = nullptr, int64_t inner = 1, const int *__restrict__ col_rest = nullptr,
+                                 int64_t C = 1) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     if (reg) {
-        const int64_t r = restart_of(i, inner, K, RK);
+        const int64_t r = restart_of(i, inner, col_rest, C);
         if (!active[r]) return;
         l1 = (S)reg[4 * r];
         l2 = (S)reg[4 * r + 1];
@@ -788,13 +863,13 @@ __global__ void __launch_bounds__(256) mu_update_vec4_kernel(float4 *__restrict_
     }
 }
 
-// s_r != nullptr (batch handles): restart restart_of(i, inner, K, RK) is scaled by s_r[r]
+// s_r != nullptr (batch handles): restart restart_of(i, inner, col_rest, C) is scaled by s_r[r]
 template <typename S>
 __global__ void scale_kernel(S *__restrict__ x, S s, int64_t n, const double *__restrict__ s_r = nullptr, int64_t inner = 1,
-                             int64_t K = 1, int64_t RK = 1) {
+                             const int *__restrict__ col_rest = nullptr, int64_t C = 1) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    if (s_r) s = (S)s_r[restart_of(i, inner, K, RK)];
+    if (s_r) s = (S)s_r[restart_of(i, inner, col_rest, C)];
     x[i] *= s;
 }
 
@@ -810,32 +885,43 @@ __global__ void dot_partial_kernel(const S *__restrict__ a, const S *__restrict_
     if (threadIdx.x == 0) partial[blockIdx.x] = s;
 }
 
-// Julia W[k + K*(n + N*l)]  <->  Wi[(l*ldk + k)*N + n]; ldk = K, or R*K for the stacked W of a batch handle, whose restart
-// blockIdx.y has its Julia block at Wj + y*K*N*L and its rows at Wi + y*K*N
+// Julia W[k + K*(n + N*l)]  <->  Wi[(l*ldk + k)*N + n]; ldk = K, or C for the stacked W of a batch handle (tab != nullptr),
+// whose restart y = blockIdx.y has K = K_r, its Julia block at Wj + off_r*N*L and its rows at Wi + off_r*N
 template <typename S>
-__global__ void w_julia_to_internal(const S *__restrict__ Wj, S *__restrict__ Wi, int64_t K, int64_t N, int64_t L, int64_t ldk) {
+__global__ void w_julia_to_internal(const S *__restrict__ Wj, S *__restrict__ Wi, int64_t K, int64_t N, int64_t L, int64_t ldk,
+                                    const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = r.K; Wj += r.off * N * L; Wi += r.off * N;
+    }
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= K * N * L) return;
-    Wj += (int64_t)blockIdx.y * K * N * L; Wi += (int64_t)blockIdx.y * K * N;
     const int64_t n = idx % N, k = (idx / N) % K, l = idx / (N * K);
     Wi[(l * ldk + k) * N + n] = Wj[k + K * (n + N * l)];
 }
 template <typename S>
-__global__ void w_internal_to_julia(const S *__restrict__ Wi, S *__restrict__ Wj, int64_t K, int64_t N, int64_t L, int64_t ldk) {
+__global__ void w_internal_to_julia(const S *__restrict__ Wi, S *__restrict__ Wj, int64_t K, int64_t N, int64_t L, int64_t ldk,
+                                    const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = r.K; Wj += r.off * N * L; Wi += r.off * N;
+    }
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= K * N * L) return;
-    Wj += (int64_t)blockIdx.y * K * N * L; Wi += (int64_t)blockIdx.y * K * N;
     const int64_t k = idx % K, n = (idx / K) % N, l = idx / (K * N);
     Wj[idx] = Wi[(l * ldk + k) * N + n];
 }
 
-// H of a batch handle: R host blocks K x T (blk[r][t][k]) <-> the stacked device array st[t][r*K + k]
+// H of a batch handle: R host blocks K_r x T one after another (restart r's [t][k] at T*off_r + t*K_r + k) <-> the stacked
+// device array st[t][off_r + k] of C = sum K_r columns
 template <typename S>
-__global__ void h_stack_kernel(const S *__restrict__ src, S *__restrict__ dst, int64_t K, int64_t T, int64_t R, int to_stacked) {
+__global__ void h_stack_kernel(const S *__restrict__ src, S *__restrict__ dst, int64_t C, int64_t T, const BatchRest *__restrict__ tab,
+                               const int *__restrict__ col_rest, int to_stacked) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;     // index into the stacked array
-    if (i >= R * K * T) return;
-    const int64_t c = i % (R * K), t = i / (R * K), r = c / K, k = c % K;
-    const int64_t b = (r * T + t) * K + k;
+    if (i >= C * T) return;
+    const int64_t c = i % C, t = i / C;
+    const BatchRest r = tab[col_rest[c]];
+    const int64_t b = T * r.off + t * r.K + (c - r.off);
     if (to_stacked) dst[i] = src[b];
     else dst[b] = src[i];
 }
@@ -850,13 +936,17 @@ __global__ void shift_stack_kernel(const S *__restrict__ H, S *__restrict__ out,
     out[e] = (t >= l) ? H[(t - l) * K + k] : S(0);
 }
 
-// restart blockIdx.y of a batch handle: H + y*K with row stride ldh, tail + y*tail_rs
+// restart y = blockIdx.y of a batch handle (tab != nullptr): K = K_r, H + off_r with row stride ldh; tail is the base of
+// exch1 and restart y's tail follows its Gram, at tail + ex_r + L K_r^2
 template <typename S>
 __global__ void h_tail_kernel(const S *__restrict__ H, double *__restrict__ tail, int64_t K, int64_t L,
-                              int64_t Tl, int is_last, int64_t ldh, int64_t tail_rs) {
+                              int64_t Tl, int is_last, int64_t ldh, const BatchRest *tab = nullptr) {
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = r.K; H += r.off; tail += r.ex + L * K * K;
+    }
     const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (L - 1) * K) return;
-    H += (int64_t)blockIdx.y * K; tail += (int64_t)blockIdx.y * tail_rs;
     const int64_t c = idx / K, k = idx % K;
     tail[idx] = is_last ? (double)H[(Tl - (L - 1) + c) * ldh + k] : 0.0;
 }

@@ -426,6 +426,16 @@ def _per_restart(name, v, R):
     return np.ascontiguousarray(a)
 
 
+def _batch_ranks(K):
+    ranks = list(K)
+    for k in ranks:
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
+            raise ValueError(f"every rank in K must be a positive integer; got {k!r}")
+    if not ranks:
+        raise ValueError("a batch needs at least one restart")
+    return [int(k) for k in ranks]
+
+
 def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, *, seeds=None, **kwargs):
     """R MultUpdate fits of the same data in ONE library handle and one device loop (cmf_fit_batch).
 
@@ -435,7 +445,11 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
     (R x K x T) are both given.  ``l1W``, ``l2W``, ``l1H``, ``l2H`` are scalars or length-R sequences.  A restart that meets
     the early stop is frozen while the others go on.  The one deliberate difference from R separate fits: ``max_time`` and
     ``time_hist`` use the batch's wall clock, so every restart has the same ``time_hist`` (cut to its own length).
-    Returns a list of R ``CNMF_results``.  MultUpdate, fp64 / fp32, one GPU, the SIMT engine."""
+    Returns a list of R ``CNMF_results``.  MultUpdate, fp64 / fp32, one GPU, the SIMT engine.
+
+    ``K`` may also be a sequence of R positive ranks (a sweep over K in one handle, cmf_create_batch_ranks): restart r
+    then has rank ``K[r]``, ``seeds`` has R entries, and ``W_init`` / ``H_init`` are sequences of R arrays of shapes
+    ``K[r] x N x L`` and ``K[r] x T``."""
     kw = _normalise_kwargs(kwargs)
     printer = kw.get("printer", print)
     verbose = kw.get("verbose", False)
@@ -449,13 +463,23 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
     if data.ndim != 2:
         raise ValueError("data must be an N x T matrix")
     N, T = data.shape
-    L, K = int(L), int(K)
+    L = int(L)
+    ranks = None if np.ndim(K) == 0 else _batch_ranks(K)
+    K = int(K) if ranks is None else None
     W0, H0 = kw.get("W_init"), kw.get("H_init")
     if seeds is not None:
         if W0 is not None or H0 is not None:
             raise ValueError("give either seeds or the W_init / H_init stacks, not both")
         seeds = list(seeds)
         R = len(seeds)
+    elif W0 is not None and H0 is not None and ranks is not None:
+        W0, H0 = [np.asarray(w) for w in W0], [np.asarray(x) for x in H0]
+        R = len(ranks)
+        if len(W0) != R or len(H0) != R:
+            raise ValueError(f"W_init and H_init need one array per rank ({R}); got {len(W0)} and {len(H0)}")
+        for r, (k, w, x) in enumerate(zip(ranks, W0, H0)):
+            if w.shape != (k, N, L) or x.shape != (k, T):
+                raise ValueError(f"W_init[{r}] must be {(k, N, L)} and H_init[{r}] {(k, T)}; got {w.shape}, {x.shape}")
     elif W0 is not None and H0 is not None:
         W0, H0 = np.asarray(W0), np.asarray(H0)
         if W0.ndim != 4 or H0.ndim != 3 or W0.shape[0] != H0.shape[0]:
@@ -467,22 +491,31 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
         raise ValueError("fit_cnmf_batch needs seeds, or both the W_init and H_init stacks")
     if R < 1:
         raise ValueError("a batch needs at least one restart")
+    if ranks is not None and len(ranks) != R:
+        raise ValueError(f"K has {len(ranks)} ranks but the batch has {R} restarts")
     regs = {k: _per_restart(k, kw.get(k, 0.0), R) for k in ("l1W", "l2W", "l1H", "l2H")}
     if int(kw.get("ngpu", 1) or 1) > 1:
         raise CMFError(3, "batched restarts run on one GPU")
 
+    Ks = [K] * R if ranks is None else ranks
     if seeds is not None:                                 # model.jl:64-67, 116-117: W drawn first, then H
-        W0, H0 = np.empty((R, K, N, L)), np.empty((R, K, T))
-        for r, seed in enumerate(seeds):
+        W0, H0 = [], []
+        for k, seed in zip(Ks, seeds):
             rng = np.random.default_rng(seed)
-            W0[r], H0[r] = rng.random((K, N, L)), rng.random((K, T))
+            W0.append(rng.random((k, N, L)))
+            H0.append(rng.random((k, T)))
     # restart-major host stacks, each block column-major (include/cmf_sm100.h)
-    Wj = julia_array(np.moveaxis(W0, 0, -1), dtype)
-    Hj = julia_array(np.moveaxis(H0, 0, -1), dtype)
+    Wj = np.concatenate([julia_array(w, dtype).ravel(order="F") for w in W0])
+    Hj = np.concatenate([julia_array(x, dtype).ravel(order="F") for x in H0])
 
     lib = _lib.load()
     h = ctypes.c_void_p()
-    check(lib.cmf_create_batch(ctypes.byref(h), N, T, K, L, dtype, rule_cls._ALG, R, device))
+    if ranks is None:
+        check(lib.cmf_create_batch(ctypes.byref(h), N, T, K, L, dtype, rule_cls._ALG, R, device))
+    else:
+        rk = np.asarray(ranks, dtype=np.int64)
+        check(lib.cmf_create_batch_ranks(ctypes.byref(h), N, T, rk.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), L, dtype,
+                                         rule_cls._ALG, R, device))
     dptr = lambda a: a.ctypes.data_as(ctypes.POINTER(ctypes.c_double))  # noqa: E731
     try:
         if kw.get("engine") is not None:
@@ -516,14 +549,17 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
                 _emit(printer, "Converged early.")        # alternating.jl:64, once per restart that stopped early
         verbose and _emit(printer, " fit!")
         dt = np_dtype(dtype)
-        Wo = np.empty((K, N, L, R), dtype=dt, order="F")
-        Ho = np.empty((K, T, R), dtype=dt, order="F")
+        Wo = np.empty(N * L * sum(Ks), dtype=dt)
+        Ho = np.empty(T * sum(Ks), dtype=dt)
         check(lib.cmf_get_factors_batch(h, fptr(Wo), fptr(Ho)))
     finally:
         lib.cmf_destroy(h)
     out = []
+    offs = np.concatenate([[0], np.cumsum(Ks)])
     for r in range(R):
-        W, H = Wo[..., r], np.asfortranarray(Ho[..., r])
+        k, o = Ks[r], int(offs[r])
+        W = Wo[N * L * o: N * L * (o + k)].reshape((k, N, L), order="F")
+        H = Ho[T * o: T * (o + k)].reshape((k, T), order="F")
         W = np.ascontiguousarray(W.transpose(2, 1, 0)) if layout == "LNK" else np.asfortranarray(W)
         nr = int(n[r])
         res = CNMF_results(data, W, H, list(time_hist[:nr]), list(loss_hist[r * cap: r * cap + nr]), layout)

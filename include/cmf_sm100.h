@@ -165,11 +165,12 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
 
 /* ---- batched restarts: R MultUpdate fits of ONE data set in one handle ------------------------
  *
- * Random restarts and regulariser sweeps fit the same data many times.  A batch handle holds R factor sets of the same
- * (K, L) over one copy of X and steps all of them with one launch per kernel: numW (mult.jl:32) and numH (mult.jl:47) of
- * all restarts are one correlation / one transposed convolution with R*K components (X is read once per step), and the
- * per-restart pieces (Gram, G*W, W*W', lag tables, denomH, ratio updates, loss) are launches with a restart index.  The
- * launches of an iteration do not depend on R.  MultUpdate, fp64 and fp32, SIMT engine (0), one GPU, a single shard.
+ * Random restarts, regulariser sweeps and rank sweeps fit the same data many times.  A batch handle holds R factor sets of
+ * one L -- of one K (cmf_create_batch) or of a rank K[r] each (cmf_create_batch_ranks) -- over one copy of X and steps all
+ * of them with one launch per kernel: numW (mult.jl:32) and numH (mult.jl:47) of all restarts are one correlation / one
+ * transposed convolution with sum K[r] components (X is read once per step), and the per-restart pieces (Gram, G*W, W*W',
+ * lag tables, denomH, ratio updates, loss) are launches with a restart index.  The launches of an iteration depend
+ * neither on R nor on the ranks.  MultUpdate, fp64 and fp32, SIMT engine (0), one GPU, a single shard.
  *
  * Host arrays hold the R restarts one after another, each in the layout of the single-set calls: W is R blocks of
  * K x N x L, H is R blocks of K x T; per-restart vectors have R entries.
@@ -187,7 +188,16 @@ int cmf_fit(cmf_handle h, int64_t max_itr, double max_time, int eval_mode, int c
  * Argument checks come before any device query, as for cmf_create. */
 int cmf_create_batch(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int dtype, int alg, int64_t R,
                      int device);
-/* W: R blocks of K x N x L, H: R blocks of K x T (restart r at W + r*K*N*L, H + r*K*T). */
+/* Like cmf_create_batch, restart r with its own rank K[r] >= 1 (same N, T, L, dtype, alg for all): a sweep over K in one
+ * handle.  MultUpdate, SIMT engine, one GPU.  Host arrays hold the restarts one after another: W is the R blocks
+ * K[r] x N x L, H the R blocks K[r] x T (restart r at W + N*L*sum_{q<r} K[q], H + T*sum_{q<r} K[q]).
+ * cmf_create_batch(..., K, ..., R, ...) is this call with K[r] = K for every r.  The footprint grows with sum K[r] and
+ * sum K[r]^2 L^2 and is checked, as for cmf_create_batch, before anything is allocated.  Checks as cmf_create_batch, plus
+ * a null K (CMF_ERR_ARG) and any K[r] < 1 (CMF_ERR_ARG). */
+int cmf_create_batch_ranks(cmf_handle *out, int64_t N, int64_t T, const int64_t *K /* R */, int64_t L, int dtype,
+                           int alg, int64_t R, int device);
+/* W: R blocks of K x N x L, H: R blocks of K x T (restart r at W + r*K*N*L, H + r*K*T); for cmf_create_batch_ranks the
+ * ragged blocks above. */
 int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H);
 int cmf_get_factors_batch(cmf_handle h, void *W_out, void *H_out);
 /* out[2r] = <X, est_r>, out[2r+1] = ||est_r||^2 (model.jl:119-120); the host applies cmf_scale_factors_batch with

@@ -217,15 +217,40 @@ equals `fit_cnmf_sm100(data; seed=seeds[r], l1W=l1W[r], ...)` -- or the fit from
 keyword the same.  `l1W`, `l2W`, `l1H`, `l2H` are scalars or length-R vectors.  A restart that meets the early stop is
 frozen while the others go on; `max_time` and `time_hist` use the batch's own clock (shared by all restarts).  Returns a
 vector of R `CNMF_results`.  MultUpdate only, one GPU.
+
+`K` may be a vector of R ranks (a rank sweep in one handle, `cmf_create_batch_ranks`): restart r then has rank `K[r]`,
+`seeds` has R entries, and `W_init` / `H_init` are vectors of R arrays of sizes `K[r] x N x L` and `K[r] x T`.
 """
-function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, max_itr=100, max_time=Inf, seeds=nothing,
+function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Union{Integer,AbstractVector{<:Integer}}=5, max_itr=100,
+                              max_time=Inf, seeds=nothing,
                               W_init=nothing, H_init=nothing, layout=:LNK, device::Integer=0, kwargs...) where {T<:Union{Float32,Float64}}
     kw = Dict{Symbol,Any}(kwargs)
     for (a, b) in ((:l1_W, :l1W), (:l2_W, :l2W), (:l1_H, :l1H), (:l2_H, :l2H))
         haskey(kw, a) && (kw[b] = pop!(kw, a))
     end
     N, Tt = size(data)
-    if seeds !== nothing
+    ranks = K isa AbstractVector ? collect(Int64, K) : nothing
+    if ranks !== nothing
+        (!isempty(ranks) && all(>=(1), ranks)) || throw(ArgumentError("K must hold one rank >= 1 per restart"))
+        R = length(ranks)
+        if seeds !== nothing
+            (W_init === nothing && H_init === nothing) || throw(ArgumentError("give seeds or the W_init / H_init arrays, not both"))
+            length(seeds) == R || throw(ArgumentError("need one seed per rank ($R)"))
+            Ws, Hs = Array{T,3}[], Matrix{T}[]
+            for (k, s) in zip(ranks, seeds)                        # the draws and rescale of fit_cnmf_sm100 (model.jl:64-70)
+                Random.seed!(s)
+                Wr, Hr = init_rand(data, L, k, tensor_conv)
+                push!(Ws, convert(Array{T,3}, Wr)); push!(Hs, convert(Matrix{T}, Hr))
+            end
+        else
+            (W_init === nothing || H_init === nothing) && throw(ArgumentError("need seeds, or both W_init and H_init"))
+            (length(W_init) == R && length(H_init) == R) || throw(ArgumentError("need one W_init and one H_init per rank ($R)"))
+            Ws = [convert(Array{T,3}, w) for w in W_init]; Hs = [convert(Matrix{T}, x) for x in H_init]
+            all(size(Ws[r]) == (ranks[r], N, L) && size(Hs[r]) == (ranks[r], Tt) for r in 1:R) ||
+                throw(ArgumentError("W_init[r] must be K[r] x N x L and H_init[r] K[r] x T"))
+        end
+        W0 = reduce(vcat, vec.(Ws)); H0 = reduce(vcat, vec.(Hs))    # restart-major host layout (include/cmf_sm100.h)
+    elseif seeds !== nothing
         (W_init === nothing && H_init === nothing) || throw(ArgumentError("give seeds or the W_init / H_init stacks, not both"))
         R = length(seeds)
         W0 = zeros(T, K, N, L, R); H0 = zeros(T, K, Tt, R)
@@ -242,8 +267,13 @@ function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, max_
     end
     regs = [per_restart(get(kw, k, 0), R) for k in (:l1W, :l2W, :l1H, :l2H)]
     out = Ref{Ptr{Cvoid}}(C_NULL)
-    check(ccall((:cmf_create_batch, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Cint, Cint, Int64, Cint),
-                out, N, Tt, K, L, dtype_code(T), CMF_MULT, R, device))
+    if ranks === nothing
+        check(ccall((:cmf_create_batch, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Cint, Cint, Int64, Cint),
+                    out, N, Tt, K, L, dtype_code(T), CMF_MULT, R, device))
+    else
+        check(ccall((:cmf_create_batch_ranks, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Ptr{Int64}, Int64, Cint, Cint, Int64, Cint),
+                    out, N, Tt, ranks, L, dtype_code(T), CMF_MULT, R, device))
+    end
     h = out[]
     try
         check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h, data, 0))
@@ -262,6 +292,17 @@ function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, max_
         end
         W = similar(W0); H = similar(H0)
         check(ccall((:cmf_get_factors_batch, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}), h, W, H))
+        if ranks !== nothing
+            offs = [0; cumsum(ranks)]
+            res = CNMF_results[]
+            for r in 1:R
+                k, o = ranks[r], offs[r]
+                Wr = reshape(W[N*L*o+1:N*L*(o+k)], k, N, L); Hr = reshape(H[Tt*o+1:Tt*(o+k)], k, Tt)
+                push!(res, CNMF_results(data, layout == :LNK ? permutedims(Wr, (3, 2, 1)) : Wr, Hr, time_hist[1:n[r]],
+                                        loss_hist[1:n[r], r]))
+            end
+            return res
+        end
         return [CNMF_results(data, layout == :LNK ? permutedims(W[:, :, :, r], (3, 2, 1)) : W[:, :, :, r], H[:, :, r],
                              time_hist[1:n[r]], loss_hist[1:n[r], r]) for r in 1:R]
     finally
