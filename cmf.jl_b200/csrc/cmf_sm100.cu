@@ -491,8 +491,6 @@ struct Ctx : RankState {
         }
         return fds.B >= 1024 ? 8 : 16;          // tiles of <= 64 KB + twiddles: three CTAs per SM (c4 at B = 1024: 44.96 -> 43.23 ms)
     }
-    // scheduling order of the 1-D grids of the transforms: 0 = tile index fastest, block count = block index fastest (CMF_FD_ORDER=1)
-    int64_t fd_order(int64_t nblocks) const { static const int o = getenv("CMF_FD_ORDER") ? atoi(getenv("CMF_FD_ORDER")) : 0; return o ? nblocks : 0; }
     // complex columns per CTA of the W-side transforms (fft_w / ifft_numW): as for the H side, 8 at B = 1024 keeps three CTAs per SM
     int fd_cols_w() const { return fds.B >= 1024 ? 8 : 16; }
     size_t fd_smem(int C) const { return ((size_t)fds.B * (size_t)C + (size_t)fds.B) * sizeof(float2); }   // tile + full-circle twiddle table
@@ -502,7 +500,7 @@ struct Ctx : RankState {
         const int C = fd_cols_h();
         fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
             fd::fft_h_kernel<decltype(lb)::value, decltype(c)::value><<<(unsigned)(nb * (fds.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                H, hi, lo, K, Tl, Tl + (L - 1), V, nb, full, t_off, fds.Kq, fd_order(nb), fds.tw.p);
+                H, hi, lo, K, Tl, Tl + (L - 1), V, nb, full, t_off, fds.Kq, fds.tw.p);
         });
     }
     // Of (blocks of row stride nblkp_) -> the owned columns of out, nb blocks of hop V
@@ -510,7 +508,7 @@ struct Ctx : RankState {
         const int C = fd_cols_h();
         fd_with_bc(fds.logB, C, [&](auto lb, auto c) {
             fd::ifft_numH_kernel<decltype(lb)::value, decltype(c)::value><<<(unsigned)(nb * (fds.Kq / 2 / C)), fd::NT, fd_smem(C), stream>>>(
-                Of, out, K, Tl, V, nblkp_, fds.Kq, fd_order(nb), fds.tw.p);
+                Of, out, K, Tl, V, nblkp_, fds.Kq, fds.tw.p);
         });
     }
     // spectrum of the Lw lags of src[(l*K+k)][Nw] -> hi / lo (see fft_w_kernel)
@@ -537,7 +535,7 @@ struct Ctx : RankState {
         dim3 grid((unsigned)(f.nblkp * cdiv(N, 32)));
         fd_with_b(f.logB, [&](auto lb) {
             fd::fft_x_kernel<decltype(lb)::value><<<grid, fd::NT, fd_smem(16), stream>>>(X.p, f.Xf_hi.p, f.Xf_lo.p, N, Tl + (L - 1), f.V, f.nblkp,
-                                                                                        fd_order(f.nblkp), f.tw.p);
+                                                                                        f.tw.p);
         });
         post_launch();
         f.x_dirty = false;
@@ -548,7 +546,6 @@ struct Ctx : RankState {
         fd_build_X();
         fd_spectrum_H();
         tc::Params q = tc_base_params();
-        q.nprod = 3;
         q.tiles_n = cdiv(N, tc::BN);
         q.nkb = f.nblkp * 2 / tc::BK;
         q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
@@ -571,7 +568,6 @@ struct Ctx : RankState {
         fd_denomH_prefetch();
         f.hf2_valid = false;                                   // consumed below; Hf is shared with the Gram / loss passes
         tc::Params q = tc_base_params();
-        q.nprod = 3;
         q.tiles_n = cdiv(f.nblk2, tc::BN);
         q.nkb = f.MR / tc::BK;
         q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
@@ -633,7 +629,6 @@ struct Ctx : RankState {
         for (int64_t b0 = 0; b0 < f.nblk; b0 += f.nbc) {
             const int64_t cur = std::min(f.nbc, f.nblk - b0);
             tc::Params q = tc_base_params();
-            q.nprod = 3;
             q.tiles_n = cdiv(cur, tc::BN);
             q.tiles_m = cdiv(N, tc::BM);
             q.nkb = f.MR / tc::BK;
@@ -645,7 +640,7 @@ struct Ctx : RankState {
             post_launch();
             fd_with_b(f.logB, [&](auto lb) {
                 fd::ifft_resid_kernel<decltype(lb)::value><<<(unsigned)(cur * ntile32), fd::NT, fd_smem(16), stream>>>(
-                    f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.V, cur, b0, fd_order(cur), f.tw.p);
+                    f.Yf.p, X.p, loss_part.p + b0 * ntile32, N, Tl, L, f.V, cur, b0, f.tw.p);
             });
             post_launch();
         }
@@ -668,7 +663,6 @@ struct Ctx : RankState {
         fd_fft_h(f.Hf_hi.p, f.Hf_lo.p, f.nblkp, f.V, 1, 0);
         post_launch();
         tc::Params q = tc_base_params();
-        q.nprod = 3;
         q.tiles_n = 1;
         q.nkb = f.nblkp * 2 / tc::BK;
         q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.mtiles;
@@ -690,7 +684,6 @@ struct Ctx : RankState {
             f.w_dirty = false;
         }
         tc::Params q = tc_base_params();
-        q.nprod = 3;
         q.tiles_n = cdiv(f.nblkp, tc::BN);
         q.nkb = cdiv(2 * N, tc::BK);
         q.MR = f.MR; q.mtiles = f.MR / tc::BM; q.units = (int64_t)f.F * q.tiles_n * q.mtiles;
@@ -787,8 +780,6 @@ struct Ctx : RankState {
         tc::Params q;
         memset(&q, 0, sizeof(q));
         q.N = N; q.K = K; q.L = L; q.Tl = Tl; q.G = tcs.G; q.Kp = tcs.Kp;
-        { const char *e = getenv("CMF_PROMO"); q.promo = e ? std::max(1, atoi(e)) : tc::PROMO; }
-        { const char *e = getenv("CMF_TC_PRODUCTS"); q.nprod = (e && atoi(e) == 2) ? 2 : 3; }   // experiment knob, default 3
         return q;
     }
 
@@ -852,7 +843,6 @@ struct Ctx : RankState {
         q.tiles_m = tcs.tiles_m; q.tiles_n = tcs.tiles_n; q.split_len = tcs.split_len; q.tau_hi = Tl + (L - 1);
         q.units = tcs.tiles_m * tcs.tiles_n * tcs.nsplit;
         q.part = corr_part.p;
-        q.corr_order = 0;   // j tiles fastest: the CTAs that run together share the X tile (A/B: 124 vs 148 ms at T=1M)
         {
             const char *e = getenv("CMF_LOCKSTEP");            // k-block window; 0 disables (diagnostics)
             const int w = e ? atoi(e) : 256;
@@ -880,7 +870,7 @@ struct Ctx : RankState {
     // plain GEMM out[m*ldo + n] = sum_k A[m][k] B[n][k] on tensor cores (operands given as hi/lo tensor maps)
     void tc_plain(const CUtensorMap *mA, const CUtensorMap *mB, S *out, int64_t Mrows, int64_t Ncols, int64_t Kdim, int64_t ldo, bool sym = false) {
         tc::Params q = tc_base_params();
-        q.sym = (sym && !getenv("CMF_S2_FULL")) ? 1 : 0;
+        q.sym = sym ? 1 : 0;
         q.tiles_n = cdiv(Ncols, tc::BN);
         q.nkb = cdiv(Kdim, tc::BK);
         q.units = q.tiles_n * cdiv(Mrows, tc::BM);
@@ -895,12 +885,8 @@ struct Ctx : RankState {
     }
     // denomW = G * Wi (mult.jl:28,33): G is built straight into bf16 planes in the K-dim order of Wc
     void tc_denomW(int64_t j0, int64_t j1) {
-        if (getenv("CMF_G_DIRECT"))          // element-wise form (kept for A/B)
-            tc::build_G_split_kernel<<<(unsigned)cdiv(KL() * tcs.KLp, 256), 256, 0, stream>>>(
-                exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
-        else
-            tc::build_G_split_diag_kernel<<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(
-                exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
+        tc::build_G_split_diag_kernel<<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(
+            exch1.p, exch1.p + L * K * K, tcs.Gc_hi.p, tcs.Gc_lo.p, K, L, tcs.Kp, tcs.KLp);
         post_launch();
         tc_split_W();
         if (j0 == 0 && j1 == KL()) {
@@ -951,22 +937,8 @@ struct Ctx : RankState {
         q.units = cdiv(Tl, q.own);
         q.out = numH.p;
         const unsigned grid = (unsigned)std::min<int64_t>(q.units, tcs.num_sms);
-        {
-            const char *e = getenv("CMF_LOCKSTEP_TRANS");      // k-block window; 0 (default) disables
-            const int w = e ? atoi(e) : 0;
-            if (w > 0 && q.units >= (int64_t)grid) {
-                if (lockstep.n == 0) lockstep.alloc(1024);
-                CK(cudaMemsetAsync(lockstep.p, 0, lockstep.n * sizeof(int), stream));
-                q.lockstep = lockstep.p; q.lockstep_window = w;
-            }
-        }
         prof_begin(PROF_TRANSCONV);
-        if (q.lockstep != nullptr) {
-            void *args[] = {&tcs.mWu[0], &tcs.mWu[1], &tcs.mXk[0], &tcs.mXk[1], &q};
-            CK(cudaLaunchCooperativeKernel((void *)tc::tc_kernel<tc::TC_TRANS>, dim3(grid), dim3(tc::THREADS), args, tc::SMEM_BYTES, stream));
-        } else {
-            tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWu[0], tcs.mWu[1], tcs.mXk[0], tcs.mXk[1], q);
-        }
+        tc::tc_kernel<tc::TC_TRANS><<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(tcs.mWu[0], tcs.mWu[1], tcs.mXk[0], tcs.mXk[1], q);
         prof_end();
         post_launch();
     }
@@ -1635,7 +1607,7 @@ struct Ctx : RankState {
     void launch_denomH_tail() {
         const int nb = (int)cdiv((2 * L - 1) * K, 256);
         const size_t smem = (size_t)8 * (size_t)(L - 1) * sizeof(double);
-        if (getenv("CMF_TAIL_DIRECT") || smem > 48 * 1024) {          // literal form (kept for A/B and very long lags)
+        if (smem > 48 * 1024) {          // literal form: the prefix sums of very long lags do not fit shared memory
             dim3 grid((unsigned)(L - 1), (unsigned)K);
             denomH_tail_kernel<S><<<grid, 256, 0, stream>>>(GS.p, H, denH.p, K, L, Tl, -(L - 1), s2_ks, s2_ld);
             post_launch();
@@ -1677,7 +1649,7 @@ struct Ctx : RankState {
         }
         int64_t nb = conv_nblocks(0, Tl);
         if (!tc_active()) launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p);  // mult.jl:55-57
-        else if constexpr (is_f32) nb = (fd_active() && !getenv("CMF_FD_LOSS_TC")) ? fd_conv_loss() : tc_conv_loss();
+        else if constexpr (is_f32) nb = fd_active() ? fd_conv_loss() : tc_conv_loss();
         reduce_scalar(loss_part.p, nb, scal.p);
         CK(cudaMemsetAsync(scal.p + 1, 0, sizeof(double), stream));
         return 1;
@@ -1699,10 +1671,7 @@ struct Ctx : RankState {
     void loss_partial_expansion_dev() {
         gram_partial();
         gram_valid = true;
-        if (getenv("CMF_G_DIRECT"))
-            s2_dot_G_kernel<S><<<1024, 256, 0, stream>>>(GS.p, s2_ks, s2_ld, exch1.p, exch1.p + L * K * K, K, L, loss_part.p + 1024);
-        else
-            s2_dot_G_diag_kernel<S><<<1024, 256, 0, stream>>>(GS.p, s2_ks, s2_ld, exch1.p, exch1.p + L * K * K, K, L, loss_part.p + 1024);
+        s2_dot_G_diag_kernel<S><<<1024, 256, 0, stream>>>(GS.p, s2_ks, s2_ld, exch1.p, exch1.p + L * K * K, K, L, loss_part.p + 1024);
         post_launch();
         reduce_scalar(loss_part.p + 1024, 1024, scal.p + 1);
         if (numH_dot_valid) {             // produced by the H update itself (consumed once: anything may happen before the next call)
@@ -1796,11 +1765,6 @@ struct Ctx : RankState {
             a.K = K; a.L = L; a.T = Tt; a.nC = nC;
             a.l1 = (float)l1H; a.l2 = (float)l2H;
             a.G = G; a.n_block_items = n_block; a.n_diag_items = n_diag; a.n_rec = n_rec;
-            DevBuf<long long> dbgbuf;
-            const bool dbg2 = getenv("CMF_HALS_DEBUG") && atoi(getenv("CMF_HALS_DEBUG")) == 1;
-            if (dbg2) dbgbuf.alloc((size_t)12 * grid);
-            a.dbg = dbg2 ? dbgbuf.p : nullptr;
-            a.dbg_mode = getenv("CMF_HALS_DBGMODE") ? atoi(getenv("CMF_HALS_DBGMODE")) : 0;
             void *args[] = {&a};
             prof_begin(PROF_SWEEP);
             CK(cudaLaunchCooperativeKernel((void *)hals2::hals2_sweep_kernel, dim3((unsigned)grid), dim3(hals2::NT), args, smem, stream));
@@ -1808,29 +1772,6 @@ struct Ctx : RankState {
             post_launch();
             hals2::hals2_finish_kernel<<<dim3((unsigned)cdiv(Tt, 32), (unsigned)cdiv(K, 32)), tb, 0, stream>>>(h2_Hcm.p, Hp, K, Tt, Tp);
             post_launch();
-            if (dbg2) {      // kcycles of work per active round (barrier waits excluded): worst and mean CTA of every role
-                std::vector<long long> hv((size_t)12 * grid);
-                CK(cudaMemcpyAsync(hv.data(), dbgbuf.p, hv.size() * sizeof(long long), cudaMemcpyDeviceToHost, stream));
-                CK(cudaStreamSynchronize(stream));
-                fprintf(stderr, "hals2: SM clock over the launch %lld MHz (clock64 / globaltimer, CTA 0)\n", hv[7]);
-                const char *names[3] = {"block items", "diagonal items", "recurrence warps"};
-                const int lo[4] = {0, n_block, n_block + n_diag, grid};
-                for (int r = 0; r < 3; ++r) {
-                    double worst = 0.0, mean = 0.0; int cnt = 0, wi = -1;
-                    double phw[5] = {0, 0, 0, 0, 0};
-                    long long mx = 0, slow = 0, rds = 0;
-                    for (int i = lo[r]; i < lo[r + 1]; ++i) {
-                        if (hv[12 * i + 1] == 0) continue;
-                        const double v = (double)hv[12 * i] / (double)hv[12 * i + 1] / 1e3;
-                        if (v > worst) { worst = v; wi = i - lo[r]; for (int q = 0; q < 5; ++q) phw[q] = (double)hv[12 * i + 2 + q] / (double)hv[12 * i + 1] / 1e3; }
-                        mean += v; ++cnt;
-                        mx = std::max(mx, hv[12 * i + 8]); slow += hv[12 * i + 9]; rds += hv[12 * i + 1];
-                    }
-                    fprintf(stderr, "hals2 %s: slowest single round %.1f kcycles, %.2f%% of the (CTA, round) pairs above 90 kcycles\n", names[r], mx / 1e3, rds ? 100.0 * slow / rds : 0.0);
-                    fprintf(stderr, "hals2 %s: %d CTAs, kcycles of work per active round: mean %.1f, worst %.1f (item %d; phases stage %.1f pull %.1f tail/store %.1f final %.1f, barrier wait %.1f); rounds %lld, chunks %lld\n",
-                            names[r], lo[r + 1] - lo[r], cnt ? mean / cnt : 0.0, worst, wi, phw[0], phw[1], phw[2], phw[3], phw[4], (long long)(nC + 4 * (K - 1) + 3), (long long)nC);
-                }
-            }
             return true;
         }
     }
@@ -1846,13 +1787,12 @@ struct Ctx : RankState {
         int *pr = progress.p;
         int64_t Kk = K, Ll = L, Tt = full ? T : Tl, ks = s2_ks, ldv = s2_ld;
         S a1 = (S)l1H, a2 = (S)l2H;
-        int dbg = getenv("CMF_HALS_DEBUG") ? atoi(getenv("CMF_HALS_DEBUG")) : 0;   // 1: phase clocks of the last component; 2 / 4: timing runs without the pull / recurrence
         // truncated lag tables of all component pairs for the pull over the last L-1 columns (skipped when they would not fit: the
         // kernel then forms them on the fly)
         const S *ct = nullptr;
         {
             const size_t need = (size_t)(L - 1) * (size_t)(2 * L - 1) * (size_t)(K * K);
-            if (L > 1 && need * sizeof(S) <= ((size_t)1 << 30) && !getenv("CMF_HALS_TAIL_DIRECT")) {
+            if (L > 1 && need * sizeof(S) <= ((size_t)1 << 30)) {
                 if (tailCt.n < need) tailCt.alloc(need);
                 hals_tail_table_kernel<S><<<(unsigned)cdiv((2 * L - 1) * K * K, 256), 256, 0, stream>>>(GS.p, tailCt.p, K, L, s2_ks, s2_ld);
                 post_launch();
@@ -1860,7 +1800,7 @@ struct Ctx : RankState {
             }
         }
         if (hals2_sweep(q, hh, Tt, ct, l1H, l2H)) return;     // round-based kernel (fp32, L <= 32, K <= 128)
-        void *args[] = {&cf, &s2, &q, &hh, &dd, &tc_, &pr, &Kk, &Ll, &Tt, &ks, &ldv, &a1, &a2, &dbg, &ct};
+        void *args[] = {&cf, &s2, &q, &hh, &dd, &tc_, &pr, &Kk, &Ll, &Tt, &ks, &ldv, &a1, &a2, &ct};
         prof_begin(PROF_SWEEP);
         CK(cudaLaunchCooperativeKernel((void *)hals_h_wave_kernel<S>, dim3((unsigned)hals_grid), dim3(HW_NT), args, smem, stream));
         prof_end();
@@ -2252,7 +2192,7 @@ void r_update_motifs(Ctx<S> &ctx, double l1W, double l2W) {
     if (ctx.alg == CMF_PGD) { ctx.pgd_update_motifs(l1W, l2W); return; }
     ctx.w_partials();
     const int64_t KL = ctx.K * ctx.L;
-    if (ctx.world() > 1 && ctx.alg == CMF_MULT && KL % ctx.world() == 0 && !getenv("CMF_W_REPLICATED")) {
+    if (ctx.world() > 1 && ctx.alg == CMF_MULT && KL % ctx.world() == 0) {
         // MultUpdate: the W update is sharded by unfolded rows j = l*K + k (contiguous row blocks of numW / W):
         // reduce-scatter of numW on the side stream while this rank forms its rows of denomW = G W, update of those
         // rows, all-gather of W.  Same bytes on the wire as an all-reduce; G W, the ratio update and the eps floor cost 1/world.

@@ -78,12 +78,12 @@ __device__ __forceinline__ void load_twiddles(float2 *tw, const float2 *__restri
     for (int m = threadIdx.x; m < B; m += NT) tw[m] = twg[m];
 }
 
-// 1-D grid over (block, tile): nbx = number of blocks when the block index runs fastest, 0 = the tile index runs fastest (ny
-// tiles).  One 32-bit division for both indices.
-__device__ __forceinline__ void grid_block_tile(int64_t nbx, int ny, int &blk, int &tile) {
-    const unsigned dv = nbx ? (unsigned)nbx : (unsigned)ny, q = blockIdx.x / dv, r = blockIdx.x - q * dv;
-    blk = (int)(nbx ? r : q);
-    tile = (int)(nbx ? q : r);
+// 1-D grid over (block, tile), the tile index (ny tiles) fastest: the CTAs that run together read neighbouring pieces of
+// the same rows.  One 32-bit division for both indices.
+__device__ __forceinline__ void grid_block_tile(int ny, int &blk, int &tile) {
+    const unsigned q = blockIdx.x / (unsigned)ny, r = blockIdx.x - q * (unsigned)ny;
+    blk = (int)q;
+    tile = (int)r;
 }
 
 template <int LOGB> __device__ __forceinline__ int rev(int x) { return (int)(__brev((unsigned)x) >> (32 - LOGB)); }
@@ -217,12 +217,12 @@ __device__ __forceinline__ void store_split2(__nv_bfloat16 *hi, __nv_bfloat16 *l
 template <int LOGB>
 __global__ void __launch_bounds__(NT, CMF_FD_MINB)
 fft_x_kernel(const float *__restrict__ X, __nv_bfloat16 *__restrict__ hi, __nv_bfloat16 *__restrict__ lo, int64_t N, int64_t xcols,
-             int V, int64_t nblkp, int64_t nbx, const float2 *__restrict__ twg) {
+             int V, int64_t nblkp, const float2 *__restrict__ twg) {
     constexpr int B = 1 << LOGB, C = 16, ISTEP = NT / C;
     extern __shared__ float2 fd_smem[];
     float2 *d = fd_smem, *tw = fd_smem + B * C;
     int b, tile;                                      // 1-D grid over (block, unit tile)
-    grid_block_tile(nbx, (int)((N + 31) / 32), b, tile);
+    grid_block_tile((int)((N + 31) / 32), b, tile);
     const int p = threadIdx.x % C;
     const int n = tile * 32 + 2 * p;
     load_twiddles<B>(tw, twg);
@@ -266,14 +266,14 @@ fft_x_kernel(const float *__restrict__ X, __nv_bfloat16 *__restrict__ hi, __nv_b
 template <int LOGB, int C>
 __global__ void __launch_bounds__(NT, CMF_FD_MINB)
 fft_h_kernel(const float *__restrict__ H, __nv_bfloat16 *__restrict__ hi, __nv_bfloat16 *__restrict__ lo, int64_t K, int64_t Tl,
-             int64_t hcols, int V, int64_t nblkp, int full, int64_t t_off, int kq, int64_t nbx,
+             int64_t hcols, int V, int64_t nblkp, int full, int64_t t_off, int kq,
              const float2 *__restrict__ twg) {
     constexpr int B = 1 << LOGB, ISTEP = NT / C;
     const int64_t KQ = kq, MROWS = 2 * kq;
     extern __shared__ float2 fd_smem[];
     float2 *d = fd_smem, *tw = fd_smem + B * C;
     int bi, tile;                                     // 1-D grid over (block, component tile)
-    grid_block_tile(nbx, (kq / 2) / C, bi, tile);
+    grid_block_tile((kq / 2) / C, bi, tile);
     const int64_t b = bi;
     const int p = threadIdx.x % C;
     const int k = 2 * (tile * C + p);
@@ -392,13 +392,13 @@ fft_w_kernel(const float *__restrict__ Wi, __nv_bfloat16 *__restrict__ hi, __nv_
 template <int LOGB, int C>
 __global__ void __launch_bounds__(NT, CMF_FD_MINB)
 ifft_numH_kernel(const float *__restrict__ Of, float *__restrict__ numH, int64_t K, int64_t Tl, int V, int64_t nblkp, int kq,
-                 int64_t nbx, const float2 *__restrict__ twg) {
+                 const float2 *__restrict__ twg) {
     constexpr int B = 1 << LOGB, FSTEP = NT / C;
     const int64_t KQ = kq, MROWS = 2 * kq;
     extern __shared__ float2 fd_smem[];
     float2 *d = fd_smem, *tw = fd_smem + B * C;
     int bi, tile;                                     // 1-D grid over (block, component tile)
-    grid_block_tile(nbx, (kq / 2) / C, bi, tile);
+    grid_block_tile((kq / 2) / C, bi, tile);
     const int64_t b = bi;
     const int p = threadIdx.x % C;
     const int k = 2 * (tile * C + p);
@@ -441,14 +441,14 @@ ifft_numH_kernel(const float *__restrict__ Of, float *__restrict__ numH, int64_t
 template <int LOGB>
 __global__ void __launch_bounds__(NT, CMF_FD_MINB)
 ifft_resid_kernel(const float *__restrict__ Yf, const float *__restrict__ X, double *__restrict__ partial, int64_t N, int64_t Tl,
-                  int64_t L, int V, int64_t nbc, int64_t b0, int64_t nbx, const float2 *__restrict__ twg) {
+                  int64_t L, int V, int64_t nbc, int64_t b0, const float2 *__restrict__ twg) {
     constexpr int B = 1 << LOGB, C = 16, FSTEP = NT / C, ISTEP = NT / C;
     extern __shared__ float2 fd_smem[];
     __shared__ double red[NT / 32];
     float2 *d = fd_smem, *tw = fd_smem + B * C;
     const int ny = (int)((N + 31) / 32);
     int bc, by;                                       // 1-D grid over (block, unit tile)
-    grid_block_tile(nbx, ny, bc, by);
+    grid_block_tile(ny, bc, by);
     const int p = threadIdx.x % C;
     const int n = by * 32 + 2 * p;
     load_twiddles<B>(tw, twg);
@@ -511,7 +511,7 @@ ifft_resid_kernel(const float *__restrict__ Yf, const float *__restrict__ X, dou
     if (threadIdx.x == 0) {
         double s = 0.0;
         for (int w = 0; w < NT / 32; ++w) s += red[w];
-        partial[(int64_t)bc * ny + by] = s;
+        partial[blockIdx.x] = s;                      // = bc * ny + by
     }
 }
 

@@ -64,9 +64,7 @@ struct Args {
     float l1, l2;
     int G;                // groups of 8 components
     int n_block_items, n_diag_items, n_rec;
-    int dbg_mode;         // timing experiments (wrong results): 2 = the recurrence skips its global loads and stores, 4 = no role does any work (barrier cost)
     unsigned *barrier;    // grid barrier counter (zero before the launch)
-    long long *dbg;       // optional [grid][12]: cycles spent working (barrier waits excluded), rounds with work
 };
 
 __device__ __forceinline__ float ldcg(const float *p) { return __ldcg(p); }
@@ -305,16 +303,6 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
     const int64_t n_rounds = nC + (int64_t)STAG * (K - 1) + 3;
     const int b = blockIdx.x, tid = threadIdx.x;
     const float eps = 2.220446049250313e-16f;
-    long long wk_cyc = 0, wk_rounds = 0, wk_t0 = 0, ph_t = 0, ph[5] = {0, 0, 0, 0, 0}, wk_max = 0, wk_slow = 0;
-    const long long kern_t0 = clock64();
-    unsigned long long kern_ns0 = 0;
-    if (a.dbg && tid == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(kern_ns0));
-#define H2_BEGIN() do { if (a.dbg && tid == 0) { wk_t0 = clock64(); ph_t = wk_t0; } } while (0)
-#define H2_END() do { if (a.dbg && tid == 0) { const long long d_ = clock64() - wk_t0; wk_cyc += d_; ++wk_rounds; if (d_ > wk_max) wk_max = d_; if (d_ > 90000) ++wk_slow; } } while (0)
-#define H2_PHASE(i) do { if (a.dbg && tid == 0) { const long long n_ = clock64(); ph[i] += n_ - ph_t; ph_t = n_; } } while (0)
-#define H2_REPORT() do { if (a.dbg && tid == 0) { a.dbg[12 * b] = wk_cyc; a.dbg[12 * b + 1] = wk_rounds; for (int i_ = 0; i_ < 5; ++i_) a.dbg[12 * b + 2 + i_] = ph[i_]; a.dbg[12 * b + 8] = wk_max; a.dbg[12 * b + 9] = wk_slow; \
-        unsigned long long ns1_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(ns1_)); \
-        a.dbg[12 * b + 7] = (long long)((double)(clock64() - kern_t0) * 1000.0 / (double)(ns1_ - kern_ns0)); } } while (0)   /* SM MHz over the launch */
 
     if (b < a.n_block_items) {
         // ============================================================ block item (g, g'), g' < g
@@ -330,22 +318,19 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
         const int nsrc = (int)(nleft < GS ? nleft : GS);
         for (int64_t s = 0; s < n_rounds; ++s) {
             const int64_t c = s + 1 - (int64_t)STAG * GS * g;
-            if (c >= 0 && c < nC && !(a.dbg_mode & 4)) {
-                H2_BEGIN();
+            if (c >= 0 && c < nC) {
                 {
                     StageRegs sr;
                     stage_load(sr, a, (int64_t)gp * GS, nsrc, c, Tint);
                     stage_store(Dwin, sr, a, nsrc, c, Tint);
                 }
                 __syncthreads();
-                H2_PHASE(0);
                 float2 acc[8][4];
 #pragma unroll
                 for (int r = 0; r < 8; ++r)
 #pragma unroll
                     for (int q = 0; q < 4; ++q) acc[r][q] = make_float2(0.f, 0.f);
                 pull_tile<4>(acc, Dwin, tab, (nsrc + 1) / 2, L, cgp, th * 4);
-                H2_PHASE(1);
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
                     const int64_t kt = (int64_t)g * GS + th * 4 + q;
@@ -356,12 +341,9 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                     }
                 }
                 __syncthreads();
-                H2_PHASE(2);
-                H2_END();
             }
             grid.sync();
         }
-        H2_REPORT();
     } else if (b < a.n_block_items + a.n_diag_items) {
         // ============================================================ diagonal item (g): finalises qeff of its 8 targets
         const int g = b - a.n_block_items;
@@ -377,13 +359,12 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
             return i < GS && k < K && c >= 0 && c < nC;
         };
         for (int64_t s = 0; s < n_rounds; ++s) {
-            H2_BEGIN();
             int buf = 0;
             {
                 // window of the first active target of the round (the later ones are loaded during the previous target's pull)
                 int first = 0;
                 while (first < GS && !active(first, s)) ++first;
-                if (first > 0 && first < GS && !(a.dbg_mode & 4)) {
+                if (first > 0 && first < GS) {
                     StageRegs sr;
                     const int64_t cf = s - (int64_t)STAG * ((int64_t)g * GS + first);
                     stage_load(sr, a, (int64_t)g * GS, first, cf, Tint);
@@ -393,7 +374,7 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
             for (int i = 0; i < GS; ++i) {
                 const int64_t k = (int64_t)g * GS + i;
                 const int64_t c = s - (int64_t)STAG * k;
-                if (k >= K || c < 0 || c >= nC || (a.dbg_mode & 4)) continue;      // uniform over the CTA
+                if (k >= K || c < 0 || c >= nC) continue;      // uniform over the CTA
                 float2 *Dwin = Dwin0 + buf * (GS / 2) * WINQ;
                 // loads of the NEXT active target's window go out now and are stored into the other buffer after this pull
                 int nxt = i + 1;
@@ -419,7 +400,6 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                 for (int r = 0; r < 8; ++r) acc[r][0] = make_float2(0.f, 0.f);
                 __syncthreads();                                // this target's window is complete in shared memory
                 if (i > 0) {
-                    H2_PHASE(0);
                     const int npair = (i + 1) / 2;              // the two thread halves split the source pairs
                     const int p_lo = th == 0 ? 0 : (npair + 1) / 2, p_hi = th == 0 ? (npair + 1) / 2 : npair;
                     if (p_hi > p_lo) pull_tile<1>(acc, Dwin + p_lo * WINQ, tab + (size_t)p_lo * (((2 * L - 1) + 7) & ~7) * 8, p_hi - p_lo, L, cgp, i);
@@ -436,7 +416,6 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                 if (nxt < GS) stage_store(Dwin0 + (buf ^ 1) * (GS / 2) * WINQ, srn, a, nxt, cn, Tint);
                 buf ^= 1;
                 __syncthreads();
-                H2_PHASE(1);
                 // ---- truncated tail: sources t >= Tint of ALL earlier components with the tables C_w (w = T - t); work item =
                 //      (target column, block of earlier components), block sums added in a fixed order (deterministic)
                 if (k > 0 && Lm > 0 && t0 + CW + Lm > Tint) {
@@ -488,7 +467,6 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                     }
                     __syncthreads();
                 }
-                H2_PHASE(2);
                 // ---- Q + the block partials in the fixed order g' = 0 .. g-1 + the own-group pull, and the hand-over
                 const float c0 = a.Cf[((int64_t)Lm * K + k) * K + k];
                 const float inv = 1.f / (c0 + eps + a.l2);
@@ -508,15 +486,10 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                     }
                     *reinterpret_cast<float4 *>(a.AD_cm + cell_at(k, t, K)) = make_float4(ov[0], ov[1], ov[2], ov[3]);
                 }
-                H2_PHASE(3);
                 __syncthreads();
             }
-            H2_END();
-            if (a.dbg && tid == 0) ph_t = clock64();
             grid.sync();
-            H2_PHASE(4);
         }
-        H2_REPORT();
     } else {
         // ============================================================ recurrence warp: lane = component
         const int rb = b - a.n_block_items - a.n_diag_items;
@@ -547,18 +520,16 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
         float *adp = a.AD_cm, *hp = a.H_cm;               // cell bases are added per round (t0 below is the offset of the cell)
         for (int64_t s = 0; s < n_rounds; ++s) {
             const int64_t c = s - 1 - (int64_t)STAG * k;
-            const bool on_ = live && c >= 0 && c < nC;
-            const bool on = on_ && !(a.dbg_mode & 2);
-            if (__any_sync(0xffffffffu, on_) && !(a.dbg_mode & 4)) {
-                H2_BEGIN();
+            const bool on = live && c >= 0 && c < nC;
+            if (__any_sync(0xffffffffu, on)) {
                 // interior columns of this chunk (the truncated tail is left to the tail job)
                 int nv = 0;
-                if (on_) { const int64_t r = Tint - c * CW; nv = (int)(r < 0 ? 0 : (r > CW ? CW : r)); }
-                const int64_t t0 = on_ ? cell_at(k, c * CW, K) : 0;      // offset of the cell inside the working arrays
+                if (on) { const int64_t r = Tint - c * CW; nv = (int)(r < 0 ? 0 : (r > CW ? CW : r)); }
+                const int64_t t0 = on ? cell_at(k, c * CW, K) : 0;      // offset of the cell inside the working arrays
                 float *ring = reinterpret_cast<float *>(smem_raw);          // [RSTG][2][32][RLS]
                 // a lane that is off (not started / finished) runs the same instructions on zeros and stores nothing; the
                 // mask-free path needs every active lane to be on a full interior chunk (all but the last chunk of a component)
-                const bool full = __all_sync(0xffffffffu, !on_ || nv == CW);
+                const bool full = __all_sync(0xffffffffu, !on || nv == CW);
 #pragma unroll 1
                 for (int h = 0; h < RPRE; ++h) rec_fetch(ring, adp, hp, t0, h, lane, on);
                 if (!on) {                                                  // zeros for the lanes that do not load
@@ -579,7 +550,6 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
                     }
                 }
                 cp_async_wait<0>();
-                H2_END();
             }
             // ---- tail job: the last L-1 columns of one component with the truncated tables, one round after its last chunk.  At most
             //      one lane of the warp has it in a given round; the whole warp works on it: lane = lag of the pending sum.
@@ -618,12 +588,7 @@ __global__ void __launch_bounds__(NT, 1) hals2_sweep_kernel(Args a) {
             }
             grid.sync();
         }
-        H2_REPORT();
     }
-#undef H2_BEGIN
-#undef H2_END
-#undef H2_REPORT
-#undef H2_PHASE
 }
 
 // coefficient pairs of the recurrence lanes: coef[k][0..31] = (cs[2m], cs[2m+1]), coef[k][32..63] = (cs[2m+1], cs[2m+2]), m = 0..15,

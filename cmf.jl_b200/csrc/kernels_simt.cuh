@@ -635,26 +635,8 @@ __global__ void build_G_kernel(const double *__restrict__ Rg, const double *__re
 }
 
 // partial[block] = sum over a grid-stride slice of S2[j][j'] * G[j][j'], with G = Htilde Htilde' formed on the fly
-// from Rg and the tail exactly as in build_G_kernel:  ||conv(W,H)||^2 = <W W', Htilde Htilde'>.
-template <typename S>
-__global__ void s2_dot_G_kernel(const S *__restrict__ S2, int64_t Ks, int64_t ld, const double *__restrict__ Rg,
-                                const double *__restrict__ Ht, int64_t K, int64_t L, double *__restrict__ partial) {
-    __shared__ double red[32];
-    const int64_t KL = K * L;
-    double acc = 0.0;
-    for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < KL * KL; idx += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t jp = idx % KL, j = idx / KL;
-        const int64_t k = j % K, l = j / K, kp = jp % K, lp = jp / K;
-        double g = (l >= lp) ? Rg[((l - lp) * K + k) * K + kp] : Rg[((lp - l) * K + kp) * K + k];
-        const int64_t m = l < lp ? l : lp;
-        for (int64_t i = 0; i < m; ++i) g -= Ht[(L - 1 - l + i) * K + k] * Ht[(L - 1 - lp + i) * K + kp];
-        acc += g * (double)S2[(l * Ks + k) * ld + lp * Ks + kp];
-    }
-    acc = block_sum(acc, red);
-    if (threadIdx.x == 0) partial[blockIdx.x] = acc;
-}
-
-// The same sum walked along the block diagonals of G: thread (d, k, k') visits (l, l') = (d+s, s) (d >= 0) or (s, s-d) (d < 0),
+// from Rg and the tail as in build_G_kernel:  ||conv(W,H)||^2 = <W W', Htilde Htilde'>.
+// The sum walks the block diagonals of G: thread (d, k, k') visits (l, l') = (d+s, s) (d >= 0) or (s, s-d) (d < 0),
 // where the Toeplitz part is constant and the tail grows by one product per step,
 //   tail(l+1, l'+1) = tail(l, l') + Ht[L-2-l][k] Ht[L-2-l'][k'],
 // so every element of S2 is read once and the (K L)^2 L tail work becomes (K L)^2.  grid-stride over (2L-1) K K diagonals.
@@ -1123,13 +1105,8 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                                                              const S *__restrict__ Q, S *__restrict__ H, S *__restrict__ D,
                                                              S *__restrict__ tailC_all /*[grid][L*L]*/, int *progress /*[K]*/,
                                                              int64_t K, int64_t L, int64_t T, int64_t Ks, int64_t ld,
-                                                             S l1, S l2, int debug, const S *__restrict__ Ct /*tail tables or nullptr*/) {
+                                                             S l1, S l2, const S *__restrict__ Ct /*tail tables or nullptr*/) {
     constexpr int HW_KB = hw_kb<S>();
-    // optional phase clocks of the last component (CMF_HALS_DEBUG): cycles of thread 0 between marks, barrier waits included
-    __shared__ long long dbg_acc[8];
-    __shared__ long long dbg_t;
-#define HW_MARK(i) do { if ((debug & 1) && threadIdx.x == 0) { const long long now_ = clock64(); dbg_acc[i] += now_ - dbg_t; dbg_t = now_; } } while (0)
-    if (threadIdx.x == 0) { for (int i = 0; i < 8; ++i) dbg_acc[i] = 0; dbg_t = clock64(); }
     extern __shared__ __align__(16) unsigned char smem_raw[];
     S *qeff = reinterpret_cast<S *>(smem_raw);       // [HW_TC]
     S *pend = qeff + HW_TC;                          // ring of RB entries
@@ -1167,7 +1144,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
         }
         bool ring_mode = false;               // true once the window lives in the shared ring (tail / partial blocks / L > 32)
 
-        if ((debug & 1) && tid == 0) { for (int i = 0; i < 8; ++i) dbg_acc[i] = 0; dbg_t = clock64(); }
         for (int64_t c = 0; c < nC; ++c) {
             const int64_t t0 = c * HW_TC;
             // ---- wait: component k-1 must have finished cell min(c+1, nC-1)
@@ -1178,7 +1154,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
             }
             __syncthreads();
             __threadfence();
-            HW_MARK(0);
             // ---- pull: corrections from all earlier components, HW_KB components at a time through shared memory.
             //      Register tiling: thread (cg, kq) owns the 8 consecutive columns 8*cg .. 8*cg+7 and a quarter of the
             //      staged components; along the lag loop the 8 Delta values slide through registers, so each step costs
@@ -1194,7 +1169,10 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                 S a8[8];
 #pragma unroll
                 for (int r = 0; r < 8; ++r) a8[r] = S(0);
-                for (int64_t kp0 = 0; kp0 < ((debug & 2) ? 0 : k); kp0 += HW_KB) {   // debug bit 1: timing without the pull (wrong results)
+                // counted in staged blocks: with kp0 < k as the loop condition, ptxas spills a fifth more in the fp64 instantiation
+                const int nsb = (int)((k + HW_KB - 1) / HW_KB);
+                for (int sb = 0; sb < nsb; ++sb) {
+                    const int64_t kp0 = (int64_t)sb * HW_KB;
                     const int kb = (int)((k - kp0 < HW_KB) ? k - kp0 : HW_KB);
                     __syncthreads();
                     // 8 loads in flight per thread: Delta comes from L2 (written by other SMs), a dependent load per
@@ -1251,7 +1229,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                         Cs[idx] = (kk < kb && j < 2 * L - 1) ? Cf[(j * K + kp0 + kk) * K + k] : S(0);
                     }
                     __syncthreads();
-                    HW_MARK(1);
                     // two staged components per pass (they share the index arithmetic); the window of 8 Delta values per
                     // component is a circular register file whose rotation is compile-time: the lag loop is unrolled by 8,
                     // slot (r - jj) & 7 holds window index ib + r - j at step j = j0 + jj, and step jj refills slot -jj.
@@ -1287,7 +1264,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                             }
                         }
                     }
-                    HW_MARK(2);
                 }
                 // reduce the component groups: red[kq][column] (reuses the Delta window space), then add Q
                 __syncthreads();
@@ -1363,7 +1339,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                 }
             }
             __syncthreads();
-            HW_MARK(3);
             // ---- sweep: the sequential recurrence of component k over this chunk (warp 0), entirely in shared
             //      memory: H of the chunk is prefetched by all threads, results are written back by all threads
             for (int col = tid; col < HW_TC; col += nthr) {
@@ -1371,8 +1346,7 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                 hch[col] = (tp < T) ? H[tp * K + k] : S(0);
             }
             __syncthreads();
-            HW_MARK(4);
-            if (tid < 32 && !(debug & 4)) {   // debug bit 2: timing without the recurrence (wrong results)
+            if (tid < 32) {
                 const int lane = tid;
                 const int n = (int)((t0 + HW_TC < T) ? HW_TC : T - t0);
                 int i = 0;
@@ -1426,7 +1400,6 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
                 }
             }
             __syncthreads();
-            HW_MARK(5);
             for (int col = tid; col < HW_TC; col += nthr) {
                 const int64_t tp = t0 + col;
                 if (tp < T) {
@@ -1439,17 +1412,10 @@ __global__ void __launch_bounds__(HW_NT) hals_h_wave_kernel(const S *__restrict_
             __threadfence();
             __syncthreads();
             if (tid == 0) atomicExch(progress + k, (int)(c + 1));
-            HW_MARK(6);
         }
-        if ((debug & 1) && tid == 0 && k == K - 1)
-            printf("hals_h_wave component %lld, %lld cells, kcycles per cell: wait %.1f  stage %.1f  pull %.1f  reduce+Q %.1f  loadH %.1f  recurrence %.1f  writeback+publish %.1f\n",
-                   (long long)k, (long long)nC, dbg_acc[0] / 1e3 / nC, dbg_acc[1] / 1e3 / nC, dbg_acc[2] / 1e3 / nC, dbg_acc[3] / 1e3 / nC,
-                   dbg_acc[4] / 1e3 / nC, dbg_acc[5] / 1e3 / nC, dbg_acc[6] / 1e3 / nC);
         __syncthreads();
     }
 }
-
-#undef HW_MARK
 
 // Projected gradient descent pieces (src/algs/pgd.jl:224-255, SquareLoss):
 //   g = 2*(den - num) + 2*l2*x + l1*sign(x)      gradient of ||conv - X||^2 plus Square/Absolute penalties (:30-32,:77-88)

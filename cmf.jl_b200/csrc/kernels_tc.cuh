@@ -56,10 +56,7 @@ struct Params {
     int64_t own;               // owned columns per t tile = BN - (G-1)
     // CORR
     int64_t split_len;         // t columns per split (multiple of BK)
-    int nprod;                 // bf16 products per logical product: 3 (hi*hi + hi*lo + lo*hi, default) or 2 (A operand in single bf16)
-    int promo;                 // k-blocks accumulated in TMEM before promotion to registers (PROMO by default)
-    int corr_order;            // 0: j tiles fastest (CTAs share the X tile), 1: n tiles fastest (CTAs share the H window)
-    int *lockstep;             // CORR/TRANS: per-CTA k-block counters (zeroed before the launch) or nullptr
+    int *lockstep;             // CORR: per-CTA k-block counters (zeroed before the launch) or nullptr
     int lockstep_window;       // a CTA may run at most this many k-blocks ahead of the slowest CTA
     int64_t tau_hi;            // valid X columns [0, tau_hi)
     // dims
@@ -248,13 +245,13 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                 if (MODE == TC_PLAIN) { nt = unit % p.tiles_n; mt = unit / p.tiles_n; }         // nt: column tile, mt: row tile
                 int64_t fq_m = 0;                                                                        // FQT / FQC: 128-row tile of the frequency
                 if (MODE == TC_FQT || MODE == TC_FQC) { fq_m = unit % p.mtiles; const int64_t r = unit / p.mtiles; nt = r % p.tiles_n; mt = r / p.tiles_n; }   // nt: column tile, mt: frequency
-                if (MODE == TC_CORR) { const int64_t r = unit % (p.tiles_m * p.tiles_n); if (p.corr_order == 0) { mt = r % p.tiles_m; nt = r / p.tiles_m; } else { nt = r % p.tiles_n; mt = r / p.tiles_n; } }
+                if (MODE == TC_CORR) { const int64_t r = unit % (p.tiles_m * p.tiles_n); mt = r % p.tiles_m; nt = r / p.tiles_m; }   // j tiles fastest: the CTAs that run together share the X tile
                 const int64_t nseg = n_segments(unit);
                 for (int64_t seg = 0; seg < nseg; ++seg) {
                     int64_t kb0, kbn;
                     segment_kb(unit, seg, kb0, kbn);
                     for (int64_t kb = kb0; kb < kb0 + kbn; ++kb) {
-                        if ((MODE == TC_CORR || MODE == TC_TRANS) && p.lockstep != nullptr) {
+                        if (MODE == TC_CORR && p.lockstep != nullptr) {
                             // The ~50 CTAs that share an X tile must stay close in time or the tile falls out of L2 and is
                             // re-read from HBM (measured: 19x the algorithmic traffic without this).  Every 64 k-blocks each
                             // CTA publishes its progress and waits while it is more than lockstep_window ahead of the slowest.
@@ -271,17 +268,17 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                         }
                         mbar_wait(&empty_bar[s], ph ^ 1);
                         unsigned char *st = smem + (size_t)s * STAGE_BYTES;
-                        mbar_expect_tx(&full_bar[s], p.nprod == 3 ? STAGE_BYTES : STAGE_BYTES - A_PLANE);
+                        mbar_expect_tx(&full_bar[s], STAGE_BYTES);
                         if (MODE == TC_CONV) {
                             const int32_t j0 = (int32_t)(kb * BK);
                             tma_load_2d(st, &mapA_hi, &full_bar[s], j0, (int32_t)(nt * BM));
-                            if (p.nprod == 3) tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], j0, (int32_t)(nt * BM));
+                            tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], j0, (int32_t)(nt * BM));
                             tma_load_2d(st + 2 * A_PLANE, &mapB_hi, &full_bar[s], j0, (int32_t)(mt * BN));
                             tma_load_2d(st + 2 * A_PLANE + B_PLANE, &mapB_lo, &full_bar[s], j0, (int32_t)(mt * BN));
                         } else if (MODE == TC_PLAIN) {
                             const int32_t k0 = (int32_t)(kb * BK);
                             tma_load_2d(st, &mapA_hi, &full_bar[s], k0, (int32_t)(mt * BM));
-                            if (p.nprod == 3) tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], k0, (int32_t)(mt * BM));
+                            tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], k0, (int32_t)(mt * BM));
                             tma_load_2d(st + 2 * A_PLANE, &mapB_hi, &full_bar[s], k0, (int32_t)(nt * BN));
                             tma_load_2d(st + 2 * A_PLANE + B_PLANE, &mapB_lo, &full_bar[s], k0, (int32_t)(nt * BN));
                         } else if (MODE == TC_TRANS) {
@@ -289,7 +286,7 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                             const int32_t c0 = (int32_t)(nb * BK);
                             const int32_t rowA = (int32_t)(g * p.G * p.Kp), rowB = (int32_t)(unit * p.own + g * p.G);   // G*Kp <= 128 rows per lag group
                             tma_load_2d(st, &mapA_hi, &full_bar[s], c0, rowA);
-                            if (p.nprod == 3) tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], c0, rowA);
+                            tma_load_2d(st + A_PLANE, &mapA_lo, &full_bar[s], c0, rowA);
                             tma_load_2d(st + 2 * A_PLANE, &mapB_hi, &full_bar[s], c0, rowB);
                             tma_load_2d(st + 2 * A_PLANE + B_PLANE, &mapB_lo, &full_bar[s], c0, rowB);
                         } else if (MODE == TC_FQT) {
@@ -320,7 +317,7 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                             // groups), so one TMA per plane fills all the 4 KB swizzle atoms of the tile
                             const int32_t trow = (int32_t)(kb * BK);
                             tma_load_3d(st, &mapA_hi, &full_bar[s], 0, trow, (int32_t)(mt * 2));
-                            if (p.nprod == 3) tma_load_3d(st + A_PLANE, &mapA_lo, &full_bar[s], 0, trow, (int32_t)(mt * 2));
+                            tma_load_3d(st + A_PLANE, &mapA_lo, &full_bar[s], 0, trow, (int32_t)(mt * 2));
                             tma_load_3d(st + 2 * A_PLANE, &mapB_hi, &full_bar[s], 0, trow, (int32_t)(nt * 4));
                             tma_load_3d(st + 2 * A_PLANE + B_PLANE, &mapB_lo, &full_bar[s], 0, trow, (int32_t)(nt * 4));
                         }
@@ -328,7 +325,7 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                     }
                 }
             }
-            if ((MODE == TC_CORR || MODE == TC_TRANS) && p.lockstep != nullptr) atomicExch(p.lockstep + blockIdx.x, 0x7fffffff);   // finished: never the slowest
+            if (MODE == TC_CORR && p.lockstep != nullptr) atomicExch(p.lockstep + blockIdx.x, 0x7fffffff);   // finished: never the slowest
         }
     } else if (warp == 1) {
         // ================================================================ MMA issuer
@@ -341,8 +338,8 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                 for (int64_t seg = 0; seg < nseg; ++seg) {
                     int64_t kb0, kbn;
                     segment_kb(unit, seg, kb0, kbn);
-                    for (int64_t c0 = 0; c0 < kbn; c0 += p.promo, ++q) {
-                        const int64_t cn = min((int64_t)p.promo, kbn - c0);
+                    for (int64_t c0 = 0; c0 < kbn; c0 += PROMO, ++q) {
+                        const int64_t cn = min((int64_t)PROMO, kbn - c0);
                         const int acc = (int)(q & 1);
                         mbar_wait(&tmem_empty[acc], (uint32_t)((q >> 1) & 1) ^ 1);
                         tc_fence_after();
@@ -372,12 +369,8 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
                                     dah = make_desc(a_hi + off, 16, 512, 4); dal = make_desc(a_lo + off, 16, 512, 4);
                                     dbh = make_desc(b_hi + off, 16, 512, 4); dbl = make_desc(b_lo + off, 16, 512, 4);
                                 }
-                                if (p.nprod == 3) {
-                                    tc_mma(d_tmem, dal, dbh, idesc, accumulate);   // lo*hi
-                                    tc_mma(d_tmem, dah, dbl, idesc, 1u);           // hi*lo
-                                } else {
-                                    tc_mma(d_tmem, dah, dbl, idesc, accumulate);   // hi*lo (A carried in single bf16)
-                                }
+                                tc_mma(d_tmem, dal, dbh, idesc, accumulate);   // lo*hi
+                                tc_mma(d_tmem, dah, dbl, idesc, 1u);           // hi*lo
                                 tc_mma(d_tmem, dah, dbh, idesc, 1u);           // hi*hi
                                 accumulate = 1u;
                             }
@@ -404,7 +397,7 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
             int64_t fq_m = 0;
             if (MODE == TC_CONV || MODE == TC_PLAIN) { nt = unit % p.tiles_n; mt = unit / p.tiles_n; }
             if (MODE == TC_FQT || MODE == TC_FQC) { fq_m = unit % p.mtiles; const int64_t r = unit / p.mtiles; nt = r % p.tiles_n; mt = r / p.tiles_n; }
-            if (MODE == TC_CORR) { sp = unit / (p.tiles_m * p.tiles_n); const int64_t r = unit % (p.tiles_m * p.tiles_n); if (p.corr_order == 0) { mt = r % p.tiles_m; nt = r / p.tiles_m; } else { nt = r % p.tiles_n; mt = r / p.tiles_n; } }
+            if (MODE == TC_CORR) { sp = unit / (p.tiles_m * p.tiles_n); const int64_t r = unit % (p.tiles_m * p.tiles_n); mt = r % p.tiles_m; nt = r / p.tiles_m; }
             const int64_t nseg = n_segments(unit);
             for (int64_t seg = 0; seg < nseg; ++seg) {
                 int64_t kb0, kbn;
@@ -412,7 +405,7 @@ tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constant__ C
 #pragma unroll
                 for (int c = 0; c < BN / 2; ++c) racc[c] = 0.f;
                 // ---- promotion: racc += TMEM partial, every PROMO k-blocks
-                for (int64_t c0 = 0; c0 < kbn; c0 += p.promo, ++q) {
+                for (int64_t c0 = 0; c0 < kbn; c0 += PROMO, ++q) {
                     const int acc = (int)(q & 1);
                     mbar_wait(&tmem_full[acc], (uint32_t)((q >> 1) & 1));
                     tc_fence_after();
@@ -619,29 +612,8 @@ __global__ void split_W_kernel(const float *__restrict__ Wi, __nv_bfloat16 *__re
 
 // G = Htilde Htilde' (see build_G_kernel) written as bf16 hi/lo planes Gc[j][jj]: rows j = l*K + k (Wi order),
 // columns jj = (L-1-l')*Kp + k' (the K-dim order of Wc), row length KLp, zero padded.      [G*W A operand]
-__global__ void build_G_split_kernel(const double *__restrict__ Rg, const double *__restrict__ Ht, __nv_bfloat16 *__restrict__ hi,
-                                     __nv_bfloat16 *__restrict__ lo, int64_t K, int64_t L, int Kp, int64_t KLp) {
-    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= K * L * KLp) return;
-    const int64_t jj = idx % KLp, j = idx / KLp;
-    const int64_t k = j % K, l = j / K;
-    const int64_t kp = jj % Kp, lrev = jj / Kp;
-    float v = 0.f;
-    if (kp < K && lrev < L) {
-        const int64_t lp = L - 1 - lrev;
-        double g = (l >= lp) ? Rg[((l - lp) * K + k) * K + kp] : Rg[((lp - l) * K + kp) * K + k];
-        const int64_t m = l < lp ? l : lp;
-        double tail = 0.0;
-        for (int64_t i = 0; i < m; ++i) tail += Ht[(L - 1 - l + i) * K + k] * Ht[(L - 1 - lp + i) * K + kp];
-        v = (float)(g - tail);
-    }
-    __nv_bfloat16 h, l_;
-    split_bf16(v, h, l_);
-    hi[idx] = h; lo[idx] = l_;
-}
-
-// The same planes written along the block diagonals (see s2_dot_G_diag_kernel): thread (d, k, k') walks (l, l') with the
-// Toeplitz part constant and the tail updated by one product per step.  The zero padding of Gc is never touched.
+// Written along the block diagonals (see s2_dot_G_diag_kernel): thread (d, k, k') walks (l, l') with the Toeplitz part
+// constant and the tail updated by one product per step.  The zero padding of Gc is never touched.
 __global__ void build_G_split_diag_kernel(const double *__restrict__ Rg, const double *__restrict__ Ht, __nv_bfloat16 *__restrict__ hi,
                                           __nv_bfloat16 *__restrict__ lo, int64_t K, int64_t L, int Kp, int64_t KLp) {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

@@ -11,7 +11,6 @@ run() { # name, env...
 run default CMF_X=0
 run cols8 CMF_FD_COLS=8
 run cols32 CMF_FD_COLS=32
-run gdirect CMF_G_DIRECT=1
 run default2 CMF_X=0
 timeout 600 python bench.py --config c3 --steps 10 --warmup 3 --no-e2e --no-cpu > gpurun_out/fd7_c3.json 2> gpurun_out/fd7_c3.err
 python -c "import json; d=json.load(open('gpurun_out/fd7_c3.json')); print('c3', d['value'], d['ms_per_step'], d['loss'], d['roofline']['kernel_ms'])"
