@@ -76,6 +76,9 @@ SIGNATURES = {
     "cmf_init_scale_partials_batch": [_h, _c.POINTER(_dbl)],
     "cmf_scale_factors_batch": [_h, _c.POINTER(_dbl)],
     "cmf_loss_batch": [_h, _c.POINTER(_dbl)],
+    "cmf_create_sparse": [_c.POINTER(_h), _i64, _i64, _i64, _i64, _int, _int, _int],
+    "cmf_create_batch_sparse": [_c.POINTER(_h), _i64, _i64, _c.POINTER(_i64), _i64, _int, _int, _i64, _int],
+    "cmf_set_data_csc": [_h, _i64, _c.POINTER(_i64), _c.POINTER(_i64), _vp, _int],
     "cmf_fit_batch": [_h, _i64, _dbl, _int, _int, _int, _dbl, _c.POINTER(_dbl), _c.POINTER(_dbl), _c.POINTER(_dbl),
                       _c.POINTER(_dbl), _c.POINTER(_dbl), _c.POINTER(_dbl), _i64, _c.POINTER(_i64), _c.POINTER(_int)],
 }

@@ -15,6 +15,7 @@ DEPS = SOURCES + [
     os.path.join(HERE, "csrc", "kernels_fd.cuh"),
     os.path.join(HERE, "csrc", "comm.h"),
     os.path.join(HERE, "csrc", "kernels_hals.cuh"),
+    os.path.join(HERE, "csrc", "kernels_sparse.cuh"),
     os.path.join(ROOT, "include", "cmf_sm100.h"),
 ]
 

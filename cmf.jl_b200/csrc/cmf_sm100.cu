@@ -27,6 +27,7 @@
 #include "kernels_tc.cuh"
 #include "kernels_fd.cuh"
 #include "kernels_hals.cuh"
+#include "kernels_sparse.cuh"
 #include "comm.h"
 
 namespace {
@@ -110,6 +111,7 @@ struct RankState {
     bool gram_valid = false;         // exchange buffer 1 holds the local Gram/tail partial of the current H
     bool have_data = false, have_factors = false;
     int64_t R = 0;                   // restarts of a batch handle (cmf_create_batch[_ranks]); 0 = a handle of one factor set
+    bool sparse = false;             // cmf_create_sparse: X is held as CSC + CSR (cmf_set_data_csc), the dense X never exists
     // optional per-kernel-class event timing (bench.py's roofline): class -> list of event pairs
     bool profiling = false;
     struct ProfEv { int which; cudaEvent_t a, b; };
@@ -278,6 +280,10 @@ struct Ctx : RankState {
     DevBuf<S> X, Hbuf, Wi, Wtmp, numW, denW, GS, Cf, numH, denH, tailC;
     DevBuf<int> progress, lockstep;
     DevBuf<S> tailCt;                  // HALS H sweep: truncated lag tables of all component pairs
+    // sparse handles (kernels_sparse.cuh): X as CSC (numH) and CSR (numW), W transposed to [n][l*K + k] for the numH gather
+    DevBuf<int64_t> sp_colptr, sp_rowptr;
+    DevBuf<int> sp_rowval, sp_colidx;
+    DevBuf<S> sp_val, sp_rval, Wt;
     int hals_grid = 0;
     DevBuf<double> exch1, corr_part, loss_part, scal;
     S *H = nullptr;  // owned column 0 inside Hbuf
@@ -311,10 +317,27 @@ struct Ctx : RankState {
     void init() {
         if (R > 0) { init_batch(); return; }
         CK(cudaSetDevice(device));
+        const int64_t hal = L - 1;
+        if (sparse) {
+            // everything below except X, plus the transposed W of the sparse numH; the CSC / CSR arrays are checked by
+            // cmf_set_data_csc, whose size depends on nnz
+            plan_split(N, Tl + hal, nsplit_w, split_w);
+            plan_split(K, Tl + hal, nsplit_g, split_g);
+            const size_t el = (size_t)((Tl + 2 * hal) * K + 5 * KL() * N + KL() * KL() + (2 * L - 1) * K * K + 2 * Tl * K);
+            const size_t dbl = (size_t)(L * K * K + hal * K + 1) +
+                               (size_t)std::max<int64_t>((int64_t)nsplit_w * KL() * N, (int64_t)nsplit_g * KL() * K) +
+                               (size_t)std::max<int64_t>(2 * cdiv(N, BN) * cdiv(Tl + hal, BT), 4096) + 8;
+            size_t free_b = 0, total_b = 0;
+            CK(cudaMemGetInfo(&free_b, &total_b));
+            const size_t need = el * sizeof(S) + dbl * sizeof(double);
+            if (need > free_b)
+                throw CmfError(CMF_ERR_ARG, "sparse handle: the factors and work buffers need " + std::to_string(need) +
+                                                " bytes of device memory; " + std::to_string(free_b) + " bytes are free");
+        }
         CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         own_stream = true;
-        const int64_t hal = L - 1;
-        X.alloc((size_t)((Tl + hal) * N));
+        if (!sparse) X.alloc((size_t)((Tl + hal) * N));
+        else Wt.alloc((size_t)(KL() * N));
         Hbuf.alloc((size_t)((Tl + 2 * hal) * K));
         H = Hbuf.p + hal * K;
         Wi.alloc((size_t)(KL() * N));
@@ -337,7 +360,7 @@ struct Ctx : RankState {
         // the tensor-core engine is set up right away only where it is the default (big contractions); small problems
         // build it lazily on cmf_set_engine(h, 1)
         if constexpr (is_f32) {
-            if (N >= 256 && Tl >= 4096 && K * L >= 256) {
+            if (!sparse && N >= 256 && Tl >= 4096 && K * L >= 256) {
                 tc_setup();
                 // frequency-domain engine by default where it wins: enough lags that 2*L direct flops per element exceed the
                 // ~8.5 of the per-frequency products, and room for the spectrum of X (CMF_ENGINE_DEFAULT=1 keeps engine 1)
@@ -1220,9 +1243,10 @@ struct Ctx : RankState {
         CK(cudaMemcpyAsync(X_out, X.p, (size_t)(cols * N) * sizeof(S), cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
     }
-    void finish_data() {
+    void finish_data() { finish_data(data_sumsq()); }
+    void finish_data(double sumsq) {
         x_changed();
-        data_sumsq_local = data_sumsq();
+        data_sumsq_local = sumsq;
         data_norm = std::sqrt(data_sumsq_local);
         pgd_cur_loss = data_norm;
         have_data = true;
@@ -1232,6 +1256,70 @@ struct Ctx : RankState {
         post_launch();
         reduce_scalar(loss_part.p, 1024, scal.p);
         return fetch_scalar(scal.p);
+    }
+
+    // X as compressed sparse columns (include/cmf_sm100.h, cmf_set_data_csc).  Every check runs on the host before anything
+    // reaches the device; the CSR copy for numW is built here, once per data set, and ||X||^2 is summed in double from nzval.
+    void set_data_csc(int64_t nnz, const int64_t *colptr, const int64_t *rowval, const void *nzval, int base) {
+        REQUIRE(base == 0 || base == 1, "cmf_set_data_csc: index_base must be 0 or 1, got " + std::to_string(base));
+        REQUIRE(nnz >= 1, "cmf_set_data_csc: nnz must be >= 1 (the relative loss of an all-zero X is undefined)");
+        REQUIRE(colptr && rowval && nzval, "cmf_set_data_csc: null pointer");
+        REQUIRE(colptr[0] == base, "cmf_set_data_csc: colptr[0] = " + std::to_string(colptr[0]) + " must equal index_base " +
+                                       std::to_string(base));
+        REQUIRE(colptr[T] == nnz + base, "cmf_set_data_csc: colptr[T] = " + std::to_string(colptr[T]) + " must equal nnz + index_base = " +
+                                             std::to_string(nnz + base));
+        std::vector<int64_t> cp((size_t)(T + 1)), rp((size_t)(N + 1), 0);
+        std::vector<int> rv((size_t)nnz);
+        for (int64_t t = 0; t < T; ++t) {
+            const int64_t a = colptr[t] - base, b = colptr[t + 1] - base;
+            REQUIRE(a <= b && b <= nnz, "cmf_set_data_csc: colptr decreases or runs past nnz at column " + std::to_string(t));
+            cp[(size_t)t] = a;
+            for (int64_t i = a; i < b; ++i) {
+                const int64_t r = rowval[i] - base;
+                REQUIRE(r >= 0 && r < N, "cmf_set_data_csc: row index of entry " + std::to_string(i) + " (column " + std::to_string(t) +
+                                             ") is out of range");
+                REQUIRE(i == a || r > rv[(size_t)i - 1], "cmf_set_data_csc: row indices do not strictly increase in column " +
+                                                             std::to_string(t) + " (entry " + std::to_string(i) + ")");
+                rv[(size_t)i] = (int)r;
+                ++rp[(size_t)r + 1];
+            }
+        }
+        cp[(size_t)T] = nnz;
+        const size_t need = (size_t)(T + 1 + N + 1) * sizeof(int64_t) + (size_t)nnz * 2 * (sizeof(int) + sizeof(S));
+        const size_t held = (sp_colptr.n + sp_rowptr.n) * sizeof(int64_t) + (sp_rowval.n + sp_colidx.n) * sizeof(int) +
+                            (sp_val.n + sp_rval.n) * sizeof(S);
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        if (need > free_b + held)
+            throw CmfError(CMF_ERR_ARG, "cmf_set_data_csc: " + std::to_string(nnz) + " nonzeros need " + std::to_string(need) +
+                                            " bytes of device memory (CSC and CSR copies); " + std::to_string(free_b + held) +
+                                            " bytes are available");
+        // CSR copy: a counting sort by row; walking the columns in order leaves every row's times increasing
+        const S *v = static_cast<const S *>(nzval);
+        for (int64_t n = 0; n < N; ++n) rp[(size_t)n + 1] += rp[(size_t)n];
+        std::vector<int64_t> fill(rp.begin(), rp.end() - 1);
+        std::vector<int> ci((size_t)nnz);
+        std::vector<S> rvv((size_t)nnz);
+        double ss = 0.0;
+        for (int64_t t = 0; t < T; ++t)
+            for (int64_t i = cp[(size_t)t]; i < cp[(size_t)t + 1]; ++i) {
+                const int64_t dst = fill[(size_t)rv[(size_t)i]]++;
+                ci[(size_t)dst] = (int)t;
+                rvv[(size_t)dst] = v[i];
+                ss += (double)v[i] * (double)v[i];
+            }
+        auto put = [&](auto &buf, const auto *src, size_t count) {
+            if (buf.n != count) buf.alloc(count);
+            CK(cudaMemcpyAsync(buf.p, src, count * sizeof(*src), cudaMemcpyHostToDevice, stream));
+        };
+        put(sp_colptr, cp.data(), cp.size());
+        put(sp_rowval, rv.data(), rv.size());
+        put(sp_val, v, (size_t)nnz);
+        put(sp_rowptr, rp.data(), rp.size());
+        put(sp_colidx, ci.data(), ci.size());
+        put(sp_rval, rvv.data(), rvv.size());
+        CK(cudaStreamSynchronize(stream));
+        finish_data(ss);
     }
 
     void synth_data(uint64_t seed, int64_t Kt, int64_t Lt, double p_h, double noise) {
@@ -1286,6 +1374,12 @@ struct Ctx : RankState {
 
     void init_scale_partials(double out[2]) {
         REQUIRE(have_data && have_factors, "init_scale_partials: data and factors must be set");
+        if (sparse) {              // <X, est> = <numH, H>, ||est||^2 = <W W', Htilde Htilde'>: the terms of the expansion loss
+            loss_partial_dev();
+            CK(cudaMemcpyAsync(out, scal.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, stream));
+            CK(cudaStreamSynchronize(stream));
+            return;
+        }
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p);
         // partial layout: [2*b] = <est, X>, [2*b+1] = ||est||^2  -> de-interleave by strided sums
@@ -1330,6 +1424,7 @@ struct Ctx : RankState {
     DevBuf<int> b_col;               // [C]: the restart that owns each stacked component
     DevBuf<double> b_reg, b_vals;    // [R][4] = (l1W, l2W, l1H, l2H) per restart; R per-restart scalars
     DevBuf<int> b_active;            // 0 = the restart has converged: the updates leave its factors alone
+    DevBuf<double> b_dots;           // sparse batches: [R] <numH_r, H_r>, then [R] <S2_r, Gram_r> (the expansion loss)
     int64_t b_exch(int64_t Kr) const { return L * Kr * Kr + (L - 1) * Kr + 1; }   // doubles of one restart's Gram + H tail block in exch1
     int64_t b_tail_blocks(int64_t Kr) const { return cdiv((2 * L - 1) * Kr, 256); }
     GemmRows b_wrows() const { return GemmRows{N, INT64_MAX, b_C * N, RANK_W}; }   // W_r: rows l*K_r + k of restart r
@@ -1358,7 +1453,8 @@ struct Ctx : RankState {
         size_t tr_need = 0;
         launch_transconv(nullptr, nullptr, nullptr, N, b_C, L, N, Tl, Tl + hal, false, 0, &tr_need);
         const int nb = conv_nblocks(0, Tl);
-        take(X, (Tl + hal) * N);
+        if (!sparse) take(X, (Tl + hal) * N);
+        else take(Wt, KLR * N);
         take(Hbuf, (Tl + 2 * hal) * b_C);
         take(Wi, KLR * N); take(Wtmp, KLR * N); take(numW, KLR * N); take(denW, KLR * N);
         take(GS, e.gs);
@@ -1366,7 +1462,8 @@ struct Ctx : RankState {
         take(numH, Tl * b_C); take(denH, Tl * b_C);
         take(exch1, e.ex);
         take(corr_part, std::max<int64_t>((int64_t)nsplit_w * KLR * N, e.cp));
-        take(loss_part, std::max<int64_t>(2 * nb * R, 4096));
+        take(loss_part, std::max<int64_t>(sparse ? 2048 * R : 2 * nb * R, 4096));
+        if (sparse) take(b_dots, 2 * R);
         take(tail_part, e.tp);
         take(tr_part, (int64_t)tr_need);
         take(scal, 8);
@@ -1430,6 +1527,12 @@ struct Ctx : RankState {
     // init_scale_partials
     void batch_scale_partials(double *out) {
         REQUIRE(have_data && have_factors, "cmf_init_scale_partials_batch: data and factors must be set");
+        if (sparse) {              // <X, est_r> = <numH_r, H_r>, ||est_r||^2 = <S2_r, Gram_r>
+            std::vector<double> d((size_t)(2 * R));
+            batch_expansion(true, d.data());
+            for (int64_t r = 0; r < R; ++r) { out[2 * r] = d[(size_t)r]; out[2 * r + 1] = d[(size_t)(R + r)]; }
+            return;
+        }
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 16, nullptr, loss_part.p, 0, 0.0, true, 2 * nb);
         std::vector<double> hp((size_t)(2 * nb * R));
@@ -1453,8 +1556,16 @@ struct Ctx : RankState {
 
     // relative loss of every restart (mult.jl:55-57): one direct conv + residual pass with a restart index, one deterministic
     // reduction per restart, one copy of R doubles
-    void batch_loss(double *out) {
+    // after_update: called right after batch_update_feature_maps, whose numH and S2 = W W' a sparse batch reuses
+    void batch_loss(double *out, bool after_update = false) {
         REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
+        if (sparse) {              // ||X||^2 - 2 <numH_r, H_r> + <S2_r, Gram_r>
+            std::vector<double> d((size_t)(2 * R));
+            batch_expansion(!after_update, d.data());
+            for (int64_t r = 0; r < R; ++r)
+                out[r] = std::sqrt(std::max(data_sumsq_local - 2.0 * d[(size_t)r] + d[(size_t)(R + r)], 0.0)) / data_norm;
+            return;
+        }
         const int nb = conv_nblocks(0, Tl);
         launch_conv(Wi.p, H, K, L, -(L - 1), Tl + (L - 1), 0, Tl, 4, nullptr, loss_part.p, 0, 0.0, true, nb);
         reduce_scalar(loss_part.p, nb, b_vals.p, (int)R);
@@ -1470,16 +1581,41 @@ struct Ctx : RankState {
         CK(cudaStreamSynchronize(stream));
     }
 
-    // update_motifs! (mult.jl:23-39) of every active restart
-    void batch_update_motifs() {
-        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, b_C, b_C);          // numW, all restarts
+    // Gram_r and the H tail block of every restart into exch1
+    void batch_gram() {
         launch_corr(H, K, b_C, Tl + (L - 1), nsplit_g, split_g, nullptr, exch1.p, H, K, b_C, true);   // Gram_r
         if (L > 1) {
             h_tail_kernel<S><<<dim3((unsigned)cdiv((L - 1) * K, 256), (unsigned)R), 256, 0, stream>>>(H, exch1.p, K, L, Tl, 1, b_C,
                                                                                                    b_tab.p);
             post_launch();
         }
+    }
+
+    // sparse batches: out[r] = <numH_r, H_r>, out[R + r] = <S2_r, Gram_r> (host, 2R doubles), each a deterministic two-stage sum
+    // as in loss_partial_expansion_dev.  fresh: numH and S2 are recomputed for the current W first.
+    void batch_expansion(bool fresh, double *out) {
+        if (fresh) {
+            sparse_transconv(b_C);
+            launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), true);   // S2_r = W_r W_r'
+        }
+        batch_gram();
+        sp_seg_dot_partial_kernel<S><<<dim3(1024, (unsigned)R), 256, 0, stream>>>(numH.p, H, Tl, b_C, b_tab.p, loss_part.p);
+        post_launch();
+        reduce_scalar(loss_part.p, 1024, b_dots.p, (int)R);
+        s2_dot_G_diag_kernel<S><<<dim3(1024, (unsigned)R), 256, 0, stream>>>(GS.p, 0, 0, exch1.p, nullptr, K, L, loss_part.p + 1024 * R,
+                                                                             b_tab.p);
+        post_launch();
+        reduce_scalar(loss_part.p + 1024 * R, 1024, b_dots.p + R, (int)R);
+        CK(cudaMemcpyAsync(out, b_dots.p, (size_t)(2 * R) * sizeof(double), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+    }
+
+    // update_motifs! (mult.jl:23-39) of every active restart
+    void batch_update_motifs() {
+        REQUIRE(have_data && have_factors, "update: data and factors must be set first");
+        if (sparse) sparse_corr(b_C);                                                                       // numW, all restarts
+        else launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr, H, b_C, b_C);
+        batch_gram();
         build_G_kernel<S><<<dim3((unsigned)cdiv(KL() * KL(), 256), (unsigned)R), 256, 0, stream>>>(exch1.p, nullptr, GS.p, K, L,
                                                                                                     b_tab.p);
         post_launch();
@@ -1492,7 +1628,8 @@ struct Ctx : RankState {
     // update_feature_maps! (mult.jl:42-58, without the loss) of every active restart
     void batch_update_feature_maps() {
         REQUIRE(have_data && have_factors, "update: data and factors must be set first");
-        launch_transconv(Wi.p, X.p, numH.p, N, b_C, L, N, Tl, Tl + (L - 1));                                // numH, all restarts
+        if (sparse) sparse_transconv(b_C);                                                                  // numH, all restarts
+        else launch_transconv(Wi.p, X.p, numH.p, N, b_C, L, N, Tl, Tl + (L - 1));
         launch_gemm_rows<true>(Wi.p, Wi.p, GS.p, KL(), KL(), N, b_wrows(), b_wrows(), b_grows(), true);       // S2_r = W_r W_r'
         lag_table_kernel<S><<<dim3((unsigned)cdiv((2 * L - 1) * K * K, 256), (unsigned)R), 256, 0, stream>>>(GS.p, Cf.p, K, L, K, KL(),
                                                                                                           b_tab.p);
@@ -1516,14 +1653,39 @@ struct Ctx : RankState {
     // Each contraction picks its engine here and nowhere else: SIMT unless the tensor cores are on (never on fp64 handles),
     // then the frequency-domain engine where it is active, the time-domain one otherwise.
 
+    // sparse handles (kernels_sparse.cuh), C components (K, or the stacked C = sum K_r of a batch): numW from the CSR copy in
+    // the time splits of the dense correlation, added in order
+    void sparse_corr(int64_t C) {
+        const int64_t LC = L * C, n = LC * N;
+        dim3 grid((unsigned)cdiv(N, SP_WARPS), (unsigned)cdiv(LC, 32 * SP_A), (unsigned)nsplit_w);
+        prof_begin(PROF_CORR);
+        sp_corr_kernel<S><<<grid, 32 * SP_WARPS, 0, stream>>>(sp_rowptr.p, sp_colidx.p, sp_rval.p, H, C, C, L, N, split_w, corr_part.p);
+        prof_end();
+        post_launch();
+        reduce_partials_kernel<S><<<(unsigned)cdiv(n, 256), 256, 0, stream>>>(corr_part.p, nsplit_w, n, numW.p, nullptr);
+        post_launch();
+    }
+    // numH from the CSC arrays and W transposed to [n][l*K + k]
+    void sparse_transconv(int64_t C) {
+        sp_w_transpose_kernel<S><<<dim3((unsigned)cdiv(N, 32), (unsigned)cdiv(L * C, 32)), dim3(32, 8), 0, stream>>>(Wi.p, Wt.p, L * C, N);
+        post_launch();
+        prof_begin(PROF_TRANSCONV);
+        sp_transconv_kernel<S><<<dim3((unsigned)cdiv(Tl, SP_WARPS), (unsigned)cdiv(C, 32)), 32 * SP_WARPS, 0, stream>>>(
+            sp_colptr.p, sp_rowval.p, sp_val.p, Wt.p, C, L, Tl, T, numH.p, C);
+        prof_end();
+        post_launch();
+    }
+
     // numW partial over the owned u (mult.jl:32): Xin = X incl. right halo
     void compute_numW() {
-        if (!tc_active()) launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
+        if (sparse) sparse_corr(K);
+        else if (!tc_active()) launch_corr(X.p, N, N, Tl + (L - 1), nsplit_w, split_w, numW.p, nullptr);
         else if constexpr (is_f32) { if (fd_active()) fd_corr(); else tc_corr(); }
     }
     // numH (mult.jl:47)
     void compute_numH() {
-        if (!tc_active()) launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
+        if (sparse) sparse_transconv(K);
+        else if (!tc_active()) launch_transconv(Wi.p, X.p, numH.p, N, K, L, N, Tl, Tl + (L - 1));
         else if constexpr (is_f32) { if (fd_active()) fd_transconv(); else tc_transconv(); }
     }
     // denomW = G * Wi (mult.jl:28,33) for the unfolded rows [j0, j1); the frequency-domain engine runs it in the time domain
@@ -1641,6 +1803,11 @@ struct Ctx : RankState {
     // scal[1] is zeroed in the direct case so that a fixed-size all-reduce of two doubles serves both.
     int loss_partial_dev() {
         REQUIRE(have_data && have_factors, "loss: data and factors must be set first");
+        if (sparse) {              // no dense X for a direct pass: always the expansion, numH and W W' recomputed when stale
+            if (!numH_valid) { compute_numH(); lag_tables(); numH_valid = true; numH_dot_valid = false; }
+            loss_partial_expansion_dev();
+            return 2;
+        }
         if (loss_mode == 1 && tc_active()) {
             // frequency-domain engine: numH and W W' are cheap, so the expansion also serves calls that find them stale
             // (the loss at the initial factors, after a W-only step, after the HALS sweep overwrote numH)
@@ -1969,7 +2136,7 @@ struct Ctx : RankState {
 // (`ranks`, non-empty) and K = their maximum.
 template <typename S>
 std::unique_ptr<Ctx<S>> make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg,
-                                 int device, const std::vector<int64_t> &ranks = {}) {
+                                 int device, const std::vector<int64_t> &ranks = {}, bool sparse = false) {
     REQUIRE(N >= 1 && K >= 1 && L >= 1 && T >= 1, "dimensions must be positive");
     REQUIRE(L <= T, "need L <= T (src/common.jl:28-31)");
     REQUIRE(0 <= t0 && t0 < t1 && t1 <= T, "bad shard range");
@@ -1992,6 +2159,8 @@ std::unique_ptr<Ctx<S>> make_ctx(int64_t N, int64_t T, int64_t t0, int64_t t1, i
     c->R = (int64_t)ranks.size();
     c->b_K = ranks;
     c->b_C = std::accumulate(ranks.begin(), ranks.end(), (int64_t)0);
+    c->sparse = sparse;
+    if (sparse) { c->loss_mode = 1; c->loss_mode_explicit = true; }   // the expansion is the only loss of sparse data
     c->init();
     return c;
 }
@@ -2158,7 +2327,7 @@ double r_loss_sumsq(Ctx<S> &ctx, bool force_direct = false, bool *expansion_used
 // at calibration points are the direct pass itself.  Every rank sees the same all-reduced numbers and takes the same branch.
 template <typename S>
 double r_guarded_loss(Ctx<S> &ctx) {
-    if (ctx.loss_mode != 1) return std::sqrt(std::max(r_loss_sumsq(ctx), 0.0)) / ctx.data_norm;
+    if (ctx.loss_mode != 1 || ctx.sparse) return std::sqrt(std::max(r_loss_sumsq(ctx), 0.0)) / ctx.data_norm;
     bool exp_used = false;
     const double se = r_loss_sumsq(ctx, false, &exp_used);
     if (!exp_used) return std::sqrt(std::max(se, 0.0)) / ctx.data_norm;
@@ -2331,6 +2500,10 @@ template <typename S>
 void r_set_engine(Ctx<S> &ctx, int engine) {
     REQUIRE(engine >= 0 && engine <= 2, "engine must be 0 (SIMT), 1 (tcgen05, time domain) or 2 (tcgen05, frequency domain)");
     if (ctx.R > 0 && engine != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles run the SIMT engine (0) only");
+    if (ctx.sparse) {
+        if (engine != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "sparse handles (cmf_create_sparse) run the SIMT engine (0) only");
+        return;
+    }
     if (engine == 2 && !ctx.fd_available())
         throw CmfError(CMF_ERR_UNSUPPORTED, "the frequency-domain engine needs an fp32 handle with K <= 128, L <= 256, N % 8 == 0 on sm_100 and room for the spectrum of X");
     if (engine < 2) ctx.fd_release();               // the spectrum of X and the time-domain planes never coexist
@@ -2387,7 +2560,7 @@ void b_fit(Ctx<S> &ctx, int64_t max_itr, double max_time, int eval_mode, int che
         auto t_start = std::chrono::steady_clock::now();
         if (!eval_mode) ctx.batch_update_motifs();
         ctx.batch_update_feature_maps();
-        ctx.batch_loss(loss.data());
+        ctx.batch_loss(loss.data(), true);
         time_hist.push_back(time_hist.back() + std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count());
         bool stopped = false;
         for (int64_t r = 0; r < R; ++r) {
@@ -2487,13 +2660,26 @@ void batch_handle(cmf_handle h) { REQUIRE(h && first(h).R > 0, "not a batch hand
 
 // a handle of one rank context (make_ctx's checks)
 cmf_ctx *make_handle(int64_t N, int64_t T, int64_t t0, int64_t t1, int64_t K, int64_t L, int dtype, int alg, int device,
-                     const std::vector<int64_t> &ranks = {}) {
-    return with_dtype(dtype, [&](auto s) { return handle_of(make_ctx<decltype(s)>(N, T, t0, t1, K, L, dtype, alg, device, ranks)); });
+                     const std::vector<int64_t> &ranks = {}, bool sparse = false) {
+    return with_dtype(dtype, [&](auto s) { return handle_of(make_ctx<decltype(s)>(N, T, t0, t1, K, L, dtype, alg, device, ranks, sparse)); });
+}
+
+// the checks cmf_create_sparse / cmf_create_batch_sparse add to make_ctx's (before any device query)
+void sparse_checks(int64_t N, int64_t T, int alg) {
+    REQUIRE(alg == CMF_MULT || alg == CMF_HALS || alg == CMF_PGD, "alg must be 0 (mult), 1 (hals) or 2 (pgd)");
+    if (alg == CMF_PGD) throw CmfError(CMF_ERR_UNSUPPORTED, "sparse data serve MultUpdate and HALSUpdate (PGD needs the dense X)");
+    REQUIRE(N <= INT32_MAX && T <= INT32_MAX, "sparse handles need N <= INT32_MAX and T <= INT32_MAX (int32 indices on the device)");
+}
+// a sparse handle refuses the calls that need the dense X
+void dense_data(cmf_handle h, const char *call) {
+    if (h && first(h).sparse)
+        throw CmfError(CMF_ERR_ARG, std::string(call) + " needs a dense X: this is a sparse handle (cmf_create_sparse), give the data with cmf_set_data_csc");
 }
 
 // cmf_create_batch and cmf_create_batch_ranks (after their checks of R): restart r has rank ranks[r].  Every check runs
 // before any device query.
-cmf_ctx *make_batch(int64_t N, int64_t T, const std::vector<int64_t> &ranks, int64_t L, int dtype, int alg, int device) {
+cmf_ctx *make_batch(int64_t N, int64_t T, const std::vector<int64_t> &ranks, int64_t L, int dtype, int alg, int device,
+                    bool sparse = false) {
     REQUIRE(alg == CMF_MULT || alg == CMF_HALS || alg == CMF_PGD, "alg must be 0 (mult), 1 (hals) or 2 (pgd)");
     if (alg != CMF_MULT)
         throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts serve MultUpdate only (HALS sweeps run sequentially per restart; PGD is not batched)");
@@ -2505,7 +2691,7 @@ cmf_ctx *make_batch(int64_t N, int64_t T, const std::vector<int64_t> &ranks, int
     const int64_t C = std::accumulate(ranks.begin(), ranks.end(), (int64_t)0), Kmax = *std::max_element(ranks.begin(), ranks.end());
     REQUIRE(C * cdiv(L, 8) <= (int64_t)CORR_PB * 65535 && C <= 4 * 65535, "R*K too large for one launch grid (the ranks of all restarts add up to " + std::to_string(C) + ")");
     if (L > 769) throw CmfError(CMF_ERR_UNSUPPORTED, "batched restarts need L <= 769");
-    return make_handle(N, T, 0, T, Kmax, L, dtype, alg, device, ranks);
+    return make_handle(N, T, 0, T, Kmax, L, dtype, alg, device, ranks, sparse);
 }
 
 }  // namespace
@@ -2660,10 +2846,21 @@ int cmf_destroy(cmf_handle h) {
 }
 
 int cmf_set_data(cmf_handle h, const void *X, int64_t first_col) {
-    return guarded([&] { on_ranks(h, [&](auto &r) { r.set_data(X, first_col); r_data_norm(r); }); });
+    return guarded([&] { dense_data(h, "cmf_set_data"); on_ranks(h, [&](auto &r) { r.set_data(X, first_col); r_data_norm(r); }); });
 }
 int cmf_synth_data(cmf_handle h, uint64_t seed, int64_t K_true, int64_t L_true, double p_h, double noise) {
-    return guarded([&] { on_ranks(h, [&](auto &r) { r.synth_data(seed, K_true, L_true, p_h, noise); r_data_norm(r); }); });
+    return guarded([&] {
+        dense_data(h, "cmf_synth_data");
+        on_ranks(h, [&](auto &r) { r.synth_data(seed, K_true, L_true, p_h, noise); r_data_norm(r); });
+    });
+}
+int cmf_set_data_csc(cmf_handle h, int64_t nnz, const int64_t *colptr, const int64_t *rowval, const void *nzval, int index_base) {
+    return guarded([&] {
+        REQUIRE(h, "null handle");
+        if (!first(h).sparse)
+            throw CmfError(CMF_ERR_ARG, "cmf_set_data_csc needs a sparse handle: create it with cmf_create_sparse or cmf_create_batch_sparse");
+        on_ranks(h, [&](auto &r) { r.set_data_csc(nnz, colptr, rowval, nzval, index_base); r_data_norm(r); });
+    });
 }
 int cmf_data_sumsq(cmf_handle h, double *out) {
     return guarded([&] {
@@ -2794,6 +2991,7 @@ int cmf_stream(cmf_handle h, void **stream_out) {
 int cmf_get_data(cmf_handle h, void *X_out, int with_halo) {
     return guarded([&] {
         REQUIRE(X_out, "null output");
+        dense_data(h, "cmf_get_data");
         on_ranks(h, [&](auto &r) {
             REQUIRE(r.have_data, "no data");
             // several rank contexts fill one N x T array: no halos
@@ -2848,7 +3046,9 @@ int cmf_set_engine(cmf_handle h, int engine) {
 int cmf_set_loss_mode(cmf_handle h, int mode) {
     return guarded([&] {
         REQUIRE(mode == 0 || mode == 1, "loss mode must be 0 (direct) or 1 (expansion)");
-        if (h && first(h).R > 0 && mode != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles evaluate the loss by the direct pass (mode 0) only");
+        if (h && first(h).sparse && mode != 1)
+            throw CmfError(CMF_ERR_UNSUPPORTED, "sparse handles evaluate the loss by the expansion (mode 1) only: the direct pass needs the dense X");
+        if (h && first(h).R > 0 && !first(h).sparse && mode != 0) throw CmfError(CMF_ERR_UNSUPPORTED, "batch handles evaluate the loss by the direct pass (mode 0) only");
         on_ranks(h, [&](auto &r) { r.loss_mode = mode; r.loss_mode_explicit = true; r.calib_reset(); });
     });
 }
@@ -2856,6 +3056,8 @@ int cmf_set_loss_guard(cmf_handle h, double guard, int max_interval) {
     return guarded([&] {
         REQUIRE(guard >= 0.0, "loss guard must be >= 0");
         REQUIRE(max_interval >= 1 && max_interval <= 1024, "calibration interval must be in [1, 1024]");
+        if (h && first(h).sparse)
+            throw CmfError(CMF_ERR_UNSUPPORTED, "sparse handles have no calibrated loss: the expansion is their only loss (no direct pass)");
         on_ranks(h, [&](auto &r) { r.loss_guard = guard; r.calib_max_interval = max_interval; r.calib_reset(); });
     });
 }
@@ -2966,6 +3168,25 @@ int cmf_create_batch_ranks(cmf_handle *out, int64_t N, int64_t T, const int64_t 
         REQUIRE(R >= 1 && R <= 32768, "R (restarts) must be in 1..32768");
         DevRestore g;
         *out = make_batch(N, T, std::vector<int64_t>(K, K + R), L, dtype, alg, device);
+    });
+}
+int cmf_create_sparse(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int dtype, int alg, int device) {
+    return guarded([&] {
+        REQUIRE(out != nullptr, "null output pointer");
+        sparse_checks(N, T, alg);
+        DevRestore g;
+        *out = make_handle(N, T, 0, T, K, L, dtype, alg, device, {}, true);
+    });
+}
+int cmf_create_batch_sparse(cmf_handle *out, int64_t N, int64_t T, const int64_t *K, int64_t L, int dtype, int alg, int64_t R,
+                            int device) {
+    return guarded([&] {
+        REQUIRE(out != nullptr, "null output pointer");
+        REQUIRE(K != nullptr, "null rank array K");
+        REQUIRE(R >= 1 && R <= 32768, "R (restarts) must be in 1..32768");
+        sparse_checks(N, T, alg);
+        DevRestore g;
+        *out = make_batch(N, T, std::vector<int64_t>(K, K + R), L, dtype, alg, device, true);
     });
 }
 int cmf_set_factors_batch(cmf_handle h, const void *W, const void *H) {

@@ -640,10 +640,18 @@ __global__ void build_G_kernel(const double *__restrict__ Rg, const double *__re
 // where the Toeplitz part is constant and the tail grows by one product per step,
 //   tail(l+1, l'+1) = tail(l, l') + Ht[L-2-l][k] Ht[L-2-l'][k'],
 // so every element of S2 is read once and the (K L)^2 L tail work becomes (K L)^2.  grid-stride over (2L-1) K K diagonals.
+// Restart y = blockIdx.y of a batch handle (tab != nullptr): K = Ks = K_r, ld = K_r L, S2 + gs_r, its Gram at Rg + ex_r with the
+// tail right after it; its partials at partial + y * gridDim.x.
 template <typename S>
 __global__ void s2_dot_G_diag_kernel(const S *__restrict__ S2, int64_t Ks, int64_t ld, const double *__restrict__ Rg,
-                                     const double *__restrict__ Ht, int64_t K, int64_t L, double *__restrict__ partial) {
+                                     const double *__restrict__ Ht, int64_t K, int64_t L, double *__restrict__ partial,
+                                     const BatchRest *tab = nullptr) {
     __shared__ double red[32];
+    if (tab) {
+        const BatchRest r = tab[blockIdx.y];
+        K = Ks = r.K; ld = r.K * L; S2 += r.gs; Rg += r.ex; Ht = Rg + L * K * K;
+        partial += (int64_t)blockIdx.y * gridDim.x;
+    }
     double acc = 0.0;
     const int64_t total = (2 * L - 1) * K * K;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {

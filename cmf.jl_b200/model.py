@@ -75,6 +75,61 @@ def num_iter(r):        # src/model.jl:30
     return len(r.loss_hist)
 
 
+class SparseData:
+    """X as canonical compressed sparse columns (column t = time bin t): ``colptr`` (T+1), ``rowval`` and ``nzval`` (nnz),
+    0-based int64 indices, rows strictly increasing in every column, no explicit zeros, values of the handle dtype."""
+
+    def __init__(self, shape, colptr, rowval, nzval):
+        self.shape, self.colptr, self.rowval, self.nzval = shape, colptr, rowval, nzval
+        self.ndim = 2
+
+    @property
+    def nnz(self):
+        return len(self.nzval)
+
+
+def _is_sparse(data):
+    return isinstance(data, SparseData) or type(data).__module__.startswith("scipy.sparse")
+
+
+def as_csc(data, dtype="f64"):
+    """Any ``scipy.sparse`` matrix or array -> ``SparseData`` in the handle dtype: duplicates summed, indices sorted, explicit
+    zeros dropped.  None for dense data (scipy is imported only here, so dense-only use does not need it)."""
+    if isinstance(data, SparseData) or not _is_sparse(data):
+        return data if isinstance(data, SparseData) else None
+    import scipy.sparse as sp
+
+    X = sp.csc_matrix(data, dtype=np.float64, copy=True)
+    X.sum_duplicates()                    # also sorts the row indices of every column
+    X = X.astype(np_dtype(parse_dtype(dtype)))
+    X.eliminate_zeros()
+    return SparseData(X.shape, X.indptr.astype(np.int64), X.indices.astype(np.int64), np.ascontiguousarray(X.data))
+
+
+def _data_shape(data):
+    """(N, T) of a dense or sparse ``data`` argument; ValueError when it is not a matrix."""
+    shape = data.shape if _is_sparse(data) else np.shape(data)
+    if len(shape) != 2:
+        raise ValueError("data must be an N x T matrix")
+    return tuple(int(d) for d in shape)
+
+
+def _check_sparse_rule(sparse, rule_cls, ngpu):
+    """Sparse data serve MultUpdate and HALSUpdate on one GPU: the same refusal (code 3) as the library's."""
+    if not sparse:
+        return
+    if rule_cls is PGDUpdate:
+        raise CMFError(3, "sparse data serve MultUpdate and HALSUpdate (PGD needs the dense X)")
+    if int(ngpu or 1) > 1:
+        raise CMFError(3, "sparse data run on one GPU")
+
+
+def _set_csc(h, csc):
+    i64 = ctypes.POINTER(ctypes.c_int64)
+    check(_lib.load().cmf_set_data_csc(h, csc.nnz, csc.colptr.ctypes.data_as(i64), csc.rowval.ctypes.data_as(i64),
+                                       fptr(csc.nzval), 0))
+
+
 def _emit(printer, s, nl=True):
     if printer is print:
         print(s, end="\n" if nl else "", flush=True)
@@ -111,22 +166,30 @@ class AbstractCFUpdate:
     def __init__(self, data, W, H, dtype="f64", device=0, sync_host=True, engine=None, loss_mode=None, ngpu=1,
                  devices=None, loss_guard=None):
         """``ngpu > 1``: the rule spans ``ngpu`` GPUs (time axis sharded inside the library, NCCL collectives driven
-        from this one thread -- cmf_create_multi); every other argument and every method is unchanged."""
-        lib = _lib.load()
+        from this one thread -- cmf_create_multi); every other argument and every method is unchanged.  ``data`` may be a
+        ``scipy.sparse`` matrix or array (MultUpdate / HALSUpdate, one GPU): the handle then holds X as compressed sparse
+        columns and never densifies it (cmf_create_sparse)."""
+        self._h = ctypes.c_void_p()
         self.dtype = parse_dtype(dtype)
-        data = np.asarray(data)
+        csc = as_csc(data, self.dtype)
+        if csc is None:
+            data = np.asarray(data)
         W = np.asarray(W)
         H = np.asarray(H)
-        if data.ndim != 2 or W.ndim != 3 or H.ndim != 2:
+        if len(data.shape) != 2 or W.ndim != 3 or H.ndim != 2:
             raise ValueError("expected data N x T, W K x N x L, H K x T")
         K, N, L = W.shape
         if data.shape[0] != N or H.shape[0] != K or H.shape[1] != data.shape[1]:
             raise ValueError(f"dimension mismatch: data {data.shape}, W {W.shape}, H {H.shape}")
+        ngpu = int(ngpu or 1)
+        _check_sparse_rule(csc is not None, type(self), ngpu)
+        lib = _lib.load()
         self.N, self.T, self.K, self.L = N, data.shape[1], K, L
         self.sync_host = sync_host
-        self._h = ctypes.c_void_p()
-        ngpu = int(ngpu or 1)
-        if ngpu > 1:
+        if csc is not None:
+            check(lib.cmf_create_sparse(ctypes.byref(self._h), N, self.T, K, L, self.dtype, self._ALG,
+                                        device if devices is None else devices[0]))
+        elif ngpu > 1:
             devs = (ctypes.c_int * ngpu)(*(devices if devices is not None else range(ngpu)))
             check(lib.cmf_create_multi(ctypes.byref(self._h), N, self.T, K, L, self.dtype, self._ALG, ngpu, devs))
         else:
@@ -138,8 +201,10 @@ class AbstractCFUpdate:
             check(lib.cmf_set_loss_mode(self._h, int(loss_mode)))
         if loss_guard is not None:
             check(lib.cmf_set_loss_guard(self._h, float(loss_guard), 16))
-        Xj = julia_array(data, self.dtype)
-        check(lib.cmf_set_data(self._h, fptr(Xj), 0))
+        if csc is not None:
+            _set_csc(self._h, csc)
+        else:
+            check(lib.cmf_set_data(self._h, fptr(julia_array(data, self.dtype)), 0))
         self.set_factors(W, H)
 
     # -- plumbing ------------------------------------------------------------------------
@@ -311,9 +376,10 @@ def fit(alg, data, L, K, W_init, H_init, verbose=False, printer=print, layout="L
 def init_rand(data, L, K, seed=None, dtype="f64", device=0):
     """src/model.jl:113-125.  Uniform draws come from numpy's Generator (Julia's stream cannot be
     reproduced outside Julia; the Julia shim keeps its own ``rand``); the conv and the two
-    reductions of the alpha rescale run on the GPU.  Returns (W K x N x L, H K x T)."""
-    data = np.asarray(data)
-    N, T = data.shape
+    reductions of the alpha rescale run on the GPU.  Returns (W K x N x L, H K x T).  ``data`` may be sparse."""
+    if not _is_sparse(data):
+        data = np.asarray(data)
+    N, T = _data_shape(data)
     rng = np.random.default_rng(seed)
     W = rng.random((K, N, L))             # W drawn first (model.jl:116), then H (:117)
     H = rng.random((K, T))
@@ -340,7 +406,9 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
 
     Extra keywords of this implementation: ``dtype`` ("f64" default, "f32"), ``device``,
     ``layout`` ("LNK" default -- W returned as L x N x K as in the README -- or "KNL"), ``ngpu`` / ``devices``
-    (the fit runs T-sharded over that many GPUs inside the same single library call; MultUpdate and HALSUpdate)."""
+    (the fit runs T-sharded over that many GPUs inside the same single library call; MultUpdate and HALSUpdate).
+    ``data`` may be a ``scipy.sparse`` matrix or array (MultUpdate / HALSUpdate, one GPU): X is then never densified;
+    ``CNMF_results.data`` is the caller's matrix."""
     kw = _normalise_kwargs(kwargs)
     printer = kw.get("printer", print)
     verbose = kw.get("verbose", False)
@@ -350,11 +418,18 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
     dtype = parse_dtype(kw.get("dtype", "f64"))
     device = kw.get("device", 0)
     rule_cls = _resolve_alg(alg)
-    data = np.asarray(data)
-    if data.ndim != 2:
-        raise ValueError("data must be an N x T matrix")
-    N, T = data.shape
+    data_in = data
+    sparse = _is_sparse(data)
+    if not sparse:
+        data = np.asarray(data)
+    N, T = _data_shape(data)
     L, K = int(L), int(K)
+    _check_sparse_rule(sparse, rule_cls, kw.get("ngpu", 1))
+    if sparse:
+        W0, H0 = kw.get("W_init"), kw.get("H_init")
+        if (W0 is not None and np.shape(W0) != (K, N, L)) or (H0 is not None and np.shape(H0) != (K, T)):
+            raise ValueError(f"W_init must be {(K, N, L)} and H_init {(K, T)}; got {np.shape(W0)}, {np.shape(H0)}")
+        data = as_csc(data, dtype)
 
     rng = np.random.default_rng(kw.get("seed"))      # model.jl:64-67
     W0 = kw.get("W_init")
@@ -412,7 +487,7 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
         rule.close()
     if layout == "LNK":
         W = np.ascontiguousarray(W.transpose(2, 1, 0))
-    res = CNMF_results(data, W, H, list(time_hist[: n.value]), list(loss_hist[: n.value]), layout)
+    res = CNMF_results(data_in, W, H, list(time_hist[: n.value]), list(loss_hist[: n.value]), layout)
     res.engine_info = stats      # not part of the reference struct: which engine / loss path produced loss_hist (ADVICE r1)
     return res
 
@@ -449,7 +524,10 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
 
     ``K`` may also be a sequence of R positive ranks (a sweep over K in one handle, cmf_create_batch_ranks): restart r
     then has rank ``K[r]``, ``seeds`` has R entries, and ``W_init`` / ``H_init`` are sequences of R arrays of shapes
-    ``K[r] x N x L`` and ``K[r] x T``."""
+    ``K[r] x N x L`` and ``K[r] x T``.
+
+    ``data`` may be a ``scipy.sparse`` matrix or array (cmf_create_batch_sparse): X is stored once as compressed sparse
+    columns and never densified."""
     kw = _normalise_kwargs(kwargs)
     printer = kw.get("printer", print)
     verbose = kw.get("verbose", False)
@@ -459,11 +537,13 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
     dtype = parse_dtype(kw.get("dtype", "f64"))
     device = kw.get("device", 0)
     rule_cls = _resolve_alg(alg)
-    data = np.asarray(data)
-    if data.ndim != 2:
-        raise ValueError("data must be an N x T matrix")
-    N, T = data.shape
+    data_in = data
+    sparse = _is_sparse(data)
+    if not sparse:
+        data = np.asarray(data)
+    N, T = _data_shape(data)
     L = int(L)
+    _check_sparse_rule(sparse, rule_cls, 1)
     ranks = None if np.ndim(K) == 0 else _batch_ranks(K)
     K = int(K) if ranks is None else None
     W0, H0 = kw.get("W_init"), kw.get("H_init")
@@ -508,9 +588,15 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
     Wj = np.concatenate([julia_array(w, dtype).ravel(order="F") for w in W0])
     Hj = np.concatenate([julia_array(x, dtype).ravel(order="F") for x in H0])
 
+    if sparse:
+        data = as_csc(data, dtype)
     lib = _lib.load()
     h = ctypes.c_void_p()
-    if ranks is None:
+    if sparse:
+        rk = np.asarray(Ks, dtype=np.int64)
+        check(lib.cmf_create_batch_sparse(ctypes.byref(h), N, T, rk.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), L, dtype,
+                                          rule_cls._ALG, R, device))
+    elif ranks is None:
         check(lib.cmf_create_batch(ctypes.byref(h), N, T, K, L, dtype, rule_cls._ALG, R, device))
     else:
         rk = np.asarray(ranks, dtype=np.int64)
@@ -522,7 +608,10 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
             check(lib.cmf_set_engine(h, int(kw["engine"])))
         if kw.get("loss_mode") is not None:
             check(lib.cmf_set_loss_mode(h, int(kw["loss_mode"])))
-        check(lib.cmf_set_data(h, fptr(julia_array(data, dtype)), 0))
+        if sparse:
+            _set_csc(h, data)
+        else:
+            check(lib.cmf_set_data(h, fptr(julia_array(data, dtype)), 0))
         check(lib.cmf_set_factors_batch(h, fptr(Wj), fptr(Hj)))
         if seeds is not None:                             # model.jl:119-122, per restart
             part = np.zeros(2 * R)
@@ -562,8 +651,9 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
         H = Ho[T * o: T * (o + k)].reshape((k, T), order="F")
         W = np.ascontiguousarray(W.transpose(2, 1, 0)) if layout == "LNK" else np.asfortranarray(W)
         nr = int(n[r])
-        res = CNMF_results(data, W, H, list(time_hist[:nr]), list(loss_hist[r * cap: r * cap + nr]), layout)
-        res.engine_info = dict(direct=nr, expansion=0, interval=0, last_err=0.0, engine=0, loss_mode=0, restarts=R)
+        res = CNMF_results(data_in, W, H, list(time_hist[:nr]), list(loss_hist[r * cap: r * cap + nr]), layout)
+        res.engine_info = dict(direct=0 if sparse else nr, expansion=nr if sparse else 0, interval=0, last_err=0.0, engine=0,
+                               loss_mode=int(sparse), restarts=R)
         out.append(res)
     return out
 

@@ -217,6 +217,48 @@ int cmf_fit_batch(cmf_handle h, int64_t max_itr, double max_time, int eval_mode,
                   double *loss_hist /* R x cap, restart-major */, double *time_hist /* cap */, int64_t cap,
                   int64_t *n_hist /* R */, int *converged_early /* R */);
 
+/* ---- sparse data: X given as compressed sparse columns, the dense N x T X never allocated ---------------------------
+ *
+ * Spike rasters and event trains are mostly zeros.  A sparse handle holds X as CSC (and a CSR copy built from it, for numW),
+ * with int32 row / time indices on the device, and computes the two contractions that read X -- numW (mult.jl:32) and numH
+ * (mult.jl:47) -- with nnz K L multiply-adds each instead of N T K L.  Everything else touches W and H only and is unchanged.
+ *
+ * Rules of a sparse handle:
+ *  - The SIMT engine (0) only: cmf_set_engine(h, 1 | 2) returns CMF_ERR_UNSUPPORTED, cmf_get_engine reports 0.
+ *  - The loss is always the expansion ||X||^2 - 2 <numH, H> + <W W', Htilde Htilde'>, each term summed in double (||X||^2 from
+ *    nzval, once per data set): the direct pass would need the dense residual.  cmf_get_loss_mode reports 1,
+ *    cmf_set_loss_mode(h, 0) and cmf_set_loss_guard return CMF_ERR_UNSUPPORTED (there is no calibration), and
+ *    cmf_get_loss_stats counts expansions.  cmf_init_scale_partials[_batch] use the same identities:
+ *    <X, est> = <numH, H>, ||est||^2 = <W W', Htilde Htilde'>.
+ *  - cmf_set_data, cmf_synth_data and cmf_get_data need the dense X and return CMF_ERR_ARG naming cmf_set_data_csc.
+ *  - Every other call works as on a dense handle of the same kind (single or batch), including the split-phase diagnostics
+ *    cmf_w_partials / cmf_h_update + cmf_exchange_buffer on a single handle.
+ *  - MultUpdate and HALSUpdate (batches: MultUpdate), one GPU, one shard.  PGD: CMF_ERR_UNSUPPORTED.
+ *  - The footprint of the factors and work buffers (as for a dense handle, without X, plus a transposed copy of W) is checked
+ *    at creation, that of the CSC and CSR arrays (2 nnz (4 + sizeof(dtype)) + 8 (N + T + 2) bytes) by cmf_set_data_csc; either
+ *    fails with CMF_ERR_ARG and a message stating the bytes needed. */
+
+/* A handle whose data are given as a sparse matrix (cmf_set_data_csc): the dense N x T X is never allocated.
+ * alg: CMF_MULT or CMF_HALS (CMF_PGD: CMF_ERR_UNSUPPORTED).  One GPU, one shard.  N <= INT32_MAX, T <= INT32_MAX.  The checks
+ * of cmf_create, all before any device query. */
+int cmf_create_sparse(cmf_handle *out, int64_t N, int64_t T, int64_t K, int64_t L, int dtype, int alg, int device);
+
+/* Batch form (R MultUpdate restarts of one sparse data set, restart r with rank K[r]); the checks of cmf_create_batch_ranks
+ * and of cmf_create_sparse.  numW and numH of all restarts are one sparse launch each (X is read once per step). */
+int cmf_create_batch_sparse(cmf_handle *out, int64_t N, int64_t T, const int64_t *K /* R */, int64_t L, int dtype, int alg,
+                            int64_t R, int device);
+
+/* X as compressed sparse columns, column t = time bin t, exactly Julia's SparseMatrixCSC{T,Int64} layout:
+ * the entries of column t are colptr[t] .. colptr[t+1]-1 (minus index_base), with row indices rowval[] and values nzval[]
+ * of the handle dtype.  index_base = 1 lets Julia pass its arrays unchanged; 0 for scipy.  Row indices strictly increasing
+ * within a column (no duplicates).  Replaces the data (any nnz).  Sparse handles only (a dense handle: CMF_ERR_ARG naming
+ * cmf_create_sparse).  Checked on the host before anything reaches the device, CMF_ERR_ARG with a message naming the first
+ * offending column or entry: index_base is 0 or 1; colptr starts at the base, never decreases and ends at nnz + base; every
+ * row index is in range; row indices strictly increase within each column; nnz >= 1 (the relative loss of an all-zero X is
+ * undefined). */
+int cmf_set_data_csc(cmf_handle h, int64_t nnz, const int64_t *colptr /* T+1 */, const int64_t *rowval /* nnz */,
+                     const void *nzval /* nnz */, int index_base);
+
 /* ---- split-phase steps for time-sharded fits (MultUpdate only) -------------------------- */
 
 /* 1. local W-side partials: numW (src/algs/mult.jl:32), the H cross-correlation that yields

@@ -6,9 +6,12 @@
 #   * `SM100MultUpdate <: CMF.AbstractCFUpdate`, `SM100HALSUpdate` -- the update-rule plugin interface
 #     (src/algs/alternating.jl:8, constructor call at src/model.jl:79, method calls at alternating.jl:52,54)
 #   * `fit_cnmf_sm100` -- replaces the whole `fit_cnmf` (src/model.jl:58-85) with ONE ccall for the loop.
+#   * every rule constructor and both fit functions also take `SparseMatrixCSC{T,Int64}` data: its colptr / rowval / nzval
+#     go to cmf_set_data_csc as they are (index_base = 1, no copy) and the dense X is never formed.
 module CMFsm100
 
 using LinearAlgebra
+using SparseArrays
 import Random
 
 const LIB = get(ENV, "LIBCMF_SM100", "libcmf_sm100")
@@ -32,9 +35,14 @@ dtype_code(::Type{Float32}) = CMF_F32
 """Opaque device handle; the finalizer releases all device memory (ownership rule of include/cmf_sm100.h)."""
 mutable struct Handle
     ptr::Ptr{Cvoid}
-    function Handle(N, T, K, L, dtype::Cint, alg::Cint, device::Integer=0; ngpu::Integer=1, devices=nothing)
+    function Handle(N, T, K, L, dtype::Cint, alg::Cint, device::Integer=0; ngpu::Integer=1, devices=nothing, sparse::Bool=false)
         out = Ref{Ptr{Cvoid}}(C_NULL)
-        if ngpu > 1
+        if sparse
+            ngpu > 1 && throw(CMFError(3, "sparse data run on one GPU"))
+            check(ccall((:cmf_create_sparse, LIB), Cint,
+                        (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Cint, Cint, Cint),
+                        out, N, T, K, L, dtype, alg, device))
+        elseif ngpu > 1
             # the fit spans `ngpu` GPUs: time axis sharded INSIDE the library (NCCL communicators, one worker thread and one
             # stream per device), driven from this one Julia task -- no `Distributed`, same calls as a single-GPU handle
             devs = devices === nothing ? C_NULL : convert(Vector{Cint}, devices)
@@ -55,6 +63,14 @@ mutable struct Handle
     end
 end
 
+const SparseData{T} = SparseMatrixCSC{T,Int64}
+
+"""X as compressed sparse columns: Julia's own arrays, 1-based, passed without a copy (cmf_set_data_csc)."""
+function set_csc!(h::Ptr{Cvoid}, data::SparseData{T}) where {T}
+    GC.@preserve data check(ccall((:cmf_set_data_csc, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Cvoid}, Cint),
+                                  h, nnz(data), data.colptr, data.rowval, data.nzval, 1))
+end
+
 # ---- update rules behind CMF.jl's own interface ------------------------------------------------
 # In CMF.jl these would be declared `<: CMF.AbstractCFUpdate`; the abstract type is re-declared here
 # only so that this file parses stand-alone.
@@ -73,11 +89,14 @@ alg_code(::Type{SM100Update{:hals}}) = CMF_HALS
 alg_code(::Type{SM100Update{:pgd}}) = CMF_PGD
 
 """`Rule(data, W, H)` -- src/model.jl:79, src/algs/mult.jl:11-20, src/algs/hals.jl:18-28."""
-function (::Type{R})(data::Matrix{T}, W::Array{T,3}, H::Matrix{T}; sync_host=true, device=0, ngpu=1, devices=nothing,
-                     loss_func=:square, mask=nothing, constrW=:nonneg, constrH=:nonneg) where {R<:SM100Update,T<:Union{Float32,Float64}}
+function (::Type{R})(data::Union{Matrix{T},SparseData{T}}, W::Array{T,3}, H::Matrix{T}; sync_host=true, device=0, ngpu=1,
+                     devices=nothing, loss_func=:square, mask=nothing, constrW=:nonneg,
+                     constrH=:nonneg) where {R<:SM100Update,T<:Union{Float32,Float64}}
     K, N, L = size(W)
     @assert size(data) == (N, size(H, 2)) && size(H, 1) == K
-    h = Handle(N, size(data, 2), K, L, dtype_code(T), alg_code(R), device; ngpu=ngpu, devices=devices)
+    sparse = data isa SparseData
+    sparse && R === SM100PGDUpdate && throw(CMFError(3, "sparse data serve MultUpdate and HALSUpdate"))
+    h = Handle(N, size(data, 2), K, L, dtype_code(T), alg_code(R), device; ngpu=ngpu, devices=devices, sparse=sparse)
     if R === SM100PGDUpdate && (loss_func != :square || mask !== nothing)
         # PGD's pluggable losses (src/algs/pgd.jl:28-70): AbsoluteLoss and / or a MaskedLoss around it, on the device
         m = mask === nothing ? nothing : convert(Matrix{T}, mask)
@@ -87,10 +106,9 @@ function (::Type{R})(data::Matrix{T}, W::Array{T,3}, H::Matrix{T}; sync_host=tru
     if R === SM100PGDUpdate && (constrW != :nonneg || constrH != :nonneg)     # UnitNormConstraint, src/algs/pgd.jl:98-110
         check(ccall((:cmf_set_pgd_constraints, LIB), Cint, (Ptr{Cvoid}, Cint, Cint), h.ptr, constrW == :unitnorm ? 1 : 0, constrH == :unitnorm ? 1 : 0))
     end
-    GC.@preserve data W H begin
-        check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h.ptr, data, 0))
-        check(ccall((:cmf_set_factors, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int64), h.ptr, W, H, 0))
-    end
+    sparse ? set_csc!(h.ptr, data) :
+        GC.@preserve data check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h.ptr, data, 0))
+    GC.@preserve W H check(ccall((:cmf_set_factors, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int64), h.ptr, W, H, 0))
     return R(h, T, sync_host)
 end
 
@@ -130,6 +148,19 @@ function init_rand(data, L, K, tensor_conv)
     return W * sqrt(abs(alpha)), H * sqrt(abs(alpha))
 end
 
+"""init_rand for sparse data: the same draws, the alpha rescale on the device through <X, est> = <numH, H> and
+||est||^2 = <W W', Htilde Htilde'> (cmf_init_scale_partials), so est is never formed."""
+function init_rand(data::SparseData{T}, L, K) where {T}
+    N, Tt = size(data)
+    W = convert(Array{T,3}, rand(K, N, L)); H = convert(Matrix{T}, rand(K, Tt))
+    rule = SM100MultUpdate(data, W, H; sync_host=false)
+    part = zeros(Cdouble, 2)
+    check(ccall((:cmf_init_scale_partials, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}), rule.h.ptr, part))
+    s = sqrt(abs(part[1] / part[2]))
+    return W * s, H * s
+end
+init_rand(data::SparseData, L, K, tensor_conv) = init_rand(data, L, K)
+
 """tensor_conv(W, H) on the device -- src/common.jl:17-34."""
 function tensor_conv(W::Array{T,3}, H::Matrix{T}) where {T}
     K, N, L = size(W); Tt = size(H, 2)
@@ -161,12 +192,13 @@ end
     fit_cnmf_sm100(data; L=10, K=5, alg=:mult, max_itr=100, max_time=Inf, ngpu=1, kwargs...)
 
 `ngpu > 1` runs the same fit T-sharded over that many GPUs inside the same single `cmf_fit` call (MultUpdate, HALSUpdate).
+`data` may be a `SparseMatrixCSC{T,Int64}` (MultUpdate, HALSUpdate, one GPU; cmf_create_sparse): X is never densified.
 
 Drop-in for `CMF.fit_cnmf` (src/model.jl:58-85).  Accepts both API generations (SURVEY.md Appendix C):
 `alg` as `:mult`/`:hals` or a rule type, regularisers as `l1_H…` (README) or `l1H…` (current src),
 inits as `W_init/H_init` (or `initW/initH`).  `layout=:LNK` (default, README layout) or `:KNL`.
 """
-function fit_cnmf_sm100(data::Matrix{T}; L::Integer=10, K::Integer=5, alg=:mult, max_itr=100, max_time=Inf,
+function fit_cnmf_sm100(data::Union{Matrix{T},SparseData{T}}; L::Integer=10, K::Integer=5, alg=:mult, max_itr=100, max_time=Inf,
                         layout=:LNK, kwargs...) where {T<:Union{Float32,Float64}}
     kw = Dict{Symbol,Any}(kwargs)
     for (a, b) in ((:l1_W, :l1W), (:l2_W, :l2W), (:l1_H, :l1H), (:l2_H, :l2H), (:initW, :W_init), (:initH, :H_init))
@@ -216,12 +248,12 @@ equals `fit_cnmf_sm100(data; seed=seeds[r], l1W=l1W[r], ...)` -- or the fit from
 (stacks K x N x L x R and K x T x R, restart last, which is the library's restart-major host layout) -- with every other
 keyword the same.  `l1W`, `l2W`, `l1H`, `l2H` are scalars or length-R vectors.  A restart that meets the early stop is
 frozen while the others go on; `max_time` and `time_hist` use the batch's own clock (shared by all restarts).  Returns a
-vector of R `CNMF_results`.  MultUpdate only, one GPU.
+vector of R `CNMF_results`.  MultUpdate only, one GPU.  `data` may be a `SparseMatrixCSC{T,Int64}` (cmf_create_batch_sparse).
 
 `K` may be a vector of R ranks (a rank sweep in one handle, `cmf_create_batch_ranks`): restart r then has rank `K[r]`,
 `seeds` has R entries, and `W_init` / `H_init` are vectors of R arrays of sizes `K[r] x N x L` and `K[r] x T`.
 """
-function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Union{Integer,AbstractVector{<:Integer}}=5, max_itr=100,
+function fit_cnmf_batch_sm100(data::Union{Matrix{T},SparseData{T}}; L::Integer=10, K::Union{Integer,AbstractVector{<:Integer}}=5, max_itr=100,
                               max_time=Inf, seeds=nothing,
                               W_init=nothing, H_init=nothing, layout=:LNK, device::Integer=0, kwargs...) where {T<:Union{Float32,Float64}}
     kw = Dict{Symbol,Any}(kwargs)
@@ -267,7 +299,11 @@ function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Union{Integer,A
     end
     regs = [per_restart(get(kw, k, 0), R) for k in (:l1W, :l2W, :l1H, :l2H)]
     out = Ref{Ptr{Cvoid}}(C_NULL)
-    if ranks === nothing
+    if data isa SparseData
+        rk = ranks === nothing ? fill(Int64(K), R) : ranks
+        check(ccall((:cmf_create_batch_sparse, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Ptr{Int64}, Int64, Cint, Cint, Int64, Cint),
+                    out, N, Tt, rk, L, dtype_code(T), CMF_MULT, R, device))
+    elseif ranks === nothing
         check(ccall((:cmf_create_batch, LIB), Cint, (Ref{Ptr{Cvoid}}, Int64, Int64, Int64, Int64, Cint, Cint, Int64, Cint),
                     out, N, Tt, K, L, dtype_code(T), CMF_MULT, R, device))
     else
@@ -276,7 +312,7 @@ function fit_cnmf_batch_sm100(data::Matrix{T}; L::Integer=10, K::Union{Integer,A
     end
     h = out[]
     try
-        check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h, data, 0))
+        data isa SparseData ? set_csc!(h, data) : check(ccall((:cmf_set_data, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Int64), h, data, 0))
         check(ccall((:cmf_set_factors_batch, LIB), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}), h, W0, H0))
         cap = isfinite(max_itr) ? Int(max_itr) + 1 : 1_000_001
         loss_hist = zeros(Cdouble, cap, R); time_hist = zeros(Cdouble, cap)
