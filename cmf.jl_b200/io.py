@@ -12,30 +12,20 @@
 """
 from __future__ import annotations
 
-import ctypes
 import itertools
 import math
 
 import numpy as np
 
-from . import _lib
-from ._lib import check, fptr, np_dtype, parse_dtype
+from ._lib import MULT, Handle, parse_dtype
 
 
 def gen_synthetic(N=100, T=500, K=3, L=20, p_h=0.5, noise_scale=1.0, seed=1234, dtype="f64", device=0):
     """N x T non-negative synthetic data with K ground-truth motifs of L lags (datasets/synthetic.jl:29-61 defaults:
     alpha = 0.1, sigma = 0.2 are fixed inside the device generator)."""
-    lib = _lib.load()
-    dt = parse_dtype(dtype)
-    h = ctypes.c_void_p()
-    check(lib.cmf_create(ctypes.byref(h), N, T, K, L, dt, _lib.MULT, device))
-    try:
-        check(lib.cmf_synth_data(h, int(seed), K, L, float(p_h), float(noise_scale)))
-        out = np.empty((N, T), dtype=np_dtype(dt), order="F")
-        check(lib.cmf_get_data(h, fptr(out), 0))
-    finally:
-        lib.cmf_destroy(h)
-    return out
+    with Handle(N, T, K, L, parse_dtype(dtype), MULT, device) as h:
+        h.synth_data(seed, K, L, p_h, noise_scale)
+        return h.get_data()
 
 
 def save_model(results, path):

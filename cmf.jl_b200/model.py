@@ -23,7 +23,7 @@ import warnings
 import numpy as np
 
 from . import _lib
-from ._lib import F32, F64, HALS, MULT, PGD, CMFError, check, fptr, julia_array, np_dtype, parse_dtype
+from ._lib import HALS, MULT, PGD, CMFError, Handle, check, fptr, julia_array, np_dtype, parse_dtype
 
 # kwargs the reference's methods read (src/algs/alternating.jl:23-31, mult.jl:23,42, hals.jl:31,37,
 # src/model.jl:64,72-73) plus the README-generation spellings (README.md:44-52) and this library's own.
@@ -147,14 +147,8 @@ def converged(loss_hist, patience, tol):
 
 # ------------------------------------------------------------------------------------------
 # update rules: the plugin boundary (abstract type AbstractCFUpdate, alternating.jl:8)
-def _loss_stats(h):
-    nd, ne, iv, le = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int(), ctypes.c_double()
-    check(_lib.load().cmf_get_loss_stats(h, ctypes.byref(nd), ctypes.byref(ne), ctypes.byref(iv), ctypes.byref(le)))
-    return dict(direct=nd.value, expansion=ne.value, interval=iv.value, last_err=le.value)
-
-
 # ------------------------------------------------------------------------------------------
-class AbstractCFUpdate:
+class AbstractCFUpdate(Handle):
     """A rule owns an opaque libcmf_sm100 handle: the constructor uploads (data, W, H) exactly like
     ``Rule(data, W, H)`` at src/model.jl:79; ``update_motifs`` / ``update_feature_maps`` run one
     device half-step each.  ``sync_host=True`` (default) copies the updated factor back into the
@@ -169,9 +163,8 @@ class AbstractCFUpdate:
         from this one thread -- cmf_create_multi); every other argument and every method is unchanged.  ``data`` may be a
         ``scipy.sparse`` matrix or array (MultUpdate / HALSUpdate, one GPU): the handle then holds X as compressed sparse
         columns and never densifies it (cmf_create_sparse)."""
-        self._h = ctypes.c_void_p()
-        self.dtype = parse_dtype(dtype)
-        csc = as_csc(data, self.dtype)
+        dtype = parse_dtype(dtype)
+        csc = as_csc(data, dtype)
         if csc is None:
             data = np.asarray(data)
         W = np.asarray(W)
@@ -183,89 +176,36 @@ class AbstractCFUpdate:
             raise ValueError(f"dimension mismatch: data {data.shape}, W {W.shape}, H {H.shape}")
         ngpu = int(ngpu or 1)
         _check_sparse_rule(csc is not None, type(self), ngpu)
-        lib = _lib.load()
-        self.N, self.T, self.K, self.L = N, data.shape[1], K, L
+        super().__init__(N, data.shape[1], K, L, dtype, self._ALG, device if devices is None else devices[0], ngpu=ngpu,
+                         devices=devices, sparse=csc is not None)
         self.sync_host = sync_host
-        if csc is not None:
-            check(lib.cmf_create_sparse(ctypes.byref(self._h), N, self.T, K, L, self.dtype, self._ALG,
-                                        device if devices is None else devices[0]))
-        elif ngpu > 1:
-            devs = (ctypes.c_int * ngpu)(*(devices if devices is not None else range(ngpu)))
-            check(lib.cmf_create_multi(ctypes.byref(self._h), N, self.T, K, L, self.dtype, self._ALG, ngpu, devs))
-        else:
-            check(lib.cmf_create(ctypes.byref(self._h), N, self.T, K, L, self.dtype, self._ALG,
-                                 device if devices is None else devices[0]))
         if engine is not None:
-            check(lib.cmf_set_engine(self._h, int(engine)))
+            self.set_engine(engine)
         if loss_mode is not None:
-            check(lib.cmf_set_loss_mode(self._h, int(loss_mode)))
+            self.set_loss_mode(loss_mode)
         if loss_guard is not None:
-            check(lib.cmf_set_loss_guard(self._h, float(loss_guard), 16))
+            self.set_loss_guard(loss_guard, 16)
         if csc is not None:
             _set_csc(self._h, csc)
         else:
-            check(lib.cmf_set_data(self._h, fptr(julia_array(data, self.dtype)), 0))
+            self.set_data(data)
         self.set_factors(W, H)
-
-    # -- plumbing ------------------------------------------------------------------------
-    def set_factors(self, W, H):
-        Wj, Hj = julia_array(W, self.dtype), julia_array(H, self.dtype)
-        check(_lib.load().cmf_set_factors(self._h, fptr(Wj), fptr(Hj), 0))
-
-    def get_factors(self):
-        """(W as K x N x L, H as K x T) numpy arrays of the handle dtype read back from the device."""
-        dt = np_dtype(self.dtype)
-        W = np.empty((self.K, self.N, self.L), dtype=dt, order="F")
-        H = np.empty((self.K, self.T), dtype=dt, order="F")
-        check(_lib.load().cmf_get_factors(self._h, fptr(W), fptr(H)))
-        return W, H
-
-    def loss(self):
-        out = ctypes.c_double()
-        check(_lib.load().cmf_loss(self._h, ctypes.byref(out)))
-        return out.value
-
-    def launch_count(self):
-        out = ctypes.c_int64()
-        check(_lib.load().cmf_launch_count(self._h, ctypes.byref(out)))
-        return out.value
-
-    def set_loss_guard(self, guard=0.25, max_interval=16):
-        """Relative loss at or below which loss mode 1 calibrates the expansion against the direct pass, and the
-        longest stretch of evaluations between two direct passes (include/cmf_sm100.h)."""
-        check(_lib.load().cmf_set_loss_guard(self._h, float(guard), int(max_interval)))
-
-    def loss_stats(self):
-        """dict(direct=, expansion=, interval=, last_err=): loss evaluations by path and the calibration state."""
-        return _loss_stats(self._h)
-
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            _lib.load().cmf_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
     # -- the interface of src/algs/alternating.jl:52,54 ---------------------------------------
     def update_motifs(self, data, W, H, l1W=0.0, l2W=0.0, **kwargs):
         """update_motifs!(rule, data, W, H; l1W, l2W)  (mult.jl:23-39 / hals.jl:31-34)."""
-        check(_lib.load().cmf_update_motifs(self._h, float(l1W), float(l2W)))
+        super().update_motifs(l1W, l2W)
         if self.sync_host and W is not None:
             Wn, _ = self.get_factors()
             W[...] = Wn
 
     def update_feature_maps(self, data, W, H, l1H=0.0, l2H=0.0, **kwargs):
         """loss = update_feature_maps!(rule, data, W, H; l1H, l2H)  (mult.jl:42-58 / hals.jl:37-42)."""
-        out = ctypes.c_double()
-        check(_lib.load().cmf_update_feature_maps(self._h, float(l1H), float(l2H), ctypes.byref(out)))
+        loss = super().update_feature_maps(l1H, l2H)
         if self.sync_host and H is not None:
             _, Hn = self.get_factors()
             H[...] = Hn
-        return out.value
+        return loss
 
     # julia-style aliases
     update_motifs_ = update_motifs
@@ -333,6 +273,36 @@ class AlternatingOptimizer:
         self.update_rule, self.max_itr, self.max_time = update_rule, max_itr, max_time
 
 
+def _alternate(loss, step, max_itr, max_time=math.inf, check_convergence=True, patience=3, tol=1e-4, tick=None):
+    """The loop of src/algs/alternating.jl:37-66: ``loss`` before the first iteration, then ``step()`` (one iteration,
+    returning its loss) until ``max_itr`` iterations, ``max_time`` seconds or convergence, with ``tick()`` after every
+    iteration.  Returns (loss_hist, time_hist, stopped_early)."""
+    loss_hist = [loss]                    # :37
+    time_hist = [0.0]                     # :38
+    itr = 1
+    while itr <= max_itr and time_hist[-1] <= max_time:   # :45
+        itr += 1
+        t0 = _time.time()
+        loss = step()
+        time_hist.append(time_hist[-1] + (_time.time() - t0))
+        loss_hist.append(loss)
+        if tick is not None:
+            tick()
+        if check_convergence and converged(loss_hist, patience, tol):
+            return loss_hist, time_hist, True
+    return loss_hist, time_hist, False
+
+
+def _results(data, W, H, time_hist, loss_hist, layout, engine_info=None):
+    """CNMF_results from the factors as the library returns them: W (K x N x L) goes to ``layout``."""
+    if layout == "LNK":
+        W = np.ascontiguousarray(W.transpose(2, 1, 0))
+    res = CNMF_results(data, W, H, list(time_hist), list(loss_hist), layout)
+    if engine_info is not None:
+        res.engine_info = engine_info      # not part of the reference struct: which engine / loss path produced loss_hist
+    return res
+
+
 def fit(alg, data, L, K, W_init, H_init, verbose=False, printer=print, layout="LNK", **kwargs):
     """src/algs/alternating.jl:16-71, stepping the rule from the host (one C-ABI call per
     half-step; factors stay on the device and are read back once at the end).  ``fit_cnmf`` uses
@@ -345,32 +315,25 @@ def fit(alg, data, L, K, W_init, H_init, verbose=False, printer=print, layout="L
     rule = alg.update_rule
     reg = {k: kwargs[k] for k in ("l1W", "l2W", "l1H", "l2H") if k in kwargs}
 
+    def step():
+        if not eval_mode:
+            rule.update_motifs(data, None, None, **reg)
+        return rule.update_feature_maps(data, None, None, **reg)
+
     rule.set_factors(W_init, H_init)      # alternating.jl:33-34 (deepcopy of the inits)
     old_sync, rule.sync_host = rule.sync_host, False
-    loss_hist = [rule.loss()]             # :37
-    time_hist = [0.0]                     # :38
-    verbose and _emit(printer, "Starting ", False)
-    itr = 1
     try:
-        while itr <= alg.max_itr and time_hist[-1] <= alg.max_time:   # :45
-            itr += 1
-            t0 = _time.time()
-            if not eval_mode:
-                rule.update_motifs(data, None, None, **reg)
-            loss = rule.update_feature_maps(data, None, None, **reg)
-            time_hist.append(time_hist[-1] + (_time.time() - t0))
-            loss_hist.append(loss)
-            verbose and _emit(printer, ".", False)
-            if check_convergence and converged(loss_hist, patience, tol):
-                _emit(printer, "Converged early.")   # :64, unconditional in the reference
-                break
+        loss0 = rule.loss()
+        verbose and _emit(printer, "Starting ", False)
+        loss_hist, time_hist, early = _alternate(loss0, step, alg.max_itr, alg.max_time, check_convergence, patience, tol,
+                                                 tick=(lambda: _emit(printer, ".", False)) if verbose else None)
     finally:
         rule.sync_host = old_sync
+    if early:
+        _emit(printer, "Converged early.")   # :64, unconditional in the reference
     verbose and _emit(printer, " fit!")
     W, H = rule.get_factors()
-    if layout == "LNK":
-        W = np.ascontiguousarray(W.transpose(2, 1, 0))
-    return CNMF_results(data, W, H, time_hist, loss_hist, layout)
+    return _results(data, W, H, time_hist, loss_hist, layout)
 
 
 def init_rand(data, L, K, seed=None, dtype="f64", device=0):
@@ -383,21 +346,64 @@ def init_rand(data, L, K, seed=None, dtype="f64", device=0):
     rng = np.random.default_rng(seed)
     W = rng.random((K, N, L))             # W drawn first (model.jl:116), then H (:117)
     H = rng.random((K, T))
-    rule = MultUpdate(data, W, H, dtype=dtype, device=device, sync_host=False)
-    try:
-        s = _rescale(rule)
-    finally:
-        rule.close()
-    return W * s, H * s
+    return _host_rescaled(data, W, H, dtype, device)
 
 
 def _rescale(rule):
-    out = (ctypes.c_double * 2)()
-    check(_lib.load().cmf_init_scale_partials(rule._h, out))
-    alpha = out[0] / out[1]               # model.jl:120
+    dot, nrm2 = rule.init_scale_partials()
+    alpha = dot / nrm2                    # model.jl:120
     s = math.sqrt(abs(alpha))             # model.jl:121-122
-    check(_lib.load().cmf_scale_factors(rule._h, s))
+    rule.scale_factors(s)
     return s
+
+
+class _FitCall:
+    """What fit_cnmf and fit_cnmf_batch share: the keywords and the checks that come before their own, the data as a
+    dense array or a ``scipy.sparse`` input, and the device loop (cmf_fit / cmf_fit_batch) with its history buffers and
+    prints."""
+
+    def __init__(self, data, alg, kwargs):
+        self.kw = kw = _normalise_kwargs(kwargs)
+        self.printer = kw.get("printer", print)
+        self.verbose = kw.get("verbose", False)
+        self.layout = kw.get("layout", "LNK")
+        if self.layout not in ("LNK", "KNL"):
+            raise ValueError("layout must be 'LNK' or 'KNL'")
+        self.dtype = parse_dtype(kw.get("dtype", "f64"))
+        self.device = kw.get("device", 0)
+        self.rule_cls = _resolve_alg(alg)
+        self.data_in = data
+        self.sparse = _is_sparse(data)
+        self.data = data if self.sparse else np.asarray(data)
+        self.N, self.T = _data_shape(self.data)
+
+    def run(self, entry, handle, regs, max_itr, max_time, R=1):
+        """``entry(handle, <loop arguments>, *regs, <history buffers>)`` for a batch of R fits (R = 1: cmf_fit).  Returns
+        (loss_hist R x cap, time_hist, iterations recorded per fit)."""
+        kw = self.kw
+        unbounded = not (max_itr < math.inf)
+        cap = 1 + (int(max_itr) if not unbounded else 1_000_000)
+        loss_hist = np.zeros(R * cap)
+        time_hist = np.zeros(cap)
+        n = np.zeros(R, dtype=np.int64)
+        early = np.zeros(R, dtype=np.int32)
+        self.verbose and _emit(self.printer, "Starting ", False)
+        check(entry(
+            handle._h, -1 if unbounded else int(max_itr), float(max_time),
+            int(bool(kw.get("eval_mode", False))), int(bool(kw.get("check_convergence", True))),
+            int(kw.get("patience", 3)), float(kw.get("tol", 1e-4)), *regs,
+            _dptr(loss_hist), _dptr(time_hist), cap, n.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+            early.ctypes.data_as(ctypes.POINTER(ctypes.c_int))))
+        self.verbose and _emit(self.printer, "." * (int(n.max()) - 1), False)
+        for r in range(R):
+            if early[r]:
+                _emit(self.printer, "Converged early.")   # alternating.jl:64, once per fit that stopped early
+        self.verbose and _emit(self.printer, " fit!")
+        return loss_hist.reshape(R, cap), time_hist, n
+
+
+def _dptr(a):
+    return a.ctypes.data_as(ctypes.POINTER(ctypes.c_double))
 
 
 def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **kwargs):
@@ -409,23 +415,12 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
     (the fit runs T-sharded over that many GPUs inside the same single library call; MultUpdate and HALSUpdate).
     ``data`` may be a ``scipy.sparse`` matrix or array (MultUpdate / HALSUpdate, one GPU): X is then never densified;
     ``CNMF_results.data`` is the caller's matrix."""
-    kw = _normalise_kwargs(kwargs)
-    printer = kw.get("printer", print)
-    verbose = kw.get("verbose", False)
-    layout = kw.get("layout", "LNK")
-    if layout not in ("LNK", "KNL"):
-        raise ValueError("layout must be 'LNK' or 'KNL'")
-    dtype = parse_dtype(kw.get("dtype", "f64"))
-    device = kw.get("device", 0)
-    rule_cls = _resolve_alg(alg)
-    data_in = data
-    sparse = _is_sparse(data)
-    if not sparse:
-        data = np.asarray(data)
-    N, T = _data_shape(data)
+    fc = _FitCall(data, alg, kwargs)
+    kw, dtype, device, rule_cls, N, T = fc.kw, fc.dtype, fc.device, fc.rule_cls, fc.N, fc.T
     L, K = int(L), int(K)
-    _check_sparse_rule(sparse, rule_cls, kw.get("ngpu", 1))
-    if sparse:
+    _check_sparse_rule(fc.sparse, rule_cls, kw.get("ngpu", 1))
+    data = fc.data
+    if fc.sparse:
         W0, H0 = kw.get("W_init"), kw.get("H_init")
         if (W0 is not None and np.shape(W0) != (K, N, L)) or (H0 is not None and np.shape(H0) != (K, T)):
             raise ValueError(f"W_init must be {(K, N, L)} and H_init {(K, T)}; got {np.shape(W0)}, {np.shape(H0)}")
@@ -450,46 +445,17 @@ def fit_cnmf(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.inf, **
     if rule_cls is PGDUpdate:
         extra = dict(loss_func=kw.get("loss_func", "square"), mask=kw.get("mask"),
                      constrW=kw.get("constrW", "nonneg"), constrH=kw.get("constrH", "nonneg"))
-    rule = rule_cls(data, W0, H0, dtype=dtype, device=device, sync_host=False,
-                    engine=kw.get("engine"), loss_mode=kw.get("loss_mode"), loss_guard=kw.get("loss_guard"),
-                    ngpu=kw.get("ngpu", 1), devices=kw.get("devices"), **extra)  # model.jl:79
-    try:
+    with rule_cls(data, W0, H0, dtype=dtype, device=device, sync_host=False,
+                  engine=kw.get("engine"), loss_mode=kw.get("loss_mode"), loss_guard=kw.get("loss_guard"),
+                  ngpu=kw.get("ngpu", 1), devices=kw.get("devices"), **extra) as rule:   # model.jl:79
         if need_rescale:
             _rescale(rule)
-        lib = _lib.load()
-        unbounded = not (max_itr < math.inf)
-        cap = 1 + (int(max_itr) if not unbounded else 1_000_000)
-        loss_hist = np.zeros(cap)
-        time_hist = np.zeros(cap)
-        n = ctypes.c_int64()
-        early = ctypes.c_int()
-        verbose and _emit(printer, "Starting ", False)
-        check(lib.cmf_fit(
-            rule._h, -1 if unbounded else int(max_itr), float(max_time),
-            int(bool(kw.get("eval_mode", False))), int(bool(kw.get("check_convergence", True))),
-            int(kw.get("patience", 3)), float(kw.get("tol", 1e-4)),
-            float(kw.get("l1W", 0.0)), float(kw.get("l2W", 1.0 if rule_cls is PGDUpdate else 0.0)),
-            float(kw.get("l1H", 0.0)), float(kw.get("l2H", 0.0)),
-            loss_hist.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
-            time_hist.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
-            cap, ctypes.byref(n), ctypes.byref(early)))
-        verbose and _emit(printer, "." * (n.value - 1), False)
-        if early.value:
-            _emit(printer, "Converged early.")          # alternating.jl:64
-        verbose and _emit(printer, " fit!")
+        regs = [float(kw.get("l1W", 0.0)), float(kw.get("l2W", 1.0 if rule_cls is PGDUpdate else 0.0)),
+                float(kw.get("l1H", 0.0)), float(kw.get("l2H", 0.0))]
+        loss_hist, time_hist, n = fc.run(_lib.load().cmf_fit, rule, regs, max_itr, max_time)
         W, H = rule.get_factors()
-        stats = rule.loss_stats()
-        eng, lm = ctypes.c_int(), ctypes.c_int()
-        check(lib.cmf_get_engine(rule._h, ctypes.byref(eng)))
-        check(lib.cmf_get_loss_mode(rule._h, ctypes.byref(lm)))
-        stats.update(engine=eng.value, loss_mode=lm.value)
-    finally:
-        rule.close()
-    if layout == "LNK":
-        W = np.ascontiguousarray(W.transpose(2, 1, 0))
-    res = CNMF_results(data_in, W, H, list(time_hist[: n.value]), list(loss_hist[: n.value]), layout)
-    res.engine_info = stats      # not part of the reference struct: which engine / loss path produced loss_hist (ADVICE r1)
-    return res
+        engine_info = dict(rule.loss_stats(), engine=rule.get_engine(), loss_mode=rule.loss_mode)
+    return _results(fc.data_in, W, H, time_hist[: n[0]], loss_hist[0, : n[0]], fc.layout, engine_info)
 
 
 def _per_restart(name, v, R):
@@ -528,22 +494,10 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
 
     ``data`` may be a ``scipy.sparse`` matrix or array (cmf_create_batch_sparse): X is stored once as compressed sparse
     columns and never densified."""
-    kw = _normalise_kwargs(kwargs)
-    printer = kw.get("printer", print)
-    verbose = kw.get("verbose", False)
-    layout = kw.get("layout", "LNK")
-    if layout not in ("LNK", "KNL"):
-        raise ValueError("layout must be 'LNK' or 'KNL'")
-    dtype = parse_dtype(kw.get("dtype", "f64"))
-    device = kw.get("device", 0)
-    rule_cls = _resolve_alg(alg)
-    data_in = data
-    sparse = _is_sparse(data)
-    if not sparse:
-        data = np.asarray(data)
-    N, T = _data_shape(data)
+    fc = _FitCall(data, alg, kwargs)
+    kw, dtype, N, T = fc.kw, fc.dtype, fc.N, fc.T
     L = int(L)
-    _check_sparse_rule(sparse, rule_cls, 1)
+    _check_sparse_rule(fc.sparse, fc.rule_cls, 1)
     ranks = None if np.ndim(K) == 0 else _batch_ranks(K)
     K = int(K) if ranks is None else None
     W0, H0 = kw.get("W_init"), kw.get("H_init")
@@ -588,82 +542,53 @@ def fit_cnmf_batch(data, L=10, K=5, alg=MultUpdate, max_itr=100, max_time=math.i
     Wj = np.concatenate([julia_array(w, dtype).ravel(order="F") for w in W0])
     Hj = np.concatenate([julia_array(x, dtype).ravel(order="F") for x in H0])
 
-    if sparse:
-        data = as_csc(data, dtype)
+    data = as_csc(fc.data, dtype) if fc.sparse else fc.data
     lib = _lib.load()
-    h = ctypes.c_void_p()
-    if sparse:
-        rk = np.asarray(Ks, dtype=np.int64)
-        check(lib.cmf_create_batch_sparse(ctypes.byref(h), N, T, rk.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), L, dtype,
-                                          rule_cls._ALG, R, device))
-    elif ranks is None:
-        check(lib.cmf_create_batch(ctypes.byref(h), N, T, K, L, dtype, rule_cls._ALG, R, device))
-    else:
-        rk = np.asarray(ranks, dtype=np.int64)
-        check(lib.cmf_create_batch_ranks(ctypes.byref(h), N, T, rk.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), L, dtype,
-                                         rule_cls._ALG, R, device))
-    dptr = lambda a: a.ctypes.data_as(ctypes.POINTER(ctypes.c_double))  # noqa: E731
-    try:
+    with Handle(N, T, K if ranks is None else ranks, L, dtype, fc.rule_cls._ALG, fc.device, sparse=fc.sparse,
+                restarts=R) as h:
         if kw.get("engine") is not None:
-            check(lib.cmf_set_engine(h, int(kw["engine"])))
+            h.set_engine(kw["engine"])
         if kw.get("loss_mode") is not None:
-            check(lib.cmf_set_loss_mode(h, int(kw["loss_mode"])))
-        if sparse:
-            _set_csc(h, data)
+            h.set_loss_mode(kw["loss_mode"])
+        if fc.sparse:
+            _set_csc(h._h, data)
         else:
-            check(lib.cmf_set_data(h, fptr(julia_array(data, dtype)), 0))
-        check(lib.cmf_set_factors_batch(h, fptr(Wj), fptr(Hj)))
+            h.set_data(data)
+        check(lib.cmf_set_factors_batch(h._h, fptr(Wj), fptr(Hj)))
         if seeds is not None:                             # model.jl:119-122, per restart
             part = np.zeros(2 * R)
-            check(lib.cmf_init_scale_partials_batch(h, dptr(part)))
+            check(lib.cmf_init_scale_partials_batch(h._h, _dptr(part)))
             s = np.sqrt(np.abs(part[0::2] / part[1::2]))
-            check(lib.cmf_scale_factors_batch(h, dptr(s)))
-        unbounded = not (max_itr < math.inf)
-        cap = 1 + (int(max_itr) if not unbounded else 1_000_000)
-        loss_hist = np.zeros(R * cap)
-        time_hist = np.zeros(cap)
-        n = np.zeros(R, dtype=np.int64)
-        early = np.zeros(R, dtype=np.int32)
-        verbose and _emit(printer, "Starting ", False)
-        check(lib.cmf_fit_batch(
-            h, -1 if unbounded else int(max_itr), float(max_time),
-            int(bool(kw.get("eval_mode", False))), int(bool(kw.get("check_convergence", True))),
-            int(kw.get("patience", 3)), float(kw.get("tol", 1e-4)),
-            dptr(regs["l1W"]), dptr(regs["l2W"]), dptr(regs["l1H"]), dptr(regs["l2H"]),
-            dptr(loss_hist), dptr(time_hist), cap, n.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
-            early.ctypes.data_as(ctypes.POINTER(ctypes.c_int))))
-        verbose and _emit(printer, "." * (int(n.max()) - 1), False)
-        for r in range(R):
-            if early[r]:
-                _emit(printer, "Converged early.")        # alternating.jl:64, once per restart that stopped early
-        verbose and _emit(printer, " fit!")
+            check(lib.cmf_scale_factors_batch(h._h, _dptr(s)))
+        loss_hist, time_hist, n = fc.run(lib.cmf_fit_batch, h, [_dptr(regs[k]) for k in ("l1W", "l2W", "l1H", "l2H")],
+                                         max_itr, max_time, R)
         dt = np_dtype(dtype)
         Wo = np.empty(N * L * sum(Ks), dtype=dt)
         Ho = np.empty(T * sum(Ks), dtype=dt)
-        check(lib.cmf_get_factors_batch(h, fptr(Wo), fptr(Ho)))
-    finally:
-        lib.cmf_destroy(h)
+        check(lib.cmf_get_factors_batch(h._h, fptr(Wo), fptr(Ho)))
     out = []
     offs = np.concatenate([[0], np.cumsum(Ks)])
     for r in range(R):
         k, o = Ks[r], int(offs[r])
         W = Wo[N * L * o: N * L * (o + k)].reshape((k, N, L), order="F")
         H = Ho[T * o: T * (o + k)].reshape((k, T), order="F")
-        W = np.ascontiguousarray(W.transpose(2, 1, 0)) if layout == "LNK" else np.asfortranarray(W)
         nr = int(n[r])
-        res = CNMF_results(data_in, W, H, list(time_hist[:nr]), list(loss_hist[r * cap: r * cap + nr]), layout)
-        res.engine_info = dict(direct=0 if sparse else nr, expansion=nr if sparse else 0, interval=0, last_err=0.0, engine=0,
-                               loss_mode=int(sparse), restarts=R)
-        out.append(res)
+        info = dict(direct=0 if fc.sparse else nr, expansion=nr if fc.sparse else 0, interval=0, last_err=0.0, engine=0,
+                    loss_mode=int(fc.sparse), restarts=R)
+        out.append(_results(fc.data_in, W, H, time_hist[:nr], loss_hist[r, :nr], fc.layout, info))
     return out
 
 
+def _temporary_rule(data, W, H, dtype, device):
+    """A MultUpdate rule for one computation on the device; use it as ``with _temporary_rule(...) as rule:``, which
+    frees its handle."""
+    return MultUpdate(data, W, H, dtype=dtype, device=device, sync_host=False)
+
+
 def _host_rescaled(data, W, H, dtype, device):
-    rule = MultUpdate(data, W, H, dtype=dtype, device=device, sync_host=False)
-    try:
+    """(W, H) times the alpha rescale of src/model.jl:119-122, computed on the device."""
+    with _temporary_rule(data, W, H, dtype, device) as rule:
         s = _rescale(rule)
-    finally:
-        rule.close()
     return W * s, H * s
 
 
@@ -726,8 +651,5 @@ def shift_and_stack(H, L, dtype="f64"):
 
 def compute_loss(data, W, H, dtype="f64", device=0):
     """src/common.jl:54-55."""
-    rule = MultUpdate(data, W, H, dtype=dtype, device=device, sync_host=False)
-    try:
+    with _temporary_rule(data, W, H, dtype, device) as rule:
         return rule.loss()
-    finally:
-        rule.close()

@@ -17,10 +17,9 @@ from __future__ import annotations
 import ctypes
 import math
 
-import numpy as np
-
 from . import _lib
-from ._lib import check, fptr, julia_array, np_dtype, parse_dtype
+from ._lib import HALS, MULT, Handle, check, parse_dtype
+from .model import _alternate, _rescale
 
 
 class ShardPlan:
@@ -58,7 +57,7 @@ class _CudaView:
         }
 
 
-class DeviceShard:
+class DeviceShard(Handle):
     """One rank's shard on one GPU: a libcmf_sm100 handle plus torch views of its exchange buffers."""
 
     def __init__(self, N, T, t0, t1, K, L, dtype="f32", device=0, use_torch_stream=True, alg="mult", comm=None,
@@ -69,33 +68,15 @@ class DeviceShard:
         import torch
 
         self.torch = torch
-        lib = _lib.load()
-        self.N, self.T, self.t0, self.t1, self.K, self.L = N, T, t0, t1, K, L
-        self.dtype = parse_dtype(dtype)
         self.device = device
-        self._h = ctypes.c_void_p()
         self.group = bool(ngpu and ngpu > 1)
         self.in_library_comm = comm is not None or self.group
-        algc = {"mult": _lib.MULT, "hals": _lib.HALS}[alg]
-        if self.group:
-            devs = (ctypes.c_int * ngpu)(*(devices if devices is not None else range(ngpu)))
-            check(lib.cmf_create_multi(ctypes.byref(self._h), N, T, K, L, self.dtype, algc, ngpu, devs))
-            self.t0, self.t1 = 0, T
-        elif comm is not None:
-            uid, rank, world = comm      # uid None: reuse the communicator this process already built for (device, rank, world)
-            buf = ctypes.create_string_buffer(bytes(uid), 128) if uid is not None else None
-            check(lib.cmf_create_rank(ctypes.byref(self._h), N, T, K, L, self.dtype, algc, device, buf, rank, world))
-            a, b = ctypes.c_int64(), ctypes.c_int64()
-            check(lib.cmf_comm_info(self._h, None, None, ctypes.byref(a), ctypes.byref(b)))
-            assert (a.value, b.value) == (t0, t1), "ShardPlan and cmf_shard_range disagree"
-        elif t0 == 0 and t1 == T:
-            check(lib.cmf_create(ctypes.byref(self._h), N, T, K, L, self.dtype, algc, device))
-        else:
-            check(lib.cmf_create_shard(ctypes.byref(self._h), N, T, t0, t1, K, L, self.dtype, algc, device))
+        super().__init__(N, T, K, L, parse_dtype(dtype), {"mult": MULT, "hals": HALS}[alg], device, t0, t1, comm=comm,
+                         ngpu=ngpu, devices=devices)
         if use_torch_stream and not self.group:
             with torch.cuda.device(device):
                 s = torch.cuda.current_stream().cuda_stream
-            check(lib.cmf_set_stream(self._h, ctypes.c_void_p(s)))
+            check(_lib.load().cmf_set_stream(self._h, ctypes.c_void_p(s)))
         if not self.group:
             self._views()
 
@@ -108,11 +89,6 @@ class DeviceShard:
 
     def exchange_halos(self):
         check(_lib.load().cmf_exchange_halos(self._h))
-
-    def loss(self):
-        out = ctypes.c_double()
-        check(_lib.load().cmf_loss(self._h, ctypes.byref(out)))
-        return out.value
 
     def _views(self):
         torch, lib = self.torch, _lib.load()
@@ -132,111 +108,8 @@ class DeviceShard:
             v = [torch.empty(0, device=dev)] * 4
         self.send_left, self.send_right, self.recv_left, self.recv_right = v
 
-    def set_engine(self, engine):
-        """0 = SIMT kernels, 1 = tcgen05 kernels in the time domain, 2 = frequency-domain engine (spectrum of X +
-        per-frequency tcgen05 products); raises if the handle cannot use the engine."""
-        check(_lib.load().cmf_set_engine(self._h, int(engine)))
-
-    def set_loss_mode(self, mode):
-        """0 = direct residual pass, 1 = algebraic expansion on resident numH / C (tcgen05 engine only)."""
-        check(_lib.load().cmf_set_loss_mode(self._h, int(mode)))
-
-    def set_loss_guard(self, guard=0.25, max_interval=16):
-        check(_lib.load().cmf_set_loss_guard(self._h, float(guard), int(max_interval)))
-
-    def loss_stats(self):
-        from .model import _loss_stats
-
-        return _loss_stats(self._h)
-
-    @property
-    def loss_mode(self):
-        out = ctypes.c_int(0)
-        check(_lib.load().cmf_get_loss_mode(self._h, ctypes.byref(out)))
-        return out.value
-
-    def fd_layout(self):
-        """(block length, hop, blocks) of the frequency-domain engine on this handle; zeros on the other engines."""
-        b, v, n = ctypes.c_int(), ctypes.c_int(), ctypes.c_int64()
-        check(_lib.load().cmf_get_fd_layout(self._h, ctypes.byref(b), ctypes.byref(v), ctypes.byref(n)))
-        return b.value, v.value, n.value
-
-    def get_engine(self):
-        out = ctypes.c_int()
-        check(_lib.load().cmf_get_engine(self._h, ctypes.byref(out)))
-        return out.value
-
     def scalar_tensor(self, values):
         return self.torch.tensor(values, dtype=self.torch.float64, device=f"cuda:{self.device}")
-
-    # data / factors --------------------------------------------------------------------------
-    def set_data(self, X, first_col=0):
-        Xj = julia_array(X, self.dtype)
-        check(_lib.load().cmf_set_data(self._h, fptr(Xj), first_col))
-
-    def synth_data(self, seed, K_true, L_true, p_h, noise):
-        check(_lib.load().cmf_synth_data(self._h, seed, K_true, L_true, p_h, noise))
-
-    def data_sumsq(self):
-        """||X||^2 of the owned columns; over ALL columns on handles whose collectives run inside the library."""
-        out = ctypes.c_double()
-        check(_lib.load().cmf_data_sumsq(self._h, ctypes.byref(out)))
-        return out.value
-
-    def get_data(self, out=None, with_halo=False):
-        """Owned columns of X (plus the right halo, clipped to T, with ``with_halo``) as a
-        Fortran-ordered N x cols array (optionally into a caller buffer)."""
-        cols = (min(self.t1 + self.L - 1, self.T) if with_halo else self.t1) - self.t0
-        if out is None:
-            out = np.empty((self.N, cols), dtype=np_dtype(self.dtype), order="F")
-        assert out.shape == (self.N, cols) and out.flags.f_contiguous
-        check(_lib.load().cmf_get_data(self._h, fptr(out), int(with_halo)))
-        return out
-
-    def profile(self, enable=True):
-        check(_lib.load().cmf_profile(self._h, int(enable)))
-
-    def profile_read(self):
-        """{class: (total_ms, launches)} for conv / transconv / corr / sweep (HALS H sweep)."""
-        res = {}
-        for which, name in enumerate(("conv", "transconv", "corr", "sweep")):
-            ms, n = ctypes.c_double(), ctypes.c_int64()
-            check(_lib.load().cmf_profile_read(self._h, which, ctypes.byref(ms), ctypes.byref(n)))
-            res[name] = (ms.value, n.value)
-        return res
-
-    def set_data_norm(self, v):
-        check(_lib.load().cmf_set_data_norm(self._h, float(v)))
-
-    def set_factors(self, W, H, first_col=0):
-        Wj, Hj = julia_array(W, self.dtype), julia_array(H, self.dtype)
-        check(_lib.load().cmf_set_factors(self._h, fptr(Wj), fptr(Hj), first_col))
-
-    def init_rand(self, seed):
-        check(_lib.load().cmf_init_rand(self._h, seed))
-
-    def init_scale_partials(self):
-        out = (ctypes.c_double * 2)()
-        check(_lib.load().cmf_init_scale_partials(self._h, out))
-        return [out[0], out[1]]
-
-    def scale_factors(self, s):
-        check(_lib.load().cmf_scale_factors(self._h, float(s)))
-
-    def get_factors(self, out=None):
-        """W (K x N x L) and the owned columns of H (K x Tl), Fortran order, handle dtype.  ``out=(W, H)`` downloads
-        into caller-owned arrays of that shape/order/dtype (e.g. views of pinned buffers)."""
-        dt = np_dtype(self.dtype)
-        if out is not None:
-            W, H = out
-            for a, shp in ((W, (self.K, self.N, self.L)), (H, (self.K, self.t1 - self.t0))):
-                if a.shape != shp or a.dtype != dt or not a.flags.f_contiguous:
-                    raise ValueError("get_factors(out=...): need Fortran-ordered arrays of the handle dtype, shapes K x N x L and K x Tl")
-        else:
-            W = np.empty((self.K, self.N, self.L), dtype=dt, order="F")
-            H = np.empty((self.K, self.t1 - self.t0), dtype=dt, order="F")
-        check(_lib.load().cmf_get_factors(self._h, fptr(W), fptr(H)))
-        return W, H            # handle dtype (no host-side conversion: H is 1 GiB at the benchmark size)
 
     # split-phase steps -------------------------------------------------------------------------
     def w_partials(self):
@@ -248,42 +121,24 @@ class DeviceShard:
     def h_update(self, l1H, l2H):
         check(_lib.load().cmf_h_update(self._h, float(l1H), float(l2H)))
 
-    def update_motifs(self, l1W=0.0, l2W=0.0):
-        """Single-shard update_motifs! (MU or HALS)."""
-        check(_lib.load().cmf_update_motifs(self._h, float(l1W), float(l2W)))
-
-    def update_feature_maps(self, l1H=0.0, l2H=0.0):
-        """Single-shard update_feature_maps! (MU or HALS); returns the relative loss."""
-        out = ctypes.c_double()
-        check(_lib.load().cmf_update_feature_maps(self._h, float(l1H), float(l2H), ctypes.byref(out)))
-        return out.value
-
     def loss_partial(self):
         out = ctypes.c_double()
         check(_lib.load().cmf_loss_partial(self._h, ctypes.byref(out)))
         return out.value
 
-    def launch_count(self):
-        out = ctypes.c_int64()
-        check(_lib.load().cmf_launch_count(self._h, ctypes.byref(out)))
-        return out.value
 
-    def sync(self):
-        check(_lib.load().cmf_sync(self._h))
+class _AlternatingFit:
+    """The fit loop shared by ShardedMultFit and LibraryFit, over their ``loss`` and ``iterate``."""
 
-    def close(self):
-        if self._h is not None and self._h.value:
-            _lib.load().cmf_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+    def fit(self, max_itr=100, check_convergence=True, patience=3, tol=1e-4, **reg):
+        """src/algs/alternating.jl:16-71 over shards (every rank takes the same branch because the
+        loss is all-reduced)."""
+        loss_hist, _, _ = _alternate(self.loss(), lambda: self.iterate(**reg), max_itr, check_convergence=check_convergence,
+                                     patience=patience, tol=tol)
+        return loss_hist
 
 
-class ShardedMultFit:
+class ShardedMultFit(_AlternatingFit):
     """The sharded MU iteration (src/algs/mult.jl:23-58 split at its three global dependencies).
 
     ``shard`` is any engine with the DeviceShard step interface; ``dist`` is torch.distributed
@@ -355,22 +210,8 @@ class ShardedMultFit:
             loss = self.loss()                   # re-evaluate with the direct pass, as the library's own loop does
         return loss
 
-    def fit(self, max_itr=100, check_convergence=True, patience=3, tol=1e-4, **reg):
-        """src/algs/alternating.jl:16-71 over shards (every rank takes the same branch because the
-        loss is all-reduced)."""
-        from .model import converged
 
-        loss_hist = [self.loss()]
-        itr = 1
-        while itr <= max_itr:
-            itr += 1
-            loss_hist.append(self.iterate(**reg))
-            if check_convergence and converged(loss_hist, patience, tol):
-                break
-        return loss_hist
-
-
-class LibraryFit:
+class LibraryFit(_AlternatingFit):
     """The same fit steps as ``ShardedMultFit`` with every collective INSIDE libcmf_sm100 (NCCL bound by the library:
     ``DeviceShard(comm=...)`` under torchrun, or ``DeviceShard(ngpu=...)`` in one process).  The host only calls the
     reference-facing entry points: update_motifs! / update_feature_maps! / compute_loss (alternating.jl:37,52,54)."""
@@ -383,10 +224,7 @@ class LibraryFit:
         return self.data_norm
 
     def rescale_init(self):
-        dot, nrm2 = self.shard.init_scale_partials()              # all-reduced by the library
-        s = math.sqrt(abs(dot / nrm2))
-        self.shard.scale_factors(s)
-        return s
+        return _rescale(self.shard)                               # the partials are all-reduced by the library
 
     def exchange_halos(self):
         self.shard.exchange_halos()
@@ -398,15 +236,3 @@ class LibraryFit:
         if not eval_mode:
             self.shard.update_motifs(l1W, l2W)
         return self.shard.update_feature_maps(l1H, l2H)
-
-    def fit(self, max_itr=100, check_convergence=True, patience=3, tol=1e-4, **reg):
-        from .model import converged
-
-        loss_hist = [self.loss()]
-        itr = 1
-        while itr <= max_itr:
-            itr += 1
-            loss_hist.append(self.iterate(**reg))
-            if check_convergence and converged(loss_hist, patience, tol):
-                break
-        return loss_hist
